@@ -5,6 +5,7 @@ threshold-kernel HBM GB/s vs peak).
     python bench.py --gpus N --steps K --warmup W                    # this repo's CUDA path, headline workload C3
     python bench.py --workload C4|C5|all ...                         # the other BASELINE.json configs (one JSON line each)
     python bench.py --impl reference --gpus N --steps K ...          # CPU arm: the C restatement of the reference (oracle/)
+    python bench.py --dump-outputs DIR ...                           # also write the last timed call's counters and markers (.npy)
 
 One step = one pass of `Detector::detect` (src/aruco.rs:52-121) over one batch of synthetic frames (aruco3_b200/synth.py):
   C3  BASELINE.json configs[2] (HEADLINE): 256 x 1920x1080 RGB8 per GPU, 20 ARUCO markers each; weak scaling
@@ -47,6 +48,7 @@ sys.path.insert(0, str(ROOT))
 import numpy as np  # noqa: E402
 
 ALGO_BYTES_PER_PIXEL = 5   # 3 B RGB read + 1 B grey written + 1 B mask written (SURVEY.md §8d)
+DUMP_LIMIT_BYTES = 64 << 20  # --dump-outputs: larger outputs are written as a seeded sample of their marker rows
 
 WORKLOADS = {
     "C3": dict(spec="C3", metric="frames_per_sec_1080p_batch256", per_gpu=256, total=None, scaling="weak", rotate=3, distinct=None,
@@ -241,6 +243,26 @@ def k1_traffic(frames_per_launch, w, h):
     return (t["dram_bytes_read"] + t["dram_bytes_write"]) * px_ratio, t["source"]
 
 
+def dump_outputs(out_dir, prefix, rec, stats):
+    """--dump-outputs: what one a3_detect_batch call hands its caller, as float64 arrays that two builds can be compared by.
+    `<prefix>_counts.npy` holds the call's a3_stats counters (n_frames, n_contours, n_contour_points, n_candidates_before_discard,
+    n_candidates, n_markers); `<prefix>_marker_<field>.npy` one field of every marker record, rows in (frame, candidate) order.
+    Marker rows beyond DUMP_LIMIT_BYTES are cut to a fixed seeded sample, still in that order."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    counts = [stats[k] for k in ("n_frames", "n_contours", "n_contour_points", "n_candidates_before_discard", "n_candidates", "n_markers")]
+    np.save(out / f"{prefix}_counts.npy", np.array(counts, np.float64))
+    rec = rec[np.lexsort((rec["candidate"], rec["frame"]))]
+    cols = {"frame": rec["frame"], "candidate": rec["candidate"], "id": rec["id"], "code": rec["code"], "rotation": rec["rot"],
+            "hamming_distance": rec["hd"], "corners": rec["corners"]}
+    max_rows = (DUMP_LIMIT_BYTES - 4096) // (8 * (6 + 8))  # six scalar fields + eight corner coordinates per row
+    rows = np.arange(len(rec))
+    if len(rec) > max_rows:
+        rows = np.sort(np.random.default_rng(0xA3D0).choice(len(rec), max_rows, replace=False))
+    for name, v in cols.items():
+        np.save(out / f"{prefix}_marker_{name}.npy", v[rows].astype(np.float64))  # ids and codes < 2^53: exact in float64
+
+
 def run_b200(args, wl_name, ctx):
     import torch
     import torch.distributed as dist
@@ -376,7 +398,9 @@ def run_b200(args, wl_name, ctx):
     dev_ptrs = [r.data_ptr() for r in resident]
     host_ptrs = [p.data_ptr() for p in pinned]
     ms_dev, acc_dev, clocks = timed(dev_ptrs, _ffi.MEM_DEVICE, args.steps, args.warmup)
-    # the timed region ended on batch (warmup + steps - 1) % rotate: its markers are still in `markers`
+    # the timed region ended on batch (warmup + steps - 1) % rotate: its markers are still in `markers`, its counters in `stats`
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, wl_name if world == 1 else f"{wl_name}_rank{rank}", marker_rows(), stats.as_dict())
     parity += check_parity((args.warmup + args.steps - 1) % rotate, check_frames, "resident")
     ms_e2e, acc_e2e, clocks_e2e = timed(host_ptrs, _ffi.MEM_HOST, args.steps, 3, stats_in_loop=False)
     parity += check_parity((3 + 2 * args.steps - 1) % rotate_host, check_frames, "e2e")
@@ -603,9 +627,15 @@ def main():
     ap.add_argument("--fast", action="store_true", help="value + pinned e2e only (skips pageable / full e2e, H2D ceiling, latency, isolated K1)")
     ap.add_argument("--chunk", type=int, default=0, help="frames per pipeline chunk (0 = library default)")
     ap.add_argument("--contours", default="device", choices=["device", "host"], help="where find_contours + quad filters run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the counters and markers of the last timed call as DIR/<workload>_*.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     names = ["C3", "C4", "C5"] if args.workload == "all" else [args.workload]
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs needs the CUDA arm: the reference arm counts markers but keeps none")
         for name in names:
             run_reference(args, name)
         return 0
