@@ -17,6 +17,7 @@ FMT_LUMAA8, FMT_LUMA16, FMT_LUMAA16, FMT_RGB16, FMT_RGBA16 = 5, 6, 7, 8, 9
 MEM_HOST, MEM_DEVICE = 0, 1
 CONTOURS_HOST, CONTOURS_DEVICE = 0, 1
 POSE_OFF, POSE_UNDISTORTED, POSE_INTRINSICS, POSE_NORMALIZED = 0, 1, 2, 3
+CORNERS_INTEGER, CORNERS_REFINED = 0, 1
 
 
 class A3Config(C.Structure):
@@ -33,7 +34,7 @@ class A3Dictionary(C.Structure):
 class A3Marker(C.Structure):
     _fields_ = [("id", C.c_uint64), ("code", C.c_uint64), ("corners", C.c_uint32 * 8), ("frame", C.c_uint32),
                 ("candidate", C.c_uint32), ("hamming_distance", C.c_uint8), ("rotation", C.c_uint8),
-                ("reserved", C.c_uint8 * 6)]
+                ("corners_refined", C.c_uint8), ("reserved", C.c_uint8 * 5)]
 
 
 class A3Decode(C.Structure):
@@ -48,7 +49,9 @@ class A3Stats(C.Structure):
                [(n, C.c_double) for n in ("ms_h2d", "ms_pixel_kernel", "ms_contour_kernels", "ms_mask_d2h", "ms_host_quads",
                                           "ms_decode_kernel", "ms_host_cpu", "ms_total")] + \
                [(n, C.c_uint32) for n in ("pixel_kernel_launches", "decode_kernel_launches", "host_threads", "contour_kernel_launches",
-                                          "host_fallback_frames", "pose_kernel_launches", "one_shot", "one_shot_retry", "input_staged", "output_staged")]
+                                          "host_fallback_frames", "pose_kernel_launches", "one_shot", "one_shot_retry", "input_staged", "output_staged",
+                                          "refine_kernel_launches")] + \
+               [("ms_refine_kernel", C.c_double)]
 
     def as_dict(self):
         return {f: getattr(self, f) for f, _ in self._fields_}
@@ -57,7 +60,8 @@ class A3Stats(C.Structure):
 class A3Outputs(C.Structure):
     _fields_ = [("grey", C.c_void_p), ("mask", C.c_void_p), ("candidates", C.c_void_p), ("candidate_frame", C.c_void_p),
                 ("homographies", C.c_void_p), ("decodes", C.c_void_p), ("cand_capacity", C.c_uint32),
-                ("n_candidates", C.c_uint32), ("frame_marker_offsets", C.c_void_p), ("marker_poses", C.c_void_p)]
+                ("n_candidates", C.c_uint32), ("frame_marker_offsets", C.c_void_p), ("marker_poses", C.c_void_p),
+                ("marker_corners", C.c_void_p)]
 
 
 class A3Pose(C.Structure):
@@ -133,6 +137,7 @@ def lib():
     L.a3_detector_create_count.restype = C.c_uint64
     L.a3_detector_set_host_threads.argtypes = [vp, u32]
     L.a3_detector_set_contour_mode.argtypes = [vp, u32]
+    L.a3_detector_set_corner_refinement.argtypes = [vp, u32]
     L.a3_detector_set_k1_tuning.argtypes = [vp, C.POINTER(A3K1Tuning)]
     L.a3_detect_batch.argtypes = [vp, vp, C.c_int, C.c_int, u32, u32, u32, sz, sz, vp, u32, C.POINTER(u32),
                                   C.POINTER(A3Outputs), C.POINTER(A3Stats)]
@@ -140,6 +145,7 @@ def lib():
     L.a3_quads_from_mask.argtypes = [C.POINTER(A3Config), vp, u32, u32, vp, u32, C.POINTER(u32), C.POINTER(A3Stats)]
     L.a3_quads_from_masks_device.argtypes = [vp, vp, u32, u32, u32, vp, u32, vp, vp, vp, vp]
     L.a3_decode_candidates.argtypes = [vp, vp, u32, u32, u32, vp, vp, u32, vp, vp]
+    L.a3_refine_corners.argtypes = [vp, vp, u32, u32, u32, vp, vp, u32, vp, vp]
     fp, f32, PK, PP = C.POINTER(C.c_float), C.c_float, C.POINTER(A3CameraIntrinsics), C.POINTER(A3Pose)
     L.a3_detector_set_pose.argtypes = [vp, u32, f32, PK]
     L.a3_solve_with_intrinsics.argtypes = [vp, vp, u32, f32, PK, vp, vp]

@@ -231,16 +231,23 @@ struct DecodeBlock {
     DevBuf<uint8_t> d_patches;
     DevBuf<a3_pose> d_pose;   // K4: two poses per quad (written for accepted candidates only)
     PinBuf<a3_pose> h_pose;
-    cudaEvent_t ev_a = nullptr, ev_b = nullptr;
+    DevBuf<float> d_ref;      // K5: refined corners per quad (accepted candidates only) and their flags
+    PinBuf<float> h_ref;
+    DevBuf<uint8_t> d_refok;
+    PinBuf<uint8_t> h_refok;
+    cudaEvent_t ev_a = nullptr, ev_b = nullptr, ev_r0 = nullptr, ev_r1 = nullptr;  // around K2, around K5
     uint32_t n_quads = 0;
-    // where the host reads this group's records: h_dec / h_pose, or the one-shot arena
+    // where the host reads this group's records: h_dec / h_pose / h_ref, or the one-shot arena
     const a3_decode *dec_view = nullptr;
     const a3_pose *pose_view = nullptr;
+    const float *ref_view = nullptr;
+    const uint8_t *refok_view = nullptr;
     void release() {
         h_quads.release(); h_qframe.release(); h_dec.release(); d_quads.release(); d_qframe.release(); d_dec.release(); d_patches.release();
         d_info.release(); d_qoff.release();
         d_pose.release(); h_pose.release();
-        for (cudaEvent_t *e : {&ev_a, &ev_b}) { if (*e) cudaEventDestroy(*e); *e = nullptr; }
+        d_ref.release(); h_ref.release(); d_refok.release(); h_refok.release();
+        for (cudaEvent_t *e : {&ev_a, &ev_b, &ev_r0, &ev_r1}) { if (*e) cudaEventDestroy(*e); *e = nullptr; }
     }
 };
 
@@ -313,6 +320,10 @@ struct a3_detector {
     a3::DevBuf<float> d_pose_in;      // standalone solve entry points: 8 x 4 bytes per marker (f32 points or u32 corners)
     a3::DevBuf<a3_pose> d_pose_out;
     a3::PinBuf<a3_pose> h_pose_out;
+    // corner refinement (K5)
+    uint32_t corner_mode = A3_CORNERS_INTEGER;
+    a3::DevBuf<float> d_refined;      // a3_refine_corners: refined corners and their flags
+    a3::DevBuf<uint8_t> d_refined_ok;
 };
 
 namespace a3 {
@@ -407,8 +418,10 @@ __global__ void __launch_bounds__(128) pack_quads_kernel(const uint32_t *quads, 
 // rotation) with their poses beside them, so the host copies one block instead of walking every candidate.
 // info[3] = number of markers.
 __global__ void __launch_bounds__(1024) assemble_markers_kernel(const a3_decode *dec, const uint32_t *quads, const uint32_t *qframe,
-                                                                const uint32_t *qoff, const a3_pose *poses, uint32_t cap, uint32_t *info,
-                                                                const uint32_t *chunk_accepted, a3_marker *markers, a3_pose *mposes) {
+                                                                const uint32_t *qoff, const a3_pose *poses, const float *refined,
+                                                                const uint8_t *refined_ok, uint32_t cap, uint32_t *info,
+                                                                const uint32_t *chunk_accepted, a3_marker *markers, a3_pose *mposes,
+                                                                float *mcorners) {
     // One CTA per 1024 quads.  The number of markers before a chunk is the sum of the accepted counts of the chunks before
     // it, which K2 accumulated while it decoded (K2Params::accept_counts; zeroed by pack_offsets_kernel): no CTA waits for
     // another, so the kernel needs no co-residency and any number of chunks is fine.
@@ -452,9 +465,12 @@ __global__ void __launch_bounds__(1024) assemble_markers_kernel(const a3_decode 
     m.candidate = k - qoff[frame];
     m.hamming_distance = dc.hamming_distance;
     m.rotation = dc.rotation;
-    for (int i = 0; i < 6; i++) m.reserved[i] = 0;
+    m.corners_refined = refined ? refined_ok[k] : 0;
+    for (int i = 0; i < 5; i++) m.reserved[i] = 0;
     markers[idx] = m;
     if (poses) { mposes[2 * (size_t)idx] = poses[2 * (size_t)k]; mposes[2 * (size_t)idx + 1] = poses[2 * (size_t)k + 1]; }
+    if (refined)  // K5 wrote them in marker order already
+        for (int i = 0; i < 8; i++) mcorners[8 * (size_t)idx + i] = refined[8 * (size_t)k + i];
 }
 
 // K1 over `p`.  LumaA8 / 16-bit frames first go through K0 (image's into_luma8 for those variants) into the detector's Luma8
@@ -477,6 +493,21 @@ K2Params k2_params(const a3_detector *d, const uint8_t *grey, uint32_t w, uint32
     p.n_codes = d->dict.n_codes; p.tau = d->dict.tau; p.filter_high_bit_errors = d->cfg.filter_high_bit_errors;
     p.resize_w = d->d_taps.p; p.resize_meta = d->d_meta.p; p.decodes = nullptr; p.patches = nullptr;
     return p;
+}
+
+// K5 on the candidates K2 just decoded (its accepted ones), bracketed by the block's events
+cudaError_t launch_refine(DecodeBlock &b, const uint8_t *grey, uint32_t w, uint32_t h, const uint32_t *quads, const uint32_t *qframe,
+                          const a3_decode *dec, uint32_t n, const uint32_t *n_dev, float *out, uint8_t *ok, cudaStream_t s) {
+    cudaError_t e = cudaSuccess;
+    if (!b.ev_r0) e = cudaEventCreate(&b.ev_r0);
+    if (e == cudaSuccess && !b.ev_r1) e = cudaEventCreate(&b.ev_r1);
+    if (e == cudaSuccess) e = cudaEventRecord(b.ev_r0, s);
+    K5Params kp{};
+    kp.grey = grey; kp.w = w; kp.h = h; kp.quads = quads; kp.quad_frame = qframe; kp.decodes = dec; kp.n = n; kp.n_dev = n_dev;
+    kp.corners = out; kp.ok = ok;
+    if (e == cudaSuccess) e = k5_corners(kp, s);
+    if (e == cudaSuccess) e = cudaEventRecord(b.ev_r1, s);
+    return e;
 }
 
 }  // namespace
@@ -596,6 +627,7 @@ void a3_detector_release(a3_detector *d) {
     // back to the state a3_detector_create leaves a handle in (the buffers stay)
     d->contour_mode = A3_CONTOURS_DEVICE;
     d->pose_mode = A3_POSE_OFF;
+    d->corner_mode = A3_CORNERS_INTEGER;
     d->has_tuning = false; d->k1_tuning = K1Tuning{}; d->chunk_override = 0;
     a3_detector *evict = nullptr;
     {
@@ -628,6 +660,7 @@ void a3_detector_destroy(a3_detector *d) {
     d->h_k3flags.release(); d->h_k3contours.release(); d->h_k3points.release(); d->h_plane.release();
     d->d_qoff.release(); d->d_k2queue.release(); d->d_shot.release(); d->h_shot.release();
     d->d_pose_in.release(); d->d_pose_out.release(); d->h_pose_out.release();
+    d->d_refined.release(); d->d_refined_ok.release();
     d->copy_pool.stop();
     d->h_stage_in.release(); d->h_stage_out.release();
     d->events.release();
@@ -644,6 +677,12 @@ a3_status a3_detector_set_host_threads(a3_detector *d, uint32_t threads) {
 a3_status a3_detector_set_contour_mode(a3_detector *d, uint32_t mode) {
     if (!d || mode > A3_CONTOURS_DEVICE) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_contour_mode: bad argument");
     d->contour_mode = mode;
+    return A3_OK;
+}
+
+a3_status a3_detector_set_corner_refinement(a3_detector *d, uint32_t mode) {
+    if (!d || mode > A3_CORNERS_REFINED) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_corner_refinement: bad argument");
+    d->corner_mode = mode;
     return A3_OK;
 }
 
@@ -796,6 +835,34 @@ a3_status a3_decode_candidates(a3_detector *d, const uint8_t *grey, uint32_t n_f
     return A3_OK;
 }
 
+a3_status a3_refine_corners(a3_detector *d, const uint8_t *grey, uint32_t n_frames, uint32_t w, uint32_t h, const uint32_t *corners,
+                            const uint32_t *corner_frame, uint32_t n, float *refined, uint8_t *ok) {
+    if (!d || !grey || (n && (!corners || !refined || !ok))) return fail(A3_ERR_INVALID_ARGUMENT, "a3_refine_corners: null argument");
+    if (n == 0) return A3_OK;
+    if (n_frames == 0 || w == 0 || h == 0) return fail(A3_ERR_INVALID_ARGUMENT, "a3_refine_corners: empty grey frames");
+    for (uint32_t i = 0; corner_frame && i < n; i++)
+        if (corner_frame[i] >= n_frames) return fail(A3_ERR_INVALID_ARGUMENT, "a3_refine_corners: corner_frame out of range");
+    A3_CUDA(cudaSetDevice(d->device));
+    cudaStream_t s = d->s_decode;
+    const size_t px = (size_t)w * h;
+    A3_CUDA(d->d_grey.reserve(px * n_frames));
+    A3_CUDA(d->d_quads.reserve((size_t)n * 8));
+    A3_CUDA(d->d_qframe.reserve(n));
+    A3_CUDA(d->d_refined.reserve((size_t)n * 8));
+    A3_CUDA(d->d_refined_ok.reserve(n));
+    A3_CUDA(cudaMemcpyAsync(d->d_grey.p, grey, px * n_frames, cudaMemcpyHostToDevice, s));
+    A3_CUDA(cudaMemcpyAsync(d->d_quads.p, corners, (size_t)n * 32, cudaMemcpyHostToDevice, s));
+    if (corner_frame) A3_CUDA(cudaMemcpyAsync(d->d_qframe.p, corner_frame, (size_t)n * 4, cudaMemcpyHostToDevice, s));
+    K5Params kp{};
+    kp.grey = d->d_grey.p; kp.w = w; kp.h = h; kp.quads = d->d_quads.p; kp.quad_frame = corner_frame ? d->d_qframe.p : nullptr;
+    kp.decodes = nullptr; kp.n = n; kp.corners = d->d_refined.p; kp.ok = d->d_refined_ok.p;
+    A3_CUDA(k5_corners(kp, s));
+    A3_CUDA(cudaMemcpyAsync(refined, d->d_refined.p, (size_t)n * 32, cudaMemcpyDeviceToHost, s));
+    A3_CUDA(cudaMemcpyAsync(ok, d->d_refined_ok.p, n, cudaMemcpyDeviceToHost, s));
+    A3_CUDA(cudaStreamSynchronize(s));
+    return A3_OK;
+}
+
 a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, a3_mem_kind mem, uint32_t n, uint32_t w,
                           uint32_t h, size_t pitch, size_t frame_stride, a3_marker *markers, uint32_t marker_capacity,
                           uint32_t *n_markers, a3_outputs *outs, a3_stats *stats) {
@@ -816,6 +883,9 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
     const size_t np = (size_t)d->cfg.homography_sample_size * d->cfg.homography_sample_size;
     const bool want_mask = outs && outs->mask, want_grey = outs && outs->grey, want_patches = outs && outs->homographies;
     const bool want_poses = outs && outs->marker_poses && markers && d->pose_mode != A3_POSE_OFF;
+    // K5 refines the markers' corners (a3_marker.corners_refined, a3_outputs.marker_corners) and K4 then solves from them
+    const bool want_refine = markers && d->corner_mode == A3_CORNERS_REFINED;
+    float *const out_corners = want_refine && outs ? outs->marker_corners : nullptr;
     const K1Tuning *tune = d->has_tuning ? &d->k1_tuning : nullptr;
     const uint8_t *src_all = static_cast<const uint8_t *>(frames);
     a3_stats st;
@@ -929,10 +999,13 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
         const bool lean = shot && markers && !(outs && (outs->candidates || outs->candidate_frame || outs->decodes || outs->homographies));
         const size_t off_stats = 16, off_markers = (off_stats + 24 * shot_c + 15) & ~(size_t)15;
         const size_t off_mposes = off_markers + (lean ? (size_t)shot_cap * sizeof(a3_marker) : 0);
-        const size_t off_quads = (off_mposes + ((lean && want_poses) ? (size_t)shot_cap * 2 * sizeof(a3_pose) : 0) + 15) & ~(size_t)15;
+        const size_t off_mcorners = off_mposes + ((lean && want_poses) ? (size_t)shot_cap * 2 * sizeof(a3_pose) : 0);  // K5's, per marker
+        const size_t off_quads = (off_mcorners + ((lean && want_refine) ? (size_t)shot_cap * 32 : 0) + 15) & ~(size_t)15;
         const size_t off_dec = off_quads + (size_t)shot_cap * 32;
         const size_t off_pose = off_dec + (size_t)shot_cap * sizeof(a3_decode);
-        const size_t shot_bytes = off_pose + (want_poses ? (size_t)shot_cap * 2 * sizeof(a3_pose) : 0);
+        const size_t off_ref = off_pose + (want_poses ? (size_t)shot_cap * 2 * sizeof(a3_pose) : 0);  // K5's, per candidate
+        const size_t off_refok = off_ref + (want_refine ? (size_t)shot_cap * 32 : 0);
+        const size_t shot_bytes = off_refok + (want_refine ? (size_t)shot_cap : 0);
         const size_t shot_copy_bytes = lean ? off_quads : shot_bytes;  // what goes back to the host
         if (shot) {
             A3_CUDA(d->d_shot.reserve(shot_bytes)); A3_CUDA(d->h_shot.reserve(shot_bytes));
@@ -1025,16 +1098,21 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             A3_CUDA(cudaEventRecord(b.ev_a, d->s_pixel));
             A3_CUDA(k2_decode(p, d->s_pixel));
             A3_CUDA(cudaEventRecord(b.ev_b, d->s_pixel));
+            float *d_ref = want_refine ? reinterpret_cast<float *>(d->d_shot.p + off_ref) : nullptr;
+            uint8_t *d_refok = want_refine ? d->d_shot.p + off_refok : nullptr;
+            if (want_refine) A3_CUDA(launch_refine(b, d->d_grey.p, w, h, d_quads, b.d_qframe.p, d_dec, cap, d_info, d_ref, d_refok, d->s_pixel));
             if (want_poses) {
                 K4Params kp{};
-                kp.mode = d->pose_mode; kp.corners = d_quads; kp.decodes = d_dec; kp.n = cap; kp.n_dev = d_info;
+                kp.mode = d->pose_mode; kp.corners = d_quads; kp.corners_f32 = d_ref; kp.decodes = d_dec; kp.n = cap; kp.n_dev = d_info;
                 kp.marker_size = d->pose_marker_size; kp.image_w = w; kp.image_h = h; kp.k = d->pose_k; kp.poses = d_pose;
                 A3_CUDA(k4_pose(kp, d->s_pixel));
             }
             if (lean) {
-                assemble_markers_kernel<<<n_chunks, 1024, 0, d->s_pixel>>>(d_dec, d_quads, b.d_qframe.p, d->d_qoff.p, want_poses ? d_pose : nullptr, cap, d_info,
-                                                                    d_chain, reinterpret_cast<a3_marker *>(d->d_shot.p + off_markers),
-                                                                    reinterpret_cast<a3_pose *>(d->d_shot.p + off_mposes));
+                assemble_markers_kernel<<<n_chunks, 1024, 0, d->s_pixel>>>(d_dec, d_quads, b.d_qframe.p, d->d_qoff.p, want_poses ? d_pose : nullptr,
+                                                                    d_ref, d_refok, cap, d_info, d_chain,
+                                                                    reinterpret_cast<a3_marker *>(d->d_shot.p + off_markers),
+                                                                    reinterpret_cast<a3_pose *>(d->d_shot.p + off_mposes),
+                                                                    reinterpret_cast<float *>(d->d_shot.p + off_mcorners));
                 A3_CUDA(cudaGetLastError());
             }
             // everything the host needs in one copy: route info, K3's counters, then either the finished markers (+ poses) or the
@@ -1053,6 +1131,8 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 b.n_quads = h_info[0];
                 b.dec_view = reinterpret_cast<const a3_decode *>(d->h_shot.p + off_dec);
                 b.pose_view = reinterpret_cast<const a3_pose *>(d->h_shot.p + off_pose);
+                b.ref_view = reinterpret_cast<const float *>(d->h_shot.p + off_ref);
+                b.refok_view = d->h_shot.p + off_refok;
                 const uint32_t *h_quads = reinterpret_cast<const uint32_t *>(d->h_shot.p + off_quads);
                 uint32_t k = 0;
                 for (uint32_t i = 0; i < sn; i++) {
@@ -1067,6 +1147,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 d->hist_nq = b.n_quads ? b.n_quads : 1;
                 st.decode_kernel_launches++;
                 if (want_poses) st.pose_kernel_launches++;
+                if (want_refine) st.refine_kernel_launches++;
                 st.one_shot = 1;
                 one_shot_done = true;
                 lean_done = lean;
@@ -1328,10 +1409,20 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             st.decode_kernel_launches++;
             A3_CUDA(cudaMemcpyAsync(b.h_dec.p, b.d_dec.p, (size_t)nq * sizeof(a3_decode), cudaMemcpyDeviceToHost, d->s_decode));
             b.dec_view = b.h_dec.p; b.pose_view = nullptr;
+            if (want_refine) {  // K5 right behind K2, on the grey, the quads and K2's records where they lie
+                A3_CUDA(b.d_ref.reserve((size_t)nq * 8)); A3_CUDA(b.h_ref.reserve((size_t)nq * 8));
+                A3_CUDA(b.d_refok.reserve(nq)); A3_CUDA(b.h_refok.reserve(nq));
+                A3_CUDA(launch_refine(b, d->d_grey.p, w, h, b.d_quads.p, b.d_qframe.p, b.d_dec.p, nq, on_device ? b.d_info.p : nullptr, b.d_ref.p,
+                                      b.d_refok.p, d->s_decode));
+                st.refine_kernel_launches++;
+                A3_CUDA(cudaMemcpyAsync(b.h_ref.p, b.d_ref.p, (size_t)nq * 32, cudaMemcpyDeviceToHost, d->s_decode));
+                A3_CUDA(cudaMemcpyAsync(b.h_refok.p, b.d_refok.p, nq, cudaMemcpyDeviceToHost, d->s_decode));
+                b.ref_view = b.h_ref.p; b.refok_view = b.h_refok.p;
+            }
             if (want_poses) {  // K4 right behind K2, on K2's records and the quads where they lie
                 A3_CUDA(b.d_pose.reserve((size_t)nq * 2)); A3_CUDA(b.h_pose.reserve((size_t)nq * 2));
                 K4Params kp{};
-                kp.mode = d->pose_mode; kp.corners = b.d_quads.p; kp.decodes = b.d_dec.p; kp.n = nq; kp.marker_size = d->pose_marker_size;
+                kp.mode = d->pose_mode; kp.corners = b.d_quads.p; kp.corners_f32 = want_refine ? b.d_ref.p : nullptr; kp.decodes = b.d_dec.p; kp.n = nq; kp.marker_size = d->pose_marker_size;
                 kp.image_w = w; kp.image_h = h; kp.k = d->pose_k; kp.poses = b.d_pose.p;
                 A3_CUDA(k4_pose(kp, d->s_decode));
                 st.pose_kernel_launches++;
@@ -1395,8 +1486,9 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 if (mem == A3_MEM_HOST || j == 0) {
                     cudaEventElapsedTime(&ms, ev_k1b[j], ev_k3[j]); st.ms_contour_kernels += ms;
                     cudaEventElapsedTime(&ms, ev_k3[j], ev_fe[j]); st.ms_mask_d2h += ms;
-                    if (one_shot_done && d->blocks[0]->n_quads) {  // the decode sits between those two events on this route
+                    if (one_shot_done && d->blocks[0]->n_quads) {  // the decode (and K5) sit between those two events on this route
                         cudaEventElapsedTime(&ms, d->blocks[0]->ev_a, d->blocks[0]->ev_b); st.ms_mask_d2h -= ms;
+                        if (want_refine) { cudaEventElapsedTime(&ms, d->blocks[0]->ev_r0, d->blocks[0]->ev_r1); st.ms_mask_d2h -= ms; }
                     }
                 }
             } else {
@@ -1425,9 +1517,11 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
         if (lean_done) {  // the markers were assembled on the device: one block copy (lean implies a single super-batch and group)
             DecodeBlock &b = *d->blocks[0];
             if (b.n_quads && stats) { cudaEventElapsedTime(&ms, b.ev_a, b.ev_b); st.ms_decode_kernel += ms; }
+            if (b.n_quads && stats && want_refine) { cudaEventElapsedTime(&ms, b.ev_r0, b.ev_r1); st.ms_refine_kernel += ms; }
             const uint32_t nm = h_info[3], take = nm < marker_capacity ? nm : marker_capacity;
             memcpy(markers, d->h_shot.p + off_markers, (size_t)take * sizeof(a3_marker));
             if (want_poses) memcpy(outs->marker_poses, d->h_shot.p + off_mposes, (size_t)take * 2 * sizeof(a3_pose));
+            if (out_corners) memcpy(out_corners, d->h_shot.p + off_mcorners, (size_t)take * 32);
             if (nm > marker_capacity) overflow = true;
             if (outs && outs->frame_marker_offsets) {
                 uint32_t i = 0;
@@ -1443,6 +1537,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
         for (uint32_t g = 0; g < ngroups; g++) {
             DecodeBlock &b = *d->blocks[g];
             if (b.n_quads && stats) { cudaEventElapsedTime(&ms, b.ev_a, b.ev_b); st.ms_decode_kernel += ms; }
+            if (b.n_quads && stats && want_refine) { cudaEventElapsedTime(&ms, b.ev_r0, b.ev_r1); st.ms_refine_kernel += ms; }
             const uint32_t f0 = g * group, f1 = f0 + group_size(g);
             if (want_patches && b.n_quads && total_cands < outs->cand_capacity) {
                 const uint32_t room = outs->cand_capacity - total_cands, m = b.n_quads < room ? b.n_quads : room;
@@ -1479,6 +1574,10 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                             mk.corners[2 * cidx + 1] = q[2 * sidx + 1];
                         }
                         if (want_poses) memcpy(outs->marker_poses + (size_t)total_markers * 2, b.pose_view + (size_t)k * 2, 2 * sizeof(a3_pose));
+                        if (want_refine) {
+                            mk.corners_refined = b.refok_view[k];
+                            if (out_corners) memcpy(out_corners + (size_t)total_markers * 8, b.ref_view + (size_t)k * 8, 32);
+                        }
                     } else {
                         overflow = true;
                     }

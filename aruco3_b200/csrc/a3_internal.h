@@ -149,6 +149,7 @@ struct K4Params {
     uint32_t mode;               // A3_POSE_UNDISTORTED / A3_POSE_INTRINSICS (corners) or A3_POSE_NORMALIZED (points)
     const float *points;         // device n*8 (NORMALIZED)
     const uint32_t *corners;     // device n*8 (other modes)
+    const float *corners_f32 = nullptr;  // device n*8 or null: f32 corners (K5's), already rotate_left(rotation), read instead of `corners`
     const a3_decode *decodes;    // device n or null; when set: only accepted items, corners.rotate_left(rotation)
     uint32_t n;
     const uint32_t *n_dev = nullptr;  // device, optional: the real number of items (<= n, which then only sizes the launch)
@@ -158,6 +159,20 @@ struct K4Params {
     a3_pose *poses;              // device n*2: [2i] best, [2i+1] alternative
 };
 cudaError_t k4_pose(const K4Params &p, cudaStream_t stream);
+
+// ---- K5: sub-pixel marker corners (k5_corners.cu; specification oracle/a3ref_refine.c) ---------------------------------
+struct K5Params {
+    const uint8_t *grey;         // device, n_frames*h*w
+    uint32_t w, h;
+    const uint32_t *quads;       // device n*8 integer corners, screen-clockwise
+    const uint32_t *quad_frame;  // device n or null (all frame 0)
+    const a3_decode *decodes;    // device n or null; when set: only accepted items, output corners.rotate_left(rotation)
+    uint32_t n;
+    const uint32_t *n_dev = nullptr;  // device, optional: the real number of items (<= n, which then only sizes the launch)
+    float *corners;              // device out n*8: refined corners, or the integer corners as f32 where it fell back
+    uint8_t *ok;                 // device out n: 1 refined, 0 fell back
+};
+cudaError_t k5_corners(const K5Params &p, cudaStream_t stream);
 
 // ---- host quad stage (host_quads.cpp) ---------------------------------------------------------------
 struct QuadStats {

@@ -174,7 +174,14 @@ __global__ void __launch_bounds__(128) k4_pose_kernel(K4Params p) {
             px[c] = p.points[(size_t)i * 8 + 2 * sidx];
             py[c] = p.points[(size_t)i * 8 + 2 * sidx + 1];
         } else {
-            const float x = (float)p.corners[(size_t)i * 8 + 2 * sidx], y = (float)p.corners[(size_t)i * 8 + 2 * sidx + 1];
+            float x, y;
+            if (p.corners_f32) {  // K5's corners: already in marker order
+                x = p.corners_f32[(size_t)i * 8 + 2 * c];
+                y = p.corners_f32[(size_t)i * 8 + 2 * c + 1];
+            } else {
+                x = (float)p.corners[(size_t)i * 8 + 2 * sidx];
+                y = (float)p.corners[(size_t)i * 8 + 2 * sidx + 1];
+            }
             if (p.mode == A3_POSE_UNDISTORTED) {  // pose.rs:59-62
                 px[c] = x / (float)p.image_w;
                 py[c] = y / (float)p.image_h;

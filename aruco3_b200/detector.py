@@ -98,6 +98,10 @@ class Marker:
     rotation: int = 0
     candidate: int = 0
     poses: tuple | None = None   # (best, alt) MarkerPose when the detector has a pose mode (Detector.set_pose)
+    # corners="refined": [(x, y)] * 4 f32 sub-pixel corners in the order of `corners` (pixel-centre convention: grey pixel
+    # (x, y) is the point (x, y)); `refined` is False where the refinement fell back to the integer corners
+    corners_refined: list | None = None
+    refined: bool = False
 
 
 @dataclass
@@ -145,7 +149,7 @@ class Detector:
     """
 
     def __init__(self, config: DetectorConfig | None = None, dictionary: ARDictionary | str = "ARUCO", device: int = 0,
-                 host_threads: int | None = None, contours: str = "device"):
+                 host_threads: int | None = None, contours: str = "device", corners: str = "integer"):
         self.config = config or DetectorConfig()
         self.dictionary = ARDictionary.new_from_named_dict(dictionary) if isinstance(dictionary, str) else dictionary
         self.device = device
@@ -158,6 +162,16 @@ class Detector:
         check(lib().a3_detector_set_contour_mode(self._h, {"host": _ffi.CONTOURS_HOST, "device": _ffi.CONTOURS_DEVICE}[contours]))
         self.last_stats: dict = {}
         self._pose_mode = _ffi.POSE_OFF
+        self._corner_mode = _ffi.CORNERS_INTEGER
+        self.set_corner_refinement(corners)
+
+    def set_corner_refinement(self, corners: str = "refined"):
+        """`"refined"`: `detect` / `detect_batch` also return each marker's sub-pixel corners (`Marker.corners_refined`,
+        kernel K5 behind the decode kernel), and the pose step (set_pose) solves from them.  `"integer"` (the default)
+        switches it off: only the reference's integer corners, and nothing more runs."""
+        mode = {"integer": _ffi.CORNERS_INTEGER, "refined": _ffi.CORNERS_REFINED}[corners]
+        check(lib().a3_detector_set_corner_refinement(self._h, mode))
+        self._corner_mode = mode
 
     def set_pose(self, marker_size_mm: float | None, camera_intrinsics=None):
         """Also solve every marker's pose pair inside `detect` / `detect_batch` (kernel K4 behind the decode kernel):
@@ -215,6 +229,10 @@ class Detector:
             if self._pose_mode != _ffi.POSE_OFF:
                 poses = (A3Pose * (2 * cap_m))()
                 outs.marker_poses = C.cast(poses, C.c_void_p).value
+            refined = None
+            if self._corner_mode == _ffi.CORNERS_REFINED:
+                refined = np.zeros((cap_m, 4, 2), np.float32)
+                outs.marker_corners = refined.ctypes.data
             if full:
                 grey = np.empty((n, h, w), np.uint8)
                 cands = np.zeros((cap_c, 8), np.uint32)
@@ -249,6 +267,9 @@ class Detector:
             if poses is not None:
                 from .pose import MarkerPose
                 dets[m.frame].markers[-1].poses = (MarkerPose.from_c(poses[2 * i]), MarkerPose.from_c(poses[2 * i + 1]))
+            if refined is not None:
+                dets[m.frame].markers[-1].corners_refined = [(refined[i, k, 0], refined[i, k, 1]) for k in range(4)]
+                dets[m.frame].markers[-1].refined = bool(m.corners_refined)
         if full:
             for f in range(n):
                 dets[f].grey = grey[f]
@@ -310,6 +331,22 @@ class Detector:
                     homography_ok=bool(decs[k].homography_ok), otsu=int(decs[k].otsu), rotation=int(decs[k].rotation),
                     hamming_distance=int(decs[k].hamming_distance), accepted=bool(decs[k].accepted)) for k in range(m)]
         return out, patches
+
+    def refine_corners(self, grey: np.ndarray, corners: np.ndarray, corner_frame: np.ndarray | None = None):
+        """The corner refinement (kernel K5) for integer corners uint32 [m,4,2] or [m,8] (screen-clockwise, as
+        `Marker.corners`) over grey [n,H,W] or [H,W] -> (refined float32 [m,4,2], ok bool [m])."""
+        g = np.ascontiguousarray(grey, dtype=np.uint8)
+        if g.ndim == 2:
+            g = g[None]
+        n, h, w = g.shape
+        c = np.ascontiguousarray(corners, dtype=np.uint32).reshape(-1, 8)
+        m = c.shape[0]
+        out = np.zeros((m, 4, 2), np.float32)
+        ok = np.zeros(m, np.uint8)
+        cf = np.ascontiguousarray(corner_frame, dtype=np.uint32) if corner_frame is not None else None
+        check(lib().a3_refine_corners(self._h, g.ctypes.data, n, w, h, c.ctypes.data, cf.ctypes.data if cf is not None else None, m,
+                                      out.ctypes.data, ok.ctypes.data))
+        return out, ok.astype(bool)
 
 
 def quads_from_mask(mask: np.ndarray, config: DetectorConfig | None = None) -> np.ndarray:

@@ -82,7 +82,9 @@ typedef struct a3_dictionary {
 } a3_dictionary;
 
 /* Marker (src/aruco.rs:8-13) plus the frame / candidate it came from and the winning rotation.
- * corners = x0,y0,...,x3,y3 after rotate_left(rotation) (src/aruco.rs:97-103). */
+ * corners = x0,y0,...,x3,y3 after rotate_left(rotation) (src/aruco.rs:97-103).
+ * corners_refined: 1 when the detector refines corners (a3_detector_set_corner_refinement) and K5 refined this marker's,
+ * 0 when refinement is off or fell back to the integer corners. */
 typedef struct a3_marker {
     uint64_t id;
     uint64_t code;
@@ -91,7 +93,8 @@ typedef struct a3_marker {
     uint32_t candidate;
     uint8_t hamming_distance;
     uint8_t rotation;
-    uint8_t reserved[6];
+    uint8_t corners_refined;
+    uint8_t reserved[5];
 } a3_marker;
 
 /* One decoded candidate (every quad, accepted or not): the intermediates of
@@ -125,6 +128,9 @@ typedef struct a3_stats {
     /* pageable memory at the boundary: 1 when this call's host frames (input) / Detection.grey (output) were not page-locked and
      * went through the library's pinned staging rings (copy threads), 0 when the DMA used the caller's memory directly */
     uint32_t input_staged, output_staged;
+    /* corner refinement (K5, a3_detector_set_corner_refinement): launches, and the sum of its CUDA-event intervals */
+    uint32_t refine_kernel_launches;
+    double ms_refine_kernel;
 } a3_stats;
 
 /* MarkerPose (src/pose.rs:8-12): scene-from-marker transform in OpenCV chirality (+Z forward, +Y down, +X right).
@@ -162,6 +168,9 @@ typedef struct a3_outputs {
     uint32_t *frame_marker_offsets; /* n+1: markers of frame f are [off[f], off[f+1]) (may be NULL) */
     a3_pose *marker_poses;      /* marker_capacity*2: [2i] best and [2i+1] alternative pose of markers[i]; filled when
                                  * the detector has a pose mode (a3_detector_set_pose), may be NULL */
+    float *marker_corners;      /* marker_capacity*8: x0,y0..x3,y3 of markers[i] in f32, the order of a3_marker.corners; filled
+                                 * when the detector refines corners (A3_CORNERS_REFINED), may be NULL.  Where a marker's
+                                 * corners_refined is 0 these are its integer corners. */
 } a3_outputs;
 
 typedef struct a3_detector a3_detector;
@@ -191,7 +200,7 @@ void a3_detector_destroy(a3_detector *det);
  * (src/aruco.rs:46-49, benches/detect_markers.rs:17-20, README.md:14-17), and so cannot own a handle: bracket each
  * detect with acquire / release.  acquire returns an idle cached handle created with exactly this config, dictionary
  * (same `codes` pointer, sizes and tau) and device — warm: streams, device / pinned buffers and the one-shot history
- * survive — and creates one only when none is idle; release puts it back (pose / contour mode / tuning reset to the
+ * survive — and creates one only when none is idle; release puts it back (pose / contour / corner mode, tuning reset to the
  * defaults) and never blocks on the GPU.  A handle is held by one caller at a time; the cache itself is thread-safe and
  * keeps at most 16 idle handles (oldest destroyed).  a3_detector_cache_clear destroys the idle ones (call before unloading).
  * a3_detector_create_count: successful a3_detector_create calls of this process so far (diagnostic: a per-frame loop over
@@ -209,6 +218,17 @@ a3_status a3_detector_set_host_threads(a3_detector *det, uint32_t threads);
  * the mode.  A3_CONTOURS_HOST: always the host stage (C++ threads), as BASELINE.json's north_star describes it. */
 enum { A3_CONTOURS_HOST = 0, A3_CONTOURS_DEVICE = 1 };
 a3_status a3_detector_set_contour_mode(a3_detector *det, uint32_t mode);
+
+/* Sub-pixel marker corners (kernel K5, queued behind the decode kernel).  A3_CORNERS_INTEGER (default): the corners are
+ * the contour pixels the reference returns, and nothing else runs.  A3_CORNERS_REFINED: a3_detect_batch also fits a line
+ * to the grey image's edge profile along each side of every marker and returns the four intersections in
+ * a3_outputs.marker_corners, in the pixel-centre convention (grey pixel (x, y) is the point (x, y)); a3_marker.corners
+ * stay the integer corners.  Where the fit is not trustworthy (too few edge samples, near-parallel sides, a quad that is
+ * not convex and clockwise, a corner moved by more than a quarter of the shortest side) the marker keeps its integer
+ * corners and corners_refined = 0.  With a pose mode set, K4 solves from these corners.  Not a field of the reference's
+ * DetectorConfig; a3_detector_release resets it. */
+enum { A3_CORNERS_INTEGER = 0, A3_CORNERS_REFINED = 1 };
+a3_status a3_detector_set_corner_refinement(a3_detector *det, uint32_t mode);
 
 /* Launch-shape knobs of the pixel kernel (benchmark sweeps and tests; results never depend on them). 0 = automatic. */
 typedef struct a3_k1_tuning {
@@ -257,6 +277,12 @@ a3_status a3_quads_from_masks_device(a3_detector *det, const uint8_t *masks, uin
 a3_status a3_decode_candidates(a3_detector *det, const uint8_t *grey, uint32_t n_frames, uint32_t width,
                                uint32_t height, const uint32_t *quads, const uint32_t *quad_frame, uint32_t n_quads,
                                a3_decode *decodes, uint8_t *patches);
+
+/* The corner refinement (kernel K5) for n sets of four integer corners over grey frames, as a probe.  HOST pointers;
+ * corners n*8 (x0,y0..x3,y3, screen-clockwise: a3_marker.corners), corner_frame n (NULL = all frame 0); refined n*8 f32
+ * in the same corner order, ok n (1 refined, 0 fell back to the integer corners). */
+a3_status a3_refine_corners(a3_detector *det, const uint8_t *grey, uint32_t n_frames, uint32_t width, uint32_t height,
+                            const uint32_t *corners, const uint32_t *corner_frame, uint32_t n, float *refined, uint8_t *ok);
 
 /* ---- pose (src/pose.rs, src/pinhole.rs): the step after detect in the reference's examples ---- */
 

@@ -97,6 +97,10 @@ struct Marker {
     uint64_t code = 0;
     std::vector<std::pair<uint32_t, uint32_t>> corners;  // 4, already rotate_left(rotation)
     uint8_t hamming_distance = 0;
+    // Detector::set_corner_refinement(true): the 4 sub-pixel corners in the order of `corners` (pixel-centre convention),
+    // empty otherwise; `refined` is false where the refinement fell back to the integer corners
+    std::vector<std::pair<float, float>> corners_refined;
+    bool refined = false;
 };
 
 struct GrayImage {  // image::GrayImage: tightly packed, row-major
@@ -128,7 +132,7 @@ inline a3_config to_c(const DetectorConfig &config) {
 // a3_detect_batch on handle `h` (host frames) unpacked into Detections; `full` fills grey / candidates / homographies,
 // otherwise only markers.
 inline std::vector<Detection> detect_batch_on(a3_detector *h_, const DetectorConfig &config, const uint8_t *frames, uint32_t n, uint32_t width,
-                                              uint32_t height, PixelFormat fmt, bool full, a3_stats *stats) {
+                                              uint32_t height, PixelFormat fmt, bool full, a3_stats *stats, bool refined = false) {
     const uint32_t bpp = (fmt == PixelFormat::Rgb8 || fmt == PixelFormat::Bgr8) ? 3 : (fmt == PixelFormat::Luma8 ? 1 : 4);
     const size_t pitch = (size_t)width * bpp, stride = pitch * height, px = (size_t)width * height;
     const size_t hs = config.homography_sample_size, np = hs * hs;
@@ -139,8 +143,10 @@ inline std::vector<Detection> detect_batch_on(a3_detector *h_, const DetectorCon
         std::vector<uint8_t> grey, patches;
         std::vector<uint32_t> cands, cframe, offsets(n + 1);
         std::vector<a3_decode> decs;
+        std::vector<float> mcorners(refined ? (size_t)cap_m * 8 : 0);
         a3_outputs o{};
         o.frame_marker_offsets = offsets.data();
+        if (refined) o.marker_corners = mcorners.data();
         if (full) {
             grey.resize(n * px); cands.resize((size_t)cap_c * 8); cframe.resize(cap_c); patches.resize((size_t)cap_c * np); decs.resize(cap_c);
             o.grey = grey.data(); o.candidates = cands.data(); o.candidate_frame = cframe.data();
@@ -160,6 +166,10 @@ inline std::vector<Detection> detect_batch_on(a3_detector *h_, const DetectorCon
             Marker mk;
             mk.id = (size_t)m.id; mk.code = m.code; mk.hamming_distance = m.hamming_distance;
             for (int k = 0; k < 4; k++) mk.corners.emplace_back(m.corners[2 * k], m.corners[2 * k + 1]);
+            if (refined) {
+                for (int k = 0; k < 4; k++) mk.corners_refined.emplace_back(mcorners[(size_t)i * 8 + 2 * k], mcorners[(size_t)i * 8 + 2 * k + 1]);
+                mk.refined = m.corners_refined != 0;
+            }
             out[m.frame].markers.push_back(std::move(mk));
         }
         if (full) {
@@ -205,6 +215,7 @@ public:
         h_ = nullptr;
         const a3_config c = to_c(config);
         check(a3_detector_create(&c, &dictionary.c(), device_, &h_));
+        if (refine_) check(a3_detector_set_corner_refinement(h_, A3_CORNERS_REFINED));
     }
 
     // Detector::detect(&self, image: DynamicImage) -> Detection (src/aruco.rs:52-121): one tightly packed image.
@@ -216,7 +227,13 @@ public:
     // The same over n equally sized frames; `full` fills grey / candidates / homographies, otherwise only markers.
     std::vector<Detection> detect_batch(const uint8_t *frames, uint32_t n, uint32_t width, uint32_t height,
                                         PixelFormat fmt = PixelFormat::Rgb8, bool full = false, a3_stats *stats = nullptr) const {
-        return detect_batch_on(h_, config, frames, n, width, height, fmt, full, stats);
+        return detect_batch_on(h_, config, frames, n, width, height, fmt, full, stats, refine_);
+    }
+
+    // Sub-pixel corners (kernel K5) in Marker::corners_refined, and poses from them; off by default.  Kept across rebuild().
+    void set_corner_refinement(bool on) {
+        check(a3_detector_set_corner_refinement(h_, on ? A3_CORNERS_REFINED : A3_CORNERS_INTEGER));
+        refine_ = on;
     }
 
     a3_detector *handle() const { return h_; }
@@ -224,6 +241,7 @@ public:
 private:
     int device_ = 0;
     a3_detector *h_ = nullptr;
+    bool refine_ = false;
 };
 
 // The reference's own shape: `Detector { config, dictionary }` is plain data built with a literal (src/aruco.rs:46-49,
@@ -235,6 +253,7 @@ struct PlainDetector {
     DetectorConfig config;
     ARDictionary dictionary;
     int device = 0;
+    bool refine_corners = false;  // wrapper-side option (not in the reference's DetectorConfig): set on the leased handle per call
 
     Detection detect(const uint8_t *pixels, uint32_t width, uint32_t height, PixelFormat fmt = PixelFormat::Rgb8) const {
         std::vector<Detection> v = detect_batch(pixels, 1, width, height, fmt, /*full=*/true);
@@ -248,7 +267,8 @@ struct PlainDetector {
         } lease;
         const a3_config c = to_c(config);
         check(a3_detector_acquire(&c, &dictionary.c(), device, &lease.h));
-        return detect_batch_on(lease.h, config, frames, n, width, height, fmt, full, stats);
+        if (refine_corners) check(a3_detector_set_corner_refinement(lease.h, A3_CORNERS_REFINED));
+        return detect_batch_on(lease.h, config, frames, n, width, height, fmt, full, stats, refine_corners);
     }
 };
 
@@ -263,6 +283,9 @@ public:
         for (int dev : devices) shards_.emplace_back(new Detector(cfg, dict, dev));
     }
     size_t size() const { return shards_.size(); }
+    void set_corner_refinement(bool on) {
+        for (auto &d : shards_) d->set_corner_refinement(on);
+    }
     static std::pair<uint32_t, uint32_t> shard_range(uint32_t n_frames, uint32_t rank, uint32_t world) {
         const uint32_t base = n_frames / world, extra = n_frames % world;
         const uint32_t lo = rank * base + (rank < extra ? rank : extra);

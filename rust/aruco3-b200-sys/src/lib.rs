@@ -57,7 +57,9 @@ pub struct a3_marker {
     pub candidate: u32,
     pub hamming_distance: u8,
     pub rotation: u8,
-    pub reserved: [u8; 6],
+    /// 1 when K5 refined this marker's corners (`a3_outputs.marker_corners`), 0 when off or fell back
+    pub corners_refined: u8,
+    pub reserved: [u8; 5],
 }
 
 #[repr(C)]
@@ -101,6 +103,8 @@ pub struct a3_stats {
     pub one_shot_retry: u32,
     pub input_staged: u32,
     pub output_staged: u32,
+    pub refine_kernel_launches: u32,
+    pub ms_refine_kernel: f64,
 }
 
 /// MarkerPose, reference `src/pose.rs:8-12`; rotation row-major
@@ -124,6 +128,8 @@ pub struct a3_camera_intrinsics {
     pub principal_y: f32,
 }
 
+pub const A3_CORNERS_INTEGER: u32 = 0;
+pub const A3_CORNERS_REFINED: u32 = 1;
 pub const A3_POSE_OFF: u32 = 0;
 pub const A3_POSE_UNDISTORTED: u32 = 1;
 pub const A3_POSE_INTRINSICS: u32 = 2;
@@ -141,6 +147,8 @@ pub struct a3_outputs {
     pub n_candidates: u32,
     pub frame_marker_offsets: *mut u32,
     pub marker_poses: *mut a3_pose,
+    /// marker_capacity * 8 f32 (A3_CORNERS_REFINED), may be null
+    pub marker_corners: *mut f32,
 }
 
 #[repr(C)]
@@ -173,6 +181,7 @@ extern "C" {
     pub fn a3_detector_create_count() -> u64;
     pub fn a3_detector_set_host_threads(det: *mut a3_detector, threads: u32) -> a3_status;
     pub fn a3_detector_set_contour_mode(det: *mut a3_detector, mode: u32) -> a3_status;
+    pub fn a3_detector_set_corner_refinement(det: *mut a3_detector, mode: u32) -> a3_status;
     pub fn a3_detect_batch(
         det: *mut a3_detector, frames: *const c_void, format: i32, mem: i32, n: u32, width: u32, height: u32, pitch: usize,
         frame_stride: usize, markers: *mut a3_marker, marker_capacity: u32, n_markers: *mut u32, outputs: *mut a3_outputs,
@@ -189,6 +198,10 @@ extern "C" {
     pub fn a3_decode_candidates(
         det: *mut a3_detector, grey: *const u8, n_frames: u32, width: u32, height: u32, quads: *const u32, quad_frame: *const u32,
         n_quads: u32, decodes: *mut a3_decode, patches: *mut u8,
+    ) -> a3_status;
+    pub fn a3_refine_corners(
+        det: *mut a3_detector, grey: *const u8, n_frames: u32, width: u32, height: u32, corners: *const u32, corner_frame: *const u32,
+        n: u32, refined: *mut f32, ok: *mut u8,
     ) -> a3_status;
 
     // pose step (reference src/pose.rs, src/pinhole.rs)

@@ -16,6 +16,9 @@ pub struct Marker {
     pub code: u64,
     pub corners: Vec<(u32, u32)>,
     pub hamming_distance: u8,
+    /// Not in the reference: the sub-pixel corners in the order of `corners` (pixel-centre convention) when this thread
+    /// asked for them (`set_corner_refinement(true)`) and the refinement held; `None` otherwise.
+    pub corners_refined: Option<[(f32, f32); 4]>,
 }
 
 /// reference `src/aruco.rs:16-21`
@@ -113,6 +116,16 @@ pub fn set_device(device: i32) {
     DEVICE.with(|d| d.set(device));
 }
 
+thread_local! {
+    /// Sub-pixel corners for this thread's `detect` calls (default off); see `set_corner_refinement`.
+    static REFINE: std::cell::Cell<bool> = std::cell::Cell::new(false);
+}
+/// Also refine every marker's corners to sub-pixel precision (kernel K5) in this thread's `detect` calls:
+/// `Marker::corners_refined`.  A wrapper-side option: the reference's `DetectorConfig` has no such field.
+pub fn set_corner_refinement(on: bool) {
+    REFINE.with(|r| r.set(on));
+}
+
 /// A handle out of the library's cache; goes back (warm) when dropped.
 pub(crate) struct Lease(pub(crate) *mut sys::a3_detector);
 impl Drop for Lease {
@@ -144,6 +157,9 @@ impl Detector {
         let st = unsafe { sys::a3_detector_acquire(&cfg, &self.dictionary.raw(), DEVICE.with(|d| d.get()), &mut h) };
         if st != sys::A3_OK {
             panic!("{}", last_error()); // threshold_window == 0 / epsilon <= 0 panic inside imageproc in the reference
+        }
+        if REFINE.with(|r| r.get()) {
+            unsafe { sys::a3_detector_set_corner_refinement(h, sys::A3_CORNERS_REFINED) }; // the release resets it
         }
         Lease(h)
     }
@@ -181,6 +197,7 @@ impl Detector {
         let hs = self.config.homography_sample_size;
         let (px, np) = ((w as usize) * (h as usize), hs * hs);
         let full = what == Outputs::Full;
+        let refine = REFINE.with(|r| r.get());
         let (mut cap_m, mut cap_c) = (64 * n as usize + 1024, if full { 128 * n as usize + 2048 } else { 0 });
         loop {
             let mut markers: Vec<sys::a3_marker> = Vec::with_capacity(cap_m);
@@ -189,28 +206,38 @@ impl Detector {
             let mut cframe = vec![0u32; cap_c];
             let mut patches = vec![0u8; cap_c * np];
             let mut decs: Vec<sys::a3_decode> = Vec::with_capacity(cap_c);
+            let mut refined = vec![0f32; if refine { cap_m * 8 } else { 0 }];
             let mut out = sys::a3_outputs {
                 grey: grey.as_mut_ptr(), mask: ptr::null_mut(), candidates: cands.as_mut_ptr(), candidate_frame: cframe.as_mut_ptr(),
                 homographies: patches.as_mut_ptr(), decodes: decs.as_mut_ptr(), cand_capacity: cap_c as u32, n_candidates: 0,
                 frame_marker_offsets: ptr::null_mut(), marker_poses: ptr::null_mut(),
+                marker_corners: if refine { refined.as_mut_ptr() } else { ptr::null_mut() },
             };
+            if !full {
+                // markers only (plus their refined corners): no per-candidate output, so the device assembles the markers
+                out = sys::a3_outputs { grey: ptr::null_mut(), candidates: ptr::null_mut(), candidate_frame: ptr::null_mut(),
+                                        homographies: ptr::null_mut(), decodes: ptr::null_mut(), cand_capacity: 0, ..out };
+            }
             let mut nm = 0u32;
             let st = unsafe {
                 sys::a3_detect_batch(hd.0, frames.as_ptr() as *const _, fmt, sys::A3_MEM_HOST, n, w, h, w as usize * bpp,
                                      w as usize * bpp * h as usize, markers.as_mut_ptr(), cap_m as u32, &mut nm,
-                                     if full { &mut out } else { ptr::null_mut() }, ptr::null_mut())
+                                     if full || refine { &mut out } else { ptr::null_mut() }, ptr::null_mut())
             };
             if st == sys::A3_ERR_CAPACITY {
                 cap_m = cap_m.max(nm as usize);
-                cap_c = cap_c.max(out.n_candidates as usize);
+                if full {
+                    cap_c = cap_c.max(out.n_candidates as usize);
+                }
                 continue;
             }
             if st != sys::A3_OK {
                 panic!("{}", last_error());
             }
+            let n_cand = if full { out.n_candidates as usize } else { 0 }; // a markers-only call reports the count only
             unsafe {
                 markers.set_len(nm as usize);
-                decs.set_len(out.n_candidates as usize);
+                decs.set_len(n_cand);
             }
             let mut dets: Vec<Detection> = (0..n).map(|_| Detection::default()).collect();
             if full {
@@ -223,7 +250,7 @@ impl Detector {
                     }
                 }
             }
-            for k in 0..out.n_candidates as usize {
+            for k in 0..n_cand {
                 let d = &mut dets[cframe[k] as usize];
                 d.candidates.push((0..4).map(|j| Point::new(cands[k * 8 + 2 * j], cands[k * 8 + 2 * j + 1])).collect());
                 d.homographies.push(if decs[k].homography_ok != 0 {
@@ -232,12 +259,14 @@ impl Detector {
                     GrayImage::new(1, 1) // reference src/aruco.rs:256
                 });
             }
-            for m in &markers {
+            for (i, m) in markers.iter().enumerate() {
+                let r = |k: usize| (refined[i * 8 + 2 * k], refined[i * 8 + 2 * k + 1]);
                 dets[m.frame as usize].markers.push(Marker {
                     id: m.id as usize,
                     code: m.code,
                     corners: (0..4).map(|k| (m.corners[2 * k], m.corners[2 * k + 1])).collect(),
                     hamming_distance: m.hamming_distance,
+                    corners_refined: if m.corners_refined != 0 { Some([r(0), r(1), r(2), r(3)]) } else { None },
                 });
             }
             return dets;
