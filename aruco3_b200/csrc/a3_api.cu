@@ -341,6 +341,13 @@ a3_status check_config(const a3_config &c) {
 
 uint32_t bytes_per_pixel(a3_format f) { return (uint32_t)fmt_bpp((int)f); }
 
+// Bytes of caller memory that `cn` consecutive frames cover: from the first frame's first pixel to the last frame's last
+// pixel.  Host input copies move exactly this much; the rest of the last frame's stride (the parent image's row tail when the
+// frames are crops, a gap after the frame) is memory the caller never passed.  The device slots stay frame_stride apart.
+size_t input_span(size_t cn, uint32_t w, uint32_t h, uint32_t bpp, size_t pitch, size_t frame_stride) {
+    return (cn - 1) * frame_stride + (size_t)(h - 1) * pitch + (size_t)w * bpp;
+}
+
 double now_ms() {
     return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count();
 }
@@ -725,8 +732,8 @@ a3_status a3_gray_threshold_batch(a3_detector *d, const void *frames, a3_format 
     for (uint32_t f0 = 0; f0 < n; f0 += (uint32_t)chunk) {
         const uint32_t c = n - f0 < chunk ? n - f0 : (uint32_t)chunk;
         A3_CUDA(d->d_src.reserve((size_t)c * frame_stride));
-        A3_CUDA(cudaMemcpyAsync(d->d_src.p, static_cast<const uint8_t *>(frames) + (size_t)f0 * frame_stride, (size_t)c * frame_stride,
-                                cudaMemcpyHostToDevice, s));
+        A3_CUDA(cudaMemcpyAsync(d->d_src.p, static_cast<const uint8_t *>(frames) + (size_t)f0 * frame_stride,
+                                input_span(c, w, h, bpp, pitch, frame_stride), cudaMemcpyHostToDevice, s));
         if (grey) A3_CUDA(d->d_grey.reserve(c * px));
         if (mask) A3_CUDA(d->d_mask.reserve(c * px));
         if (mask_bits) A3_CUDA(d->d_bits.reserve(c * wpr * h));
@@ -1259,7 +1266,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                     }
                 }
                 const uint32_t f0 = c * (uint32_t)fe, cn = sn - f0 < fe ? sn - f0 : (uint32_t)fe;
-                const size_t bytes = (size_t)cn * frame_stride;
+                const size_t bytes = input_span(cn, w, h, bpp, pitch, frame_stride);
                 const uint32_t pieces = (uint32_t)((bytes + kPiece - 1) / kPiece);
                 const uint8_t *src = src_all + (size_t)(s0 + f0) * frame_stride;
                 uint8_t *dst = d->h_stage_in.p + (size_t)(c % kHostRing) * in_slot_bytes;
@@ -1287,7 +1294,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             }
             if (j >= kStaging) A3_CUDA(cudaStreamWaitEvent(d->s_copy, ev_k1b[j - kStaging], 0));  // the slot's previous K1 is done
             A3_CUDA(cudaEventRecord(ev_h2da[j], d->s_copy));
-            A3_CUDA(cudaMemcpyAsync(slot, from, (size_t)cn * frame_stride, cudaMemcpyHostToDevice, d->s_copy));
+            A3_CUDA(cudaMemcpyAsync(slot, from, input_span(cn, w, h, bpp, pitch, frame_stride), cudaMemcpyHostToDevice, d->s_copy));
             A3_CUDA(cudaEventRecord(ev_h2db[j], d->s_copy));
             return A3_OK;
         };
