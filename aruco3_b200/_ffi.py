@@ -51,7 +51,7 @@ class A3Stats(C.Structure):
                [(n, C.c_uint32) for n in ("pixel_kernel_launches", "decode_kernel_launches", "host_threads", "contour_kernel_launches",
                                           "host_fallback_frames", "pose_kernel_launches", "one_shot", "one_shot_retry", "input_staged", "output_staged",
                                           "refine_kernel_launches")] + \
-               [("ms_refine_kernel", C.c_double)]
+               [("ms_refine_kernel", C.c_double), ("board_kernel_launches", C.c_uint32), ("ms_board_kernel", C.c_double)]
 
     def as_dict(self):
         return {f: getattr(self, f) for f, _ in self._fields_}
@@ -61,11 +61,19 @@ class A3Outputs(C.Structure):
     _fields_ = [("grey", C.c_void_p), ("mask", C.c_void_p), ("candidates", C.c_void_p), ("candidate_frame", C.c_void_p),
                 ("homographies", C.c_void_p), ("decodes", C.c_void_p), ("cand_capacity", C.c_uint32),
                 ("n_candidates", C.c_uint32), ("frame_marker_offsets", C.c_void_p), ("marker_poses", C.c_void_p),
-                ("marker_corners", C.c_void_p)]
+                ("marker_corners", C.c_void_p), ("board_poses", C.c_void_p)]
 
 
 class A3Pose(C.Structure):
     _fields_ = [("error", C.c_float), ("rotation", C.c_float * 9), ("translation", C.c_float * 3)]
+
+
+class A3Board(C.Structure):
+    _fields_ = [("n_markers", C.c_uint32), ("ids", C.POINTER(C.c_uint64)), ("corners", C.POINTER(C.c_float))]
+
+
+class A3BoardPose(C.Structure):
+    _fields_ = [("best", A3Pose), ("alt", A3Pose), ("n_markers", C.c_uint32), ("ok", C.c_uint8), ("reserved", C.c_uint8 * 3)]
 
 
 class A3CameraIntrinsics(C.Structure):
@@ -148,6 +156,8 @@ def lib():
     L.a3_refine_corners.argtypes = [vp, vp, u32, u32, u32, vp, vp, u32, vp, vp]
     fp, f32, PK, PP = C.POINTER(C.c_float), C.c_float, C.POINTER(A3CameraIntrinsics), C.POINTER(A3Pose)
     L.a3_detector_set_pose.argtypes = [vp, u32, f32, PK]
+    L.a3_detector_set_board.argtypes = [vp, C.POINTER(A3Board), u32, PK]
+    L.a3_solve_board.argtypes = [vp, vp, vp, vp, u32, u32, u32, u32, vp]
     L.a3_solve_with_intrinsics.argtypes = [vp, vp, u32, f32, PK, vp, vp]
     L.a3_solve_with_undistorted_points.argtypes = [vp, vp, u32, f32, u32, u32, vp, vp]
     L.a3_solve_with_normalized_points.argtypes = [vp, vp, u32, f32, vp, vp]

@@ -29,6 +29,7 @@
 #include <vector>
 
 #include "a3_internal.h"
+#include "k6_board_spec.h"
 
 namespace a3 {
 
@@ -235,19 +236,24 @@ struct DecodeBlock {
     PinBuf<float> h_ref;
     DevBuf<uint8_t> d_refok;
     PinBuf<uint8_t> h_refok;
-    cudaEvent_t ev_a = nullptr, ev_b = nullptr, ev_r0 = nullptr, ev_r1 = nullptr;  // around K2, around K5
+    DevBuf<a3_board_pose> d_board;  // K6: one board pose per frame of the group
+    PinBuf<a3_board_pose> h_board;
+    PinBuf<uint32_t> h_qoff;        // K6: per-frame quad offsets of a group whose quads came from the host
+    cudaEvent_t ev_a = nullptr, ev_b = nullptr, ev_r0 = nullptr, ev_r1 = nullptr, ev_k6a = nullptr, ev_k6b = nullptr;  // around K2, K5, K6
     uint32_t n_quads = 0;
     // where the host reads this group's records: h_dec / h_pose / h_ref, or the one-shot arena
     const a3_decode *dec_view = nullptr;
     const a3_pose *pose_view = nullptr;
     const float *ref_view = nullptr;
     const uint8_t *refok_view = nullptr;
+    const a3_board_pose *board_view = nullptr;
     void release() {
         h_quads.release(); h_qframe.release(); h_dec.release(); d_quads.release(); d_qframe.release(); d_dec.release(); d_patches.release();
         d_info.release(); d_qoff.release();
         d_pose.release(); h_pose.release();
         d_ref.release(); h_ref.release(); d_refok.release(); h_refok.release();
-        for (cudaEvent_t *e : {&ev_a, &ev_b, &ev_r0, &ev_r1}) { if (*e) cudaEventDestroy(*e); *e = nullptr; }
+        d_board.release(); h_board.release(); h_qoff.release();
+        for (cudaEvent_t *e : {&ev_a, &ev_b, &ev_r0, &ev_r1, &ev_k6a, &ev_k6b}) { if (*e) cudaEventDestroy(*e); *e = nullptr; }
     }
 };
 
@@ -324,6 +330,14 @@ struct a3_detector {
     uint32_t corner_mode = A3_CORNERS_INTEGER;
     a3::DevBuf<float> d_refined;      // a3_refine_corners: refined corners and their flags
     a3::DevBuf<uint8_t> d_refined_ok;
+    // board pose (K6): the board as its id -> slot table and points on the device; board_n = 0 is off
+    uint32_t board_n = 0, board_mode = A3_POSE_OFF;
+    a3_camera_intrinsics board_k{};
+    a3::DevBuf<uint16_t> d_board_slots;
+    a3::DevBuf<float> d_board_pts;
+    a3::DevBuf<uint64_t> d_probe_ids;  // a3_solve_board
+    a3::DevBuf<uint32_t> d_probe_off;
+    a3::DevBuf<a3_board_pose> d_probe_out;
 };
 
 namespace a3 {
@@ -517,6 +531,23 @@ cudaError_t launch_refine(DecodeBlock &b, const uint8_t *grey, uint32_t w, uint3
     return e;
 }
 
+// K6 over the frames [0, n_frames) of a decode group or of the one-shot arena, bracketed by the block's events
+cudaError_t launch_board(const a3_detector *d, DecodeBlock &b, const a3_decode *dec, const uint32_t *quads, const float *ref,
+                         const uint32_t *offsets, const uint32_t *skip, uint32_t n_frames, uint32_t w, uint32_t h, a3_board_pose *out,
+                         cudaStream_t s) {
+    cudaError_t e = cudaSuccess;
+    if (!b.ev_k6a) e = cudaEventCreate(&b.ev_k6a);
+    if (e == cudaSuccess && !b.ev_k6b) e = cudaEventCreate(&b.ev_k6b);
+    if (e == cudaSuccess) e = cudaEventRecord(b.ev_k6a, s);
+    K6Params kp;
+    kp.decodes = dec; kp.quads = quads; kp.corners_f32 = ref; kp.offsets = offsets; kp.skip = skip; kp.n_frames = n_frames;
+    kp.slots = d->d_board_slots.p; kp.n_codes = d->dict.n_codes; kp.board = d->d_board_pts.p; kp.n_board = d->board_n;
+    kp.mode = d->board_mode; kp.image_w = w; kp.image_h = h; kp.k = d->board_k; kp.out = out;
+    if (e == cudaSuccess) e = k6_board(kp, s);
+    if (e == cudaSuccess) e = cudaEventRecord(b.ev_k6b, s);
+    return e;
+}
+
 }  // namespace
 }  // namespace a3
 
@@ -635,6 +666,7 @@ void a3_detector_release(a3_detector *d) {
     d->contour_mode = A3_CONTOURS_DEVICE;
     d->pose_mode = A3_POSE_OFF;
     d->corner_mode = A3_CORNERS_INTEGER;
+    d->board_n = 0; d->board_mode = A3_POSE_OFF;
     d->has_tuning = false; d->k1_tuning = K1Tuning{}; d->chunk_override = 0;
     a3_detector *evict = nullptr;
     {
@@ -668,6 +700,7 @@ void a3_detector_destroy(a3_detector *d) {
     d->d_qoff.release(); d->d_k2queue.release(); d->d_shot.release(); d->h_shot.release();
     d->d_pose_in.release(); d->d_pose_out.release(); d->h_pose_out.release();
     d->d_refined.release(); d->d_refined_ok.release();
+    d->d_board_slots.release(); d->d_board_pts.release(); d->d_probe_ids.release(); d->d_probe_off.release(); d->d_probe_out.release();
     d->copy_pool.stop();
     d->h_stage_in.release(); d->h_stage_out.release();
     d->events.release();
@@ -890,9 +923,11 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
     const size_t np = (size_t)d->cfg.homography_sample_size * d->cfg.homography_sample_size;
     const bool want_mask = outs && outs->mask, want_grey = outs && outs->grey, want_patches = outs && outs->homographies;
     const bool want_poses = outs && outs->marker_poses && markers && d->pose_mode != A3_POSE_OFF;
-    // K5 refines the markers' corners (a3_marker.corners_refined, a3_outputs.marker_corners) and K4 then solves from them
-    const bool want_refine = markers && d->corner_mode == A3_CORNERS_REFINED;
-    float *const out_corners = want_refine && outs ? outs->marker_corners : nullptr;
+    // K6 solves the board's pose per frame (a3_outputs.board_poses), whatever else the caller asked for
+    const bool want_board = d->board_n > 0 && outs && outs->board_poses;  // no board: the field is never read
+    // K5 refines the markers' corners (a3_marker.corners_refined, a3_outputs.marker_corners); K4 and K6 then solve from them
+    const bool want_refine = (markers || want_board) && d->corner_mode == A3_CORNERS_REFINED;
+    float *const out_corners = want_refine && markers && outs ? outs->marker_corners : nullptr;
     const K1Tuning *tune = d->has_tuning ? &d->k1_tuning : nullptr;
     const uint8_t *src_all = static_cast<const uint8_t *>(frames);
     a3_stats st;
@@ -1007,7 +1042,8 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
         const size_t off_stats = 16, off_markers = (off_stats + 24 * shot_c + 15) & ~(size_t)15;
         const size_t off_mposes = off_markers + (lean ? (size_t)shot_cap * sizeof(a3_marker) : 0);
         const size_t off_mcorners = off_mposes + ((lean && want_poses) ? (size_t)shot_cap * 2 * sizeof(a3_pose) : 0);  // K5's, per marker
-        const size_t off_quads = (off_mcorners + ((lean && want_refine) ? (size_t)shot_cap * 32 : 0) + 15) & ~(size_t)15;
+        const size_t off_board = off_mcorners + ((lean && want_refine) ? (size_t)shot_cap * 32 : 0);  // K6's, per frame
+        const size_t off_quads = (off_board + (want_board ? (size_t)sn * sizeof(a3_board_pose) : 0) + 15) & ~(size_t)15;
         const size_t off_dec = off_quads + (size_t)shot_cap * 32;
         const size_t off_pose = off_dec + (size_t)shot_cap * sizeof(a3_decode);
         const size_t off_ref = off_pose + (want_poses ? (size_t)shot_cap * 2 * sizeof(a3_pose) : 0);  // K5's, per candidate
@@ -1114,6 +1150,9 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 kp.marker_size = d->pose_marker_size; kp.image_w = w; kp.image_h = h; kp.k = d->pose_k; kp.poses = d_pose;
                 A3_CUDA(k4_pose(kp, d->s_pixel));
             }
+            if (want_board)
+                A3_CUDA(launch_board(d, b, d_dec, d_quads, d_ref, d->d_qoff.p, d_info + 1, sn, w, h,
+                                     reinterpret_cast<a3_board_pose *>(d->d_shot.p + off_board), d->s_pixel));
             if (lean) {
                 assemble_markers_kernel<<<n_chunks, 1024, 0, d->s_pixel>>>(d_dec, d_quads, b.d_qframe.p, d->d_qoff.p, want_poses ? d_pose : nullptr,
                                                                     d_ref, d_refok, cap, d_info, d_chain,
@@ -1140,6 +1179,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 b.pose_view = reinterpret_cast<const a3_pose *>(d->h_shot.p + off_pose);
                 b.ref_view = reinterpret_cast<const float *>(d->h_shot.p + off_ref);
                 b.refok_view = d->h_shot.p + off_refok;
+                b.board_view = reinterpret_cast<const a3_board_pose *>(d->h_shot.p + off_board);
                 const uint32_t *h_quads = reinterpret_cast<const uint32_t *>(d->h_shot.p + off_quads);
                 uint32_t k = 0;
                 for (uint32_t i = 0; i < sn; i++) {
@@ -1155,6 +1195,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 st.decode_kernel_launches++;
                 if (want_poses) st.pose_kernel_launches++;
                 if (want_refine) st.refine_kernel_launches++;
+                if (want_board) st.board_kernel_launches++;
                 st.one_shot = 1;
                 one_shot_done = true;
                 lean_done = lean;
@@ -1368,7 +1409,16 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             b.n_quads = nq;
             if (one_shot && ngroups == 1) { d->hist_nq = nq ? nq : 1; d->hist_nq_n = n; d->hist_nq_w = w; d->hist_nq_h = h; }
             if (!b.ev_a) { A3_CUDA(cudaEventCreate(&b.ev_a)); A3_CUDA(cudaEventCreate(&b.ev_b)); }
-            if (nq == 0) return A3_OK;
+            if (nq == 0) {
+                if (want_board) {  // no candidates: every frame of the group has the empty board pose
+                    A3_CUDA(b.h_board.reserve(f1 - f0));
+                    a3_board_pose e{};
+                    a3_pose_default(&e.best); a3_pose_default(&e.alt);
+                    for (uint32_t i = 0; i < f1 - f0; i++) b.h_board.p[i] = e;
+                    b.board_view = b.h_board.p;
+                }
+                return A3_OK;
+            }
             A3_CUDA(b.h_quads.reserve((size_t)nq * 8)); A3_CUDA(b.h_qframe.reserve(nq)); A3_CUDA(b.h_dec.reserve(nq));
             A3_CUDA(b.d_quads.reserve((size_t)nq * 8)); A3_CUDA(b.d_qframe.reserve(nq)); A3_CUDA(b.d_dec.reserve(nq));
             if (want_patches) A3_CUDA(b.d_patches.reserve(nq * np));
@@ -1398,6 +1448,13 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 }
                 A3_CUDA(cudaMemcpyAsync(b.d_quads.p, b.h_quads.p, (size_t)nq * 32, cudaMemcpyHostToDevice, d->s_decode));
                 A3_CUDA(cudaMemcpyAsync(b.d_qframe.p, b.h_qframe.p, (size_t)nq * 4, cudaMemcpyHostToDevice, d->s_decode));
+                if (want_board) {  // K6's per-frame offsets travel with the quads
+                    A3_CUDA(b.h_qoff.reserve((size_t)(f1 - f0) + 1)); A3_CUDA(b.d_qoff.reserve((size_t)(f1 - f0) + 1));
+                    uint32_t o = 0;
+                    for (uint32_t i = f0; i < f1; i++) { b.h_qoff.p[i - f0] = o; o += (uint32_t)(frame_quads[i].size() / 8); }
+                    b.h_qoff.p[f1 - f0] = o;
+                    A3_CUDA(cudaMemcpyAsync(b.d_qoff.p, b.h_qoff.p, (size_t)(f1 - f0 + 1) * 4, cudaMemcpyHostToDevice, d->s_decode));
+                }
             }
             p.quads = b.d_quads.p; p.quad_frame = b.d_qframe.p; p.n_quads = nq; p.decodes = b.d_dec.p;
             p.patches = want_patches ? b.d_patches.p : nullptr;
@@ -1435,6 +1492,15 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 st.pose_kernel_launches++;
                 A3_CUDA(cudaMemcpyAsync(b.h_pose.p, b.d_pose.p, (size_t)nq * 2 * sizeof(a3_pose), cudaMemcpyDeviceToHost, d->s_decode));
                 b.pose_view = b.h_pose.p;
+            }
+            if (want_board) {  // K6 behind K2 (and K5), on the records, the quads or K5's corners where they lie
+                const uint32_t gn = f1 - f0;
+                A3_CUDA(b.d_board.reserve(gn)); A3_CUDA(b.h_board.reserve(gn));
+                A3_CUDA(launch_board(d, b, b.d_dec.p, b.d_quads.p, want_refine ? b.d_ref.p : nullptr, b.d_qoff.p, nullptr, gn, w, h, b.d_board.p,
+                                     d->s_decode));
+                st.board_kernel_launches++;
+                A3_CUDA(cudaMemcpyAsync(b.h_board.p, b.d_board.p, (size_t)gn * sizeof(a3_board_pose), cudaMemcpyDeviceToHost, d->s_decode));
+                b.board_view = b.h_board.p;
             }
             return A3_OK;
         };
@@ -1496,6 +1562,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                     if (one_shot_done && d->blocks[0]->n_quads) {  // the decode (and K5) sit between those two events on this route
                         cudaEventElapsedTime(&ms, d->blocks[0]->ev_a, d->blocks[0]->ev_b); st.ms_mask_d2h -= ms;
                         if (want_refine) { cudaEventElapsedTime(&ms, d->blocks[0]->ev_r0, d->blocks[0]->ev_r1); st.ms_mask_d2h -= ms; }
+                        if (want_board) { cudaEventElapsedTime(&ms, d->blocks[0]->ev_k6a, d->blocks[0]->ev_k6b); st.ms_mask_d2h -= ms; }
                     }
                 }
             } else {
@@ -1525,6 +1592,8 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             DecodeBlock &b = *d->blocks[0];
             if (b.n_quads && stats) { cudaEventElapsedTime(&ms, b.ev_a, b.ev_b); st.ms_decode_kernel += ms; }
             if (b.n_quads && stats && want_refine) { cudaEventElapsedTime(&ms, b.ev_r0, b.ev_r1); st.ms_refine_kernel += ms; }
+            if (stats && want_board) { cudaEventElapsedTime(&ms, b.ev_k6a, b.ev_k6b); st.ms_board_kernel += ms; }
+            if (want_board) memcpy(outs->board_poses, b.board_view, (size_t)sn * sizeof(a3_board_pose));
             const uint32_t nm = h_info[3], take = nm < marker_capacity ? nm : marker_capacity;
             memcpy(markers, d->h_shot.p + off_markers, (size_t)take * sizeof(a3_marker));
             if (want_poses) memcpy(outs->marker_poses, d->h_shot.p + off_mposes, (size_t)take * 2 * sizeof(a3_pose));
@@ -1546,6 +1615,10 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             if (b.n_quads && stats) { cudaEventElapsedTime(&ms, b.ev_a, b.ev_b); st.ms_decode_kernel += ms; }
             if (b.n_quads && stats && want_refine) { cudaEventElapsedTime(&ms, b.ev_r0, b.ev_r1); st.ms_refine_kernel += ms; }
             const uint32_t f0 = g * group, f1 = f0 + group_size(g);
+            if (want_board) {
+                if (b.n_quads && stats) { cudaEventElapsedTime(&ms, b.ev_k6a, b.ev_k6b); st.ms_board_kernel += ms; }
+                memcpy(outs->board_poses + s0 + f0, b.board_view, (size_t)(f1 - f0) * sizeof(a3_board_pose));
+            }
             if (want_patches && b.n_quads && total_cands < outs->cand_capacity) {
                 const uint32_t room = outs->cand_capacity - total_cands, m = b.n_quads < room ? b.n_quads : room;
                 A3_CUDA(cudaMemcpy(outs->homographies + (size_t)total_cands * np, b.d_patches.p, (size_t)m * np, cudaMemcpyDeviceToHost));
@@ -1614,6 +1687,83 @@ a3_status a3_detector_set_pose(a3_detector *d, uint32_t mode, float marker_size_
     d->pose_mode = mode;
     d->pose_marker_size = marker_size_mm;
     if (k) d->pose_k = *k;
+    return A3_OK;
+}
+
+// ---- board pose (K6) ------------------------------------------------------------------------------------------------
+
+a3_status a3_detector_set_board(a3_detector *d, const a3_board *board, uint32_t mode, const a3_camera_intrinsics *k) {
+    if (!d) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: null detector");
+    if (!board) {
+        d->board_n = 0;
+        d->board_mode = A3_POSE_OFF;
+        return A3_OK;
+    }
+    if (mode != A3_POSE_UNDISTORTED && mode != A3_POSE_INTRINSICS)
+        return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: mode must be UNDISTORTED or INTRINSICS");
+    if (mode == A3_POSE_INTRINSICS && !k) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: intrinsics required");
+    const uint32_t m = board->n_markers;
+    if (m == 0 || m > A3_K6_MAX_MARKERS) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: a board has 1 to 1024 markers");
+    if (!board->ids || !board->corners) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: null ids or corners");
+    if (d->dict.n_codes > A3_K6_MAX_CODES) return fail(A3_ERR_UNSUPPORTED, "a3_detector_set_board: dictionaries of more than 8192 codes");
+    std::vector<uint16_t> slots(d->dict.n_codes ? d->dict.n_codes : 1, (uint16_t)A3_K6_NO_SLOT);
+    for (uint32_t i = 0; i < m; i++) {
+        const uint64_t id = board->ids[i];
+        if (id >= d->dict.n_codes) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: id not below the dictionary's code count");
+        if (slots[id] != A3_K6_NO_SLOT) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: duplicate id");
+        slots[id] = (uint16_t)i;
+    }
+    for (size_t i = 0; i < (size_t)m * 8; i++)
+        if (!isfinite(board->corners[i])) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: non-finite coordinate");
+    A3_CUDA(cudaSetDevice(d->device));
+    A3_CUDA(d->d_board_slots.reserve(slots.size()));
+    A3_CUDA(d->d_board_pts.reserve((size_t)m * 8));
+    // the decode stream reads the previous board until its work is done; these copies are ordered behind it
+    A3_CUDA(cudaStreamSynchronize(d->s_decode));
+    A3_CUDA(cudaStreamSynchronize(d->s_pixel));
+    A3_CUDA(cudaMemcpy(d->d_board_slots.p, slots.data(), slots.size() * sizeof(uint16_t), cudaMemcpyHostToDevice));
+    A3_CUDA(cudaMemcpy(d->d_board_pts.p, board->corners, (size_t)m * 32, cudaMemcpyHostToDevice));
+    d->board_n = m;
+    d->board_mode = mode;
+    if (k) d->board_k = *k;
+    return A3_OK;
+}
+
+a3_status a3_solve_board(a3_detector *d, const uint64_t *ids, const float *corners, const uint32_t *frame, uint32_t n, uint32_t n_frames,
+                         uint32_t image_w, uint32_t image_h, a3_board_pose *out) {
+    if (!d || (n && (!ids || !corners)) || (n_frames && !out)) return fail(A3_ERR_INVALID_ARGUMENT, "a3_solve_board: null argument");
+    if (d->board_n == 0) return fail(A3_ERR_INVALID_ARGUMENT, "a3_solve_board: the detector has no board (a3_detector_set_board)");
+    if (n_frames == 0) {
+        if (n) return fail(A3_ERR_INVALID_ARGUMENT, "a3_solve_board: markers but no frames");
+        return A3_OK;
+    }
+    if (d->board_mode == A3_POSE_UNDISTORTED && (image_w == 0 || image_h == 0))
+        return fail(A3_ERR_INVALID_ARGUMENT, "a3_solve_board: undistorted mode needs the frame size");
+    std::vector<uint32_t> off((size_t)n_frames + 1, 0);
+    for (uint32_t i = 0; i < n; i++) {
+        const uint32_t f = frame ? frame[i] : 0;
+        if (f >= n_frames || (i && frame && f < frame[i - 1])) return fail(A3_ERR_INVALID_ARGUMENT, "a3_solve_board: frame out of range or decreasing");
+        off[f + 1]++;
+    }
+    for (uint32_t f = 0; f < n_frames; f++) off[f + 1] += off[f];
+    A3_CUDA(cudaSetDevice(d->device));
+    cudaStream_t s = d->s_decode;
+    A3_CUDA(d->d_probe_ids.reserve(n ? n : 1));
+    A3_CUDA(d->d_refined.reserve(n ? (size_t)n * 8 : 1));
+    A3_CUDA(d->d_probe_off.reserve(off.size()));
+    A3_CUDA(d->d_probe_out.reserve(n_frames));
+    if (n) {
+        A3_CUDA(cudaMemcpyAsync(d->d_probe_ids.p, ids, (size_t)n * 8, cudaMemcpyHostToDevice, s));
+        A3_CUDA(cudaMemcpyAsync(d->d_refined.p, corners, (size_t)n * 32, cudaMemcpyHostToDevice, s));
+    }
+    A3_CUDA(cudaMemcpyAsync(d->d_probe_off.p, off.data(), off.size() * 4, cudaMemcpyHostToDevice, s));
+    K6Params kp;
+    kp.ids = d->d_probe_ids.p; kp.corners_f32 = d->d_refined.p; kp.offsets = d->d_probe_off.p; kp.n_frames = n_frames;
+    kp.slots = d->d_board_slots.p; kp.n_codes = d->dict.n_codes; kp.board = d->d_board_pts.p; kp.n_board = d->board_n;
+    kp.mode = d->board_mode; kp.image_w = image_w; kp.image_h = image_h; kp.k = d->board_k; kp.out = d->d_probe_out.p;
+    A3_CUDA(k6_board(kp, s));
+    A3_CUDA(cudaMemcpyAsync(out, d->d_probe_out.p, (size_t)n_frames * sizeof(a3_board_pose), cudaMemcpyDeviceToHost, s));
+    A3_CUDA(cudaStreamSynchronize(s));
     return A3_OK;
 }
 

@@ -174,6 +174,27 @@ struct K5Params {
 };
 cudaError_t k5_corners(const K5Params &p, cudaStream_t stream);
 
+// ---- K6: one pose per frame from every visible marker of a planar board (k6_board.cu; specification oracle/a3ref_board.c)
+struct K6Params {
+    const a3_decode *decodes = nullptr;     // device n or null; when set: accepted items only, id from the record, integer corners
+                                            //   rotate_left(rotation)
+    const uint64_t *ids = nullptr;          // device n: the items' ids when decodes is null (probe; every item counts)
+    const uint32_t *quads = nullptr;        // device n*8 integer corners (screen order), read when corners_f32 is null
+    const float *corners_f32 = nullptr;     // device n*8 or null: f32 corners already in marker order (K5's, or the probe's)
+    const uint32_t *offsets = nullptr;      // device n_frames + 1: items of frame f are [offsets[f], offsets[f + 1])
+    const uint32_t *skip = nullptr;         // device flag or null: non-zero = the launch writes nothing (a one-shot route that did not hold)
+    uint32_t n_frames = 0;
+    const uint16_t *slots = nullptr;        // device n_codes: board slot of each id, A3_K6_NO_SLOT when the id is not on the board
+    uint32_t n_codes = 0;
+    const float *board = nullptr;           // device n_board*8: board points of each slot, the order of a3_marker.corners
+    uint32_t n_board = 0;
+    uint32_t mode = 0;                      // A3_POSE_UNDISTORTED / A3_POSE_INTRINSICS
+    uint32_t image_w = 0, image_h = 0;
+    a3_camera_intrinsics k{};
+    a3_board_pose *out = nullptr;           // device n_frames
+};
+cudaError_t k6_board(const K6Params &p, cudaStream_t stream);
+
 // ---- host quad stage (host_quads.cpp) ---------------------------------------------------------------
 struct QuadStats {
     uint64_t n_contours = 0, n_contour_points = 0, n_before_discard = 0;

@@ -114,6 +114,7 @@ class Detection:
     # extras for stage-by-stage parity checks (not in the reference struct)
     mask: np.ndarray | None = None
     decodes: list = field(default_factory=list)
+    board_pose: object | None = None  # BoardPose of the detector's board (Detector.set_board), else None
 
 
 _FMT = {("rgb", 3): _ffi.FMT_RGB8, ("rgb", 4): _ffi.FMT_RGBA8, ("bgr", 3): _ffi.FMT_BGR8, ("bgr", 4): _ffi.FMT_BGRA8}
@@ -149,7 +150,8 @@ class Detector:
     """
 
     def __init__(self, config: DetectorConfig | None = None, dictionary: ARDictionary | str = "ARUCO", device: int = 0,
-                 host_threads: int | None = None, contours: str = "device", corners: str = "integer"):
+                 host_threads: int | None = None, contours: str = "device", corners: str = "integer", board=None,
+                 board_intrinsics=None):
         self.config = config or DetectorConfig()
         self.dictionary = ARDictionary.new_from_named_dict(dictionary) if isinstance(dictionary, str) else dictionary
         self.device = device
@@ -164,6 +166,24 @@ class Detector:
         self._pose_mode = _ffi.POSE_OFF
         self._corner_mode = _ffi.CORNERS_INTEGER
         self.set_corner_refinement(corners)
+        self._board = None
+        if board is not None:
+            self.set_board(board, board_intrinsics)
+
+    def set_board(self, board, camera_intrinsics=None):
+        """Also solve the pose of a planar `Board` in every frame inside `detect` / `detect_batch` (kernel K6 behind the
+        decode kernel and K5) into `Detection.board_pose`, from every accepted marker on the board: its refined corners when
+        the detector refines corners, else the integer ones.  Normalisation as `set_pose`: `camera_intrinsics`, or
+        undistorted at the frame size when None.  `board=None` switches it off."""
+        if board is None:
+            check(lib().a3_detector_set_board(self._h, None, _ffi.POSE_OFF, None))
+            self._board = None
+            return
+        mode = _ffi.POSE_INTRINSICS if camera_intrinsics is not None else _ffi.POSE_UNDISTORTED
+        c = board.to_c()
+        check(lib().a3_detector_set_board(self._h, C.byref(c), mode,
+                                          C.byref(camera_intrinsics._c) if camera_intrinsics is not None else None))
+        self._board = board
 
     def set_corner_refinement(self, corners: str = "refined"):
         """`"refined"`: `detect` / `detect_batch` also return each marker's sub-pixel corners (`Marker.corners_refined`,
@@ -233,6 +253,10 @@ class Detector:
             if self._corner_mode == _ffi.CORNERS_REFINED:
                 refined = np.zeros((cap_m, 4, 2), np.float32)
                 outs.marker_corners = refined.ctypes.data
+            bposes = None
+            if self._board is not None:
+                bposes = (_ffi.A3BoardPose * n)()
+                outs.board_poses = C.cast(bposes, C.c_void_p).value
             if full:
                 grey = np.empty((n, h, w), np.uint8)
                 cands = np.zeros((cap_c, 8), np.uint32)
@@ -270,6 +294,10 @@ class Detector:
             if refined is not None:
                 dets[m.frame].markers[-1].corners_refined = [(refined[i, k, 0], refined[i, k, 1]) for k in range(4)]
                 dets[m.frame].markers[-1].refined = bool(m.corners_refined)
+        if bposes is not None:
+            from .board import BoardPose
+            for f in range(n):
+                dets[f].board_pose = BoardPose.from_c(bposes[f])
         if full:
             for f in range(n):
                 dets[f].grey = grey[f]
@@ -347,6 +375,21 @@ class Detector:
         check(lib().a3_refine_corners(self._h, g.ctypes.data, n, w, h, c.ctypes.data, cf.ctypes.data if cf is not None else None, m,
                                       out.ctypes.data, ok.ctypes.data))
         return out, ok.astype(bool)
+
+    def solve_board(self, ids, corners, frame=None, n_frames: int | None = None, image_size=None) -> list:
+        """The board solve (kernel K6) with this detector's board and mode, as a probe: markers' ids [m], f32 corners
+        [m, 4, 2] (image pixels, the order of `Marker.corners`), non-decreasing frame index [m] (None = all frame 0);
+        image_size (w, h) for undistorted mode -> [BoardPose] * n_frames."""
+        from .board import BoardPose
+        i = np.ascontiguousarray(np.asarray(ids, np.uint64).reshape(-1))
+        c = np.ascontiguousarray(np.asarray(corners, np.float32).reshape(-1, 8))
+        f = np.ascontiguousarray(np.asarray(frame, np.uint32).reshape(-1)) if frame is not None else None
+        nf = n_frames if n_frames is not None else (int(f.max()) + 1 if f is not None and f.size else 1)
+        out = (_ffi.A3BoardPose * max(nf, 1))()
+        w, h = image_size if image_size is not None else (0, 0)
+        check(lib().a3_solve_board(self._h, i.ctypes.data, c.ctypes.data, f.ctypes.data if f is not None else None, i.size, nf, w, h,
+                                   C.cast(out, C.c_void_p)))
+        return [BoardPose.from_c(out[k]) for k in range(nf)]
 
 
 def quads_from_mask(mask: np.ndarray, config: DetectorConfig | None = None) -> np.ndarray:

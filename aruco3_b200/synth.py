@@ -238,3 +238,67 @@ def render_batch(spec, n_frames: int, first_index: int = 0, out: np.ndarray | No
         out[i] = img
         truths.append(truth)
     return out, truths
+
+
+# ---- planar boards seen from a known pose (kernel K6) ------------------------------------------------------------------
+def project_points(points: np.ndarray, R: np.ndarray, t: np.ndarray, k: tuple) -> np.ndarray:
+    """Board points [n, 2] (z = 0) -> image points [n, 2] under X = R p + t and the pinhole k = (fx, fy, cx, cy), in the
+    pixel-centre convention (grey pixel (x, y) is the point (x, y))."""
+    p = np.asarray(points, np.float64).reshape(-1, 2)
+    X = p @ np.asarray(R, np.float64)[:, :2].T + np.asarray(t, np.float64)
+    fx, fy, cx, cy = k
+    return np.stack([fx * X[:, 0] / X[:, 2] + cx, fy * X[:, 1] / X[:, 2] + cy], axis=1)
+
+
+def render_board_frame(board_ids, board_corners, R, t, k: tuple, width: int, height: int, dictionary: str = "ARUCO",
+                       extra_ids=(), noise: int = 0, seed: int = 0):
+    """A planar board seen from pose (R, t) with pinhole k = (fx, fy, cx, cy) -> (uint8 [H, W, 3], [TruthMarker]).
+
+    A pinhole view of a plane is a homography, so drawing each marker on its projected quad is exact.  There is no sheet
+    around the markers (its outline would become a quad of its own).  `extra_ids`: markers that are not on the board, drawn
+    in the frame's corners (keep the board away from them).  Truth corners are in draw_marker's convention (+0.5 px from the
+    pixel-centre convention of project_points and of refined corners)."""
+    table = dictionaries.table(dictionary)
+    spec = FrameSpec("board", 0, width, height)
+    img = np.empty((height, width, 3), dtype=np.uint8)
+    img[:] = np.array(spec.background, dtype=np.uint8)
+    truth = []
+    for mid, corners in zip(np.asarray(board_ids).reshape(-1), np.asarray(board_corners, np.float64).reshape(-1, 4, 2)):
+        quad = project_points(corners, R, t, k) + 0.5
+        draw_marker(img, marker_cells(table, int(mid)), quad, spec.white, spec.black)
+        truth.append(TruthMarker(int(mid), quad))
+    side = 0.12 * min(width, height)
+    spots = [(0.04 * width, 0.04 * height), (width - 0.04 * width - side, 0.04 * height),
+             (0.04 * width, height - 0.04 * height - side), (width - 0.04 * width - side, height - 0.04 * height - side)]
+    for mid, (x0, y0) in zip(extra_ids, spots):
+        quad = np.array([[x0, y0], [x0 + side, y0], [x0 + side, y0 + side], [x0, y0 + side]])
+        draw_marker(img, marker_cells(table, int(mid)), quad, spec.white, spec.black)
+        truth.append(TruthMarker(int(mid), quad))
+    if noise:
+        rng = Rng(seed)
+        nz = rng.bytes(img.size).reshape(img.shape)
+        delta = (nz % np.uint8(2 * noise + 1)).astype(np.int16) - noise
+        img = np.clip(img.astype(np.int16) + delta, 0, 255).astype(np.uint8)
+    return img, truth
+
+
+def board_views(n: int, seed: int = 0, distance: tuple = (300.0, 420.0), tilt: float = 0.45):
+    """n seeded poses (R, t) of a board facing the camera: board y up -> image y down, the board's face toward the camera,
+    tilted by up to `tilt` radians about each in-plane axis, at `distance` along the optical axis."""
+    rng = Rng(seed)
+    out = []
+    for _ in range(n):
+        u = rng.uniform(6)
+        ax, ay, az = (u[0] * 2 - 1) * tilt, (u[1] * 2 - 1) * tilt, (u[2] * 2 - 1) * 0.5
+        cx_, sx_ = np.cos(ax), np.sin(ax)
+        cy_, sy_ = np.cos(ay), np.sin(ay)
+        cz_, sz_ = np.cos(az), np.sin(az)
+        rx = np.array([[1, 0, 0], [0, cx_, -sx_], [0, sx_, cx_]])
+        ry = np.array([[cy_, 0, sy_], [0, 1, 0], [-sy_, 0, cy_]])
+        rz = np.array([[cz_, -sz_, 0], [sz_, cz_, 0], [0, 0, 1]])
+        facing = np.diag([1.0, -1.0, -1.0])
+        R = rz @ ry @ rx @ facing
+        z = distance[0] + (distance[1] - distance[0]) * u[3]
+        t = np.array([(u[4] * 2 - 1) * 0.05 * z, (u[5] * 2 - 1) * 0.05 * z, z])
+        out.append((R, t))
+    return out

@@ -131,6 +131,9 @@ typedef struct a3_stats {
     /* corner refinement (K5, a3_detector_set_corner_refinement): launches, and the sum of its CUDA-event intervals */
     uint32_t refine_kernel_launches;
     double ms_refine_kernel;
+    /* board pose (K6, a3_detector_set_board): launches, and the sum of its CUDA-event intervals */
+    uint32_t board_kernel_launches;
+    double ms_board_kernel;
 } a3_stats;
 
 /* MarkerPose (src/pose.rs:8-12): scene-from-marker transform in OpenCV chirality (+Z forward, +Y down, +X right).
@@ -171,6 +174,8 @@ typedef struct a3_outputs {
     float *marker_corners;      /* marker_capacity*8: x0,y0..x3,y3 of markers[i] in f32, the order of a3_marker.corners; filled
                                  * when the detector refines corners (A3_CORNERS_REFINED), may be NULL.  Where a marker's
                                  * corners_refined is 0 these are its integer corners. */
+    struct a3_board_pose *board_poses; /* n: the board's pose in each frame; filled when the detector has a board
+                                        * (a3_detector_set_board), may be NULL */
 } a3_outputs;
 
 typedef struct a3_detector a3_detector;
@@ -300,6 +305,44 @@ a3_status a3_solve_with_undistorted_points(a3_detector *det, const uint32_t *cor
                                            uint32_t image_width, uint32_t image_height, a3_pose *best, a3_pose *alt);
 a3_status a3_solve_with_normalized_points(a3_detector *det, const float *points, uint32_t n, float marker_size_mm,
                                           a3_pose *best, a3_pose *alt);
+
+/* ---- board pose: one pose per frame from every visible marker of a planar board (kernel K6) ---- */
+
+/* A rigid planar board: n_markers (1..1024) distinct ids below the dictionary's code count, and for each marker its four
+ * corners (x, y) on the board plane (z = 0), in any length unit, in the order of a3_marker.corners (the marker's own TL, TR,
+ * BR, BL).  x to the right and y up on the board's face: one marker of side L centred at the origin has TL = (-L/2, +L/2),
+ * the square the single-marker solve uses. */
+typedef struct a3_board {
+    uint32_t n_markers;
+    const uint64_t *ids;   /* n_markers */
+    const float *corners;  /* n_markers*8: x0,y0..x3,y3 */
+} a3_board;
+
+/* The board's pose in one frame: the map from board points (x, y, 0) to camera coordinates, in the chirality and row-major
+ * layout of a3_pose.  best has the smaller error, alt is the other branch of the planar ambiguity.  error = RMS reprojection
+ * distance over the used corners in normalised units (unlike a3_pose.error of one marker, a sum over its 4 corners).  A
+ * branch that failed (non-finite value, singular system, translation z <= 0) is a3_pose_default (error 1e31).  n_markers =
+ * markers the solve used; ok = 0 when both branches failed or no board marker was seen (then both are the default). */
+typedef struct a3_board_pose {
+    a3_pose best, alt;
+    uint32_t n_markers;
+    uint8_t ok;
+    uint8_t reserved[3];
+} a3_board_pose;
+
+/* Make a3_detect_batch also solve the board's pose in every frame (kernel K6, queued behind the decode kernel and K5) into
+ * a3_outputs.board_poses.  Every accepted marker whose id is on the board contributes its four corners, in candidate
+ * order: K5's corners when the detector refines corners (A3_CORNERS_REFINED), else the integer corners.  An id detected more
+ * than once in a frame is skipped there.  mode: A3_POSE_UNDISTORTED (image size = the frame size) or A3_POSE_INTRINSICS (k
+ * required).  The board is copied to the device.  board = NULL switches it off; a3_detector_release resets it.  Invalid: duplicate ids, an
+ * id >= the dictionary's code count, 0 or more than 1024 markers, a non-finite coordinate, mode OFF or NORMALIZED. */
+a3_status a3_detector_set_board(a3_detector *det, const a3_board *board, uint32_t mode, const a3_camera_intrinsics *k);
+
+/* The board solve (kernel K6) as a probe, with the detector's board and mode, over n markers: ids n, corners n*8 f32 (the
+ * order of a3_marker.corners, image pixels), frame n (non-decreasing frame index of each marker, < n_frames; NULL = all
+ * frame 0).  HOST pointers; out: n_frames board poses.  image_w / image_h: the frame size (A3_POSE_UNDISTORTED). */
+a3_status a3_solve_board(a3_detector *det, const uint64_t *ids, const float *corners, const uint32_t *frame, uint32_t n,
+                         uint32_t n_frames, uint32_t image_w, uint32_t image_h, a3_board_pose *out);
 
 /* Plain host helpers (constructors and one-point conversions; nothing here is on the hot path). */
 void a3_pose_default(a3_pose *p);                                                   /* src/pose.rs:42-50        */

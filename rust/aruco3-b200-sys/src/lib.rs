@@ -105,6 +105,9 @@ pub struct a3_stats {
     pub output_staged: u32,
     pub refine_kernel_launches: u32,
     pub ms_refine_kernel: f64,
+    /// board pose (K6, `a3_detector_set_board`): launches and the sum of its CUDA-event intervals
+    pub board_kernel_launches: u32,
+    pub ms_board_kernel: f64,
 }
 
 /// MarkerPose, reference `src/pose.rs:8-12`; rotation row-major
@@ -149,6 +152,28 @@ pub struct a3_outputs {
     pub marker_poses: *mut a3_pose,
     /// marker_capacity * 8 f32 (A3_CORNERS_REFINED), may be null
     pub marker_corners: *mut f32,
+    /// n board poses (`a3_detector_set_board`), may be null
+    pub board_poses: *mut a3_board_pose,
+}
+
+/// A rigid planar board: `n_markers` distinct ids and their corners on the board plane (x right, y up), `n_markers * 8`
+/// f32 in the order of `a3_marker.corners`
+#[repr(C)]
+pub struct a3_board {
+    pub n_markers: u32,
+    pub ids: *const u64,
+    pub corners: *const f32,
+}
+
+/// The board's pose in one frame (kernel K6): board points `(x, y, 0)` -> camera; error = RMS reprojection distance
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct a3_board_pose {
+    pub best: a3_pose,
+    pub alt: a3_pose,
+    pub n_markers: u32,
+    pub ok: u8,
+    pub reserved: [u8; 3],
 }
 
 #[repr(C)]
@@ -216,6 +241,12 @@ extern "C" {
     ) -> a3_status;
     pub fn a3_solve_with_normalized_points(
         det: *mut a3_detector, points: *const f32, n: u32, marker_size_mm: f32, best: *mut a3_pose, alt: *mut a3_pose,
+    ) -> a3_status;
+    // board pose (kernel K6)
+    pub fn a3_detector_set_board(det: *mut a3_detector, board: *const a3_board, mode: u32, k: *const a3_camera_intrinsics) -> a3_status;
+    pub fn a3_solve_board(
+        det: *mut a3_detector, ids: *const u64, corners: *const f32, frame: *const u32, n: u32, n_frames: u32, image_w: u32,
+        image_h: u32, out: *mut a3_board_pose,
     ) -> a3_status;
     pub fn a3_pose_default(p: *mut a3_pose);
     pub fn a3_pose_apply_transform(p: *const a3_pose, points: *const f32, n: u32, inverse: i32, out: *mut f32);

@@ -28,6 +28,8 @@ pub struct Detection {
     pub candidates: Vec<Vec<Point<u32>>>,
     pub homographies: Vec<GrayImage>,
     pub markers: Vec<Marker>,
+    /// Not in the reference: the pose of this thread's board (`set_board`) in this frame; `None` when no board is set.
+    pub board_pose: Option<pose::BoardPose>,
 }
 
 /// reference `src/aruco.rs:23-43`
@@ -126,6 +128,43 @@ pub fn set_corner_refinement(on: bool) {
     REFINE.with(|r| r.set(on));
 }
 
+/// A rigid planar board (kernel K6): distinct `ids` and, per marker, its four corners `x0,y0..x3,y3` on the board plane
+/// (z = 0, x right, y up, any length unit) in the order of `Marker::corners`.
+#[derive(Clone, Debug)]
+pub struct Board {
+    pub ids: Vec<u64>,
+    pub corners: Vec<[f32; 8]>,
+}
+
+impl Board {
+    /// `cols` x `rows` square markers `separation` apart, centred on the origin; row 0 at the top, ids row-major from `first_id`.
+    pub fn grid(cols: u32, rows: u32, marker_size: f32, separation: f32, first_id: u64) -> Board {
+        let pitch = marker_size + separation;
+        let w = cols as f32 * marker_size + (cols as f32 - 1.0) * separation;
+        let h = rows as f32 * marker_size + (rows as f32 - 1.0) * separation;
+        let (mut ids, mut corners) = (Vec::new(), Vec::new());
+        for r in 0..rows {
+            for c in 0..cols {
+                let (x0, y0) = (-w / 2.0 + c as f32 * pitch, h / 2.0 - r as f32 * pitch);
+                ids.push(first_id + (r * cols + c) as u64);
+                corners.push([x0, y0, x0 + marker_size, y0, x0 + marker_size, y0 - marker_size, x0, y0 - marker_size]);
+            }
+        }
+        Board { ids, corners }
+    }
+}
+
+thread_local! {
+    /// The board this thread's `detect` calls solve, with the intrinsics (`None`: undistorted at the frame size).
+    static BOARD: std::cell::RefCell<Option<(Board, Option<pose::CameraIntrinsics>)>> = std::cell::RefCell::new(None);
+}
+/// Also solve the pose of `board` in every frame of this thread's `detect` calls (kernel K6): `Detection::board_pose`.
+/// `k = None` normalises by the frame size, as `solve_with_undistorted_points`; `board = None` switches it off.  Like
+/// `set_corner_refinement`, a wrapper-side option, set on each leased handle (the release resets it).
+pub fn set_board(board: Option<Board>, k: Option<pose::CameraIntrinsics>) {
+    BOARD.with(|b| *b.borrow_mut() = board.map(|b| (b, k)));
+}
+
 /// A handle out of the library's cache; goes back (warm) when dropped.
 pub(crate) struct Lease(pub(crate) *mut sys::a3_detector);
 impl Drop for Lease {
@@ -161,6 +200,19 @@ impl Detector {
         if REFINE.with(|r| r.get()) {
             unsafe { sys::a3_detector_set_corner_refinement(h, sys::A3_CORNERS_REFINED) }; // the release resets it
         }
+        BOARD.with(|b| {
+            if let Some((board, k)) = &*b.borrow() {
+                let raw = sys::a3_board { n_markers: board.ids.len() as u32, ids: board.ids.as_ptr(), corners: board.corners.as_ptr() as *const f32 };
+                let (mode, kp) = match k {
+                    Some(k) => (sys::A3_POSE_INTRINSICS, k as *const sys::a3_camera_intrinsics),
+                    None => (sys::A3_POSE_UNDISTORTED, ptr::null()),
+                };
+                if unsafe { sys::a3_detector_set_board(h, &raw, mode, kp) } != sys::A3_OK {
+                    unsafe { sys::a3_detector_release(h) };
+                    panic!("{}", last_error());
+                }
+            }
+        });
         Lease(h)
     }
 
@@ -198,6 +250,7 @@ impl Detector {
         let (px, np) = ((w as usize) * (h as usize), hs * hs);
         let full = what == Outputs::Full;
         let refine = REFINE.with(|r| r.get());
+        let board = BOARD.with(|b| b.borrow().is_some());
         let (mut cap_m, mut cap_c) = (64 * n as usize + 1024, if full { 128 * n as usize + 2048 } else { 0 });
         loop {
             let mut markers: Vec<sys::a3_marker> = Vec::with_capacity(cap_m);
@@ -207,11 +260,13 @@ impl Detector {
             let mut patches = vec![0u8; cap_c * np];
             let mut decs: Vec<sys::a3_decode> = Vec::with_capacity(cap_c);
             let mut refined = vec![0f32; if refine { cap_m * 8 } else { 0 }];
+            let mut boards: Vec<sys::a3_board_pose> = Vec::with_capacity(if board { n as usize } else { 0 });
             let mut out = sys::a3_outputs {
                 grey: grey.as_mut_ptr(), mask: ptr::null_mut(), candidates: cands.as_mut_ptr(), candidate_frame: cframe.as_mut_ptr(),
                 homographies: patches.as_mut_ptr(), decodes: decs.as_mut_ptr(), cand_capacity: cap_c as u32, n_candidates: 0,
                 frame_marker_offsets: ptr::null_mut(), marker_poses: ptr::null_mut(),
                 marker_corners: if refine { refined.as_mut_ptr() } else { ptr::null_mut() },
+                board_poses: if board { boards.as_mut_ptr() } else { ptr::null_mut() },
             };
             if !full {
                 // markers only (plus their refined corners): no per-candidate output, so the device assembles the markers
@@ -222,7 +277,7 @@ impl Detector {
             let st = unsafe {
                 sys::a3_detect_batch(hd.0, frames.as_ptr() as *const _, fmt, sys::A3_MEM_HOST, n, w, h, w as usize * bpp,
                                      w as usize * bpp * h as usize, markers.as_mut_ptr(), cap_m as u32, &mut nm,
-                                     if full || refine { &mut out } else { ptr::null_mut() }, ptr::null_mut())
+                                     if full || refine || board { &mut out } else { ptr::null_mut() }, ptr::null_mut())
             };
             if st == sys::A3_ERR_CAPACITY {
                 cap_m = cap_m.max(nm as usize);
@@ -238,6 +293,9 @@ impl Detector {
             unsafe {
                 markers.set_len(nm as usize);
                 decs.set_len(n_cand);
+                if board {
+                    boards.set_len(n as usize);
+                }
             }
             let mut dets: Vec<Detection> = (0..n).map(|_| Detection::default()).collect();
             if full {
@@ -268,6 +326,9 @@ impl Detector {
                     hamming_distance: m.hamming_distance,
                     corners_refined: if m.corners_refined != 0 { Some([r(0), r(1), r(2), r(3)]) } else { None },
                 });
+            }
+            for (d, b) in dets.iter_mut().zip(boards.iter()) {
+                d.board_pose = Some(pose::BoardPose::from_raw(b));
             }
             return dets;
         }
@@ -320,6 +381,24 @@ pub mod pose {
         /// reference `src/pose.rs:30-33`
         pub fn apply_inverse_transform_to_points(&self, points: &Vec<(f32, f32, f32)>) -> Vec<(f32, f32, f32)> {
             self.apply(points, 1)
+        }
+    }
+
+    /// The pose of a `Board` in one frame (kernel K6): `best` has the smaller error (RMS reprojection distance over the used
+    /// corners, normalised units), `alt` is the other branch of the planar ambiguity; `ok` is false when both failed or no
+    /// board marker was seen.
+    #[derive(Clone, Debug)]
+    pub struct BoardPose {
+        pub best: MarkerPose,
+        pub alt: MarkerPose,
+        pub n_markers: u32,
+        pub ok: bool,
+    }
+
+    impl BoardPose {
+        pub(crate) fn from_raw(b: &sys::a3_board_pose) -> BoardPose {
+            let p = |q: &sys::a3_pose| MarkerPose { error: q.error, rotation: q.rotation, translation: q.translation };
+            BoardPose { best: p(&b.best), alt: p(&b.alt), n_markers: b.n_markers, ok: b.ok != 0 }
         }
     }
 
