@@ -90,9 +90,9 @@ __device__ bool solve8_warp(double (*a)[9], int lane) {
 __device__ void make_projection(const uint32_t *quad, float hs, double (*a)[9], Proj *out, int lane) {
     if (lane < 8) {
         const int k = lane >> 1;
-        const float to[8] = {0.0f, 0.0f, hs, 0.0f, hs, hs, 0.0f, hs};
+        // to = {(0,0), (hs,0), (hs,hs), (0,hs)}, chosen by select: a table indexed by lane would live in local memory
         const double xf = (double)(float)quad[2 * k], yf = (double)(float)quad[2 * k + 1];
-        const double x = (double)to[2 * k], y = (double)to[2 * k + 1];
+        const double x = (double)(k == 1 || k == 2 ? hs : 0.0f), y = (double)(k >= 2 ? hs : 0.0f);
         if (lane & 1) {
             const double r1[9] = {xf, yf, 1.0, 0.0, 0.0, 0.0, -x * xf, -x * yf, x};
             for (int i = 0; i < 9; i++) a[lane][i] = r1[i];
@@ -136,42 +136,122 @@ __device__ void make_projection(const uint32_t *quad, float hs, double (*a)[9], 
     out->ok = 1;
 }
 
-// <u8 as Clamp<f32>>::clamp followed by `as u8`: x < 255 ? (x > 0 ? trunc(x) : 0) : 255, so NaN gives 255.  The
-// float-to-unsigned conversion (cvt.rzi.u32.f32) already saturates: negatives and NaN give 0, large values 2^32 - 1.
-__device__ __forceinline__ uint8_t clamp_u8_trunc(float x) {
-    const uint32_t v = min(__float2uint_rz(x), 255u);
-    return (uint8_t)(x != x ? 255u : v);
-}
+// An integer 0 <= v < 2^23 as f32 without the conversion pipe: 2^23 + v is exact, so is the subtraction.
+__device__ __forceinline__ float small_to_f32(uint32_t v) { return __uint_as_float(0x4B000000u | v) - 8388608.0f; }
 
-// warp_into's per-pixel body: projective map + interpolate_bilinear with default 0 (SURVEY A.7).
-__device__ __forceinline__ uint8_t sample(const uint8_t *grey, uint32_t w, uint32_t h, const float *t, int cls, uint32_t ox,
-                                          uint32_t oy) {
-    float x = (float)ox, y = (float)oy, px, py;
-    if (cls == 2) {
+// <u8 as Clamp<f32>>::clamp followed by `as u8` (x < 255 ? (x > 0 ? trunc(x) : 0) : 255, so NaN gives 255) for a blend of
+// interpolate_bilinear, which is +-0, positive or NaN; returns 2^23 + the byte.  x + 2^23 rounded toward zero is 2^23 + trunc(x)
+// exactly for 0 <= x < 2^23 (floats in [2^23, 2^24) are the integers), larger x and +inf stay at or above 2^23 + 255, and fminf
+// returns its other operand for NaN.
+__device__ __forceinline__ float clamp_u8_trunc_biased(float x) { return fminf(__fadd_rz(x, 8388608.0f), 8388608.0f + 255.0f); }
+
+// First half of warp_into's per-pixel body (projective map + interpolate_bilinear with default 0, SURVEY A.7) for patch pixel
+// (x, y): the bilinear weights, the frame offset of the top-left texel and whether the sample is outside the frame (result 0).
+// The reference's test `left < 0 || right >= w || top < 0 || bottom >= h` with left = floor(px), right = left + 1 is
+// `px < 0 || px >= w - 1` (and the same in y): floor(px) < 0 iff px < 0, and floor(px) + 1 >= w iff px >= w - 1 since w - 1 is
+// an integer (from 2^24 on, where left + 1 rounds, both hold).  +-inf is outside.  NaN fails every comparison, as in Rust, and is
+// not outside: its blend is 255 or a function of the finite weight alone, whatever bytes it reads, so it reads offset 0.
+// Inside the frame 0 <= px < 2^16, where px + 2^23 rounded down is 2^23 + floor(px) exactly: the floors and their integer values
+// come without FRND or F2I.  (For px = -0 the weight becomes -0 where the reference has +0; every blend that weight enters is
+// >= +0 either way and clamps to the same byte.)
+struct Tap {
+    float rw, bw;
+    uint32_t off;
+    bool out;
+};
+template <int CLS>
+__device__ __forceinline__ Tap locate(const float *t, float x, float y, float wm1, float hm1, uint32_t w) {
+    float px, py;
+    if constexpr (CLS == 2) {
         float d = t[6] * x + t[7] * y + t[8];
         px = (t[0] * x + t[1] * y + t[2]) / d;
         py = (t[3] * x + t[4] * y + t[5]) / d;
-    } else if (cls == 1) {
+    } else if constexpr (CLS == 1) {
         px = t[0] * x + t[1] * y + t[2];
         py = t[3] * x + t[4] * y + t[5];
     } else {
         px = x + t[2];
         py = y + t[5];
     }
-    float left = floorf(px), right = left + 1.0f, top = floorf(py), bottom = top + 1.0f;
-    float rw = px - left, bw = py - top;
-    if (left < 0.0f || right >= (float)w || top < 0.0f || bottom >= (float)h) return 0;
-    // NaN coordinates fall through every comparison (as in Rust) and `NaN as u32` is 0 there and here (cvt.rzi.u32.f32 gives 0
-    // for NaN; everything else is inside the frame after the test above).
-    const uint32_t l = __float2uint_rz(left), r = __float2uint_rz(right), tp = __float2uint_rz(top), b = __float2uint_rz(bottom);
-    float tl = (float)grey[(size_t)tp * w + l], tr = (float)grey[(size_t)tp * w + r];
-    float bl = (float)grey[(size_t)b * w + l], br = (float)grey[(size_t)b * w + r];
-    uint8_t topv = clamp_u8_trunc((1.0f - rw) * tl + rw * tr);
-    uint8_t botv = clamp_u8_trunc((1.0f - rw) * bl + rw * br);
-    return clamp_u8_trunc((1.0f - bw) * (float)topv + bw * (float)botv);
+    const float fx = __fadd_rd(px, 8388608.0f), fy = __fadd_rd(py, 8388608.0f);
+    const bool in = px >= 0.0f && px < wm1 && py >= 0.0f && py < hm1;
+    Tap s;
+    s.rw = px - (fx - 8388608.0f);
+    s.bw = py - (fy - 8388608.0f);
+    s.out = px < 0.0f || px >= wm1 || py < 0.0f || py >= hm1;
+    s.off = in ? (__float_as_uint(fy) - 0x4B000000u) * w + (__float_as_uint(fx) - 0x4B000000u) : 0u;
+    return s;
 }
 
-constexpr int kInFlight = 4;  // samples per lane whose gathers are issued before any is consumed
+// Second half: blend_bilinear on the texels at off, off + 1, off + w, off + w + 1, in the reference's operation order.
+__device__ __forceinline__ uint32_t blend(const Tap &s, uint32_t tl8, uint32_t tr8, uint32_t bl8, uint32_t br8) {
+    const float tl = small_to_f32(tl8), tr = small_to_f32(tr8), bl = small_to_f32(bl8), br = small_to_f32(br8);
+    const float topv = clamp_u8_trunc_biased((1.0f - s.rw) * tl + s.rw * tr) - 8388608.0f;
+    const float botv = clamp_u8_trunc_biased((1.0f - s.rw) * bl + s.rw * br) - 8388608.0f;
+    const uint32_t v = __float_as_uint(clamp_u8_trunc_biased((1.0f - s.bw) * topv + s.bw * botv)) - 0x4B000000u;
+    return s.out ? 0u : v;
+}
+
+// Samples per thread whose gathers are issued before any is consumed.  Eight spill at 80 registers and were slower (K2 on
+// 256 x C3 0.215 against 0.194 ms on a B200); so was building for 4 CTAs per SM (64 registers: spills, 0.52 ms), with or
+// without a warp-aggregated (__match_any_sync) histogram update, which alone also lost (0.197 ms).
+constexpr int kInFlight = 4;
+
+// Read by the discarded loads of frames under 2 x 2 pixels, which have no sample inside them.
+__device__ uint8_t k2_no_frame[2];
+
+// The ps x ps patch of one candidate into `patch` and its histogram: this thread takes samples first, first + stride, ...  Each
+// group of kInFlight samples is located first, then all 4 kInFlight byte loads of the group are issued with no branch between
+// them, so that their latencies overlap, then the group is blended.
+template <int CLS>
+__device__ __forceinline__ void sample_patch(const uint8_t *grey, uint32_t w, uint32_t h, const float *inv, uint32_t ps,
+                                             uint32_t first, uint32_t stride, uint8_t *patch, uint32_t *hist) {
+    const uint32_t np = ps * ps;
+    const bool any_inside = w >= 2 && h >= 2;
+    const uint8_t *src = any_inside ? grey : k2_no_frame;
+    const uint32_t row = any_inside ? w : 0u;
+    const float wm1 = (float)w - 1.0f, hm1 = (float)h - 1.0f;
+    // (column, row) of sample i without a division per sample: a step of `stride` adds sq rows and sr < ps columns, which wrap
+    // at most once
+    const uint32_t sq = stride / ps, sr = stride % ps;
+    uint32_t ox = first % ps, oy = first / ps;
+    for (uint32_t base = first; base < np; base += stride * kInFlight) {
+        Tap s[kInFlight];
+#pragma unroll
+        for (int u = 0; u < kInFlight; u++) {
+            s[u] = locate<CLS>(inv, small_to_f32(ox), small_to_f32(oy), wm1, hm1, w);
+            ox += sr;
+            oy += sq;
+            if (ox >= ps) { ox -= ps; oy++; }
+        }
+        uint32_t b[kInFlight][4];
+#pragma unroll
+        for (int u = 0; u < kInFlight; u++) {
+            const uint8_t *t0 = src + s[u].off, *t1 = t0 + row;
+            b[u][0] = t0[0];
+            b[u][1] = t0[1];
+            b[u][2] = t1[0];
+            b[u][3] = t1[1];
+        }
+#pragma unroll
+        for (int u = 0; u < kInFlight; u++) {
+            const uint32_t i = base + stride * u;
+            const uint32_t v = blend(s[u], b[u][0], b[u][1], b[u][2], b[u][3]);
+            if (i < np) {
+                patch[i] = (uint8_t)v;
+                atomicAdd(&hist[v], 1u);
+            }
+        }
+    }
+}
+
+// the loop is specialised per projection class (translation, affine, projective) so that no sample branches on it
+__device__ __forceinline__ void sample_patch(const uint8_t *grey, uint32_t w, uint32_t h, const float *inv, int cls, uint32_t ps,
+                                             uint32_t first, uint32_t stride, uint8_t *patch, uint32_t *hist) {
+    if (cls == 2) sample_patch<2>(grey, w, h, inv, ps, first, stride, patch, hist);
+    else if (cls == 1) sample_patch<1>(grey, w, h, inv, ps, first, stride, patch, hist);
+    else sample_patch<0>(grey, w, h, inv, ps, first, stride, patch, hist);
+}
 
 // Per-warp scratch in shared memory.
 struct WarpScratch {
@@ -195,10 +275,12 @@ __global__ void __launch_bounds__(kThreads, 3) k2_kernel(const K2Params p, const
     uint64_t *dict = reinterpret_cast<uint64_t *>(smem);                       // n_codes
     float *taps = reinterpret_cast<float *>(dict + p.n_codes);                // ms * max_taps
     int *meta = reinterpret_cast<int *>(taps + ms * max_taps);                // 2 * ms
-    uintptr_t cur = (reinterpret_cast<uintptr_t>(meta + 2 * ms) + 15) & ~(uintptr_t)15;
+    // the slices are addressed from `smem` itself, not through an integer, so that the compiler keeps them in the shared
+    // space: the patch stores and histogram atomics of the sampling loop are then STS / ATOMS instead of generic ST / ATOM
+    const size_t head = ((size_t)p.n_codes * 8 + (size_t)ms * max_taps * 4 + (size_t)2 * ms * 4 + 15) & ~(size_t)15;
     const uint32_t warp_bytes = k2_warp_bytes(ps, ms);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    uint8_t *mine = reinterpret_cast<uint8_t *>(cur) + (size_t)(WIDE ? 0 : warp) * warp_bytes;
+    uint8_t *mine = smem + head + (size_t)(WIDE ? 0 : warp) * warp_bytes;
     WarpScratch *ws = reinterpret_cast<WarpScratch *>(mine);
     float *tmp = reinterpret_cast<float *>(mine + sizeof(WarpScratch));       // ms * ps  (vertical pass, f32)
     uint8_t *reduced = reinterpret_cast<uint8_t *>(tmp + ms * ps);            // ms * ms (padded to x4)
@@ -235,23 +317,7 @@ __global__ void __launch_bounds__(kThreads, 3) k2_kernel(const K2Params p, const
                 float inv[9];
 #pragma unroll
                 for (int k = 0; k < 9; k++) inv[k] = ws->proj.inv[k];
-                const int cls = ws->proj.cls;
-                for (uint32_t base = threadIdx.x; base < np; base += blockDim.x * kInFlight) {
-                    uint8_t v[kInFlight];
-#pragma unroll
-                    for (int u = 0; u < kInFlight; u++) {
-                        const uint32_t i = base + blockDim.x * u;
-                        v[u] = i < np ? sample(grey, p.w, p.h, inv, cls, i % ps, i / ps) : 0;
-                    }
-#pragma unroll
-                    for (int u = 0; u < kInFlight; u++) {
-                        const uint32_t i = base + blockDim.x * u;
-                        if (i < np) {
-                            patch[i] = v[u];
-                            atomicAdd(&ws->hist[v[u]], 1u);
-                        }
-                    }
-                }
+                sample_patch(grey, p.w, p.h, inv, ws->proj.cls, ps, threadIdx.x, blockDim.x, patch, ws->hist);
             }
             __syncthreads();   // the patch and its histogram are complete
             if (warp != 0) {   // the other warps wait for warp 0 at the end of the round
@@ -261,37 +327,13 @@ __global__ void __launch_bounds__(kThreads, 3) k2_kernel(const K2Params p, const
         }
         if (ok) {
             if constexpr (!WIDE) {
-            // ---- warp: ps*ps bilinear samples, histogram on the fly ----
-            // The inverse map goes into registers first: it lives in shared memory next to the histogram the loop updates
-            // with atomics, so the compiler would otherwise reload all nine coefficients (generic loads) for every sample.
-            float inv[9];
+                // ---- warp: ps*ps bilinear samples, histogram on the fly ----
+                // The inverse map goes into registers first: it lives in shared memory next to the histogram the loop updates
+                // with atomics, so the compiler would otherwise reload all nine coefficients for every sample.
+                float inv[9];
 #pragma unroll
-            for (int k = 0; k < 9; k++) inv[k] = ws->proj.inv[k];
-            const int cls = ws->proj.cls;
-            const uint32_t fw = p.w, fh = p.h;
-            // four samples per lane in flight: the 16 gathers of a group are independent, so their latencies overlap (eight
-            // measured no faster).  The kernel is built for 3 CTAs per SM (80 registers): at 4 CTAs (64 registers) this
-            // loop spills, and the spill traffic made the whole kernel 1.8x slower.
-            // (patch column, row) of sample `base + 32 u` without a division per sample: advance by 32 with wrap-around
-            uint32_t ox = (uint32_t)lane % ps, oy = (uint32_t)lane / ps;
-            for (uint32_t base = lane; base < np; base += 32 * kInFlight) {
-                uint8_t v[kInFlight];
-#pragma unroll
-                for (int u = 0; u < kInFlight; u++) {
-                    const uint32_t i = base + 32 * u;
-                    v[u] = i < np ? sample(grey, fw, fh, inv, cls, ox, oy) : 0;
-                    ox += 32;
-                    while (ox >= ps) { ox -= ps; oy++; }
-                }
-#pragma unroll
-                for (int u = 0; u < kInFlight; u++) {
-                    const uint32_t i = base + 32 * u;
-                    if (i < np) {
-                        patch[i] = v[u];
-                        atomicAdd(&ws->hist[v[u]], 1u);
-                    }
-                }
-            }
+                for (int k = 0; k < 9; k++) inv[k] = ws->proj.inv[k];
+                sample_patch(grey, p.w, p.h, inv, ws->proj.cls, ps, lane, 32, patch, ws->hist);
             }
             __syncwarp();
             // ---- otsu_level (SURVEY A.8): integer prefix sums are exact; the f64 expression keeps the reference's order ----
