@@ -8,7 +8,7 @@ from .detector import (ARDictionary, Detection, Detector, DetectorConfig, Marker
                        quads_from_mask)
 from ._ffi import A3Error  # noqa: F401
 from . import pose  # noqa: F401
-from .pose import CameraIntrinsics, MarkerPose  # noqa: F401
+from .pose import CameraDistortion, CameraIntrinsics, MarkerPose  # noqa: F401
 from .board import Board, BoardPose  # noqa: F401
 
 __version__ = "0.1.0"

@@ -51,7 +51,8 @@ class A3Stats(C.Structure):
                [(n, C.c_uint32) for n in ("pixel_kernel_launches", "decode_kernel_launches", "host_threads", "contour_kernel_launches",
                                           "host_fallback_frames", "pose_kernel_launches", "one_shot", "one_shot_retry", "input_staged", "output_staged",
                                           "refine_kernel_launches")] + \
-               [("ms_refine_kernel", C.c_double), ("board_kernel_launches", C.c_uint32), ("ms_board_kernel", C.c_double)]
+               [("ms_refine_kernel", C.c_double), ("board_kernel_launches", C.c_uint32), ("ms_board_kernel", C.c_double),
+                ("undistort_kernel_launches", C.c_uint32), ("ms_undistort_kernel", C.c_double)]
 
     def as_dict(self):
         return {f: getattr(self, f) for f, _ in self._fields_}
@@ -79,6 +80,10 @@ class A3BoardPose(C.Structure):
 class A3CameraIntrinsics(C.Structure):
     _fields_ = [("image_width", C.c_uint32), ("image_height", C.c_uint32), ("focal_x", C.c_float), ("focal_y", C.c_float),
                 ("principal_x", C.c_float), ("principal_y", C.c_float)]
+
+
+class A3CameraDistortion(C.Structure):
+    _fields_ = [(n, C.c_float) for n in ("k1", "k2", "p1", "p2", "k3")]
 
 
 class A3K1Tuning(C.Structure):
@@ -158,6 +163,9 @@ def lib():
     L.a3_detector_set_pose.argtypes = [vp, u32, f32, PK]
     L.a3_detector_set_board.argtypes = [vp, C.POINTER(A3Board), u32, PK]
     L.a3_solve_board.argtypes = [vp, vp, vp, vp, u32, u32, u32, u32, vp]
+    PD = C.POINTER(A3CameraDistortion)
+    L.a3_detector_set_distortion.argtypes = [vp, PD]
+    L.a3_undistort_points.argtypes = [vp, vp, u32, PK, PD, vp, vp]
     L.a3_solve_with_intrinsics.argtypes = [vp, vp, u32, f32, PK, vp, vp]
     L.a3_solve_with_undistorted_points.argtypes = [vp, vp, u32, f32, u32, u32, vp, vp]
     L.a3_solve_with_normalized_points.argtypes = [vp, vp, u32, f32, vp, vp]

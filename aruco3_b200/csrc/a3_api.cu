@@ -239,7 +239,10 @@ struct DecodeBlock {
     DevBuf<a3_board_pose> d_board;  // K6: one board pose per frame of the group
     PinBuf<a3_board_pose> h_board;
     PinBuf<uint32_t> h_qoff;        // K6: per-frame quad offsets of a group whose quads came from the host
+    DevBuf<float> d_norm;           // K7: normalised undistorted corners per quad, one set per distinct intrinsics, and their flags
+    DevBuf<uint8_t> d_nok;
     cudaEvent_t ev_a = nullptr, ev_b = nullptr, ev_r0 = nullptr, ev_r1 = nullptr, ev_k6a = nullptr, ev_k6b = nullptr;  // around K2, K5, K6
+    cudaEvent_t ev_u0 = nullptr, ev_u1 = nullptr;  // around K7
     uint32_t n_quads = 0;
     // where the host reads this group's records: h_dec / h_pose / h_ref, or the one-shot arena
     const a3_decode *dec_view = nullptr;
@@ -253,7 +256,8 @@ struct DecodeBlock {
         d_pose.release(); h_pose.release();
         d_ref.release(); h_ref.release(); d_refok.release(); h_refok.release();
         d_board.release(); h_board.release(); h_qoff.release();
-        for (cudaEvent_t *e : {&ev_a, &ev_b, &ev_r0, &ev_r1, &ev_k6a, &ev_k6b}) { if (*e) cudaEventDestroy(*e); *e = nullptr; }
+        d_norm.release(); d_nok.release();
+        for (cudaEvent_t *e : {&ev_a, &ev_b, &ev_r0, &ev_r1, &ev_k6a, &ev_k6b, &ev_u0, &ev_u1}) { if (*e) cudaEventDestroy(*e); *e = nullptr; }
     }
 };
 
@@ -338,6 +342,11 @@ struct a3_detector {
     a3::DevBuf<uint64_t> d_probe_ids;  // a3_solve_board
     a3::DevBuf<uint32_t> d_probe_off;
     a3::DevBuf<a3_board_pose> d_probe_out;
+    // lens distortion (K7) of the intrinsics of the pose and board modes; off unless set
+    bool dist_on = false;
+    a3_camera_distortion dist{};
+    a3::DevBuf<float> d_und_in, d_und_out;  // a3_undistort_points, and K7's points for a3_solve_board
+    a3::DevBuf<uint8_t> d_und_ok;
 };
 
 namespace a3 {
@@ -531,10 +540,46 @@ cudaError_t launch_refine(DecodeBlock &b, const uint8_t *grey, uint32_t w, uint3
     return e;
 }
 
-// K6 over the frames [0, n_frames) of a decode group or of the one-shot arena, bracketed by the block's events
+// Which undistorted corner sets K7 writes for a call: one for K4 (the pose intrinsics) and one for K6 (the board
+// intrinsics), shared when the two intrinsics are the same.  The setters allow distortion only with INTRINSICS modes.
+struct UndistortPlan {
+    bool pose = false, board = false;
+    uint32_t sets = 0, board_set = 0;  // corner sets (0 = K7 does not run), and the one K6 reads
+};
+UndistortPlan undistort_plan(const a3_detector *d, bool want_poses, bool want_board) {
+    UndistortPlan u;
+    if (!d->dist_on) return u;
+    u.pose = want_poses;
+    u.board = want_board;
+    const bool shared = u.pose && u.board && memcmp(&d->pose_k, &d->board_k, sizeof(a3_camera_intrinsics)) == 0;
+    u.sets = (u.pose ? 1u : 0u) + ((u.board && !shared) ? 1u : 0u);
+    u.board_set = (u.pose && !shared) ? 1u : 0u;
+    return u;
+}
+
+// K7 for every set of the plan on n items (set j at norm + 8 n j, ok + n j), bracketed by the block's events
+cudaError_t launch_undistort(const a3_detector *d, DecodeBlock &b, const UndistortPlan &u, const uint32_t *quads, const float *ref,
+                             const a3_decode *dec, uint32_t n, const uint32_t *n_dev, float *norm, uint8_t *ok, cudaStream_t s) {
+    cudaError_t e = cudaSuccess;
+    if (!b.ev_u0) e = cudaEventCreate(&b.ev_u0);
+    if (e == cudaSuccess && !b.ev_u1) e = cudaEventCreate(&b.ev_u1);
+    if (e == cudaSuccess) e = cudaEventRecord(b.ev_u0, s);
+    for (uint32_t j = 0; j < u.sets && e == cudaSuccess; j++) {
+        K7Params kp;
+        kp.quads = quads; kp.corners_f32 = ref; kp.decodes = dec; kp.n = n; kp.n_dev = n_dev;
+        kp.k = (j == 0 && u.pose) ? d->pose_k : d->board_k; kp.dist = d->dist;
+        kp.out = norm + (size_t)n * 8 * j; kp.ok = ok + (size_t)n * j;
+        e = k7_undistort(kp, s);
+    }
+    if (e == cudaSuccess) e = cudaEventRecord(b.ev_u1, s);
+    return e;
+}
+
+// K6 over the frames [0, n_frames) of a decode group or of the one-shot arena, bracketed by the block's events; norm / nok:
+// K7's points when the board's intrinsics have a distortion
 cudaError_t launch_board(const a3_detector *d, DecodeBlock &b, const a3_decode *dec, const uint32_t *quads, const float *ref,
                          const uint32_t *offsets, const uint32_t *skip, uint32_t n_frames, uint32_t w, uint32_t h, a3_board_pose *out,
-                         cudaStream_t s) {
+                         cudaStream_t s, const float *norm = nullptr, const uint8_t *nok = nullptr) {
     cudaError_t e = cudaSuccess;
     if (!b.ev_k6a) e = cudaEventCreate(&b.ev_k6a);
     if (e == cudaSuccess && !b.ev_k6b) e = cudaEventCreate(&b.ev_k6b);
@@ -543,6 +588,7 @@ cudaError_t launch_board(const a3_detector *d, DecodeBlock &b, const a3_decode *
     kp.decodes = dec; kp.quads = quads; kp.corners_f32 = ref; kp.offsets = offsets; kp.skip = skip; kp.n_frames = n_frames;
     kp.slots = d->d_board_slots.p; kp.n_codes = d->dict.n_codes; kp.board = d->d_board_pts.p; kp.n_board = d->board_n;
     kp.mode = d->board_mode; kp.image_w = w; kp.image_h = h; kp.k = d->board_k; kp.out = out;
+    kp.norm = norm; kp.norm_ok = nok;
     if (e == cudaSuccess) e = k6_board(kp, s);
     if (e == cudaSuccess) e = cudaEventRecord(b.ev_k6b, s);
     return e;
@@ -667,6 +713,7 @@ void a3_detector_release(a3_detector *d) {
     d->pose_mode = A3_POSE_OFF;
     d->corner_mode = A3_CORNERS_INTEGER;
     d->board_n = 0; d->board_mode = A3_POSE_OFF;
+    d->dist_on = false; d->dist = a3_camera_distortion{};
     d->has_tuning = false; d->k1_tuning = K1Tuning{}; d->chunk_override = 0;
     a3_detector *evict = nullptr;
     {
@@ -701,6 +748,7 @@ void a3_detector_destroy(a3_detector *d) {
     d->d_pose_in.release(); d->d_pose_out.release(); d->h_pose_out.release();
     d->d_refined.release(); d->d_refined_ok.release();
     d->d_board_slots.release(); d->d_board_pts.release(); d->d_probe_ids.release(); d->d_probe_off.release(); d->d_probe_out.release();
+    d->d_und_in.release(); d->d_und_out.release(); d->d_und_ok.release();
     d->copy_pool.stop();
     d->h_stage_in.release(); d->h_stage_out.release();
     d->events.release();
@@ -928,6 +976,8 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
     // K5 refines the markers' corners (a3_marker.corners_refined, a3_outputs.marker_corners); K4 and K6 then solve from them
     const bool want_refine = (markers || want_board) && d->corner_mode == A3_CORNERS_REFINED;
     float *const out_corners = want_refine && markers && outs ? outs->marker_corners : nullptr;
+    // K7 undistorts the corners K4 and K6 read when their intrinsics have a distortion
+    const UndistortPlan und = undistort_plan(d, want_poses, want_board);
     const K1Tuning *tune = d->has_tuning ? &d->k1_tuning : nullptr;
     const uint8_t *src_all = static_cast<const uint8_t *>(frames);
     a3_stats st;
@@ -1048,7 +1098,10 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
         const size_t off_pose = off_dec + (size_t)shot_cap * sizeof(a3_decode);
         const size_t off_ref = off_pose + (want_poses ? (size_t)shot_cap * 2 * sizeof(a3_pose) : 0);  // K5's, per candidate
         const size_t off_refok = off_ref + (want_refine ? (size_t)shot_cap * 32 : 0);
-        const size_t shot_bytes = off_refok + (want_refine ? (size_t)shot_cap : 0);
+        const size_t off_norm = und.sets ? (off_refok + (want_refine ? (size_t)shot_cap : 0) + 15) & ~(size_t)15  // K7's, per candidate
+                                         : off_refok + (want_refine ? (size_t)shot_cap : 0);
+        const size_t off_nok = off_norm + (size_t)und.sets * shot_cap * 32;
+        const size_t shot_bytes = off_nok + (size_t)und.sets * shot_cap;
         const size_t shot_copy_bytes = lean ? off_quads : shot_bytes;  // what goes back to the host
         if (shot) {
             A3_CUDA(d->d_shot.reserve(shot_bytes)); A3_CUDA(d->h_shot.reserve(shot_bytes));
@@ -1144,15 +1197,21 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             float *d_ref = want_refine ? reinterpret_cast<float *>(d->d_shot.p + off_ref) : nullptr;
             uint8_t *d_refok = want_refine ? d->d_shot.p + off_refok : nullptr;
             if (want_refine) A3_CUDA(launch_refine(b, d->d_grey.p, w, h, d_quads, b.d_qframe.p, d_dec, cap, d_info, d_ref, d_refok, d->s_pixel));
+            float *d_norm = und.sets ? reinterpret_cast<float *>(d->d_shot.p + off_norm) : nullptr;
+            uint8_t *d_nok = und.sets ? d->d_shot.p + off_nok : nullptr;
+            if (und.sets) A3_CUDA(launch_undistort(d, b, und, d_quads, d_ref, d_dec, cap, d_info, d_norm, d_nok, d->s_pixel));
             if (want_poses) {
                 K4Params kp{};
                 kp.mode = d->pose_mode; kp.corners = d_quads; kp.corners_f32 = d_ref; kp.decodes = d_dec; kp.n = cap; kp.n_dev = d_info;
                 kp.marker_size = d->pose_marker_size; kp.image_w = w; kp.image_h = h; kp.k = d->pose_k; kp.poses = d_pose;
+                if (und.pose) { kp.mode = A3_POSE_NORMALIZED; kp.points = d_norm; kp.points_ok = d_nok; }
                 A3_CUDA(k4_pose(kp, d->s_pixel));
             }
             if (want_board)
                 A3_CUDA(launch_board(d, b, d_dec, d_quads, d_ref, d->d_qoff.p, d_info + 1, sn, w, h,
-                                     reinterpret_cast<a3_board_pose *>(d->d_shot.p + off_board), d->s_pixel));
+                                     reinterpret_cast<a3_board_pose *>(d->d_shot.p + off_board), d->s_pixel,
+                                     und.board ? d_norm + (size_t)cap * 8 * und.board_set : nullptr,
+                                     und.board ? d_nok + (size_t)cap * und.board_set : nullptr));
             if (lean) {
                 assemble_markers_kernel<<<n_chunks, 1024, 0, d->s_pixel>>>(d_dec, d_quads, b.d_qframe.p, d->d_qoff.p, want_poses ? d_pose : nullptr,
                                                                     d_ref, d_refok, cap, d_info, d_chain,
@@ -1196,6 +1255,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 if (want_poses) st.pose_kernel_launches++;
                 if (want_refine) st.refine_kernel_launches++;
                 if (want_board) st.board_kernel_launches++;
+                st.undistort_kernel_launches += und.sets;
                 st.one_shot = 1;
                 one_shot_done = true;
                 lean_done = lean;
@@ -1483,11 +1543,18 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 A3_CUDA(cudaMemcpyAsync(b.h_refok.p, b.d_refok.p, nq, cudaMemcpyDeviceToHost, d->s_decode));
                 b.ref_view = b.h_ref.p; b.refok_view = b.h_refok.p;
             }
+            if (und.sets) {  // K7 behind K2 (and K5), on the corners K4 and K6 read
+                A3_CUDA(b.d_norm.reserve((size_t)und.sets * nq * 8)); A3_CUDA(b.d_nok.reserve((size_t)und.sets * nq));
+                A3_CUDA(launch_undistort(d, b, und, b.d_quads.p, want_refine ? b.d_ref.p : nullptr, b.d_dec.p, nq, on_device ? b.d_info.p : nullptr,
+                                         b.d_norm.p, b.d_nok.p, d->s_decode));
+                st.undistort_kernel_launches += und.sets;
+            }
             if (want_poses) {  // K4 right behind K2, on K2's records and the quads where they lie
                 A3_CUDA(b.d_pose.reserve((size_t)nq * 2)); A3_CUDA(b.h_pose.reserve((size_t)nq * 2));
                 K4Params kp{};
                 kp.mode = d->pose_mode; kp.corners = b.d_quads.p; kp.corners_f32 = want_refine ? b.d_ref.p : nullptr; kp.decodes = b.d_dec.p; kp.n = nq; kp.marker_size = d->pose_marker_size;
                 kp.image_w = w; kp.image_h = h; kp.k = d->pose_k; kp.poses = b.d_pose.p;
+                if (und.pose) { kp.mode = A3_POSE_NORMALIZED; kp.points = b.d_norm.p; kp.points_ok = b.d_nok.p; }
                 A3_CUDA(k4_pose(kp, d->s_decode));
                 st.pose_kernel_launches++;
                 A3_CUDA(cudaMemcpyAsync(b.h_pose.p, b.d_pose.p, (size_t)nq * 2 * sizeof(a3_pose), cudaMemcpyDeviceToHost, d->s_decode));
@@ -1497,7 +1564,8 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 const uint32_t gn = f1 - f0;
                 A3_CUDA(b.d_board.reserve(gn)); A3_CUDA(b.h_board.reserve(gn));
                 A3_CUDA(launch_board(d, b, b.d_dec.p, b.d_quads.p, want_refine ? b.d_ref.p : nullptr, b.d_qoff.p, nullptr, gn, w, h, b.d_board.p,
-                                     d->s_decode));
+                                     d->s_decode, und.board ? b.d_norm.p + (size_t)nq * 8 * und.board_set : nullptr,
+                                     und.board ? b.d_nok.p + (size_t)nq * und.board_set : nullptr));
                 st.board_kernel_launches++;
                 A3_CUDA(cudaMemcpyAsync(b.h_board.p, b.d_board.p, (size_t)gn * sizeof(a3_board_pose), cudaMemcpyDeviceToHost, d->s_decode));
                 b.board_view = b.h_board.p;
@@ -1563,6 +1631,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                         cudaEventElapsedTime(&ms, d->blocks[0]->ev_a, d->blocks[0]->ev_b); st.ms_mask_d2h -= ms;
                         if (want_refine) { cudaEventElapsedTime(&ms, d->blocks[0]->ev_r0, d->blocks[0]->ev_r1); st.ms_mask_d2h -= ms; }
                         if (want_board) { cudaEventElapsedTime(&ms, d->blocks[0]->ev_k6a, d->blocks[0]->ev_k6b); st.ms_mask_d2h -= ms; }
+                        if (und.sets) { cudaEventElapsedTime(&ms, d->blocks[0]->ev_u0, d->blocks[0]->ev_u1); st.ms_mask_d2h -= ms; }
                     }
                 }
             } else {
@@ -1593,6 +1662,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             if (b.n_quads && stats) { cudaEventElapsedTime(&ms, b.ev_a, b.ev_b); st.ms_decode_kernel += ms; }
             if (b.n_quads && stats && want_refine) { cudaEventElapsedTime(&ms, b.ev_r0, b.ev_r1); st.ms_refine_kernel += ms; }
             if (stats && want_board) { cudaEventElapsedTime(&ms, b.ev_k6a, b.ev_k6b); st.ms_board_kernel += ms; }
+            if (stats && und.sets) { cudaEventElapsedTime(&ms, b.ev_u0, b.ev_u1); st.ms_undistort_kernel += ms; }
             if (want_board) memcpy(outs->board_poses, b.board_view, (size_t)sn * sizeof(a3_board_pose));
             const uint32_t nm = h_info[3], take = nm < marker_capacity ? nm : marker_capacity;
             memcpy(markers, d->h_shot.p + off_markers, (size_t)take * sizeof(a3_marker));
@@ -1614,6 +1684,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             DecodeBlock &b = *d->blocks[g];
             if (b.n_quads && stats) { cudaEventElapsedTime(&ms, b.ev_a, b.ev_b); st.ms_decode_kernel += ms; }
             if (b.n_quads && stats && want_refine) { cudaEventElapsedTime(&ms, b.ev_r0, b.ev_r1); st.ms_refine_kernel += ms; }
+            if (b.n_quads && stats && und.sets) { cudaEventElapsedTime(&ms, b.ev_u0, b.ev_u1); st.ms_undistort_kernel += ms; }
             const uint32_t f0 = g * group, f1 = f0 + group_size(g);
             if (want_board) {
                 if (b.n_quads && stats) { cudaEventElapsedTime(&ms, b.ev_k6a, b.ev_k6b); st.ms_board_kernel += ms; }
@@ -1684,6 +1755,8 @@ a3_status a3_detector_set_pose(a3_detector *d, uint32_t mode, float marker_size_
     if (mode != A3_POSE_OFF && mode != A3_POSE_UNDISTORTED && mode != A3_POSE_INTRINSICS)
         return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_pose: mode must be OFF, UNDISTORTED or INTRINSICS");
     if (mode == A3_POSE_INTRINSICS && !k) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_pose: intrinsics required");
+    if (d->dist_on && mode == A3_POSE_UNDISTORTED)
+        return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_pose: the detector has a lens distortion, which needs INTRINSICS (or OFF)");
     d->pose_mode = mode;
     d->pose_marker_size = marker_size_mm;
     if (k) d->pose_k = *k;
@@ -1702,6 +1775,8 @@ a3_status a3_detector_set_board(a3_detector *d, const a3_board *board, uint32_t 
     if (mode != A3_POSE_UNDISTORTED && mode != A3_POSE_INTRINSICS)
         return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: mode must be UNDISTORTED or INTRINSICS");
     if (mode == A3_POSE_INTRINSICS && !k) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: intrinsics required");
+    if (d->dist_on && mode != A3_POSE_INTRINSICS)
+        return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: the detector has a lens distortion, which needs INTRINSICS");
     const uint32_t m = board->n_markers;
     if (m == 0 || m > A3_K6_MAX_MARKERS) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: a board has 1 to 1024 markers");
     if (!board->ids || !board->corners) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: null ids or corners");
@@ -1761,8 +1836,50 @@ a3_status a3_solve_board(a3_detector *d, const uint64_t *ids, const float *corne
     kp.ids = d->d_probe_ids.p; kp.corners_f32 = d->d_refined.p; kp.offsets = d->d_probe_off.p; kp.n_frames = n_frames;
     kp.slots = d->d_board_slots.p; kp.n_codes = d->dict.n_codes; kp.board = d->d_board_pts.p; kp.n_board = d->board_n;
     kp.mode = d->board_mode; kp.image_w = image_w; kp.image_h = image_h; kp.k = d->board_k; kp.out = d->d_probe_out.p;
+    if (d->dist_on && n) {  // K7 first, as a3_detect_batch runs it
+        A3_CUDA(d->d_und_out.reserve((size_t)n * 8)); A3_CUDA(d->d_und_ok.reserve(n));
+        K7Params up;
+        up.corners_f32 = d->d_refined.p; up.n = n; up.k = d->board_k; up.dist = d->dist; up.out = d->d_und_out.p; up.ok = d->d_und_ok.p;
+        A3_CUDA(k7_undistort(up, s));
+        kp.norm = d->d_und_out.p; kp.norm_ok = d->d_und_ok.p;
+    }
     A3_CUDA(k6_board(kp, s));
     A3_CUDA(cudaMemcpyAsync(out, d->d_probe_out.p, (size_t)n_frames * sizeof(a3_board_pose), cudaMemcpyDeviceToHost, s));
+    A3_CUDA(cudaStreamSynchronize(s));
+    return A3_OK;
+}
+
+// ---- lens distortion (K7) ------------------------------------------------------------------------------------------
+
+a3_status a3_detector_set_distortion(a3_detector *d, const a3_camera_distortion *dist) {
+    if (!d) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_distortion: null detector");
+    if (!dist || (dist->k1 == 0.0f && dist->k2 == 0.0f && dist->p1 == 0.0f && dist->p2 == 0.0f && dist->k3 == 0.0f)) {
+        d->dist_on = false;
+        d->dist = a3_camera_distortion{};
+        return A3_OK;
+    }
+    if (!isfinite(dist->k1) || !isfinite(dist->k2) || !isfinite(dist->p1) || !isfinite(dist->p2) || !isfinite(dist->k3))
+        return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_distortion: non-finite coefficient");
+    if (d->pose_mode == A3_POSE_UNDISTORTED || d->pose_mode == A3_POSE_NORMALIZED)
+        return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_distortion: the pose mode does not use the intrinsics (set INTRINSICS or OFF first)");
+    if (d->board_n && d->board_mode != A3_POSE_INTRINSICS)
+        return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_distortion: the board mode does not use the intrinsics (set INTRINSICS first)");
+    d->dist_on = true;
+    d->dist = *dist;
+    return A3_OK;
+}
+
+a3_status a3_undistort_points(a3_detector *d, const float *points, uint32_t n, const a3_camera_intrinsics *k, const a3_camera_distortion *dist,
+                              float *out, uint8_t *ok) {
+    if (!d || !k || !dist || (n && (!points || !out || !ok))) return fail(A3_ERR_INVALID_ARGUMENT, "a3_undistort_points: null argument");
+    if (n == 0) return A3_OK;
+    A3_CUDA(cudaSetDevice(d->device));
+    cudaStream_t s = d->s_decode;
+    A3_CUDA(d->d_und_in.reserve((size_t)n * 2)); A3_CUDA(d->d_und_out.reserve((size_t)n * 2)); A3_CUDA(d->d_und_ok.reserve(n));
+    A3_CUDA(cudaMemcpyAsync(d->d_und_in.p, points, (size_t)n * 8, cudaMemcpyHostToDevice, s));
+    A3_CUDA(k7_undistort_points(d->d_und_in.p, n, *k, *dist, d->d_und_out.p, d->d_und_ok.p, s));
+    A3_CUDA(cudaMemcpyAsync(out, d->d_und_out.p, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
+    A3_CUDA(cudaMemcpyAsync(ok, d->d_und_ok.p, n, cudaMemcpyDeviceToHost, s));
     A3_CUDA(cudaStreamSynchronize(s));
     return A3_OK;
 }

@@ -150,6 +150,7 @@ struct K4Params {
     const float *points;         // device n*8 (NORMALIZED)
     const uint32_t *corners;     // device n*8 (other modes)
     const float *corners_f32 = nullptr;  // device n*8 or null: f32 corners (K5's), already rotate_left(rotation), read instead of `corners`
+    const uint8_t *points_ok = nullptr;  // device n or null (NORMALIZED): K7's flags; an item with 0 gets two default poses
     const a3_decode *decodes;    // device n or null; when set: only accepted items, corners.rotate_left(rotation)
     uint32_t n;
     const uint32_t *n_dev = nullptr;  // device, optional: the real number of items (<= n, which then only sizes the launch)
@@ -181,6 +182,9 @@ struct K6Params {
     const uint64_t *ids = nullptr;          // device n: the items' ids when decodes is null (probe; every item counts)
     const uint32_t *quads = nullptr;        // device n*8 integer corners (screen order), read when corners_f32 is null
     const float *corners_f32 = nullptr;     // device n*8 or null: f32 corners already in marker order (K5's, or the probe's)
+    const float *norm = nullptr;            // device n*8 or null: K7's normalised undistorted corners (K7's layout), read instead of
+                                            //   both corner sources and of the mode's normalisation
+    const uint8_t *norm_ok = nullptr;       // device n, with norm: K7's flags; an item with 0 is left out as if not detected
     const uint32_t *offsets = nullptr;      // device n_frames + 1: items of frame f are [offsets[f], offsets[f + 1])
     const uint32_t *skip = nullptr;         // device flag or null: non-zero = the launch writes nothing (a one-shot route that did not hold)
     uint32_t n_frames = 0;
@@ -194,6 +198,24 @@ struct K6Params {
     a3_board_pose *out = nullptr;           // device n_frames
 };
 cudaError_t k6_board(const K6Params &p, cudaStream_t stream);
+
+// ---- K7: lens undistortion of marker corners (k7_undistort.cu; specification k7_undistort_spec.h, oracle/a3ref_distort.c)
+struct K7Params {
+    const uint32_t *quads = nullptr;        // device n*8 integer corners (screen order), read when corners_f32 is null
+    const float *corners_f32 = nullptr;     // device n*8 or null: f32 corners already in marker order (K5's, or the probe's)
+    const a3_decode *decodes = nullptr;     // device n or null; when set: accepted items only, rotation from the record
+    uint32_t n = 0;
+    const uint32_t *n_dev = nullptr;        // device, optional: the real number of items (<= n, which then only sizes the launch)
+    a3_camera_intrinsics k{};
+    a3_camera_distortion dist{};
+    float *out = nullptr;                   // device out n*8: marker corner c at [8 i + 2 ((c + rotation) & 3)], the slot K4's
+                                            //   A3_POSE_NORMALIZED read and K6 take it from
+    uint8_t *ok = nullptr;                  // device out n: 1 when all four corners undistorted
+};
+cudaError_t k7_undistort(const K7Params &p, cudaStream_t stream);
+// the probe: n points (x, y) -> n normalised undistorted points and their flags
+cudaError_t k7_undistort_points(const float *pts, uint32_t n, const a3_camera_intrinsics &k, const a3_camera_distortion &dist, float *out,
+                                uint8_t *ok, cudaStream_t stream);
 
 // ---- host quad stage (host_quads.cpp) ---------------------------------------------------------------
 struct QuadStats {

@@ -122,6 +122,16 @@ __global__ void __launch_bounds__(128) k4_pose_kernel(K4Params p) {
         if (!dc.accepted) return;
         rot = dc.rotation & 3;
     }
+    if (p.points_ok && !p.points_ok[i]) {  // a corner K7 could not undistort: the default pair (pose.rs:42-50)
+        for (int b = 0; b < 2; b++) {
+            a3_pose *o = p.poses + (size_t)i * 2 + b;
+            o->error = 1e31f;
+#pragma unroll
+            for (int j = 0; j < 9; j++) o->rotation[j] = (j % 4 == 0) ? 1.0f : 0.0f;
+            o->translation[0] = o->translation[1] = o->translation[2] = 0.0f;
+        }
+        return;
+    }
     float px[4], py[4];
 #pragma unroll
     for (int c = 0; c < 4; c++) {

@@ -31,10 +31,19 @@ struct Frame {
     double r[9], t[3], r2[9];
 };
 
-// point q of the frame: normalised image point (u, v) and board point (x, y), as f32 the way K4 normalises corners
+// point q of the frame: normalised image point (u, v) and board point (x, y): K7's point, or the corner normalised in f32
+// the way K4 normalises corners
 __device__ __forceinline__ void point(const Frame &f, uint32_t q, double &u, double &v, double &x, double &y) {
     const K6Params &p = *f.p;
     const uint32_t k = f.used[q >> 2], c = q & 3u, s = f.slot[q >> 2];
+    x = (double)p.board[(size_t)s * 8 + 2 * c];
+    y = (double)p.board[(size_t)s * 8 + 2 * c + 1];
+    if (p.norm) {  // K7's points, already normalised and undistorted, where K4 reads them
+        const uint32_t sidx = (c + (p.decodes ? p.decodes[k].rotation & 3u : 0u)) & 3u;
+        u = (double)p.norm[(size_t)k * 8 + 2 * sidx];
+        v = (double)p.norm[(size_t)k * 8 + 2 * sidx + 1];
+        return;
+    }
     float px, py;
     if (p.corners_f32) {
         px = p.corners_f32[(size_t)k * 8 + 2 * c];
@@ -54,8 +63,6 @@ __device__ __forceinline__ void point(const Frame &f, uint32_t q, double &u, dou
     }
     u = (double)nu;
     v = (double)nv;
-    x = (double)p.board[(size_t)s * 8 + 2 * c];
-    y = (double)p.board[(size_t)s * 8 + 2 * c + 1];
 }
 
 // sums of K per-point values over n points: lane-strided, then the xor tree (the oracle's warp_sums)
@@ -335,6 +342,7 @@ __global__ void __launch_bounds__(32) k6_board_kernel(K6Params p) {
         } else {
             id = p.ids[i];
         }
+        if (p.norm_ok && !p.norm_ok[i]) return A3_K6_NO_SLOT;  // a corner K7 could not undistort: as if not detected
         return id < p.n_codes ? s_slots[id] : A3_K6_NO_SLOT;
     };
     for (uint32_t i = o0 + lane; i < o1; i += 32) {

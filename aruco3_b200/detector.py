@@ -151,7 +151,7 @@ class Detector:
 
     def __init__(self, config: DetectorConfig | None = None, dictionary: ARDictionary | str = "ARUCO", device: int = 0,
                  host_threads: int | None = None, contours: str = "device", corners: str = "integer", board=None,
-                 board_intrinsics=None):
+                 board_intrinsics=None, distortion=None):
         self.config = config or DetectorConfig()
         self.dictionary = ARDictionary.new_from_named_dict(dictionary) if isinstance(dictionary, str) else dictionary
         self.device = device
@@ -169,6 +169,15 @@ class Detector:
         self._board = None
         if board is not None:
             self.set_board(board, board_intrinsics)
+        self.set_distortion(distortion)
+
+    def set_distortion(self, distortion=None):
+        """Give the camera intrinsics of the pose and board modes a lens distortion (`pose.CameraDistortion`): `detect` /
+        `detect_batch` then undistort every corner the pose kernels read (kernel K7) and the marker and board poses solve from
+        the undistorted points.  Only with intrinsics modes (`set_pose` / `set_board` with `camera_intrinsics`); `None` or all
+        coefficients zero switches it off."""
+        check(lib().a3_detector_set_distortion(self._h, C.byref(distortion._c) if distortion is not None else None))
+        self._distortion = distortion
 
     def set_board(self, board, camera_intrinsics=None):
         """Also solve the pose of a planar `Board` in every frame inside `detect` / `detect_batch` (kernel K6 behind the
@@ -374,6 +383,17 @@ class Detector:
         cf = np.ascontiguousarray(corner_frame, dtype=np.uint32) if corner_frame is not None else None
         check(lib().a3_refine_corners(self._h, g.ctypes.data, n, w, h, c.ctypes.data, cf.ctypes.data if cf is not None else None, m,
                                       out.ctypes.data, ok.ctypes.data))
+        return out, ok.astype(bool)
+
+    def undistort_points(self, points, camera_intrinsics, distortion):
+        """The undistortion (kernel K7's device function) as a probe: pixels [n, 2] (pixel-centre convention) -> (normalised
+        undistorted float32 [n, 2], ok bool [n]); a point that fails (fold of the model, no convergence, non-finite) reads
+        (0, 0).  `pose.solve_with_normalized_points` on its result is what the marker pose with distortion computes."""
+        p = np.ascontiguousarray(np.asarray(points, np.float32).reshape(-1, 2))
+        out = np.zeros_like(p)
+        ok = np.zeros(p.shape[0], np.uint8)
+        check(lib().a3_undistort_points(self._h, p.ctypes.data, p.shape[0], C.byref(camera_intrinsics._c), C.byref(distortion._c),
+                                        out.ctypes.data, ok.ctypes.data))
         return out, ok.astype(bool)
 
     def solve_board(self, ids, corners, frame=None, n_frames: int | None = None, image_size=None) -> list:

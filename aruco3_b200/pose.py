@@ -5,6 +5,7 @@
   `solve_with_undistorted_points`   /root/reference/src/pose.rs:59-62
   `solve_with_normalized_points`    /root/reference/src/pose.rs:64-81
   `CameraIntrinsics`                /root/reference/src/pinhole.rs:11-94
+  `CameraDistortion`                not in the reference: OpenCV's five lens coefficients (kernel K7)
 
 The solvers run on the device (kernel K4, csrc/k4_pose.cu) and therefore need a `Detector` handle; each accepts one
 marker (4 corners, returns `(best, alt)` like the reference) or a batch [n,4,2] (returns two lists).  With
@@ -18,7 +19,7 @@ from dataclasses import dataclass, field
 import numpy as np
 
 from . import _ffi
-from ._ffi import A3CameraIntrinsics, A3Pose, check, lib
+from ._ffi import A3CameraDistortion, A3CameraIntrinsics, A3Pose, check, lib
 
 
 @dataclass
@@ -113,6 +114,28 @@ class CameraIntrinsics:
     def to_matrix3x4(self) -> np.ndarray:
         """`From<CameraIntrinsics> for Matrix3x4<f32>` (src/pinhole.rs:107-115)"""
         return np.concatenate([self.to_matrix3(), np.zeros((3, 1), np.float32)], axis=1)
+
+
+class CameraDistortion:
+    """A lens distortion: OpenCV's five-coefficient Brown-Conrady model in OpenCV's order (the `distCoeffs` of
+    `calibrateCamera`), on the normalised coordinates of `CameraIntrinsics`.  Give it to `Detector(distortion=...)` /
+    `Detector.set_distortion` and the marker and board poses in intrinsics mode solve from undistorted corners."""
+
+    def __init__(self, k1: float = 0.0, k2: float = 0.0, p1: float = 0.0, p2: float = 0.0, k3: float = 0.0):
+        self._c = A3CameraDistortion(k1, k2, p1, p2, k3)
+
+    k1 = property(lambda s: float(s._c.k1))
+    k2 = property(lambda s: float(s._c.k2))
+    p1 = property(lambda s: float(s._c.p1))
+    p2 = property(lambda s: float(s._c.p2))
+    k3 = property(lambda s: float(s._c.k3))
+
+    def coefficients(self) -> np.ndarray:
+        """(k1, k2, p1, p2, k3) as f32, OpenCV's distCoeffs"""
+        return np.array([self._c.k1, self._c.k2, self._c.p1, self._c.p2, self._c.k3], np.float32)
+
+    def __repr__(self):
+        return "CameraDistortion(k1={}, k2={}, p1={}, p2={}, k3={})".format(*self.coefficients().tolist())
 
 
 def _solve(detector, mode, pts, dtype, marker_size_mm, extra):

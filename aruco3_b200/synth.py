@@ -241,31 +241,118 @@ def render_batch(spec, n_frames: int, first_index: int = 0, out: np.ndarray | No
 
 
 # ---- planar boards seen from a known pose (kernel K6) ------------------------------------------------------------------
-def project_points(points: np.ndarray, R: np.ndarray, t: np.ndarray, k: tuple) -> np.ndarray:
+def _coefficients(distortion) -> np.ndarray:
+    """(k1, k2, p1, p2, k3) in f64 from a pose.CameraDistortion or a sequence of five numbers"""
+    c = distortion.coefficients() if hasattr(distortion, "coefficients") else distortion
+    return np.asarray(c, np.float64).reshape(5)
+
+
+def distort_normalized(x: np.ndarray, y: np.ndarray, distortion):
+    """OpenCV's forward model (k1 k2 p1 p2 k3) on normalised points, f64."""
+    k1, k2, p1, p2, k3 = _coefficients(distortion)
+    r2 = x * x + y * y
+    rad = 1.0 + r2 * (k1 + r2 * (k2 + r2 * k3))
+    return x * rad + 2.0 * p1 * x * y + p2 * (r2 + 2.0 * x * x), y * rad + p1 * (r2 + 2.0 * y * y) + 2.0 * p2 * x * y
+
+
+def undistort_normalized(xd: np.ndarray, yd: np.ndarray, distortion, iters: int = 30):
+    """The inverse of distort_normalized by a vectorised f64 Newton solve from the distorted point -> (x, y, ok); ok is
+    False where the model folds (Jacobian determinant <= 0) or the solve does not converge to 1e-12."""
+    k1, k2, p1, p2, k3 = _coefficients(distortion)
+    x, y = xd.astype(np.float64).copy(), yd.astype(np.float64).copy()
+    ok = np.isfinite(x) & np.isfinite(y)
+    for _ in range(iters):
+        r2 = x * x + y * y
+        rad = 1.0 + r2 * (k1 + r2 * (k2 + r2 * k3))
+        fx = x * rad + 2.0 * p1 * x * y + p2 * (r2 + 2.0 * x * x) - xd
+        fy = y * rad + p1 * (r2 + 2.0 * y * y) + 2.0 * p2 * x * y - yd
+        if not (np.maximum(np.abs(fx), np.abs(fy))[ok] > 1e-12).any():
+            break
+        dr = k1 + r2 * (2.0 * k2 + 3.0 * k3 * r2)
+        j00 = rad + 2.0 * x * x * dr + 2.0 * p1 * y + 6.0 * p2 * x
+        j01 = 2.0 * x * y * dr + 2.0 * p1 * x + 2.0 * p2 * y
+        j11 = rad + 2.0 * y * y * dr + 6.0 * p1 * y + 2.0 * p2 * x
+        det = j00 * j11 - j01 * j01
+        ok &= det > 0
+        det = np.where(ok, det, 1.0)
+        x = np.where(ok, x - (fx * j11 - fy * j01) / det, x)
+        y = np.where(ok, y - (j00 * fy - j01 * fx) / det, y)
+    r2 = x * x + y * y
+    rad = 1.0 + r2 * (k1 + r2 * (k2 + r2 * k3))
+    res = np.maximum(np.abs(x * rad + 2.0 * p1 * x * y + p2 * (r2 + 2.0 * x * x) - xd),
+                     np.abs(y * rad + p1 * (r2 + 2.0 * y * y) + 2.0 * p2 * x * y - yd))
+    return x, y, ok & (res <= 1e-12)
+
+
+def project_points(points: np.ndarray, R: np.ndarray, t: np.ndarray, k: tuple, distortion=None) -> np.ndarray:
     """Board points [n, 2] (z = 0) -> image points [n, 2] under X = R p + t and the pinhole k = (fx, fy, cx, cy), in the
-    pixel-centre convention (grey pixel (x, y) is the point (x, y))."""
+    pixel-centre convention (grey pixel (x, y) is the point (x, y)).  `distortion` (pose.CameraDistortion or OpenCV's
+    five coefficients): the lens model applied to the normalised point before the pinhole, as cv2.projectPoints does."""
     p = np.asarray(points, np.float64).reshape(-1, 2)
     X = p @ np.asarray(R, np.float64)[:, :2].T + np.asarray(t, np.float64)
     fx, fy, cx, cy = k
-    return np.stack([fx * X[:, 0] / X[:, 2] + cx, fy * X[:, 1] / X[:, 2] + cy], axis=1)
+    x, y = X[:, 0] / X[:, 2], X[:, 1] / X[:, 2]
+    if distortion is not None:
+        x, y = distort_normalized(x, y, distortion)
+    return np.stack([fx * x + cx, fy * y + cy], axis=1)
+
+
+def _render_distorted(board_ids, board_corners, R, t, k: tuple, width: int, height: int, table, spec, distortion, ss: int):
+    """The board through pinhole k and the lens model: every output pixel is the mean of ss x ss samples, each undistorted
+    (f64 Newton) onto a pinhole image of the board rendered at ss times the resolution and read bilinearly there."""
+    fx, fy, cx, cy = k
+    sub = (np.arange(ss, dtype=np.float64) + 0.5) / ss - 0.5  # sample offsets in the pixel-centre convention
+    gx = (np.arange(width, dtype=np.float64)[:, None] + sub[None, :]).reshape(-1)
+    gy = (np.arange(height, dtype=np.float64)[:, None] + sub[None, :]).reshape(-1)
+    X, Y = np.meshgrid(gx, gy)  # [H ss, W ss]
+    xu, yu, ok = undistort_normalized((X - cx) / fx, (Y - cy) / fy, distortion)
+    qx, qy = fx * xu + cx, fy * yu + cy  # pinhole pixel of every sample (pixel-centre convention)
+    lo_x, hi_x = np.floor(qx[ok].min()) - 2, np.ceil(qx[ok].max()) + 2
+    lo_y, hi_y = np.floor(qy[ok].min()) - 2, np.ceil(qy[ok].max()) + 2
+    cw, ch = int((hi_x - lo_x) * ss) + 1, int((hi_y - lo_y) * ss) + 1
+    canvas = np.empty((ch, cw, 3), dtype=np.uint8)
+    canvas[:] = np.array(spec.background, dtype=np.uint8)
+    for mid, corners in zip(np.asarray(board_ids).reshape(-1), np.asarray(board_corners, np.float64).reshape(-1, 4, 2)):
+        quad = (project_points(corners, R, t, k) + 0.5 - np.array([lo_x, lo_y])) * ss  # draw_marker's convention on the canvas
+        draw_marker(canvas, marker_cells(table, int(mid)), quad, spec.white, spec.black)
+    # canvas pixel (i, j) is sampled at pinhole pixel-centre point ((i + 0.5) / ss + lo - 0.5)
+    u = np.where(ok, (qx - lo_x + 0.5) * ss - 0.5, 0.0)
+    v = np.where(ok, (qy - lo_y + 0.5) * ss - 0.5, 0.0)
+    i0 = np.clip(np.floor(u).astype(np.int64), 0, cw - 2)
+    j0 = np.clip(np.floor(v).astype(np.int64), 0, ch - 2)
+    a = np.clip(u - i0, 0.0, 1.0)[..., None]
+    b = np.clip(v - j0, 0.0, 1.0)[..., None]
+    c = canvas.astype(np.float32)
+    a, b = a.astype(np.float32), b.astype(np.float32)
+    val = (c[j0, i0] * (1 - a) + c[j0, i0 + 1] * a) * (1 - b) + (c[j0 + 1, i0] * (1 - a) + c[j0 + 1, i0 + 1] * a) * b
+    val[~ok] = np.array(spec.background, np.float32)
+    img = val.reshape(height, ss, width, ss, 3).mean(axis=(1, 3))
+    return np.clip(np.rint(img), 0, 255).astype(np.uint8)
 
 
 def render_board_frame(board_ids, board_corners, R, t, k: tuple, width: int, height: int, dictionary: str = "ARUCO",
-                       extra_ids=(), noise: int = 0, seed: int = 0):
+                       extra_ids=(), noise: int = 0, seed: int = 0, distortion=None, supersample: int = 2):
     """A planar board seen from pose (R, t) with pinhole k = (fx, fy, cx, cy) -> (uint8 [H, W, 3], [TruthMarker]).
 
     A pinhole view of a plane is a homography, so drawing each marker on its projected quad is exact.  There is no sheet
     around the markers (its outline would become a quad of its own).  `extra_ids`: markers that are not on the board, drawn
     in the frame's corners (keep the board away from them).  Truth corners are in draw_marker's convention (+0.5 px from the
-    pixel-centre convention of project_points and of refined corners)."""
+    pixel-centre convention of project_points and of refined corners).
+
+    `distortion` (pose.CameraDistortion or OpenCV's five coefficients): the view through that lens.  It is no longer a
+    homography, so the frame is rendered by inverse mapping (`supersample`^2 samples per pixel, see _render_distorted) and
+    the truth corners are the distorted projections.  The extra markers are drawn undistorted on top."""
     table = dictionaries.table(dictionary)
     spec = FrameSpec("board", 0, width, height)
     img = np.empty((height, width, 3), dtype=np.uint8)
     img[:] = np.array(spec.background, dtype=np.uint8)
     truth = []
+    if distortion is not None:
+        img = _render_distorted(board_ids, board_corners, R, t, k, width, height, table, spec, distortion, supersample)
     for mid, corners in zip(np.asarray(board_ids).reshape(-1), np.asarray(board_corners, np.float64).reshape(-1, 4, 2)):
-        quad = project_points(corners, R, t, k) + 0.5
-        draw_marker(img, marker_cells(table, int(mid)), quad, spec.white, spec.black)
+        quad = project_points(corners, R, t, k, distortion) + 0.5
+        if distortion is None:
+            draw_marker(img, marker_cells(table, int(mid)), quad, spec.white, spec.black)
         truth.append(TruthMarker(int(mid), quad))
     side = 0.12 * min(width, height)
     spots = [(0.04 * width, 0.04 * height), (width - 0.04 * width - side, 0.04 * height),

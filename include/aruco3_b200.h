@@ -134,6 +134,9 @@ typedef struct a3_stats {
     /* board pose (K6, a3_detector_set_board): launches, and the sum of its CUDA-event intervals */
     uint32_t board_kernel_launches;
     double ms_board_kernel;
+    /* corner undistortion (K7, a3_detector_set_distortion): launches, and the sum of its CUDA-event intervals */
+    uint32_t undistort_kernel_launches;
+    double ms_undistort_kernel;
 } a3_stats;
 
 /* MarkerPose (src/pose.rs:8-12): scene-from-marker transform in OpenCV chirality (+Z forward, +Y down, +X right).
@@ -149,6 +152,14 @@ typedef struct a3_camera_intrinsics {
     uint32_t image_width, image_height;
     float focal_x, focal_y, principal_x, principal_y;
 } a3_camera_intrinsics;
+
+/* Lens distortion: OpenCV's five-coefficient Brown-Conrady model, in OpenCV's order (calibrateCamera's distCoeffs), on the
+ * normalised coordinates of a3_camera_intrinsics: with r2 = x^2 + y^2, a normalised undistorted point (x, y) is seen at
+ *     x (1 + k1 r2 + k2 r2^2 + k3 r2^3) + 2 p1 x y + p2 (r2 + 2 x^2),   y (1 + k1 r2 + k2 r2^2 + k3 r2^3) + p1 (r2 + 2 y^2) + 2 p2 x y.
+ * Not part of the reference's pinhole model. */
+typedef struct a3_camera_distortion {
+    float k1, k2, p1, p2, k3;
+} a3_camera_distortion;
 
 /* How image corners become the normalised points the pose solver works on. */
 enum {
@@ -343,6 +354,25 @@ a3_status a3_detector_set_board(a3_detector *det, const a3_board *board, uint32_
  * frame 0).  HOST pointers; out: n_frames board poses.  image_w / image_h: the frame size (A3_POSE_UNDISTORTED). */
 a3_status a3_solve_board(a3_detector *det, const uint64_t *ids, const float *corners, const uint32_t *frame, uint32_t n,
                          uint32_t n_frames, uint32_t image_w, uint32_t image_h, a3_board_pose *out);
+
+/* ---- lens distortion: undistorted marker corners for the pose kernels (kernel K7) ---- */
+
+/* Give the detector's intrinsics a lens distortion.  It applies exactly where A3_POSE_INTRINSICS is used: the marker pose
+ * (a3_detector_set_pose), the board pose (a3_detector_set_board) and a3_solve_board.  a3_detect_batch then undistorts every
+ * corner those kernels read once (kernel K7, queued behind the decode kernel and K5: K5's corners when the detector refines
+ * corners, else the integer corners), by Newton's method on the model (k7_undistort_spec.h), and K4 / K6 solve from the
+ * normalised undistorted points.  A marker with a corner that does not undistort (the model folds there, no convergence, a
+ * non-finite value) gets two a3_pose_default poses and is left out of the board solve as if it had not been detected.
+ * d = NULL, or all five coefficients zero, switches it off: nothing more runs.  a3_detector_release resets it.  Invalid:
+ * a non-finite coefficient; distortion together with an A3_POSE_UNDISTORTED or A3_POSE_NORMALIZED pose or board mode,
+ * whichever of the setters is called last.  a3_solve_with_intrinsics stays the reference's pinhole solve. */
+a3_status a3_detector_set_distortion(a3_detector *det, const a3_camera_distortion *d);
+
+/* The undistortion (K7's device function) as a probe.  HOST pointers; points n*2 pixel coordinates (pixel-centre
+ * convention), out n*2 normalised undistorted coordinates, ok n (1 converged, 0 failed).  Followed by
+ * a3_solve_with_normalized_points, this is what the marker pose with distortion computes. */
+a3_status a3_undistort_points(a3_detector *det, const float *points, uint32_t n, const a3_camera_intrinsics *k,
+                              const a3_camera_distortion *d, float *out, uint8_t *ok);
 
 /* Plain host helpers (constructors and one-point conversions; nothing here is on the hot path). */
 void a3_pose_default(a3_pose *p);                                                   /* src/pose.rs:42-50        */

@@ -204,6 +204,23 @@ struct Board {
     a3_board c() const { return a3_board{(uint32_t)ids.size(), ids.data(), corners.empty() ? nullptr : corners[0].data()}; }
 };
 
+// A lens distortion of the intrinsics (a3_camera_distortion): OpenCV's k1 k2 p1 p2 k3.  With it the pose kernels solve
+// from undistorted corners (kernel K7); only with intrinsics modes.
+struct CameraDistortion {
+    float k1 = 0, k2 = 0, p1 = 0, p2 = 0, k3 = 0;
+    a3_camera_distortion c() const { return a3_camera_distortion{k1, k2, p1, p2, k3}; }
+};
+
+// a3_detector_set_distortion on `h` (nullptr = off)
+inline void set_distortion_on(a3_detector *h, const CameraDistortion *d) {
+    if (!d) {
+        check(a3_detector_set_distortion(h, nullptr));
+        return;
+    }
+    const a3_camera_distortion c = d->c();
+    check(a3_detector_set_distortion(h, &c));
+}
+
 // a3_detector_set_board on `h` (nullptr board = off; nullptr k = undistorted at the frame size)
 inline void set_board_on(a3_detector *h, const Board *board, const CameraIntrinsics *k) {
     if (!board) {
@@ -346,6 +363,7 @@ public:
         check(a3_detector_create(&c, &dictionary.c(), device_, &h_));
         if (refine_) check(a3_detector_set_corner_refinement(h_, A3_CORNERS_REFINED));
         if (board_) set_board_on(h_, &*board_, board_k_ ? &*board_k_ : nullptr);
+        if (dist_) set_distortion_on(h_, &*dist_);
     }
 
     // Detector::detect(&self, image: DynamicImage) -> Detection (src/aruco.rs:52-121): one tightly packed image.
@@ -374,6 +392,13 @@ public:
         board_k_ = k ? std::optional<CameraIntrinsics>(*k) : std::nullopt;
     }
 
+    // A lens distortion of the board's intrinsics (kernel K7 undistorts the corners K6 reads); nullptr switches it off.
+    // Copied and kept across rebuild().
+    void set_distortion(const CameraDistortion *d) {
+        set_distortion_on(h_, d);
+        dist_ = d ? std::optional<CameraDistortion>(*d) : std::nullopt;
+    }
+
     a3_detector *handle() const { return h_; }
 
 private:
@@ -382,6 +407,7 @@ private:
     bool refine_ = false;
     std::optional<Board> board_;
     std::optional<CameraIntrinsics> board_k_;
+    std::optional<CameraDistortion> dist_;
 };
 
 // The reference's own shape: `Detector { config, dictionary }` is plain data built with a literal (src/aruco.rs:46-49,
@@ -396,6 +422,7 @@ struct PlainDetector {
     bool refine_corners = false;  // wrapper-side option (not in the reference's DetectorConfig): set on the leased handle per call
     std::optional<Board> board;   // likewise: the board whose pose every frame gets (kernel K6)
     std::optional<CameraIntrinsics> board_intrinsics;  // empty: undistorted at the frame size
+    std::optional<CameraDistortion> distortion;        // likewise: the lens of board_intrinsics (kernel K7)
 
     Detection detect(const uint8_t *pixels, uint32_t width, uint32_t height, PixelFormat fmt = PixelFormat::Rgb8) const {
         std::vector<Detection> v = detect_batch(pixels, 1, width, height, fmt, /*full=*/true);
@@ -411,6 +438,7 @@ struct PlainDetector {
         check(a3_detector_acquire(&c, &dictionary.c(), device, &lease.h));
         if (refine_corners) check(a3_detector_set_corner_refinement(lease.h, A3_CORNERS_REFINED));
         if (board) set_board_on(lease.h, &*board, board_intrinsics ? &*board_intrinsics : nullptr);  // the release resets it
+        if (distortion) set_distortion_on(lease.h, &*distortion);                                      // and this
         return detect_batch_on(lease.h, config, frames, n, width, height, fmt, full, stats, refine_corners, board.has_value());
     }
 };
@@ -431,6 +459,9 @@ public:
     }
     void set_board(const Board *board, const CameraIntrinsics *k = nullptr) {
         for (auto &d : shards_) d->set_board(board, k);
+    }
+    void set_distortion(const CameraDistortion *dist) {
+        for (auto &d : shards_) d->set_distortion(dist);
     }
     static std::pair<uint32_t, uint32_t> shard_range(uint32_t n_frames, uint32_t rank, uint32_t world) {
         const uint32_t base = n_frames / world, extra = n_frames % world;

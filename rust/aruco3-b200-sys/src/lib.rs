@@ -108,6 +108,9 @@ pub struct a3_stats {
     /// board pose (K6, `a3_detector_set_board`): launches and the sum of its CUDA-event intervals
     pub board_kernel_launches: u32,
     pub ms_board_kernel: f64,
+    /// corner undistortion (K7, `a3_detector_set_distortion`): launches and the sum of its CUDA-event intervals
+    pub undistort_kernel_launches: u32,
+    pub ms_undistort_kernel: f64,
 }
 
 /// MarkerPose, reference `src/pose.rs:8-12`; rotation row-major
@@ -129,6 +132,17 @@ pub struct a3_camera_intrinsics {
     pub focal_y: f32,
     pub principal_x: f32,
     pub principal_y: f32,
+}
+
+/// Lens distortion of the intrinsics: OpenCV's k1 k2 p1 p2 k3 (not in the reference's pinhole model).
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
+pub struct a3_camera_distortion {
+    pub k1: f32,
+    pub k2: f32,
+    pub p1: f32,
+    pub p2: f32,
+    pub k3: f32,
 }
 
 pub const A3_CORNERS_INTEGER: u32 = 0;
@@ -247,6 +261,12 @@ extern "C" {
     pub fn a3_solve_board(
         det: *mut a3_detector, ids: *const u64, corners: *const f32, frame: *const u32, n: u32, n_frames: u32, image_w: u32,
         image_h: u32, out: *mut a3_board_pose,
+    ) -> a3_status;
+    // lens distortion (kernel K7)
+    pub fn a3_detector_set_distortion(det: *mut a3_detector, d: *const a3_camera_distortion) -> a3_status;
+    pub fn a3_undistort_points(
+        det: *mut a3_detector, points: *const f32, n: u32, k: *const a3_camera_intrinsics, d: *const a3_camera_distortion, out: *mut f32,
+        ok: *mut u8,
     ) -> a3_status;
     pub fn a3_pose_default(p: *mut a3_pose);
     pub fn a3_pose_apply_transform(p: *const a3_pose, points: *const f32, n: u32, inverse: i32, out: *mut f32);

@@ -165,6 +165,17 @@ pub fn set_board(board: Option<Board>, k: Option<pose::CameraIntrinsics>) {
     BOARD.with(|b| *b.borrow_mut() = board.map(|b| (b, k)));
 }
 
+thread_local! {
+    /// The lens distortion of this thread's pose and board intrinsics (`None`: the pinhole).
+    static DISTORTION: std::cell::Cell<Option<sys::a3_camera_distortion>> = std::cell::Cell::new(None);
+}
+/// Give the intrinsics of this thread's board (`set_board`) a lens distortion, OpenCV's `k1 k2 p1 p2 k3`: the board pose
+/// then solves from undistorted corners (kernel K7).  Needs intrinsics; `None` switches it off.  Like `set_board`, a
+/// wrapper-side option, set on each leased handle (the release resets it).
+pub fn set_distortion(d: Option<sys::a3_camera_distortion>) {
+    DISTORTION.with(|x| x.set(d));
+}
+
 /// A handle out of the library's cache; goes back (warm) when dropped.
 pub(crate) struct Lease(pub(crate) *mut sys::a3_detector);
 impl Drop for Lease {
@@ -213,6 +224,12 @@ impl Detector {
                 }
             }
         });
+        if let Some(d) = DISTORTION.with(|x| x.get()) {
+            if unsafe { sys::a3_detector_set_distortion(h, &d) } != sys::A3_OK {
+                unsafe { sys::a3_detector_release(h) };
+                panic!("{}", last_error());
+            }
+        }
         Lease(h)
     }
 
