@@ -44,10 +44,15 @@ a3_status cuda_fail(cudaError_t e, const char *what) {
 
 namespace {
 
+// Device / pinned buffers that only grow; freed with their owner (the detector's device must be current then).
 template <typename T>
 struct DevBuf {
     T *p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { if (p) cudaFree(p); }
     cudaError_t reserve(size_t n) {
         if (n <= cap) return cudaSuccess;
         if (p) cudaFree(p);
@@ -56,12 +61,15 @@ struct DevBuf {
         if (e == cudaSuccess) cap = n;
         return e;
     }
-    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
 };
 template <typename T>
 struct PinBuf {
     T *p = nullptr;
     size_t cap = 0;
+    PinBuf() = default;
+    PinBuf(const PinBuf &) = delete;
+    PinBuf &operator=(const PinBuf &) = delete;
+    ~PinBuf() { if (p) cudaFreeHost(p); }
     cudaError_t reserve(size_t n) {
         if (n <= cap) return cudaSuccess;
         if (p) cudaFreeHost(p);
@@ -70,7 +78,6 @@ struct PinBuf {
         if (e == cudaSuccess) cap = n;
         return e;
     }
-    void release() { if (p) cudaFreeHost(p); p = nullptr; cap = 0; }
 };
 
 // Persistent host threads.  A job is a function of a frame index; indices [0, ready) may be claimed.
@@ -223,47 +230,87 @@ struct StageState {
     std::deque<Out> out;                                // per grey sub-chunk, in issue order (deque: stable addresses)
 };
 
+// The post-decode stages a call runs, in this order behind K2: K5 (refine), K7 (und_sets sets of undistorted corners), K4
+// (poses), K6 (board).  K7 writes one set for K4 (the pose intrinsics) and one for K6 (the board intrinsics), shared when the
+// two intrinsics are the same; the setters allow distortion only with INTRINSICS modes.
+struct StagePlan {
+    bool poses = false, refine = false, board = false;
+    bool und_pose = false, und_board = false;  // K4 / K6 read K7's points
+    uint32_t und_sets = 0, und_board_set = 0;  // corner sets (0 = K7 does not run), and the one K6 reads
+    void count(a3_stats &st) const {  // the chain's launches
+        st.decode_kernel_launches++;
+        if (refine) st.refine_kernel_launches++;
+        st.undistort_kernel_launches += und_sets;
+        if (poses) st.pose_kernel_launches++;
+        if (board) st.board_kernel_launches++;
+    }
+};
+
+size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
+
+// Byte offsets of a decode group's outputs in one buffer, for `cap` candidates of `n_frames` frames: K6's board pose per frame,
+// K2's records, K4's two poses, K5's corners and flags (accepted candidates only), then K7's points and flags, set j at
+// norm + 32 cap j and nok + cap j.  The board comes first so that [board, dec) is the per-frame part alone, and K7's points last
+// so that [0, host_end) is everything the host reads.
+struct OutLayout {
+    size_t board = 0, dec, pose, ref, refok, host_end, norm, nok, bytes;
+};
+OutLayout out_layout(const StagePlan &sp, uint32_t cap, uint32_t n_frames) {
+    OutLayout l;
+    l.dec = align16(sp.board ? (size_t)n_frames * sizeof(a3_board_pose) : 0);
+    l.pose = l.dec + (size_t)cap * sizeof(a3_decode);
+    l.ref = l.pose + (sp.poses ? (size_t)cap * 2 * sizeof(a3_pose) : 0);
+    l.refok = l.ref + (sp.refine ? (size_t)cap * 32 : 0);
+    l.host_end = l.refok + (sp.refine ? cap : 0);
+    l.norm = sp.und_sets ? align16(l.host_end) : l.host_end;
+    l.nok = l.norm + (size_t)sp.und_sets * cap * 32;
+    l.bytes = l.nok + (size_t)sp.und_sets * cap;
+    return l;
+}
+
+// Timed stages of the chain (K4 is not timed), and the a3_stats field of each one's time
+enum Stage { kDecode, kRefine, kUndistort, kBoard, kStages };
+using StatsMs = double a3_stats::*;
+constexpr StatsMs kStageMs[kStages] = {&a3_stats::ms_decode_kernel, &a3_stats::ms_refine_kernel, &a3_stats::ms_undistort_kernel,
+                                       &a3_stats::ms_board_kernel};
+
 // Buffers of one decode group (the quads of a few frames); kept for reuse across calls.
 struct DecodeBlock {
     PinBuf<uint32_t> h_quads, h_qframe;
-    PinBuf<a3_decode> h_dec;
+    PinBuf<uint32_t> h_qoff;  // K6: per-frame quad offsets of a group whose quads came from the host
     DevBuf<uint32_t> d_quads, d_qframe, d_info, d_qoff;  // d_info / d_qoff: the device-side gather of K3's quads for this group
-    DevBuf<a3_decode> d_dec;
     DevBuf<uint8_t> d_patches;
-    DevBuf<a3_pose> d_pose;   // K4: two poses per quad (written for accepted candidates only)
-    PinBuf<a3_pose> h_pose;
-    DevBuf<float> d_ref;      // K5: refined corners per quad (accepted candidates only) and their flags
-    PinBuf<float> h_ref;
-    DevBuf<uint8_t> d_refok;
-    PinBuf<uint8_t> h_refok;
-    DevBuf<a3_board_pose> d_board;  // K6: one board pose per frame of the group
-    PinBuf<a3_board_pose> h_board;
-    PinBuf<uint32_t> h_qoff;        // K6: per-frame quad offsets of a group whose quads came from the host
-    DevBuf<float> d_norm;           // K7: normalised undistorted corners per quad, one set per distinct intrinsics, and their flags
-    DevBuf<uint8_t> d_nok;
-    cudaEvent_t ev_a = nullptr, ev_b = nullptr, ev_r0 = nullptr, ev_r1 = nullptr, ev_k6a = nullptr, ev_k6b = nullptr;  // around K2, K5, K6
-    cudaEvent_t ev_u0 = nullptr, ev_u1 = nullptr;  // around K7
+    DevBuf<uint8_t> d_out;  // the group's outputs (OutLayout), and their host copy
+    PinBuf<uint8_t> h_out;
+    cudaEvent_t ev[kStages][2] = {};  // around each timed stage; created with the block
+    uint32_t timed = 0;               // bit per Stage: its pair was recorded in this call
     uint32_t n_quads = 0;
-    // where the host reads this group's records: h_dec / h_pose / h_ref, or the one-shot arena
+    // where the host reads this group's records: h_out, or the one-shot arena
     const a3_decode *dec_view = nullptr;
     const a3_pose *pose_view = nullptr;
     const float *ref_view = nullptr;
     const uint8_t *refok_view = nullptr;
     const a3_board_pose *board_view = nullptr;
-    void release() {
-        h_quads.release(); h_qframe.release(); h_dec.release(); d_quads.release(); d_qframe.release(); d_dec.release(); d_patches.release();
-        d_info.release(); d_qoff.release();
-        d_pose.release(); h_pose.release();
-        d_ref.release(); h_ref.release(); d_refok.release(); h_refok.release();
-        d_board.release(); h_board.release(); h_qoff.release();
-        d_norm.release(); d_nok.release();
-        for (cudaEvent_t *e : {&ev_a, &ev_b, &ev_r0, &ev_r1, &ev_k6a, &ev_k6b, &ev_u0, &ev_u1}) { if (*e) cudaEventDestroy(*e); *e = nullptr; }
+    void set_views(const uint8_t *base, const OutLayout &l) {
+        dec_view = reinterpret_cast<const a3_decode *>(base + l.dec);
+        pose_view = reinterpret_cast<const a3_pose *>(base + l.pose);
+        ref_view = reinterpret_cast<const float *>(base + l.ref);
+        refok_view = base + l.refok;
+        board_view = reinterpret_cast<const a3_board_pose *>(base + l.board);
+    }
+    ~DecodeBlock() {
+        for (auto &pair : ev)
+            for (cudaEvent_t e : pair) if (e) cudaEventDestroy(e);
     }
 };
 
 struct EventPool {
     std::vector<cudaEvent_t> ev;
     size_t used = 0;
+    EventPool() = default;
+    EventPool(const EventPool &) = delete;
+    EventPool &operator=(const EventPool &) = delete;
+    ~EventPool() { for (auto e : ev) cudaEventDestroy(e); }
     cudaError_t get(cudaEvent_t *out) {
         if (used == ev.size()) {
             cudaEvent_t e;
@@ -275,7 +322,27 @@ struct EventPool {
         return cudaSuccess;
     }
     void reset() { used = 0; }
-    void release() { for (auto e : ev) cudaEventDestroy(e); ev.clear(); used = 0; }
+};
+
+// The options a handle's setters change; a3_detector_release puts back these defaults, the state a3_detector_create leaves.
+struct Options {
+    uint32_t contour_mode = A3_CONTOURS_DEVICE;
+    // pose step (K4)
+    uint32_t pose_mode = A3_POSE_OFF;
+    float pose_marker_size = 0.0f;
+    a3_camera_intrinsics pose_k{};
+    // corner refinement (K5)
+    uint32_t corner_mode = A3_CORNERS_INTEGER;
+    // board pose (K6): board_n = 0 is off; the board itself is in the detector's d_board_slots / d_board_pts
+    uint32_t board_n = 0, board_mode = A3_POSE_OFF;
+    a3_camera_intrinsics board_k{};
+    // lens distortion (K7) of the intrinsics of the pose and board modes; off unless set
+    bool dist_on = false;
+    a3_camera_distortion dist{};
+    // K1 launch tuning and the front-end chunk size (a3_detector_set_k1_tuning)
+    bool has_tuning = false;
+    K1Tuning k1_tuning{};
+    uint32_t chunk_override = 0;
 };
 
 }  // namespace
@@ -288,9 +355,7 @@ struct a3_detector {
     uint32_t host_threads = 1;
     uint32_t mark_size = 0;
     uint32_t max_taps = 0;
-    a3::K1Tuning k1_tuning{};
-    bool has_tuning = false;
-    uint32_t chunk_override = 0;
+    a3::Options opt;
     cudaStream_t s_copy = nullptr, s_pixel = nullptr, s_decode = nullptr;
     a3::DevBuf<uint8_t> d_src, d_grey, d_mask, d_patches, d_luma;  // d_luma: K0's Luma8 copy of LumaA8 / 16-bit frames
     a3::DevBuf<uint32_t> d_bits, d_quads, d_qframe;
@@ -306,7 +371,6 @@ struct a3_detector {
     a3::CopyPool copy_pool;
     a3::PinBuf<uint8_t> h_stage_in, h_stage_out;
     // GPU contour stage (K3)
-    uint32_t contour_mode = A3_CONTOURS_DEVICE;
     a3::K3Workspace k3;
     a3::DevBuf<uint32_t> d_planes, d_k3quads, d_k3counts, d_k3before, d_k3flags, d_k3contours;
     a3::DevBuf<unsigned long long> d_k3points;
@@ -319,32 +383,21 @@ struct a3_detector {
     a3::DevBuf<uint32_t> d_qoff;
     a3::DevBuf<uint32_t> d_k2queue;  // K2's work counter where the one-shot arena does not provide it
     // arena of the one-shot route, one device-to-host copy per call: [0] quads in total, [1] route unusable; K3's per-frame
-    // counters; the gathered quads; K2's records; K4's poses
+    // counters; the markers (lean calls); the decode group's outputs (OutLayout); the gathered quads
     a3::DevBuf<uint8_t> d_shot;
     a3::PinBuf<uint8_t> h_shot;
     uint32_t hist_nq = 0, hist_nq_n = 0, hist_nq_w = 0, hist_nq_h = 0;  // quads of the previous call with this geometry (0 = none)
-    // pose step (K4)
-    uint32_t pose_mode = A3_POSE_OFF;
-    float pose_marker_size = 0.0f;
-    a3_camera_intrinsics pose_k{};
     a3::DevBuf<float> d_pose_in;      // standalone solve entry points: 8 x 4 bytes per marker (f32 points or u32 corners)
     a3::DevBuf<a3_pose> d_pose_out;
     a3::PinBuf<a3_pose> h_pose_out;
-    // corner refinement (K5)
-    uint32_t corner_mode = A3_CORNERS_INTEGER;
     a3::DevBuf<float> d_refined;      // a3_refine_corners: refined corners and their flags
     a3::DevBuf<uint8_t> d_refined_ok;
-    // board pose (K6): the board as its id -> slot table and points on the device; board_n = 0 is off
-    uint32_t board_n = 0, board_mode = A3_POSE_OFF;
-    a3_camera_intrinsics board_k{};
+    // board pose (K6): the board as its id -> slot table and points on the device
     a3::DevBuf<uint16_t> d_board_slots;
     a3::DevBuf<float> d_board_pts;
     a3::DevBuf<uint64_t> d_probe_ids;  // a3_solve_board
     a3::DevBuf<uint32_t> d_probe_off;
     a3::DevBuf<a3_board_pose> d_probe_out;
-    // lens distortion (K7) of the intrinsics of the pose and board modes; off unless set
-    bool dist_on = false;
-    a3_camera_distortion dist{};
     a3::DevBuf<float> d_und_in, d_und_out;  // a3_undistort_points, and K7's points for a3_solve_board
     a3::DevBuf<uint8_t> d_und_ok;
 };
@@ -525,73 +578,114 @@ K2Params k2_params(const a3_detector *d, const uint8_t *grey, uint32_t w, uint32
     return p;
 }
 
-// K5 on the candidates K2 just decoded (its accepted ones), bracketed by the block's events
-cudaError_t launch_refine(DecodeBlock &b, const uint8_t *grey, uint32_t w, uint32_t h, const uint32_t *quads, const uint32_t *qframe,
-                          const a3_decode *dec, uint32_t n, const uint32_t *n_dev, float *out, uint8_t *ok, cudaStream_t s) {
-    cudaError_t e = cudaSuccess;
-    if (!b.ev_r0) e = cudaEventCreate(&b.ev_r0);
-    if (e == cudaSuccess && !b.ev_r1) e = cudaEventCreate(&b.ev_r1);
-    if (e == cudaSuccess) e = cudaEventRecord(b.ev_r0, s);
-    K5Params kp{};
-    kp.grey = grey; kp.w = w; kp.h = h; kp.quads = quads; kp.quad_frame = qframe; kp.decodes = dec; kp.n = n; kp.n_dev = n_dev;
-    kp.corners = out; kp.ok = ok;
-    if (e == cudaSuccess) e = k5_corners(kp, s);
-    if (e == cudaSuccess) e = cudaEventRecord(b.ev_r1, s);
+StagePlan plan_stages(const a3_detector *d, bool poses, bool refine, bool board) {
+    StagePlan sp;
+    sp.poses = poses; sp.refine = refine; sp.board = board;
+    if (!d->opt.dist_on) return sp;
+    sp.und_pose = poses;
+    sp.und_board = board;
+    const bool shared = poses && board && memcmp(&d->opt.pose_k, &d->opt.board_k, sizeof(a3_camera_intrinsics)) == 0;
+    sp.und_sets = (poses ? 1u : 0u) + ((board && !shared) ? 1u : 0u);
+    sp.und_board_set = (poses && !shared) ? 1u : 0u;
+    return sp;
+}
+
+// K2's work counter: beyond one wave of warps (2048 quads) the warps share the quads out through a counter that is zero at
+// launch: `zeroed` when the caller has one, else the detector's own after a memset on `s`.  Null below that.
+cudaError_t k2_queue(a3_detector *d, uint32_t n_quads, uint32_t *zeroed, cudaStream_t s, uint32_t **queue) {
+    *queue = nullptr;
+    if (n_quads <= 2048) return cudaSuccess;
+    if (zeroed) { *queue = zeroed; return cudaSuccess; }
+    cudaError_t e = d->d_k2queue.reserve(1);
+    if (e == cudaSuccess) e = cudaMemsetAsync(d->d_k2queue.p, 0, 4, s);
+    if (e == cudaSuccess) *queue = d->d_k2queue.p;
     return e;
 }
 
-// Which undistorted corner sets K7 writes for a call: one for K4 (the pose intrinsics) and one for K6 (the board
-// intrinsics), shared when the two intrinsics are the same.  The setters allow distortion only with INTRINSICS modes.
-struct UndistortPlan {
-    bool pose = false, board = false;
-    uint32_t sets = 0, board_set = 0;  // corner sets (0 = K7 does not run), and the one K6 reads
+// What the post-decode chain reads: n candidates (quads, their frames) on the grey frames, and per-route extras
+struct ChainIn {
+    const uint8_t *grey = nullptr;
+    uint32_t w = 0, h = 0;
+    const uint32_t *quads = nullptr, *qframe = nullptr;
+    uint32_t n = 0;                       // launch size
+    const uint32_t *n_dev = nullptr;      // device, optional: the real number of candidates
+    uint32_t *queue = nullptr;            // K2's work counter (k2_queue) or null
+    uint32_t *accept_counts = nullptr;    // K2's accepted count per 1024 quads (assemble_markers_kernel) or null
+    uint8_t *patches = nullptr;           // K2's sampled patches or null
+    const uint32_t *offsets = nullptr;    // K6: candidates of frame f are [offsets[f], offsets[f + 1])
+    const uint32_t *skip = nullptr;       // K6: device flag or null, non-zero = write nothing
+    uint32_t n_frames = 0;
 };
-UndistortPlan undistort_plan(const a3_detector *d, bool want_poses, bool want_board) {
-    UndistortPlan u;
-    if (!d->dist_on) return u;
-    u.pose = want_poses;
-    u.board = want_board;
-    const bool shared = u.pose && u.board && memcmp(&d->pose_k, &d->board_k, sizeof(a3_camera_intrinsics)) == 0;
-    u.sets = (u.pose ? 1u : 0u) + ((u.board && !shared) ? 1u : 0u);
-    u.board_set = (u.pose && !shared) ? 1u : 0u;
-    return u;
-}
 
-// K7 for every set of the plan on n items (set j at norm + 8 n j, ok + n j), bracketed by the block's events
-cudaError_t launch_undistort(const a3_detector *d, DecodeBlock &b, const UndistortPlan &u, const uint32_t *quads, const float *ref,
-                             const a3_decode *dec, uint32_t n, const uint32_t *n_dev, float *norm, uint8_t *ok, cudaStream_t s) {
-    cudaError_t e = cudaSuccess;
-    if (!b.ev_u0) e = cudaEventCreate(&b.ev_u0);
-    if (e == cudaSuccess && !b.ev_u1) e = cudaEventCreate(&b.ev_u1);
-    if (e == cudaSuccess) e = cudaEventRecord(b.ev_u0, s);
-    for (uint32_t j = 0; j < u.sets && e == cudaSuccess; j++) {
-        K7Params kp;
-        kp.quads = quads; kp.corners_f32 = ref; kp.decodes = dec; kp.n = n; kp.n_dev = n_dev;
-        kp.k = (j == 0 && u.pose) ? d->pose_k : d->board_k; kp.dist = d->dist;
-        kp.out = norm + (size_t)n * 8 * j; kp.ok = ok + (size_t)n * j;
-        e = k7_undistort(kp, s);
+// The post-decode stages of one decode group on stream s: K2 -> K5 -> K7 (each set) -> K4 -> K6, into `out` laid out by `l`.
+// Each timed stage is bracketed by the block's pair of events and marked as recorded.
+cudaError_t enqueue_chain(const a3_detector *d, const StagePlan &sp, const ChainIn &in, uint8_t *out, const OutLayout &l, DecodeBlock &b,
+                          cudaStream_t s) {
+    const Options &o = d->opt;
+    a3_decode *dec = reinterpret_cast<a3_decode *>(out + l.dec);
+    float *ref = sp.refine ? reinterpret_cast<float *>(out + l.ref) : nullptr;
+    float *norm = reinterpret_cast<float *>(out + l.norm);
+    uint8_t *nok = out + l.nok;
+    auto timed = [&](Stage st, auto &&launch) {
+        cudaError_t e = cudaEventRecord(b.ev[st][0], s);
+        if (e == cudaSuccess) e = launch();
+        if (e == cudaSuccess) e = cudaEventRecord(b.ev[st][1], s);
+        if (e == cudaSuccess) b.timed |= 1u << st;
+        return e;
+    };
+    K2Params p2 = k2_params(d, in.grey, in.w, in.h);
+    p2.quads = in.quads; p2.quad_frame = in.qframe; p2.n_quads = in.n; p2.n_quads_dev = in.n_dev; p2.queue = in.queue;
+    p2.accept_counts = in.accept_counts; p2.decodes = dec; p2.patches = in.patches;
+    cudaError_t e = timed(kDecode, [&] { return k2_decode(p2, s); });
+    if (e == cudaSuccess && sp.refine) {  // on K2's accepted candidates
+        K5Params p5{};
+        p5.grey = in.grey; p5.w = in.w; p5.h = in.h; p5.quads = in.quads; p5.quad_frame = in.qframe; p5.decodes = dec;
+        p5.n = in.n; p5.n_dev = in.n_dev; p5.corners = ref; p5.ok = out + l.refok;
+        e = timed(kRefine, [&] { return k5_corners(p5, s); });
     }
-    if (e == cudaSuccess) e = cudaEventRecord(b.ev_u1, s);
+    if (e == cudaSuccess && sp.und_sets)  // the corners K4 and K6 read
+        e = timed(kUndistort, [&] {
+            cudaError_t r = cudaSuccess;
+            for (uint32_t j = 0; j < sp.und_sets && r == cudaSuccess; j++) {
+                K7Params p7;
+                p7.quads = in.quads; p7.corners_f32 = ref; p7.decodes = dec; p7.n = in.n; p7.n_dev = in.n_dev;
+                p7.k = (j == 0 && sp.und_pose) ? o.pose_k : o.board_k; p7.dist = o.dist;
+                p7.out = norm + (size_t)in.n * 8 * j; p7.ok = nok + (size_t)in.n * j;
+                r = k7_undistort(p7, s);
+            }
+            return r;
+        });
+    if (e == cudaSuccess && sp.poses) {
+        K4Params p4{};
+        p4.mode = o.pose_mode; p4.corners = in.quads; p4.corners_f32 = ref; p4.decodes = dec; p4.n = in.n; p4.n_dev = in.n_dev;
+        p4.marker_size = o.pose_marker_size; p4.image_w = in.w; p4.image_h = in.h; p4.k = o.pose_k;
+        p4.poses = reinterpret_cast<a3_pose *>(out + l.pose);
+        if (sp.und_pose) { p4.mode = A3_POSE_NORMALIZED; p4.points = norm; p4.points_ok = nok; }
+        e = k4_pose(p4, s);
+    }
+    if (e == cudaSuccess && sp.board) {
+        K6Params p6;
+        p6.decodes = dec; p6.quads = in.quads; p6.corners_f32 = ref; p6.offsets = in.offsets; p6.skip = in.skip; p6.n_frames = in.n_frames;
+        p6.slots = d->d_board_slots.p; p6.n_codes = d->dict.n_codes; p6.board = d->d_board_pts.p; p6.n_board = o.board_n;
+        p6.mode = o.board_mode; p6.image_w = in.w; p6.image_h = in.h; p6.k = o.board_k;
+        p6.out = reinterpret_cast<a3_board_pose *>(out + l.board);
+        if (sp.und_board) { p6.norm = norm + (size_t)in.n * 8 * sp.und_board_set; p6.norm_ok = nok + (size_t)in.n * sp.und_board_set; }
+        e = timed(kBoard, [&] { return k6_board(p6, s); });
+    }
     return e;
 }
 
-// K6 over the frames [0, n_frames) of a decode group or of the one-shot arena, bracketed by the block's events; norm / nok:
-// K7's points when the board's intrinsics have a distortion
-cudaError_t launch_board(const a3_detector *d, DecodeBlock &b, const a3_decode *dec, const uint32_t *quads, const float *ref,
-                         const uint32_t *offsets, const uint32_t *skip, uint32_t n_frames, uint32_t w, uint32_t h, a3_board_pose *out,
-                         cudaStream_t s, const float *norm = nullptr, const uint8_t *nok = nullptr) {
-    cudaError_t e = cudaSuccess;
-    if (!b.ev_k6a) e = cudaEventCreate(&b.ev_k6a);
-    if (e == cudaSuccess && !b.ev_k6b) e = cudaEventCreate(&b.ev_k6b);
-    if (e == cudaSuccess) e = cudaEventRecord(b.ev_k6a, s);
-    K6Params kp;
-    kp.decodes = dec; kp.quads = quads; kp.corners_f32 = ref; kp.offsets = offsets; kp.skip = skip; kp.n_frames = n_frames;
-    kp.slots = d->d_board_slots.p; kp.n_codes = d->dict.n_codes; kp.board = d->d_board_pts.p; kp.n_board = d->board_n;
-    kp.mode = d->board_mode; kp.image_w = w; kp.image_h = h; kp.k = d->board_k; kp.out = out;
-    kp.norm = norm; kp.norm_ok = nok;
-    if (e == cudaSuccess) e = k6_board(kp, s);
-    if (e == cudaSuccess) e = cudaEventRecord(b.ev_k6b, s);
-    return e;
+// The stage times the block recorded in this call, summed; each is also added to its a3_stats field when `st` is given
+double stage_ms(const DecodeBlock &b, a3_stats *st) {
+    double sum = 0;
+    for (int i = 0; i < kStages; i++) {
+        if (!(b.timed >> i & 1u)) continue;
+        float ms = 0;
+        cudaEventElapsedTime(&ms, b.ev[i][0], b.ev[i][1]);
+        sum += ms;
+        if (st) st->*kStageMs[i] += ms;
+    }
+    return sum;
 }
 
 }  // namespace
@@ -708,13 +802,7 @@ a3_status a3_detector_acquire(const a3_config *cfg, const a3_dictionary *dict, i
 
 void a3_detector_release(a3_detector *d) {
     if (!d) return;
-    // back to the state a3_detector_create leaves a handle in (the buffers stay)
-    d->contour_mode = A3_CONTOURS_DEVICE;
-    d->pose_mode = A3_POSE_OFF;
-    d->corner_mode = A3_CORNERS_INTEGER;
-    d->board_n = 0; d->board_mode = A3_POSE_OFF;
-    d->dist_on = false; d->dist = a3_camera_distortion{};
-    d->has_tuning = false; d->k1_tuning = K1Tuning{}; d->chunk_override = 0;
+    d->opt = Options{};  // back to the state a3_detector_create leaves a handle in (the buffers stay)
     a3_detector *evict = nullptr;
     {
         std::lock_guard<std::mutex> lk(g_cache_mu);
@@ -738,22 +826,8 @@ void a3_detector_destroy(a3_detector *d) {
     cudaSetDevice(d->device);
     for (cudaStream_t s : {d->s_copy, d->s_pixel, d->s_decode})
         if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); }
-    d->d_src.release(); d->d_grey.release(); d->d_mask.release(); d->d_patches.release(); d->d_luma.release();
-    d->d_bits.release(); d->d_quads.release(); d->d_qframe.release(); d->d_dec.release(); d->h_bits.release();
-    d->d_codes.release(); d->d_taps.release(); d->d_meta.release();
-    d->d_planes.release(); d->d_k3quads.release(); d->d_k3counts.release(); d->d_k3before.release(); d->d_k3flags.release();
-    d->d_k3contours.release(); d->d_k3points.release(); d->h_k3quads.release(); d->h_k3counts.release(); d->h_k3before.release();
-    d->h_k3flags.release(); d->h_k3contours.release(); d->h_k3points.release(); d->h_plane.release();
-    d->d_qoff.release(); d->d_k2queue.release(); d->d_shot.release(); d->h_shot.release();
-    d->d_pose_in.release(); d->d_pose_out.release(); d->h_pose_out.release();
-    d->d_refined.release(); d->d_refined_ok.release();
-    d->d_board_slots.release(); d->d_board_pts.release(); d->d_probe_ids.release(); d->d_probe_off.release(); d->d_probe_out.release();
-    d->d_und_in.release(); d->d_und_out.release(); d->d_und_ok.release();
-    d->copy_pool.stop();
-    d->h_stage_in.release(); d->h_stage_out.release();
-    d->events.release();
-    for (auto &b : d->blocks) b->release();
-    delete d;
+    d->copy_pool.stop();  // its tasks use the staging rings, which go with the handle
+    delete d;             // buffers and events free themselves, on the device set above
 }
 
 a3_status a3_detector_set_host_threads(a3_detector *d, uint32_t threads) {
@@ -764,25 +838,25 @@ a3_status a3_detector_set_host_threads(a3_detector *d, uint32_t threads) {
 
 a3_status a3_detector_set_contour_mode(a3_detector *d, uint32_t mode) {
     if (!d || mode > A3_CONTOURS_DEVICE) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_contour_mode: bad argument");
-    d->contour_mode = mode;
+    d->opt.contour_mode = mode;
     return A3_OK;
 }
 
 a3_status a3_detector_set_corner_refinement(a3_detector *d, uint32_t mode) {
     if (!d || mode > A3_CORNERS_REFINED) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_corner_refinement: bad argument");
-    d->corner_mode = mode;
+    d->opt.corner_mode = mode;
     return A3_OK;
 }
 
 a3_status a3_detector_set_k1_tuning(a3_detector *d, const a3_k1_tuning *t) {
     if (!d) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_k1_tuning: null detector");
-    d->has_tuning = t != nullptr;
-    d->k1_tuning = K1Tuning{};
-    d->chunk_override = 0;
+    d->opt.has_tuning = t != nullptr;
+    d->opt.k1_tuning = K1Tuning{};
+    d->opt.chunk_override = 0;
     if (t) {
-        d->k1_tuning.strip_cols = t->strip_cols; d->k1_tuning.seg_rows = t->seg_rows; d->k1_tuning.force_no_tma = (int)t->force_no_tma;
-        d->k1_tuning.force_generic = (int)t->force_generic;
-        d->chunk_override = t->chunk_frames;
+        d->opt.k1_tuning.strip_cols = t->strip_cols; d->opt.k1_tuning.seg_rows = t->seg_rows; d->opt.k1_tuning.force_no_tma = (int)t->force_no_tma;
+        d->opt.k1_tuning.force_generic = (int)t->force_generic;
+        d->opt.chunk_override = t->chunk_frames;
     }
     return A3_OK;
 }
@@ -796,7 +870,7 @@ a3_status a3_gray_threshold_batch(a3_detector *d, const void *frames, a3_format 
     const uint32_t bpp = bytes_per_pixel(format);
     if (pitch < (size_t)w * bpp || frame_stride < pitch * h) return fail(A3_ERR_INVALID_ARGUMENT, "pitch / frame_stride too small");
     A3_CUDA(cudaSetDevice(d->device));
-    const K1Tuning *tune = d->has_tuning ? &d->k1_tuning : nullptr;
+    const K1Tuning *tune = d->opt.has_tuning ? &d->opt.k1_tuning : nullptr;
     K1Params p;
     p.format = format; p.n = n; p.w = w; p.h = h; p.pitch = pitch; p.frame_stride = frame_stride; p.radius = d->cfg.threshold_window;
     if (mem == A3_MEM_DEVICE) {
@@ -911,11 +985,7 @@ a3_status a3_decode_candidates(a3_detector *d, const uint8_t *grey, uint32_t n_f
     K2Params p = k2_params(d, d->d_grey.p, w, h);
     p.quads = d->d_quads.p; p.quad_frame = quad_frame ? d->d_qframe.p : nullptr; p.n_quads = n_quads;
     p.decodes = d->d_dec.p; p.patches = patches ? d->d_patches.p : nullptr;
-    if (n_quads > 2048) {  // more quads than one wave of warps: let the warps share them out
-        A3_CUDA(d->d_k2queue.reserve(1));
-        A3_CUDA(cudaMemsetAsync(d->d_k2queue.p, 0, 4, s));
-        p.queue = d->d_k2queue.p;
-    }
+    A3_CUDA(k2_queue(d, n_quads, nullptr, s, &p.queue));
     A3_CUDA(k2_decode(p, s));
     A3_CUDA(cudaMemcpyAsync(decodes, d->d_dec.p, (size_t)n_quads * sizeof(a3_decode), cudaMemcpyDeviceToHost, s));
     if (patches) A3_CUDA(cudaMemcpyAsync(patches, d->d_patches.p, n_quads * np, cudaMemcpyDeviceToHost, s));
@@ -970,15 +1040,15 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
     const size_t px = (size_t)w * h, wpr = (w + 31) / 32, bits_words = wpr * h;
     const size_t np = (size_t)d->cfg.homography_sample_size * d->cfg.homography_sample_size;
     const bool want_mask = outs && outs->mask, want_grey = outs && outs->grey, want_patches = outs && outs->homographies;
-    const bool want_poses = outs && outs->marker_poses && markers && d->pose_mode != A3_POSE_OFF;
+    const bool want_poses = outs && outs->marker_poses && markers && d->opt.pose_mode != A3_POSE_OFF;
     // K6 solves the board's pose per frame (a3_outputs.board_poses), whatever else the caller asked for
-    const bool want_board = d->board_n > 0 && outs && outs->board_poses;  // no board: the field is never read
+    const bool want_board = d->opt.board_n > 0 && outs && outs->board_poses;  // no board: the field is never read
     // K5 refines the markers' corners (a3_marker.corners_refined, a3_outputs.marker_corners); K4 and K6 then solve from them
-    const bool want_refine = (markers || want_board) && d->corner_mode == A3_CORNERS_REFINED;
+    const bool want_refine = (markers || want_board) && d->opt.corner_mode == A3_CORNERS_REFINED;
     float *const out_corners = want_refine && markers && outs ? outs->marker_corners : nullptr;
     // K7 undistorts the corners K4 and K6 read when their intrinsics have a distortion
-    const UndistortPlan und = undistort_plan(d, want_poses, want_board);
-    const K1Tuning *tune = d->has_tuning ? &d->k1_tuning : nullptr;
+    const StagePlan plan = plan_stages(d, want_poses, want_refine, want_board);
+    const K1Tuning *tune = d->opt.has_tuning ? &d->opt.k1_tuning : nullptr;
     const uint8_t *src_all = static_cast<const uint8_t *>(frames);
     a3_stats st;
     memset(&st, 0, sizeof(st));
@@ -1005,14 +1075,14 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
     if (sb < 1) sb = 1;
     if (sb > n) sb = n;
     size_t fe = ((size_t)96 << 20) / (frame_stride ? frame_stride : 1);           // ~96 MB of input per front-end chunk
-    if (d->chunk_override) fe = d->chunk_override;
+    if (d->opt.chunk_override) fe = d->opt.chunk_override;
     if (fe < 1) fe = 1;
     if (fe > 64) fe = 64;
     if (fe > sb) fe = sb;
     uint32_t group = 32;          // frames per decode launch
     const uint32_t kStaging = 3;  // staging ring depth (host input)
     // contour stage on the device (K3) unless the caller asked for the host stage or the frame is too large for K3's 16-bit points
-    const bool gpu_contours = d->contour_mode == A3_CONTOURS_DEVICE && w <= 65535 && h <= 65535 && (uint64_t)w * h < (1ull << 29);
+    const bool gpu_contours = d->opt.contour_mode == A3_CONTOURS_DEVICE && w <= 65535 && h <= 65535 && (uint64_t)w * h < (1ull << 29);
     // resident input + device contours: every quad of the super-batch is known at once, so one decode launch keeps the
     // whole GPU busy (K2 is latency-bound: what counts is candidates in flight)
     if (gpu_contours && mem == A3_MEM_DEVICE) {
@@ -1064,7 +1134,13 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
         }
         if (want_mask) A3_CUDA(d->d_mask.reserve(sn * px));
         if (mem == A3_MEM_HOST) A3_CUDA(d->d_src.reserve((size_t)kStaging * fe * frame_stride));
-        while (d->blocks.size() < ngroups) d->blocks.emplace_back(new DecodeBlock());
+        while (d->blocks.size() < ngroups) {
+            std::unique_ptr<DecodeBlock> b(new DecodeBlock());
+            for (auto &pair : b->ev)
+                for (cudaEvent_t &e : pair) A3_CUDA(cudaEventCreate(&e));
+            d->blocks.push_back(std::move(b));
+        }
+        for (uint32_t g = 0; g < ngroups; g++) d->blocks[g]->timed = 0;
         // pinned rings for pageable memory: kHostRing front-end chunks of input, kOutRing sub-chunks (<= 32 MB) of grey
         constexpr uint32_t kHostRing = 6, kOutRing = 4;
         const size_t kPiece = (size_t)1 << 20;  // bytes per copy task
@@ -1092,17 +1168,12 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
         const size_t off_stats = 16, off_markers = (off_stats + 24 * shot_c + 15) & ~(size_t)15;
         const size_t off_mposes = off_markers + (lean ? (size_t)shot_cap * sizeof(a3_marker) : 0);
         const size_t off_mcorners = off_mposes + ((lean && want_poses) ? (size_t)shot_cap * 2 * sizeof(a3_pose) : 0);  // K5's, per marker
-        const size_t off_board = off_mcorners + ((lean && want_refine) ? (size_t)shot_cap * 32 : 0);  // K6's, per frame
-        const size_t off_quads = (off_board + (want_board ? (size_t)sn * sizeof(a3_board_pose) : 0) + 15) & ~(size_t)15;
-        const size_t off_dec = off_quads + (size_t)shot_cap * 32;
-        const size_t off_pose = off_dec + (size_t)shot_cap * sizeof(a3_decode);
-        const size_t off_ref = off_pose + (want_poses ? (size_t)shot_cap * 2 * sizeof(a3_pose) : 0);  // K5's, per candidate
-        const size_t off_refok = off_ref + (want_refine ? (size_t)shot_cap * 32 : 0);
-        const size_t off_norm = und.sets ? (off_refok + (want_refine ? (size_t)shot_cap : 0) + 15) & ~(size_t)15  // K7's, per candidate
-                                         : off_refok + (want_refine ? (size_t)shot_cap : 0);
-        const size_t off_nok = off_norm + (size_t)und.sets * shot_cap * 32;
-        const size_t shot_bytes = off_nok + (size_t)und.sets * shot_cap;
-        const size_t shot_copy_bytes = lean ? off_quads : shot_bytes;  // what goes back to the host
+        const size_t off_out = align16(off_mcorners + ((lean && want_refine) ? (size_t)shot_cap * 32 : 0));  // the decode group's outputs
+        const OutLayout shot_out = out_layout(plan, shot_cap, sn);
+        const size_t off_quads = align16(off_out + shot_out.bytes);
+        const size_t shot_bytes = off_quads + (size_t)shot_cap * 32;
+        // what goes back to the host: lean calls stop before the per-candidate outputs, after the board poses
+        const size_t shot_copy_bytes = lean ? off_out + shot_out.dec : shot_bytes;
         if (shot) {
             A3_CUDA(d->d_shot.reserve(shot_bytes)); A3_CUDA(d->h_shot.reserve(shot_bytes));
             auto carve = [&](uint8_t *base, uint32_t *&c, uint32_t *&b, uint32_t *&f, uint32_t *&k, unsigned long long *&pt) {
@@ -1169,59 +1240,37 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                                       cudaMemcpyDeviceToHost, d->s_pixel));
             return A3_OK;
         };
-        // gather K3's quads on the device, decode them (K2, K4) and copy everything back, all on the pixel stream
+        // gather K3's quads on the device, run the decode chain on them and copy everything back, all on the pixel stream
         auto enqueue_one_shot = [&]() -> a3_status {
             DecodeBlock &b = *d->blocks[0];
-            const uint32_t cap = shot_cap;
+            const uint32_t cap = shot_cap, n_chunks = (cap + 1023) / 1024;
             uint32_t *d_quads = reinterpret_cast<uint32_t *>(d->d_shot.p + off_quads);
-            a3_decode *d_dec = reinterpret_cast<a3_decode *>(d->d_shot.p + off_dec);
-            a3_pose *d_pose = reinterpret_cast<a3_pose *>(d->d_shot.p + off_pose);
-            const uint32_t n_chunks = (cap + 1023) / 1024;
+            uint8_t *d_out = d->d_shot.p + off_out;
             A3_CUDA(d->d_qoff.reserve((size_t)sn + 1 + n_chunks));  // frame offsets of the quads, then the accepted count of every 1024 quads
-            uint32_t *d_chain = d->d_qoff.p + sn + 1;
+            uint32_t *d_accepted = d->d_qoff.p + sn + 1;
             A3_CUDA(b.d_qframe.reserve(cap));
             if (want_patches) A3_CUDA(b.d_patches.reserve(cap * np));
-            if (!b.ev_a) { A3_CUDA(cudaEventCreate(&b.ev_a)); A3_CUDA(cudaEventCreate(&b.ev_b)); }
             pack_offsets_kernel<<<1, 1024, 0, d->s_pixel>>>(ds_counts, ds_flags, sn, quad_cap, cap, k3_speculation_failed_flag(d->k3), d->d_qoff.p, d_info,
-                                                            d_chain, n_chunks);
+                                                            d_accepted, n_chunks);
             A3_CUDA(cudaGetLastError());
             pack_quads_kernel<<<sn, 128, 0, d->s_pixel>>>(d->d_k3quads.p, d->d_qoff.p, quad_cap, cap, d_info, d_quads, b.d_qframe.p, 0u);
             A3_CUDA(cudaGetLastError());
-            K2Params p = k2_params(d, d->d_grey.p, w, h);
-            p.quads = d_quads; p.quad_frame = b.d_qframe.p; p.n_quads = cap; p.n_quads_dev = d_info; p.queue = d_info + 2; p.decodes = d_dec;
-            p.accept_counts = lean ? d_chain : nullptr;
-            p.patches = want_patches ? b.d_patches.p : nullptr;
-            A3_CUDA(cudaEventRecord(b.ev_a, d->s_pixel));
-            A3_CUDA(k2_decode(p, d->s_pixel));
-            A3_CUDA(cudaEventRecord(b.ev_b, d->s_pixel));
-            float *d_ref = want_refine ? reinterpret_cast<float *>(d->d_shot.p + off_ref) : nullptr;
-            uint8_t *d_refok = want_refine ? d->d_shot.p + off_refok : nullptr;
-            if (want_refine) A3_CUDA(launch_refine(b, d->d_grey.p, w, h, d_quads, b.d_qframe.p, d_dec, cap, d_info, d_ref, d_refok, d->s_pixel));
-            float *d_norm = und.sets ? reinterpret_cast<float *>(d->d_shot.p + off_norm) : nullptr;
-            uint8_t *d_nok = und.sets ? d->d_shot.p + off_nok : nullptr;
-            if (und.sets) A3_CUDA(launch_undistort(d, b, und, d_quads, d_ref, d_dec, cap, d_info, d_norm, d_nok, d->s_pixel));
-            if (want_poses) {
-                K4Params kp{};
-                kp.mode = d->pose_mode; kp.corners = d_quads; kp.corners_f32 = d_ref; kp.decodes = d_dec; kp.n = cap; kp.n_dev = d_info;
-                kp.marker_size = d->pose_marker_size; kp.image_w = w; kp.image_h = h; kp.k = d->pose_k; kp.poses = d_pose;
-                if (und.pose) { kp.mode = A3_POSE_NORMALIZED; kp.points = d_norm; kp.points_ok = d_nok; }
-                A3_CUDA(k4_pose(kp, d->s_pixel));
-            }
-            if (want_board)
-                A3_CUDA(launch_board(d, b, d_dec, d_quads, d_ref, d->d_qoff.p, d_info + 1, sn, w, h,
-                                     reinterpret_cast<a3_board_pose *>(d->d_shot.p + off_board), d->s_pixel,
-                                     und.board ? d_norm + (size_t)cap * 8 * und.board_set : nullptr,
-                                     und.board ? d_nok + (size_t)cap * und.board_set : nullptr));
+            ChainIn in;
+            in.grey = d->d_grey.p; in.w = w; in.h = h; in.quads = d_quads; in.qframe = b.d_qframe.p; in.n = cap; in.n_dev = d_info;
+            in.queue = d_info + 2; in.accept_counts = lean ? d_accepted : nullptr; in.patches = want_patches ? b.d_patches.p : nullptr;
+            in.offsets = d->d_qoff.p; in.skip = d_info + 1; in.n_frames = sn;
+            A3_CUDA(enqueue_chain(d, plan, in, d_out, shot_out, b, d->s_pixel));
             if (lean) {
-                assemble_markers_kernel<<<n_chunks, 1024, 0, d->s_pixel>>>(d_dec, d_quads, b.d_qframe.p, d->d_qoff.p, want_poses ? d_pose : nullptr,
-                                                                    d_ref, d_refok, cap, d_info, d_chain,
-                                                                    reinterpret_cast<a3_marker *>(d->d_shot.p + off_markers),
-                                                                    reinterpret_cast<a3_pose *>(d->d_shot.p + off_mposes),
-                                                                    reinterpret_cast<float *>(d->d_shot.p + off_mcorners));
+                assemble_markers_kernel<<<n_chunks, 1024, 0, d->s_pixel>>>(
+                    reinterpret_cast<const a3_decode *>(d_out + shot_out.dec), d_quads, b.d_qframe.p, d->d_qoff.p,
+                    want_poses ? reinterpret_cast<const a3_pose *>(d_out + shot_out.pose) : nullptr,
+                    want_refine ? reinterpret_cast<const float *>(d_out + shot_out.ref) : nullptr, want_refine ? d_out + shot_out.refok : nullptr, cap,
+                    d_info, d_accepted, reinterpret_cast<a3_marker *>(d->d_shot.p + off_markers), reinterpret_cast<a3_pose *>(d->d_shot.p + off_mposes),
+                    reinterpret_cast<float *>(d->d_shot.p + off_mcorners));
                 A3_CUDA(cudaGetLastError());
             }
-            // everything the host needs in one copy: route info, K3's counters, then either the finished markers (+ poses) or the
-            // quads, K2's records and K4's poses
+            // everything the host needs in one copy: route info, K3's counters, then either the finished markers (+ poses) and
+            // the board poses, or the group's outputs and the quads
             A3_CUDA(cudaMemcpyAsync(d->h_shot.p, d->d_shot.p, shot_copy_bytes, cudaMemcpyDeviceToHost, d->s_pixel));
             one_shot_enqueued = true; one_shot_cap = cap;
             return A3_OK;
@@ -1234,11 +1283,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             if (held && one_shot_enqueued && h_info[1] == 0 && h_info[0] <= one_shot_cap) {
                 DecodeBlock &b = *d->blocks[0];
                 b.n_quads = h_info[0];
-                b.dec_view = reinterpret_cast<const a3_decode *>(d->h_shot.p + off_dec);
-                b.pose_view = reinterpret_cast<const a3_pose *>(d->h_shot.p + off_pose);
-                b.ref_view = reinterpret_cast<const float *>(d->h_shot.p + off_ref);
-                b.refok_view = d->h_shot.p + off_refok;
-                b.board_view = reinterpret_cast<const a3_board_pose *>(d->h_shot.p + off_board);
+                b.set_views(d->h_shot.p + off_out, shot_out);
                 const uint32_t *h_quads = reinterpret_cast<const uint32_t *>(d->h_shot.p + off_quads);
                 uint32_t k = 0;
                 for (uint32_t i = 0; i < sn; i++) {
@@ -1251,11 +1296,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 }
                 group_done[0].store(sn);
                 d->hist_nq = b.n_quads ? b.n_quads : 1;
-                st.decode_kernel_launches++;
-                if (want_poses) st.pose_kernel_launches++;
-                if (want_refine) st.refine_kernel_launches++;
-                if (want_board) st.board_kernel_launches++;
-                st.undistort_kernel_launches += und.sets;
+                plan.count(st);
                 st.one_shot = 1;
                 one_shot_done = true;
                 lean_done = lean;
@@ -1263,6 +1304,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             }
             if (!held || one_shot_enqueued) st.one_shot_retry = 1;
             one_shot_enqueued = false;
+            d->blocks[0]->timed = 0;  // the ordinary route times its own chain
             if (!held) {
                 A3_CUDA(k3_finish(d->k3, k3_last, d->s_pixel));
                 if (a3_status s = k3_stats_d2h(0, sn)) return s;
@@ -1463,24 +1505,24 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
         auto launch_group = [&](uint32_t g) -> a3_status {
             DecodeBlock &b = *d->blocks[g];
             if (one_shot_done && g == 0) return A3_OK;  // decoded on the device behind K3 already
-            const uint32_t f0 = g * group, f1 = f0 + group_size(g);
+            const uint32_t f0 = g * group, f1 = f0 + group_size(g), gn = f1 - f0;
             uint32_t nq = 0;
             for (uint32_t i = f0; i < f1; i++) nq += (uint32_t)(frame_quads[i].size() / 8);
             b.n_quads = nq;
             if (one_shot && ngroups == 1) { d->hist_nq = nq ? nq : 1; d->hist_nq_n = n; d->hist_nq_w = w; d->hist_nq_h = h; }
-            if (!b.ev_a) { A3_CUDA(cudaEventCreate(&b.ev_a)); A3_CUDA(cudaEventCreate(&b.ev_b)); }
+            const OutLayout lay = out_layout(plan, nq, gn);
+            A3_CUDA(b.h_out.reserve(lay.bytes));
+            b.set_views(b.h_out.p, lay);
             if (nq == 0) {
                 if (want_board) {  // no candidates: every frame of the group has the empty board pose
-                    A3_CUDA(b.h_board.reserve(f1 - f0));
                     a3_board_pose e{};
                     a3_pose_default(&e.best); a3_pose_default(&e.alt);
-                    for (uint32_t i = 0; i < f1 - f0; i++) b.h_board.p[i] = e;
-                    b.board_view = b.h_board.p;
+                    for (uint32_t i = 0; i < gn; i++) reinterpret_cast<a3_board_pose *>(b.h_out.p + lay.board)[i] = e;
                 }
                 return A3_OK;
             }
-            A3_CUDA(b.h_quads.reserve((size_t)nq * 8)); A3_CUDA(b.h_qframe.reserve(nq)); A3_CUDA(b.h_dec.reserve(nq));
-            A3_CUDA(b.d_quads.reserve((size_t)nq * 8)); A3_CUDA(b.d_qframe.reserve(nq)); A3_CUDA(b.d_dec.reserve(nq));
+            A3_CUDA(b.h_quads.reserve((size_t)nq * 8)); A3_CUDA(b.h_qframe.reserve(nq));
+            A3_CUDA(b.d_quads.reserve((size_t)nq * 8)); A3_CUDA(b.d_qframe.reserve(nq)); A3_CUDA(b.d_out.reserve(lay.bytes));
             if (want_patches) A3_CUDA(b.d_patches.reserve(nq * np));
             uint32_t k = 0;
             // Device contour stage: K3's quads of these frames are still in device memory, so they are gathered there (the same two
@@ -1488,9 +1530,8 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             // the copy engine and hold the decode back by whole chunks.  Groups with a frame the host stage redid take the copy.
             bool on_device = gpu_contours;
             for (uint32_t i = f0; i < f1 && on_device; i++) on_device = hs_flags[i] == 0 && frame_quads[i].size() / 8 == (hs_counts[i] < quad_cap ? hs_counts[i] : quad_cap);
-            K2Params p = k2_params(d, d->d_grey.p, w, h);
             if (on_device) {
-                const uint32_t gn = f1 - f0, n_chunks = (nq + 1023) / 1024;
+                const uint32_t n_chunks = (nq + 1023) / 1024;
                 A3_CUDA(b.d_info.reserve(4)); A3_CUDA(b.d_qoff.reserve((size_t)gn + 1 + n_chunks));
                 pack_offsets_kernel<<<1, 1024, 0, d->s_decode>>>(ds_counts + f0, ds_flags + f0, gn, quad_cap, nq, nullptr, b.d_qoff.p, b.d_info.p,
                                                                 b.d_qoff.p + gn + 1, n_chunks);
@@ -1498,7 +1539,6 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 pack_quads_kernel<<<gn, 128, 0, d->s_decode>>>(d->d_k3quads.p + (size_t)f0 * quad_cap * 8, b.d_qoff.p, quad_cap, nq, b.d_info.p,
                                                               b.d_quads.p, b.d_qframe.p, f0);
                 A3_CUDA(cudaGetLastError());
-                p.n_quads_dev = b.d_info.p;
             } else {
                 for (uint32_t i = f0; i < f1; i++) {
                     const uint32_t m = (uint32_t)(frame_quads[i].size() / 8);
@@ -1509,67 +1549,21 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 A3_CUDA(cudaMemcpyAsync(b.d_quads.p, b.h_quads.p, (size_t)nq * 32, cudaMemcpyHostToDevice, d->s_decode));
                 A3_CUDA(cudaMemcpyAsync(b.d_qframe.p, b.h_qframe.p, (size_t)nq * 4, cudaMemcpyHostToDevice, d->s_decode));
                 if (want_board) {  // K6's per-frame offsets travel with the quads
-                    A3_CUDA(b.h_qoff.reserve((size_t)(f1 - f0) + 1)); A3_CUDA(b.d_qoff.reserve((size_t)(f1 - f0) + 1));
+                    A3_CUDA(b.h_qoff.reserve((size_t)gn + 1)); A3_CUDA(b.d_qoff.reserve((size_t)gn + 1));
                     uint32_t o = 0;
                     for (uint32_t i = f0; i < f1; i++) { b.h_qoff.p[i - f0] = o; o += (uint32_t)(frame_quads[i].size() / 8); }
-                    b.h_qoff.p[f1 - f0] = o;
-                    A3_CUDA(cudaMemcpyAsync(b.d_qoff.p, b.h_qoff.p, (size_t)(f1 - f0 + 1) * 4, cudaMemcpyHostToDevice, d->s_decode));
+                    b.h_qoff.p[gn] = o;
+                    A3_CUDA(cudaMemcpyAsync(b.d_qoff.p, b.h_qoff.p, (size_t)(gn + 1) * 4, cudaMemcpyHostToDevice, d->s_decode));
                 }
             }
-            p.quads = b.d_quads.p; p.quad_frame = b.d_qframe.p; p.n_quads = nq; p.decodes = b.d_dec.p;
-            p.patches = want_patches ? b.d_patches.p : nullptr;
-            if (nq > 2048) {  // more quads than one wave of warps: let the warps share them out
-                if (on_device) {
-                    p.queue = b.d_info.p + 2;  // zeroed by pack_offsets_kernel
-                } else {
-                    A3_CUDA(d->d_k2queue.reserve(1));
-                    A3_CUDA(cudaMemsetAsync(d->d_k2queue.p, 0, 4, d->s_decode));
-                    p.queue = d->d_k2queue.p;
-                }
-            }
-            A3_CUDA(cudaEventRecord(b.ev_a, d->s_decode));
-            A3_CUDA(k2_decode(p, d->s_decode));
-            A3_CUDA(cudaEventRecord(b.ev_b, d->s_decode));
-            st.decode_kernel_launches++;
-            A3_CUDA(cudaMemcpyAsync(b.h_dec.p, b.d_dec.p, (size_t)nq * sizeof(a3_decode), cudaMemcpyDeviceToHost, d->s_decode));
-            b.dec_view = b.h_dec.p; b.pose_view = nullptr;
-            if (want_refine) {  // K5 right behind K2, on the grey, the quads and K2's records where they lie
-                A3_CUDA(b.d_ref.reserve((size_t)nq * 8)); A3_CUDA(b.h_ref.reserve((size_t)nq * 8));
-                A3_CUDA(b.d_refok.reserve(nq)); A3_CUDA(b.h_refok.reserve(nq));
-                A3_CUDA(launch_refine(b, d->d_grey.p, w, h, b.d_quads.p, b.d_qframe.p, b.d_dec.p, nq, on_device ? b.d_info.p : nullptr, b.d_ref.p,
-                                      b.d_refok.p, d->s_decode));
-                st.refine_kernel_launches++;
-                A3_CUDA(cudaMemcpyAsync(b.h_ref.p, b.d_ref.p, (size_t)nq * 32, cudaMemcpyDeviceToHost, d->s_decode));
-                A3_CUDA(cudaMemcpyAsync(b.h_refok.p, b.d_refok.p, nq, cudaMemcpyDeviceToHost, d->s_decode));
-                b.ref_view = b.h_ref.p; b.refok_view = b.h_refok.p;
-            }
-            if (und.sets) {  // K7 behind K2 (and K5), on the corners K4 and K6 read
-                A3_CUDA(b.d_norm.reserve((size_t)und.sets * nq * 8)); A3_CUDA(b.d_nok.reserve((size_t)und.sets * nq));
-                A3_CUDA(launch_undistort(d, b, und, b.d_quads.p, want_refine ? b.d_ref.p : nullptr, b.d_dec.p, nq, on_device ? b.d_info.p : nullptr,
-                                         b.d_norm.p, b.d_nok.p, d->s_decode));
-                st.undistort_kernel_launches += und.sets;
-            }
-            if (want_poses) {  // K4 right behind K2, on K2's records and the quads where they lie
-                A3_CUDA(b.d_pose.reserve((size_t)nq * 2)); A3_CUDA(b.h_pose.reserve((size_t)nq * 2));
-                K4Params kp{};
-                kp.mode = d->pose_mode; kp.corners = b.d_quads.p; kp.corners_f32 = want_refine ? b.d_ref.p : nullptr; kp.decodes = b.d_dec.p; kp.n = nq; kp.marker_size = d->pose_marker_size;
-                kp.image_w = w; kp.image_h = h; kp.k = d->pose_k; kp.poses = b.d_pose.p;
-                if (und.pose) { kp.mode = A3_POSE_NORMALIZED; kp.points = b.d_norm.p; kp.points_ok = b.d_nok.p; }
-                A3_CUDA(k4_pose(kp, d->s_decode));
-                st.pose_kernel_launches++;
-                A3_CUDA(cudaMemcpyAsync(b.h_pose.p, b.d_pose.p, (size_t)nq * 2 * sizeof(a3_pose), cudaMemcpyDeviceToHost, d->s_decode));
-                b.pose_view = b.h_pose.p;
-            }
-            if (want_board) {  // K6 behind K2 (and K5), on the records, the quads or K5's corners where they lie
-                const uint32_t gn = f1 - f0;
-                A3_CUDA(b.d_board.reserve(gn)); A3_CUDA(b.h_board.reserve(gn));
-                A3_CUDA(launch_board(d, b, b.d_dec.p, b.d_quads.p, want_refine ? b.d_ref.p : nullptr, b.d_qoff.p, nullptr, gn, w, h, b.d_board.p,
-                                     d->s_decode, und.board ? b.d_norm.p + (size_t)nq * 8 * und.board_set : nullptr,
-                                     und.board ? b.d_nok.p + (size_t)nq * und.board_set : nullptr));
-                st.board_kernel_launches++;
-                A3_CUDA(cudaMemcpyAsync(b.h_board.p, b.d_board.p, (size_t)gn * sizeof(a3_board_pose), cudaMemcpyDeviceToHost, d->s_decode));
-                b.board_view = b.h_board.p;
-            }
+            ChainIn in;
+            in.grey = d->d_grey.p; in.w = w; in.h = h; in.quads = b.d_quads.p; in.qframe = b.d_qframe.p; in.n = nq;
+            in.n_dev = on_device ? b.d_info.p : nullptr;
+            A3_CUDA(k2_queue(d, nq, on_device ? b.d_info.p + 2 : nullptr, d->s_decode, &in.queue));  // d_info[2]: zeroed by pack_offsets_kernel
+            in.patches = want_patches ? b.d_patches.p : nullptr; in.offsets = b.d_qoff.p; in.n_frames = gn;
+            A3_CUDA(enqueue_chain(d, plan, in, b.d_out.p, lay, b, d->s_decode));
+            plan.count(st);
+            A3_CUDA(cudaMemcpyAsync(b.h_out.p, b.d_out.p, lay.host_end, cudaMemcpyDeviceToHost, d->s_decode));
             return A3_OK;
         };
         auto drain = [&](a3_status s) {  // an error: let the pool and the streams finish before the buffers go away
@@ -1627,12 +1621,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 if (mem == A3_MEM_HOST || j == 0) {
                     cudaEventElapsedTime(&ms, ev_k1b[j], ev_k3[j]); st.ms_contour_kernels += ms;
                     cudaEventElapsedTime(&ms, ev_k3[j], ev_fe[j]); st.ms_mask_d2h += ms;
-                    if (one_shot_done && d->blocks[0]->n_quads) {  // the decode (and K5) sit between those two events on this route
-                        cudaEventElapsedTime(&ms, d->blocks[0]->ev_a, d->blocks[0]->ev_b); st.ms_mask_d2h -= ms;
-                        if (want_refine) { cudaEventElapsedTime(&ms, d->blocks[0]->ev_r0, d->blocks[0]->ev_r1); st.ms_mask_d2h -= ms; }
-                        if (want_board) { cudaEventElapsedTime(&ms, d->blocks[0]->ev_k6a, d->blocks[0]->ev_k6b); st.ms_mask_d2h -= ms; }
-                        if (und.sets) { cudaEventElapsedTime(&ms, d->blocks[0]->ev_u0, d->blocks[0]->ev_u1); st.ms_mask_d2h -= ms; }
-                    }
+                    if (one_shot_done) st.ms_mask_d2h -= stage_ms(*d->blocks[0], nullptr);  // the decode chain sits between those two events here
                 }
             } else {
                 cudaEventElapsedTime(&ms, (mem == A3_MEM_HOST || j == 0) ? ev_k1b[j] : ev_fe[j - 1], ev_fe[j]);
@@ -1659,10 +1648,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
         }
         if (lean_done) {  // the markers were assembled on the device: one block copy (lean implies a single super-batch and group)
             DecodeBlock &b = *d->blocks[0];
-            if (b.n_quads && stats) { cudaEventElapsedTime(&ms, b.ev_a, b.ev_b); st.ms_decode_kernel += ms; }
-            if (b.n_quads && stats && want_refine) { cudaEventElapsedTime(&ms, b.ev_r0, b.ev_r1); st.ms_refine_kernel += ms; }
-            if (stats && want_board) { cudaEventElapsedTime(&ms, b.ev_k6a, b.ev_k6b); st.ms_board_kernel += ms; }
-            if (stats && und.sets) { cudaEventElapsedTime(&ms, b.ev_u0, b.ev_u1); st.ms_undistort_kernel += ms; }
+            if (stats) stage_ms(b, &st);
             if (want_board) memcpy(outs->board_poses, b.board_view, (size_t)sn * sizeof(a3_board_pose));
             const uint32_t nm = h_info[3], take = nm < marker_capacity ? nm : marker_capacity;
             memcpy(markers, d->h_shot.p + off_markers, (size_t)take * sizeof(a3_marker));
@@ -1682,14 +1668,9 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
         }
         for (uint32_t g = 0; g < ngroups; g++) {
             DecodeBlock &b = *d->blocks[g];
-            if (b.n_quads && stats) { cudaEventElapsedTime(&ms, b.ev_a, b.ev_b); st.ms_decode_kernel += ms; }
-            if (b.n_quads && stats && want_refine) { cudaEventElapsedTime(&ms, b.ev_r0, b.ev_r1); st.ms_refine_kernel += ms; }
-            if (b.n_quads && stats && und.sets) { cudaEventElapsedTime(&ms, b.ev_u0, b.ev_u1); st.ms_undistort_kernel += ms; }
+            if (stats) stage_ms(b, &st);
             const uint32_t f0 = g * group, f1 = f0 + group_size(g);
-            if (want_board) {
-                if (b.n_quads && stats) { cudaEventElapsedTime(&ms, b.ev_k6a, b.ev_k6b); st.ms_board_kernel += ms; }
-                memcpy(outs->board_poses + s0 + f0, b.board_view, (size_t)(f1 - f0) * sizeof(a3_board_pose));
-            }
+            if (want_board) memcpy(outs->board_poses + s0 + f0, b.board_view, (size_t)(f1 - f0) * sizeof(a3_board_pose));
             if (want_patches && b.n_quads && total_cands < outs->cand_capacity) {
                 const uint32_t room = outs->cand_capacity - total_cands, m = b.n_quads < room ? b.n_quads : room;
                 A3_CUDA(cudaMemcpy(outs->homographies + (size_t)total_cands * np, b.d_patches.p, (size_t)m * np, cudaMemcpyDeviceToHost));
@@ -1755,11 +1736,11 @@ a3_status a3_detector_set_pose(a3_detector *d, uint32_t mode, float marker_size_
     if (mode != A3_POSE_OFF && mode != A3_POSE_UNDISTORTED && mode != A3_POSE_INTRINSICS)
         return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_pose: mode must be OFF, UNDISTORTED or INTRINSICS");
     if (mode == A3_POSE_INTRINSICS && !k) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_pose: intrinsics required");
-    if (d->dist_on && mode == A3_POSE_UNDISTORTED)
+    if (d->opt.dist_on && mode == A3_POSE_UNDISTORTED)
         return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_pose: the detector has a lens distortion, which needs INTRINSICS (or OFF)");
-    d->pose_mode = mode;
-    d->pose_marker_size = marker_size_mm;
-    if (k) d->pose_k = *k;
+    d->opt.pose_mode = mode;
+    d->opt.pose_marker_size = marker_size_mm;
+    if (k) d->opt.pose_k = *k;
     return A3_OK;
 }
 
@@ -1768,14 +1749,14 @@ a3_status a3_detector_set_pose(a3_detector *d, uint32_t mode, float marker_size_
 a3_status a3_detector_set_board(a3_detector *d, const a3_board *board, uint32_t mode, const a3_camera_intrinsics *k) {
     if (!d) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: null detector");
     if (!board) {
-        d->board_n = 0;
-        d->board_mode = A3_POSE_OFF;
+        d->opt.board_n = 0;
+        d->opt.board_mode = A3_POSE_OFF;
         return A3_OK;
     }
     if (mode != A3_POSE_UNDISTORTED && mode != A3_POSE_INTRINSICS)
         return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: mode must be UNDISTORTED or INTRINSICS");
     if (mode == A3_POSE_INTRINSICS && !k) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: intrinsics required");
-    if (d->dist_on && mode != A3_POSE_INTRINSICS)
+    if (d->opt.dist_on && mode != A3_POSE_INTRINSICS)
         return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: the detector has a lens distortion, which needs INTRINSICS");
     const uint32_t m = board->n_markers;
     if (m == 0 || m > A3_K6_MAX_MARKERS) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_board: a board has 1 to 1024 markers");
@@ -1798,21 +1779,21 @@ a3_status a3_detector_set_board(a3_detector *d, const a3_board *board, uint32_t 
     A3_CUDA(cudaStreamSynchronize(d->s_pixel));
     A3_CUDA(cudaMemcpy(d->d_board_slots.p, slots.data(), slots.size() * sizeof(uint16_t), cudaMemcpyHostToDevice));
     A3_CUDA(cudaMemcpy(d->d_board_pts.p, board->corners, (size_t)m * 32, cudaMemcpyHostToDevice));
-    d->board_n = m;
-    d->board_mode = mode;
-    if (k) d->board_k = *k;
+    d->opt.board_n = m;
+    d->opt.board_mode = mode;
+    if (k) d->opt.board_k = *k;
     return A3_OK;
 }
 
 a3_status a3_solve_board(a3_detector *d, const uint64_t *ids, const float *corners, const uint32_t *frame, uint32_t n, uint32_t n_frames,
                          uint32_t image_w, uint32_t image_h, a3_board_pose *out) {
     if (!d || (n && (!ids || !corners)) || (n_frames && !out)) return fail(A3_ERR_INVALID_ARGUMENT, "a3_solve_board: null argument");
-    if (d->board_n == 0) return fail(A3_ERR_INVALID_ARGUMENT, "a3_solve_board: the detector has no board (a3_detector_set_board)");
+    if (d->opt.board_n == 0) return fail(A3_ERR_INVALID_ARGUMENT, "a3_solve_board: the detector has no board (a3_detector_set_board)");
     if (n_frames == 0) {
         if (n) return fail(A3_ERR_INVALID_ARGUMENT, "a3_solve_board: markers but no frames");
         return A3_OK;
     }
-    if (d->board_mode == A3_POSE_UNDISTORTED && (image_w == 0 || image_h == 0))
+    if (d->opt.board_mode == A3_POSE_UNDISTORTED && (image_w == 0 || image_h == 0))
         return fail(A3_ERR_INVALID_ARGUMENT, "a3_solve_board: undistorted mode needs the frame size");
     std::vector<uint32_t> off((size_t)n_frames + 1, 0);
     for (uint32_t i = 0; i < n; i++) {
@@ -1834,12 +1815,12 @@ a3_status a3_solve_board(a3_detector *d, const uint64_t *ids, const float *corne
     A3_CUDA(cudaMemcpyAsync(d->d_probe_off.p, off.data(), off.size() * 4, cudaMemcpyHostToDevice, s));
     K6Params kp;
     kp.ids = d->d_probe_ids.p; kp.corners_f32 = d->d_refined.p; kp.offsets = d->d_probe_off.p; kp.n_frames = n_frames;
-    kp.slots = d->d_board_slots.p; kp.n_codes = d->dict.n_codes; kp.board = d->d_board_pts.p; kp.n_board = d->board_n;
-    kp.mode = d->board_mode; kp.image_w = image_w; kp.image_h = image_h; kp.k = d->board_k; kp.out = d->d_probe_out.p;
-    if (d->dist_on && n) {  // K7 first, as a3_detect_batch runs it
+    kp.slots = d->d_board_slots.p; kp.n_codes = d->dict.n_codes; kp.board = d->d_board_pts.p; kp.n_board = d->opt.board_n;
+    kp.mode = d->opt.board_mode; kp.image_w = image_w; kp.image_h = image_h; kp.k = d->opt.board_k; kp.out = d->d_probe_out.p;
+    if (d->opt.dist_on && n) {  // K7 first, as a3_detect_batch runs it
         A3_CUDA(d->d_und_out.reserve((size_t)n * 8)); A3_CUDA(d->d_und_ok.reserve(n));
         K7Params up;
-        up.corners_f32 = d->d_refined.p; up.n = n; up.k = d->board_k; up.dist = d->dist; up.out = d->d_und_out.p; up.ok = d->d_und_ok.p;
+        up.corners_f32 = d->d_refined.p; up.n = n; up.k = d->opt.board_k; up.dist = d->opt.dist; up.out = d->d_und_out.p; up.ok = d->d_und_ok.p;
         A3_CUDA(k7_undistort(up, s));
         kp.norm = d->d_und_out.p; kp.norm_ok = d->d_und_ok.p;
     }
@@ -1854,18 +1835,18 @@ a3_status a3_solve_board(a3_detector *d, const uint64_t *ids, const float *corne
 a3_status a3_detector_set_distortion(a3_detector *d, const a3_camera_distortion *dist) {
     if (!d) return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_distortion: null detector");
     if (!dist || (dist->k1 == 0.0f && dist->k2 == 0.0f && dist->p1 == 0.0f && dist->p2 == 0.0f && dist->k3 == 0.0f)) {
-        d->dist_on = false;
-        d->dist = a3_camera_distortion{};
+        d->opt.dist_on = false;
+        d->opt.dist = a3_camera_distortion{};
         return A3_OK;
     }
     if (!isfinite(dist->k1) || !isfinite(dist->k2) || !isfinite(dist->p1) || !isfinite(dist->p2) || !isfinite(dist->k3))
         return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_distortion: non-finite coefficient");
-    if (d->pose_mode == A3_POSE_UNDISTORTED || d->pose_mode == A3_POSE_NORMALIZED)
+    if (d->opt.pose_mode == A3_POSE_UNDISTORTED || d->opt.pose_mode == A3_POSE_NORMALIZED)
         return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_distortion: the pose mode does not use the intrinsics (set INTRINSICS or OFF first)");
-    if (d->board_n && d->board_mode != A3_POSE_INTRINSICS)
+    if (d->opt.board_n && d->opt.board_mode != A3_POSE_INTRINSICS)
         return fail(A3_ERR_INVALID_ARGUMENT, "a3_detector_set_distortion: the board mode does not use the intrinsics (set INTRINSICS first)");
-    d->dist_on = true;
-    d->dist = *dist;
+    d->opt.dist_on = true;
+    d->opt.dist = *dist;
     return A3_OK;
 }
 
