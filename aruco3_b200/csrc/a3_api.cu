@@ -44,42 +44,6 @@ a3_status cuda_fail(cudaError_t e, const char *what) {
 
 namespace {
 
-// Device / pinned buffers that only grow; freed with their owner (the detector's device must be current then).
-template <typename T>
-struct DevBuf {
-    T *p = nullptr;
-    size_t cap = 0;
-    DevBuf() = default;
-    DevBuf(const DevBuf &) = delete;
-    DevBuf &operator=(const DevBuf &) = delete;
-    ~DevBuf() { if (p) cudaFree(p); }
-    cudaError_t reserve(size_t n) {
-        if (n <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr; cap = 0;
-        cudaError_t e = cudaMalloc(&p, n * sizeof(T));
-        if (e == cudaSuccess) cap = n;
-        return e;
-    }
-};
-template <typename T>
-struct PinBuf {
-    T *p = nullptr;
-    size_t cap = 0;
-    PinBuf() = default;
-    PinBuf(const PinBuf &) = delete;
-    PinBuf &operator=(const PinBuf &) = delete;
-    ~PinBuf() { if (p) cudaFreeHost(p); }
-    cudaError_t reserve(size_t n) {
-        if (n <= cap) return cudaSuccess;
-        if (p) cudaFreeHost(p);
-        p = nullptr; cap = 0;
-        cudaError_t e = cudaHostAlloc(&p, n * sizeof(T), cudaHostAllocDefault);
-        if (e == cudaSuccess) cap = n;
-        return e;
-    }
-};
-
 // Persistent host threads.  A job is a function of a frame index; indices [0, ready) may be claimed.
 class WorkerPool {
 public:
@@ -372,10 +336,10 @@ struct a3_detector {
     a3::PinBuf<uint8_t> h_stage_in, h_stage_out;
     // GPU contour stage (K3)
     a3::K3Workspace k3;
-    a3::DevBuf<uint32_t> d_planes, d_k3quads, d_k3counts, d_k3before, d_k3flags, d_k3contours;
-    a3::DevBuf<unsigned long long> d_k3points;
-    a3::PinBuf<uint32_t> h_k3quads, h_k3counts, h_k3before, h_k3flags, h_k3contours, h_plane;
-    a3::PinBuf<unsigned long long> h_k3points;
+    a3::DevBuf<uint32_t> d_planes, d_k3quads;
+    a3::PinBuf<uint32_t> h_k3quads, h_plane;
+    a3::DevBuf<uint8_t> d_k3frames;  // K3's per-frame outputs (K3Frames) outside the one-shot arena, and their host copy
+    a3::PinBuf<uint8_t> h_k3frames;
     size_t planes_zeroed_words = 0;
     uint32_t planes_w = 0, planes_h = 0;
     std::vector<std::vector<uint32_t>> frame_quads;  // per-frame quads of the batch in flight (capacity reused across calls)
@@ -426,6 +390,39 @@ size_t input_span(size_t cn, uint32_t w, uint32_t h, uint32_t bpp, size_t pitch,
 
 double now_ms() {
     return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count();
+}
+
+// K3's per-frame outputs of n frames in one block of bytes(n): counts, before-discard, flags and contours as c-word sections
+// (c = n rounded up to even), then the points (u64) at word 4c.
+struct K3Frames {
+    uint32_t *counts, *before, *flags, *contours;
+    unsigned long long *points;
+    static size_t words(uint32_t n) { return ((size_t)n + 1) & ~(size_t)1; }
+    static size_t bytes(uint32_t n) { return 24 * words(n); }
+    K3Frames(void *base, uint32_t n) {
+        uint32_t *q = static_cast<uint32_t *>(base);
+        const size_t c = words(n);
+        counts = q; before = q + c; flags = q + 2 * c; contours = q + 3 * c; points = reinterpret_cast<unsigned long long *>(q + 4 * c);
+    }
+    void stats(uint32_t i, QuadStats &qs) const {
+        qs.n_contours = contours[i]; qs.n_contour_points = points[i]; qs.n_before_discard = before[i];
+    }
+};
+
+// K3's parameters for frames [f0, f0 + n) of guarded planes, quads and per-frame outputs that start at frame 0
+K3Params k3_params(const a3_config &cfg, const uint32_t *planes, uint32_t w, uint32_t h, uint32_t f0, uint32_t n, uint32_t *quads,
+                   uint32_t quad_cap, const K3Frames &out) {
+    const uint32_t mn = w < h ? w : h;
+    K3Params kp;
+    kp.planes = planes + (size_t)f0 * ((w + 31) / 32 + 2) * (h + 2); kp.n = n; kp.w = w; kp.h = h;
+    kp.eps_factor = cfg.contour_simplification_epsilon;
+    kp.min_edge_length = (uint32_t)((float)mn * cfg.min_side_length_factor);  // src/aruco.rs:55
+    kp.min_corner_separation = (float)mn * cfg.min_corner_separation_factor;   // src/aruco.rs:56
+    kp.min_points = (uint32_t)floor(sqrt(2.0 * (double)kp.min_edge_length));
+    kp.quad_cap = quad_cap; kp.quads = quads + (size_t)f0 * quad_cap * 8;
+    kp.quad_counts = out.counts + f0; kp.before_discard = out.before + f0; kp.frame_flags = out.flags + f0;
+    kp.frame_contours = out.contours + f0; kp.frame_points = out.points + f0;
+    return kp;
 }
 
 // ---- K3 -> K2 on the device -----------------------------------------------------------------------------------------
@@ -942,24 +939,15 @@ a3_status a3_quads_from_masks_device(a3_detector *d, const uint8_t *masks, uint3
     d->planes_zeroed_words = 0;  // the pipeline's guard words are overwritten below
     A3_CUDA(d->d_planes.reserve(planes.size()));
     A3_CUDA(d->d_k3quads.reserve((size_t)n * quad_capacity * 8));
-    A3_CUDA(d->d_k3counts.reserve(n)); A3_CUDA(d->d_k3before.reserve(n)); A3_CUDA(d->d_k3flags.reserve(n));
-    A3_CUDA(d->d_k3contours.reserve(n)); A3_CUDA(d->d_k3points.reserve(n));
+    A3_CUDA(d->d_k3frames.reserve(K3Frames::bytes(n)));
     A3_CUDA(cudaMemcpyAsync(d->d_planes.p, planes.data(), planes.size() * 4, cudaMemcpyHostToDevice, s));
-    const uint32_t mn = w < h ? w : h;
-    K3Params kp;
-    kp.planes = d->d_planes.p; kp.n = n; kp.w = w; kp.h = h;
-    kp.eps_factor = d->cfg.contour_simplification_epsilon;
-    kp.min_edge_length = (uint32_t)((float)mn * d->cfg.min_side_length_factor);
-    kp.min_corner_separation = (float)mn * d->cfg.min_corner_separation_factor;
-    kp.min_points = (uint32_t)floor(sqrt(2.0 * (double)kp.min_edge_length));
-    kp.quad_cap = quad_capacity; kp.quads = d->d_k3quads.p; kp.quad_counts = d->d_k3counts.p; kp.before_discard = d->d_k3before.p;
-    kp.frame_flags = d->d_k3flags.p; kp.frame_contours = d->d_k3contours.p; kp.frame_points = d->d_k3points.p;
-    A3_CUDA(k3_quads(d->k3, kp, s));
+    const K3Frames k3f(d->d_k3frames.p, n);
+    A3_CUDA(k3_quads(d->k3, k3_params(d->cfg, d->d_planes.p, w, h, 0, n, d->d_k3quads.p, quad_capacity, k3f), s));
     A3_CUDA(cudaMemcpyAsync(quads, d->d_k3quads.p, (size_t)n * quad_capacity * 32, cudaMemcpyDeviceToHost, s));
-    A3_CUDA(cudaMemcpyAsync(counts, d->d_k3counts.p, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
-    A3_CUDA(cudaMemcpyAsync(flags, d->d_k3flags.p, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
-    if (contours) A3_CUDA(cudaMemcpyAsync(contours, d->d_k3contours.p, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
-    if (points) A3_CUDA(cudaMemcpyAsync(points, d->d_k3points.p, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
+    A3_CUDA(cudaMemcpyAsync(counts, k3f.counts, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
+    A3_CUDA(cudaMemcpyAsync(flags, k3f.flags, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
+    if (contours) A3_CUDA(cudaMemcpyAsync(contours, k3f.contours, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
+    if (points) A3_CUDA(cudaMemcpyAsync(points, k3f.points, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
     A3_CUDA(cudaStreamSynchronize(s));
     return A3_OK;
 }
@@ -1099,9 +1087,6 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
     const size_t plane_words = (size_t)(wpr + 2) * Hp;       // words per frame
     const uint32_t quad_cap = 1024;                          // quads per frame K3 can return (more -> host stage)
     const uint32_t quad_head = 64;                           // quads per frame copied back unconditionally
-    const uint32_t mn = w < h ? w : h;
-    const uint32_t min_edge_length = (uint32_t)((float)mn * d->cfg.min_side_length_factor);   // src/aruco.rs:55
-    const float min_corner_separation = (float)mn * d->cfg.min_corner_separation_factor;      // src/aruco.rs:56
 
     uint32_t total_markers = 0, total_cands = 0;
     bool overflow = false;
@@ -1122,11 +1107,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 d->planes_zeroed_words = d->d_planes.cap; d->planes_w = w; d->planes_h = h;
             }
             A3_CUDA(d->d_k3quads.reserve((size_t)sn * quad_cap * 8)); A3_CUDA(d->h_k3quads.reserve((size_t)sn * quad_cap * 8));
-            A3_CUDA(d->d_k3counts.reserve(sn)); A3_CUDA(d->h_k3counts.reserve(sn));
-            A3_CUDA(d->d_k3before.reserve(sn)); A3_CUDA(d->h_k3before.reserve(sn));
-            A3_CUDA(d->d_k3flags.reserve(sn)); A3_CUDA(d->h_k3flags.reserve(sn));
-            A3_CUDA(d->d_k3contours.reserve(sn)); A3_CUDA(d->h_k3contours.reserve(sn));
-            A3_CUDA(d->d_k3points.reserve(sn)); A3_CUDA(d->h_k3points.reserve(sn));
+            A3_CUDA(d->d_k3frames.reserve(K3Frames::bytes(sn))); A3_CUDA(d->h_k3frames.reserve(K3Frames::bytes(sn)));
             A3_CUDA(d->h_plane.reserve(plane_words));
         } else {
             A3_CUDA(d->d_bits.reserve(sn * bits_words));
@@ -1154,18 +1135,12 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             for (uint32_t j = 0; j < nfe; j++) stg->in_left[j].store(0);
         }
         uint32_t stage_submitted = 0;  // front-end chunks whose stage-in tasks are in the copy pool
-        // K3's per-frame counters: separate buffers, or (one-shot route) sections of the arena that goes back in one copy
-        uint32_t *ds_counts = d->d_k3counts.p, *ds_before = d->d_k3before.p, *ds_flags = d->d_k3flags.p, *ds_contours = d->d_k3contours.p;
-        unsigned long long *ds_points = d->d_k3points.p;
-        uint32_t *hs_counts = d->h_k3counts.p, *hs_before = d->h_k3before.p, *hs_flags = d->h_k3flags.p, *hs_contours = d->h_k3contours.p;
-        unsigned long long *hs_points = d->h_k3points.p;
         const bool shot = one_shot && s0 == 0 && sn == n;
         const bool shot_hist = shot && d->hist_nq && d->hist_nq_n == n && d->hist_nq_w == w && d->hist_nq_h == h;
         const uint32_t shot_cap = shot_hist ? d->hist_nq + d->hist_nq / 8 + 256 : 0;  // quads the arena holds
-        const size_t shot_c = ((size_t)sn + 1) & ~(size_t)1;
         // markers only (no per-candidate outputs requested): the device also assembles the markers, and the copy stops after them
         const bool lean = shot && markers && !(outs && (outs->candidates || outs->candidate_frame || outs->decodes || outs->homographies));
-        const size_t off_stats = 16, off_markers = (off_stats + 24 * shot_c + 15) & ~(size_t)15;
+        const size_t off_stats = 16, off_markers = align16(off_stats + K3Frames::bytes(sn));
         const size_t off_mposes = off_markers + (lean ? (size_t)shot_cap * sizeof(a3_marker) : 0);
         const size_t off_mcorners = off_mposes + ((lean && want_poses) ? (size_t)shot_cap * 2 * sizeof(a3_pose) : 0);  // K5's, per marker
         const size_t off_out = align16(off_mcorners + ((lean && want_refine) ? (size_t)shot_cap * 32 : 0));  // the decode group's outputs
@@ -1176,13 +1151,11 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
         const size_t shot_copy_bytes = lean ? off_out + shot_out.dec : shot_bytes;
         if (shot) {
             A3_CUDA(d->d_shot.reserve(shot_bytes)); A3_CUDA(d->h_shot.reserve(shot_bytes));
-            auto carve = [&](uint8_t *base, uint32_t *&c, uint32_t *&b, uint32_t *&f, uint32_t *&k, unsigned long long *&pt) {
-                uint32_t *q = reinterpret_cast<uint32_t *>(base + off_stats);
-                c = q; b = q + shot_c; f = q + 2 * shot_c; k = q + 3 * shot_c; pt = reinterpret_cast<unsigned long long *>(q + 4 * shot_c);
-            };
-            carve(d->d_shot.p, ds_counts, ds_before, ds_flags, ds_contours, ds_points);
-            carve(d->h_shot.p, hs_counts, hs_before, hs_flags, hs_contours, hs_points);
         }
+        // K3's per-frame outputs: their own block, or (one-shot route) a section of the arena that goes back in one copy
+        uint8_t *const ds_base = shot ? d->d_shot.p + off_stats : d->d_k3frames.p;
+        uint8_t *const hs_base = shot ? d->h_shot.p + off_stats : d->h_k3frames.p;
+        const K3Frames ds(ds_base, sn), hs(hs_base, sn);
         uint32_t *const d_info = reinterpret_cast<uint32_t *>(d->d_shot.p);
         const uint32_t *const h_info = reinterpret_cast<const uint32_t *>(d->h_shot.p);
         d->events.reset();
@@ -1222,15 +1195,15 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
         bool k3_spec_inflight = false, one_shot_enqueued = false, one_shot_done = false, lean_done = false;
         uint32_t one_shot_cap = 0;
         auto k3_stats_d2h = [&](uint32_t f0, uint32_t kn) -> a3_status {
-            if (shot) {  // the counters are one block of the arena
-                A3_CUDA(cudaMemcpyAsync(d->h_shot.p + off_stats, d->d_shot.p + off_stats, 24 * shot_c, cudaMemcpyDeviceToHost, d->s_pixel));
+            if (kn == sn) {  // K3 covered the whole super-batch (every one-shot call, resident input): the block in one copy
+                A3_CUDA(cudaMemcpyAsync(hs_base, ds_base, K3Frames::bytes(sn), cudaMemcpyDeviceToHost, d->s_pixel));
                 return A3_OK;
             }
-            A3_CUDA(cudaMemcpyAsync(hs_counts + f0, ds_counts + f0, (size_t)kn * 4, cudaMemcpyDeviceToHost, d->s_pixel));
-            A3_CUDA(cudaMemcpyAsync(hs_before + f0, ds_before + f0, (size_t)kn * 4, cudaMemcpyDeviceToHost, d->s_pixel));
-            A3_CUDA(cudaMemcpyAsync(hs_flags + f0, ds_flags + f0, (size_t)kn * 4, cudaMemcpyDeviceToHost, d->s_pixel));
-            A3_CUDA(cudaMemcpyAsync(hs_contours + f0, ds_contours + f0, (size_t)kn * 4, cudaMemcpyDeviceToHost, d->s_pixel));
-            A3_CUDA(cudaMemcpyAsync(hs_points + f0, ds_points + f0, (size_t)kn * 8, cudaMemcpyDeviceToHost, d->s_pixel));
+            A3_CUDA(cudaMemcpyAsync(hs.counts + f0, ds.counts + f0, (size_t)kn * 4, cudaMemcpyDeviceToHost, d->s_pixel));
+            A3_CUDA(cudaMemcpyAsync(hs.before + f0, ds.before + f0, (size_t)kn * 4, cudaMemcpyDeviceToHost, d->s_pixel));
+            A3_CUDA(cudaMemcpyAsync(hs.flags + f0, ds.flags + f0, (size_t)kn * 4, cudaMemcpyDeviceToHost, d->s_pixel));
+            A3_CUDA(cudaMemcpyAsync(hs.contours + f0, ds.contours + f0, (size_t)kn * 4, cudaMemcpyDeviceToHost, d->s_pixel));
+            A3_CUDA(cudaMemcpyAsync(hs.points + f0, ds.points + f0, (size_t)kn * 8, cudaMemcpyDeviceToHost, d->s_pixel));
             return A3_OK;
         };
         auto k3_head_d2h = [&](uint32_t f0, uint32_t kn) -> a3_status {
@@ -1250,7 +1223,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             uint32_t *d_accepted = d->d_qoff.p + sn + 1;
             A3_CUDA(b.d_qframe.reserve(cap));
             if (want_patches) A3_CUDA(b.d_patches.reserve(cap * np));
-            pack_offsets_kernel<<<1, 1024, 0, d->s_pixel>>>(ds_counts, ds_flags, sn, quad_cap, cap, k3_speculation_failed_flag(d->k3), d->d_qoff.p, d_info,
+            pack_offsets_kernel<<<1, 1024, 0, d->s_pixel>>>(ds.counts, ds.flags, sn, quad_cap, cap, k3_speculation_failed_flag(d->k3), d->d_qoff.p, d_info,
                                                             d_accepted, n_chunks);
             A3_CUDA(cudaGetLastError());
             pack_quads_kernel<<<sn, 128, 0, d->s_pixel>>>(d->d_k3quads.p, d->d_qoff.p, quad_cap, cap, d_info, d_quads, b.d_qframe.p, 0u);
@@ -1287,11 +1260,9 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 const uint32_t *h_quads = reinterpret_cast<const uint32_t *>(d->h_shot.p + off_quads);
                 uint32_t k = 0;
                 for (uint32_t i = 0; i < sn; i++) {
-                    const uint32_t m = hs_counts[i] < quad_cap ? hs_counts[i] : quad_cap;
+                    const uint32_t m = hs.counts[i] < quad_cap ? hs.counts[i] : quad_cap;
                     if (!lean) frame_quads[i].assign(h_quads + (size_t)k * 8, h_quads + (size_t)(k + m) * 8);
-                    frame_stats[i].n_contours = hs_contours[i];
-                    frame_stats[i].n_contour_points = hs_points[i];
-                    frame_stats[i].n_before_discard = hs_before[i];
+                    hs.stats(i, frame_stats[i]);
                     k += m;
                 }
                 group_done[0].store(sn);
@@ -1353,14 +1324,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             if (gpu_contours) {
                 if (mem == A3_MEM_HOST || j == 0) {  // K3 over the frames K1 just produced (everything for resident input)
                     const uint32_t kn = mem == A3_MEM_HOST ? cn : sn;
-                    K3Params kp;
-                    kp.planes = d->d_planes.p + (size_t)f0 * plane_words; kp.n = kn; kp.w = w; kp.h = h;
-                    kp.eps_factor = d->cfg.contour_simplification_epsilon; kp.min_edge_length = min_edge_length;
-                    kp.min_corner_separation = min_corner_separation;
-                    kp.min_points = (uint32_t)floor(sqrt(2.0 * (double)min_edge_length));
-                    kp.quad_cap = quad_cap; kp.quads = d->d_k3quads.p + (size_t)f0 * quad_cap * 8; kp.quad_counts = ds_counts + f0;
-                    kp.before_discard = ds_before + f0; kp.frame_flags = ds_flags + f0;
-                    kp.frame_contours = ds_contours + f0; kp.frame_points = ds_points + f0;
+                    const K3Params kp = k3_params(d->cfg, d->d_planes.p, w, h, f0, kn, d->d_k3quads.p, quad_cap, ds);
                     A3_CUDA(k3_begin(d->k3, kp, d->s_pixel));
                     bool spec = false;
                     if (shot) A3_CUDA(k3_finish_speculative(d->k3, kp, d->s_pixel, &spec));
@@ -1475,17 +1439,15 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
         }
         // device-contour mode: take frame i's quads from K3's output, or redo the frame on the host when K3 flagged it
         auto take_k3_frame = [&](uint32_t i) -> a3_status {
-            if (hs_flags[i] == 0) {
-                const uint32_t m = hs_counts[i];
+            if (hs.flags[i] == 0) {
+                const uint32_t m = hs.counts[i];
                 if (m > quad_head) {  // rare (decode-stress scenes): the tail of this frame's quads
                     A3_CUDA(cudaMemcpyAsync(d->h_k3quads.p + ((size_t)i * quad_cap + quad_head) * 8, d->d_k3quads.p + ((size_t)i * quad_cap + quad_head) * 8,
                                             (size_t)(m - quad_head) * 32, cudaMemcpyDeviceToHost, d->s_decode));
                     A3_CUDA(cudaStreamSynchronize(d->s_decode));
                 }
                 frame_quads[i].assign(d->h_k3quads.p + (size_t)i * quad_cap * 8, d->h_k3quads.p + (size_t)i * quad_cap * 8 + (size_t)m * 8);
-                frame_stats[i].n_contours = hs_contours[i];
-                frame_stats[i].n_contour_points = hs_points[i];
-                frame_stats[i].n_before_discard = hs_before[i];
+                hs.stats(i, frame_stats[i]);
             } else {
                 const double t0 = now_ms();
                 A3_CUDA(cudaMemcpyAsync(d->h_plane.p, d->d_planes.p + (size_t)i * plane_words, plane_words * 4, cudaMemcpyDeviceToHost, d->s_decode));
@@ -1529,11 +1491,11 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             // kernels as on the one-shot route) — a small host-to-device copy would queue behind the frame chunks in flight on
             // the copy engine and hold the decode back by whole chunks.  Groups with a frame the host stage redid take the copy.
             bool on_device = gpu_contours;
-            for (uint32_t i = f0; i < f1 && on_device; i++) on_device = hs_flags[i] == 0 && frame_quads[i].size() / 8 == (hs_counts[i] < quad_cap ? hs_counts[i] : quad_cap);
+            for (uint32_t i = f0; i < f1 && on_device; i++) on_device = hs.flags[i] == 0 && frame_quads[i].size() / 8 == (hs.counts[i] < quad_cap ? hs.counts[i] : quad_cap);
             if (on_device) {
                 const uint32_t n_chunks = (nq + 1023) / 1024;
                 A3_CUDA(b.d_info.reserve(4)); A3_CUDA(b.d_qoff.reserve((size_t)gn + 1 + n_chunks));
-                pack_offsets_kernel<<<1, 1024, 0, d->s_decode>>>(ds_counts + f0, ds_flags + f0, gn, quad_cap, nq, nullptr, b.d_qoff.p, b.d_info.p,
+                pack_offsets_kernel<<<1, 1024, 0, d->s_decode>>>(ds.counts + f0, ds.flags + f0, gn, quad_cap, nq, nullptr, b.d_qoff.p, b.d_info.p,
                                                                 b.d_qoff.p + gn + 1, n_chunks);
                 A3_CUDA(cudaGetLastError());
                 pack_quads_kernel<<<gn, 128, 0, d->s_decode>>>(d->d_k3quads.p + (size_t)f0 * quad_cap * 8, b.d_qoff.p, quad_cap, nq, b.d_info.p,

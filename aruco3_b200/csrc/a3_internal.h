@@ -5,6 +5,7 @@
 #include <stddef.h>
 #include <stdint.h>
 
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -34,6 +35,42 @@ a3_status cuda_fail(cudaError_t e, const char *what);
         cudaError_t e__ = (expr);                                        \
         if (e__ != cudaSuccess) return ::a3::cuda_fail(e__, #expr);      \
     } while (0)
+
+// Device / pinned buffers that only grow; freed with their owner (the owner's device must be current then).
+template <typename T>
+struct DevBuf {
+    T *p = nullptr;
+    size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { if (p) cudaFree(p); }
+    cudaError_t reserve(size_t n) {
+        if (n <= cap) return cudaSuccess;
+        if (p) cudaFree(p);
+        p = nullptr; cap = 0;
+        cudaError_t e = cudaMalloc(&p, n * sizeof(T));
+        if (e == cudaSuccess) cap = n;
+        return e;
+    }
+};
+template <typename T>
+struct PinBuf {
+    T *p = nullptr;
+    size_t cap = 0;
+    PinBuf() = default;
+    PinBuf(const PinBuf &) = delete;
+    PinBuf &operator=(const PinBuf &) = delete;
+    ~PinBuf() { if (p) cudaFreeHost(p); }
+    cudaError_t reserve(size_t n) {
+        if (n <= cap) return cudaSuccess;
+        if (p) cudaFreeHost(p);
+        p = nullptr; cap = 0;
+        cudaError_t e = cudaHostAlloc(&p, n * sizeof(T), cudaHostAllocDefault);
+        if (e == cudaSuccess) cap = n;
+        return e;
+    }
+};
 
 // ---- K1: fused into_luma8 + adaptive_threshold (k1_threshold.cu) -------------------------------
 struct K1Params {
@@ -126,11 +163,9 @@ struct K3Params {
 };
 struct K3Workspace {
     struct Impl;
-    Impl *impl;
+    std::unique_ptr<Impl> impl;
     K3Workspace();
     ~K3Workspace();
-    K3Workspace(const K3Workspace &) = delete;
-    K3Workspace &operator=(const K3Workspace &) = delete;
 };
 cudaError_t k3_quads(K3Workspace &ws, const K3Params &p, cudaStream_t stream);  // k3_begin + k3_finish
 // The two halves, so that several batches (each with its own workspace and stream) can be in flight: k3_begin only

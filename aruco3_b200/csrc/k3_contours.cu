@@ -37,6 +37,9 @@
 #include <stdio.h>
 #include <stdlib.h>
 
+#include <algorithm>
+#include <optional>
+
 #include "a3_internal.h"
 
 namespace a3 {
@@ -177,7 +180,15 @@ struct Ckpt { uint32_t walker, pos, xy, state; };
 constexpr uint32_t kCkptBackward = 0x80000000u;
 
 enum { kDead = 0, kSurvivor = 1, kUndecided = 2 };
-constexpr uint32_t kSpecFail = 5;  // index into Lists::counters: the speculative finish gave up (k3_spec_prepare)
+// slots of Lists::counters
+constexpr uint32_t kNumWalkers = 0;    // entries of `walkers`
+constexpr uint32_t kNumLong = 1;       // long borders
+constexpr uint32_t kOverflow = 2;      // non-zero: a list overflowed
+constexpr uint32_t kNumCands = 3;      // entries of `cands`
+constexpr uint32_t kNumCkpts = 4;      // checkpoints
+constexpr uint32_t kSpecFail = 5;      // the speculative finish gave up (k3_spec_prepare)
+constexpr uint32_t kNumRelays = 6;     // relay cracks
+constexpr uint32_t kMaxFrameLong = 7;  // most long borders in one frame
 
 // Work lists shared by the kernels of one k3_quads call.
 struct Lists {
@@ -186,8 +197,7 @@ struct Lists {
     unsigned long long *walkers;       // candidates undecided after kBudget steps: the same key
     unsigned long long *long_keys;     // surviving borders with >= min_points points: the same key ...
     uint32_t *long_n;                  // ... and their number of points
-    uint32_t *counters;                // [0] walkers, [1] long borders, [2] overflow of a list, [3] candidates, [4] checkpoints,
-                                       // [5] speculative finish gave up, [6] relay cracks, [7] most long borders in one frame
+    uint32_t *counters;                // 8 words, slots kNumWalkers ... kMaxFrameLong
     uint32_t *long_slot;               // value array of the sort: the border's slot in long_keys / long_n
     uint32_t *walker_slot;             // per entry of `walkers`: slot of the border it survived as, or 0xffffffff
     Ckpt *ckpts;                       // checkpoints dropped by k3_walkers
@@ -198,13 +208,13 @@ struct Lists {
     unsigned long long *frame_points;  // per frame: their points
     uint32_t *frame_flags;             // per frame: bit 0 barred start (host redo), bit 1 rdp stack overflow, bit 2 quad capacity
     uint32_t *long_off_slot;           // per slot of long_keys: where the border's points go (allocated with one atomic add)
-    // the same long borders listed per frame, frame_cap entries each (0 = not kept): what k3_order ranks; counters[7] = the
+    // the same long borders listed per frame, frame_cap entries each (0 = not kept): what k3_order ranks; counters[kMaxFrameLong] = the
     // largest number of long borders any frame has
     uint32_t frame_cap;
     uint32_t *frame_long_count;
     unsigned long long *frame_keys;
     uint32_t *frame_slots;
-    // relays (tools/relay_proto.py is the spec): the west / east cracks on every (1 << relay_shift)-th row.  counters[6] = how many
+    // relays (tools/relay_proto.py is the spec): the west / east cracks on every (1 << relay_shift)-th row.  counters[kNumRelays] = how many
     uint2 *relays;                     // per relay crack: {x | y << 16, frame << 1 | side (0 west, 1 east)}
     struct Seg *segs;                  // per relay crack: its segment of the border (k3_segments), then its place in it (k3_cycles)
     uint32_t *relay_base;              // per (frame, relay row, word column): index of the word's first relay crack
@@ -316,7 +326,7 @@ __device__ __forceinline__ uint32_t record_survivor(const Lists &l, uint32_t fra
     atomicAdd(&l.frame_points[frame], (unsigned long long)n);
     if (kind == 0 && !first_pixel) atomicOr(&l.frame_flags[frame], 1u);  // a west start below the top of its border: barred natural start
     if (n >= min_points && n >= 4) {
-        const uint32_t slot = atomicAdd(&l.counters[1], 1u);
+        const uint32_t slot = atomicAdd(&l.counters[kNumLong], 1u);
         if (slot < l.long_cap) {
             l.long_keys[slot] = key;
             l.long_n[slot] = relay ? (n | kRelayFlag) : n;
@@ -328,11 +338,11 @@ __device__ __forceinline__ uint32_t record_survivor(const Lists &l, uint32_t fra
                     l.frame_keys[(size_t)frame * l.frame_cap + j] = key;
                     l.frame_slots[(size_t)frame * l.frame_cap + j] = slot;
                 }
-                atomicMax(&l.counters[7], j + 1);
+                atomicMax(&l.counters[kMaxFrameLong], j + 1);
             }
             return slot;
         }
-        atomicOr(&l.counters[2], 1u);
+        atomicOr(&l.counters[kOverflow], 1u);
     }
     return 0xffffffffu;
 }
@@ -385,7 +395,7 @@ __global__ void __launch_bounds__(256) k3_candidates(const Geo g, const StepTabl
                 const uint32_t y = base + (uint32_t)u * stride;
                 if (RELAY && (og[u] | hg[u]) && (y & ((1u << l.relay_shift) - 1u)) == 0u) {
                     const uint32_t cnt = (uint32_t)(__popc(og[u]) + __popc(hg[u]));
-                    uint32_t j = atomicAdd(&l.counters[6], cnt);
+                    uint32_t j = atomicAdd(&l.counters[kNumRelays], cnt);
                     l.relay_base[((size_t)frame * l.nrr + (y >> l.relay_shift)) * g.wpr + k] = j;
                     if (j + cnt <= l.relay_cap) {
                         for (uint32_t pending = og[u] | hg[u]; pending; pending &= pending - 1) {
@@ -394,7 +404,7 @@ __global__ void __launch_bounds__(256) k3_candidates(const Geo g, const StepTabl
                             if ((hg[u] >> bit) & 1u) l.relays[j++] = make_uint2(xy, (frame << 1) | 1u);
                         }
                     } else {
-                        atomicOr(&l.counters[2], 1u);
+                        atomicOr(&l.counters[kOverflow], 1u);
                     }
                 }
             }
@@ -454,7 +464,7 @@ __global__ void __launch_bounds__(256) k3_candidates(const Geo g, const StepTabl
             if (lane >= off) incl += up;
         }
         uint32_t first = 0;
-        if (lane == 31) first = atomicAdd(&l.counters[3], incl);
+        if (lane == 31) first = atomicAdd(&l.counters[kNumCands], incl);
         first = __shfl_sync(0xffffffffu, first, 31);
         uint32_t slot = first + incl - mine;
         if (!mine) continue;
@@ -478,9 +488,9 @@ __global__ void __launch_bounds__(256) k3_candidates(const Geo g, const StepTabl
                         if (r == kSurvivor) {
                             record_survivor(l, frame, key, (int)kind, n, first_pixel, min_points);
                         } else if (r == kUndecided) {
-                            const uint32_t ws = atomicAdd(&l.counters[0], 1u);
+                            const uint32_t ws = atomicAdd(&l.counters[kNumWalkers], 1u);
                             if (ws < l.walkers_cap) l.walkers[ws] = key;
-                            else atomicOr(&l.counters[2], 1u);
+                            else atomicOr(&l.counters[kOverflow], 1u);
                         }
                     }
                     slot++;
@@ -517,7 +527,7 @@ __global__ void __launch_bounds__(128) k3_walk_short(const Geo g, const StepTabl
         (&bwd[0][0])[i] = (&tables->bwd[0][0])[i];
     }
     __syncthreads();
-    const uint32_t total = min(l.counters[3], l.cands_cap);
+    const uint32_t total = min(l.counters[kNumCands], l.cands_cap);
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
         const unsigned long long key = l.cands[i];
         uint32_t frame, n;
@@ -529,9 +539,9 @@ __global__ void __launch_bounds__(128) k3_walk_short(const Geo g, const StepTabl
         if (r == kSurvivor) {
             record_survivor(l, frame, key, kind, n, first_pixel, min_points);
         } else if (r == kUndecided) {
-            const uint32_t slot = atomicAdd(&l.counters[0], 1u);
+            const uint32_t slot = atomicAdd(&l.counters[kNumWalkers], 1u);
             if (slot < l.walkers_cap) l.walkers[slot] = key;
-            else atomicOr(&l.counters[2], 1u);
+            else atomicOr(&l.counters[kOverflow], 1u);
         }
     }
 }
@@ -558,8 +568,8 @@ __global__ void __launch_bounds__(128) k3_segments(const Geo g, const StepTables
     __shared__ uint16_t fwd[8][512];
     for (int i = threadIdx.x; i < 8 * 512; i += blockDim.x) (&fwd[0][0])[i] = (&tables->fwd[0][0])[i];
     __syncthreads();
-    if (l.counters[6] > l.relay_cap) return;  // the list overflowed: every frame of the call goes to the host stage
-    const uint32_t total = l.counters[6], rmask = (1u << l.relay_shift) - 1u;
+    if (l.counters[kNumRelays] > l.relay_cap) return;  // the list overflowed: every frame of the call goes to the host stage
+    const uint32_t total = l.counters[kNumRelays], rmask = (1u << l.relay_shift) - 1u;
     const unsigned char *lut = reinterpret_cast<const unsigned char *>(&fwd[0][0]);
     const int w = (int)g.w, o_max = w + 30;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
@@ -610,8 +620,8 @@ __global__ void __launch_bounds__(128) k3_segments(const Geo g, const StepTables
 // reference bench's noise frame has well over a thousand segments.  So first every relay sums up the `jump_hops` segments after it
 // (all relays at once, jump_hops dependent steps).
 __global__ void __launch_bounds__(256) k3_jumps(const Lists l) {
-    if (l.counters[6] > l.relay_cap) return;
-    const uint32_t total = l.counters[6];
+    if (l.counters[kNumRelays] > l.relay_cap) return;
+    const uint32_t total = l.counters[kNumRelays];
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
         Seg q = l.segs[i];
         if (q.len == 0) continue;
@@ -640,8 +650,8 @@ __global__ void __launch_bounds__(256) k3_jumps(const Lists l) {
 // holds the border's slot and the position of the start visit.  Everything left on the way is merged with an atomic minimum:
 // the leader has the smallest index and passes everything, so its values are what remains.
 __global__ void __launch_bounds__(256) k3_cycles(const Geo g, const uint32_t min_points, const Lists l) {
-    if (l.counters[6] > l.relay_cap) return;
-    const uint32_t total = l.counters[6];
+    if (l.counters[kNumRelays] > l.relay_cap) return;
+    const uint32_t total = l.counters[kNumRelays];
     const size_t words_per_frame = (size_t)g.h * g.wpr;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
         if (l.segs[i].len == 0) continue;
@@ -680,8 +690,8 @@ __global__ void __launch_bounds__(256) k3_cycles(const Geo g, const uint32_t min
 
 // A relay that was jumped from hands (walker, visits so far) on to the jump_hops segments after it.
 __global__ void __launch_bounds__(256) k3_spread(const Lists l) {
-    if (l.counters[6] > l.relay_cap) return;
-    const uint32_t total = l.counters[6];
+    if (l.counters[kNumRelays] > l.relay_cap) return;
+    const uint32_t total = l.counters[kNumRelays];
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
         const unsigned long long a = l.anchor_owner[i];
         if (a == ~0ull) continue;
@@ -714,7 +724,7 @@ __global__ void __launch_bounds__(128) k3_walkers(const Geo g, const StepTables 
         (&bwd[0][0])[i] = (&tables->bwd[0][0])[i];
     }
     __syncthreads();
-    const uint32_t total = min(l.counters[0], l.walkers_cap);
+    const uint32_t total = min(l.counters[kNumWalkers], l.walkers_cap);
     const uint32_t tid = blockIdx.x * blockDim.x + threadIdx.x, back = tid & 1u;
     const uint32_t pair_mask = 3u << (threadIdx.x & 30u);   // the two lanes of this pair: they never diverge from each other
     const unsigned char *lut = reinterpret_cast<const unsigned char *>(back ? &bwd[0][0] : &fwd[0][0]);
@@ -780,9 +790,9 @@ __global__ void __launch_bounds__(128) k3_walkers(const Geo g, const StepTables 
                 // checkpoints for k3_emit: forwards at index kSeg, 2 kSeg, ...; backwards kSeg, 2 kSeg, ... points before the end
                 const uint32_t walked = back ? s0 + k + 1 : s0 + k;
                 if (walked && walked % kSeg == 0) {
-                    const uint32_t c = atomicAdd(&l.counters[4], 1u);
+                    const uint32_t c = atomicAdd(&l.counters[kNumCkpts], 1u);
                     if (c < l.ckpt_cap) l.ckpts[c] = Ckpt{i, walked, (uint32_t)(o - 31) | ((uint32_t)y << 16), fstate | (back ? kCkptBackward : 0u)};
-                    else atomicOr(&l.counters[2], 1u);
+                    else atomicOr(&l.counters[kOverflow], 1u);
                 }
                 const int dx = (int)((e >> 5) & 3u) - 1, dy = (int)((e >> 7) & 3u) - 1;
                 o += dx; y += dy;
@@ -817,10 +827,10 @@ __global__ void __launch_bounds__(128) k3_walkers(const Geo g, const StepTables 
             // the meeting point is where the forward lane stands: one more checkpoint there closes the gap between the last
             // forward and the first backward segment (they may overlap: every segment writes the same values)
             if (n > kSeg) {
-                const uint32_t c = atomicAdd(&l.counters[4], 1u);
+                const uint32_t c = atomicAdd(&l.counters[kNumCkpts], 1u);
                 const uint32_t mp = meet_id >> 3, my = mp / (uint32_t)w, mx = mp - my * (uint32_t)w;
                 if (c < l.ckpt_cap) l.ckpts[c] = Ckpt{i, n / 2, mx | (my << 16), meet_id & 7u};
-                else atomicOr(&l.counters[2], 1u);
+                else atomicOr(&l.counters[kOverflow], 1u);
             }
             slot = record_survivor(l, frame, key, kind, n, min_pix == start_pix, min_points);
         }
@@ -878,17 +888,17 @@ __global__ void __launch_bounds__(256) k3_order(const Lists l, uint32_t n_frames
 }
 
 // Speculative finish (k3_finish_speculative): the second half of the stage is enqueued before the list sizes are known on
-// the host, sized from the previous call.  counters[5] = 1 when the real sizes do not fit (every later kernel of the chain
+// the host, sized from the previous call.  counters[kSpecFail] = 1 when the real sizes do not fit (every later kernel of the chain
 // then returns at once and the host, which sees the same counters after its next synchronisation, redoes the second half
 // exactly); the sort input is padded to its speculated size with keys that sort last.
 __global__ void __launch_bounds__(256) k3_spec_prepare(unsigned long long *long_keys, uint32_t *long_slot, uint32_t *counters,
                                                        const unsigned long long *long_points, uint32_t cap_long, uint32_t cap_ckpts,
                                                        unsigned long long cap_points, uint32_t cap_frame_long, uint32_t cap_relays) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    const uint32_t n_long = counters[1];
+    const uint32_t n_long = counters[kNumLong];
     if (i == 0)
-        counters[kSpecFail] = (counters[2] || n_long > cap_long || counters[4] > cap_ckpts || *long_points > cap_points ||
-                               counters[7] > cap_frame_long || counters[6] > cap_relays) ? 1u : 0u;
+        counters[kSpecFail] = (counters[kOverflow] || n_long > cap_long || counters[kNumCkpts] > cap_ckpts || *long_points > cap_points ||
+                               counters[kMaxFrameLong] > cap_frame_long || counters[kNumRelays] > cap_relays) ? 1u : 0u;
     if (i >= n_long && i < cap_long) {
         long_keys[i] = ~0ull;
         long_slot[i] = 0xffffffffu;
@@ -911,7 +921,7 @@ __global__ void __launch_bounds__(128) k3_emit(const Geo g, const StepTables *ta
     __shared__ uint16_t fwd[8][512];
     if (dyn) {  // speculative finish: the real sizes are on the device only
         if (dyn[kSpecFail]) return;
-        n_contours = dyn[1]; n_ckpts = dyn[4]; n_relays = min(n_relays, dyn[6]);
+        n_contours = dyn[kNumLong]; n_ckpts = dyn[kNumCkpts]; n_relays = min(n_relays, dyn[kNumRelays]);
         if (blockIdx.x * blockDim.x >= n_contours + n_ckpts + n_relays) return;
     }
     for (int i = threadIdx.x; i < 8 * 512; i += blockDim.x) (&fwd[0][0])[i] = (&tables->fwd[0][0])[i];
@@ -1078,7 +1088,7 @@ __global__ void __launch_bounds__(128) k3_rdp(const Contour *contours, const uin
     const uint32_t ci = blockIdx.x * 4 + wid;
     if (dyn) {
         if (dyn[kSpecFail]) return;
-        n_contours = dyn[1];
+        n_contours = dyn[kNumLong];
     }
     if (ci >= n_contours) return;
     const Contour c = contours[ci];
@@ -1221,7 +1231,7 @@ __global__ void __launch_bounds__(32) k3_finalize(const uint32_t *contour_quads,
                                                   uint32_t *frame_flags, uint8_t *dead_scratch, const uint32_t *dyn) {
     if (dyn) {
         if (dyn[kSpecFail]) return;
-        total_contours = dyn[1];
+        total_contours = dyn[kNumLong];
     }
     extern __shared__ uint32_t sq[];  // quad_cap * 8 words of quads, then quad_cap floats of perimeters, then quad_cap dead bytes
     float *sper = reinterpret_cast<float *>(sq + (size_t)quad_cap * 8);
@@ -1325,60 +1335,50 @@ __global__ void __launch_bounds__(32) k3_finalize(const uint32_t *contour_quads,
 
 }  // namespace
 
+namespace {
+// List sizes of one call, as k3_begin's counters report them.  The same struct carries the sizes a second half is enqueued
+// with: the real ones (k3_finish) or capacities (k3_finish_speculative); frame_long above the per-frame lists' capacity
+// orders the borders with the radix sort.
+struct ListSizes {
+    uint32_t n_long = 0, ckpts = 0, relays = 0, frame_long = 0;
+    unsigned long long points = 0;
+    bool overflow = false;  // a list overflowed: every frame of the call is flagged for the host stage
+    // the test k3_spec_prepare makes on the device
+    bool fits(const ListSizes &cap) const {
+        return !overflow && n_long <= cap.n_long && ckpts <= cap.ckpts && points <= cap.points && frame_long <= cap.frame_long &&
+               relays <= cap.relays;
+    }
+};
+}  // namespace
+
 struct K3Workspace::Impl {
-    StepTables *d_tables = nullptr;
+    DevBuf<StepTables> tables;
     // work lists
-    unsigned long long *cands = nullptr, *walkers = nullptr, *long_keys = nullptr, *long_keys_sorted = nullptr, *long_points = nullptr, *frame_points = nullptr;
-    uint32_t *long_n = nullptr, *long_n_sorted = nullptr, *long_off = nullptr, *counters = nullptr, *frame_contours = nullptr;
-    uint32_t *long_slot = nullptr, *long_slot_sorted = nullptr, *long_rank = nullptr, *walker_slot = nullptr;
-    uint32_t *long_off_slot = nullptr, *frame_long_count = nullptr, *frame_slots = nullptr;
-    unsigned long long *frame_keys = nullptr;
-    size_t frame_lists_cap = 0;              // frames the per-frame lists are allocated for
-    Ckpt *ckpts = nullptr;
-    uint2 *relays = nullptr;
-    Seg *segs = nullptr;
-    unsigned long long *seg_owner = nullptr, *anchor_owner = nullptr;
-    Jump *jumps = nullptr;
-    uint32_t *relay_base = nullptr;
-    size_t relay_cap = 0, relay_base_cap = 0;
-    uint32_t hist_relays = 0, spec_relays = 0;
-    size_t cands_cap = 0, walkers_cap = 0, long_cap = 0, frames_cap = 0, ckpt_cap = 0;
-    void *cub_tmp = nullptr;
-    size_t cub_bytes = 0;
-    Contour *contours = nullptr;
-    uint32_t *contour_quads = nullptr;
-    size_t contours_cap = 0;
-    uint32_t *points = nullptr;
-    size_t points_cap = 0;
-    uint8_t *dead = nullptr;
-    size_t dead_cap = 0;
-    unsigned long long *h_counts = nullptr;  // pinned: [0..3] the eight 32-bit counters, [4] long_points
-    Geo g;                                   // state handed from k3_begin to k3_finish
+    DevBuf<unsigned long long> cands, walkers, long_keys, long_keys_sorted, long_points, frame_points, frame_keys, seg_owner, anchor_owner;
+    DevBuf<uint32_t> counters, walker_slot, long_n, long_n_sorted, long_off, long_slot, long_slot_sorted, long_rank, long_off_slot;
+    DevBuf<uint32_t> frame_contours, frame_long_count, frame_slots, relay_base;
+    DevBuf<Ckpt> ckpts;
+    DevBuf<uint2> relays;
+    DevBuf<Seg> segs;
+    DevBuf<Jump> jumps;
+    DevBuf<uint8_t> cub_tmp;
+    DevBuf<Contour> contours;
+    DevBuf<uint32_t> contour_quads, points;
+    DevBuf<uint8_t> dead;
+    PinBuf<unsigned long long> h_counts;  // [0..3] the eight 32-bit counters, [4] long_points
+    Geo g;                                // state handed from k3_begin to the second half
     Lists l;
-    int sms = 148;
-    // list sizes of the previous call with this geometry: what k3_finish_speculative sizes its launches from
-    bool hist_valid = false;
-    uint32_t hist_n = 0, hist_w = 0, hist_h = 0, hist_long = 0, hist_ckpts = 0;
-    unsigned long long hist_points = 0;
-    // capacities the speculative finish in flight was enqueued with (0 = none in flight)
-    uint32_t spec_long = 0, spec_ckpts = 0, spec_frame_long = 0;
-    unsigned long long spec_points = 0;
-    uint32_t hist_frame_long = 0;            // most long borders in one frame, previous call
+    // the previous call with this geometry: what k3_finish_speculative sizes its launches from
+    struct History {
+        uint32_t n = 0, w = 0, h = 0;
+        ListSizes sizes;
+        bool valid = false;
+    } hist;
+    std::optional<ListSizes> spec;        // capacities of the speculative finish in flight
 };
 
 K3Workspace::K3Workspace() : impl(new Impl()) {}
-K3Workspace::~K3Workspace() {
-    if (!impl) return;
-    for (void *p : {(void *)impl->d_tables, (void *)impl->cands, (void *)impl->walkers, (void *)impl->long_keys, (void *)impl->long_keys_sorted, (void *)impl->long_points,
-                    (void *)impl->frame_points, (void *)impl->long_n, (void *)impl->long_n_sorted, (void *)impl->long_off, (void *)impl->counters,
-                    (void *)impl->frame_contours, impl->cub_tmp, (void *)impl->contours, (void *)impl->contour_quads, (void *)impl->points,
-                    (void *)impl->dead, (void *)impl->long_slot, (void *)impl->long_slot_sorted, (void *)impl->long_rank, (void *)impl->walker_slot,
-                    (void *)impl->ckpts, (void *)impl->long_off_slot, (void *)impl->frame_long_count, (void *)impl->frame_slots, (void *)impl->frame_keys,
-                    (void *)impl->relays, (void *)impl->segs, (void *)impl->relay_base, (void *)impl->seg_owner, (void *)impl->anchor_owner, (void *)impl->jumps})
-        if (p) cudaFree(p);
-    if (impl->h_counts) cudaFreeHost(impl->h_counts);
-    delete impl;
-}
+K3Workspace::~K3Workspace() = default;
 
 #define K3_CUDA(expr)                              \
     do {                                           \
@@ -1386,26 +1386,9 @@ K3Workspace::~K3Workspace() {
         if (e__ != cudaSuccess) return e__;        \
     } while (0)
 
-template <typename T>
-static cudaError_t grow(T *&p, size_t &cap, size_t need) {
-    if (need <= cap) return cudaSuccess;
-    if (p) cudaFree(p);
-    p = nullptr; cap = 0;
-    const size_t want = need + need / 4 + 1024;
-    cudaError_t e = cudaMalloc(&p, want * sizeof(T));
-    if (e == cudaSuccess) cap = want;
-    return e;
-}
-template <typename T>
-static cudaError_t alloc_exact(T *&p, size_t n) {
-    if (p) cudaFree(p);
-    p = nullptr;
-    return cudaMalloc(&p, n * sizeof(T));
-}
-
 static __global__ void k3_flag_all(uint32_t *frame_flags, uint32_t n, const uint32_t *counters, int force) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n && (force || counters[2])) frame_flags[i] |= 8u;  // a work list overflowed: every frame of this call goes to the host stage
+    if (i < n && (force || counters[kOverflow])) frame_flags[i] |= 8u;  // a work list overflowed: every frame of this call goes to the host stage
 }
 
 // A3_K3_TIMING=1 in the environment: print the device time of every phase of a k3_quads call (debug aid)
@@ -1434,13 +1417,6 @@ struct PhaseTimer {
     }
 };
 
-// k3_emit's step: the register window when many segments are in flight (256 x 1080p: 0.094 ms against 0.115 ms), the walkers'
-// lighter step for calls of a few frames, where the chain of one segment is what is waited for (noise frame: 0.025 against 0.040 ms)
-static bool emit_light(uint32_t n_frames) {
-    static const char *v = getenv("A3_K3_EMIT_LIGHT");  // experiment switch: 0 / 1 forces the variant
-    return v ? v[0] == '1' : n_frames <= 4;
-}
-
 cudaError_t k3_quads(K3Workspace &ws, const K3Params &p, cudaStream_t stream) {
     cudaError_t e = k3_begin(ws, p, stream);
     return e == cudaSuccess ? k3_finish(ws, p, stream) : e;
@@ -1456,17 +1432,16 @@ cudaError_t k3_begin(K3Workspace &ws, const K3Params &p, cudaStream_t stream) {
     Geo g;
     g.planes = p.planes; g.n = p.n; g.w = p.w; g.h = p.h; g.wpr = (p.w + 31) / 32; g.Hp = p.h + 2;
     g.frame_words = (size_t)(g.wpr + 2) * g.Hp;
-    const size_t words_per_frame = (size_t)g.h * g.wpr, nwords = words_per_frame * p.n;
-    if (!w.d_tables) {
+    if (!w.tables.p) {
         StepTables *t = new StepTables();
         build_tables(*t);
-        cudaError_t e = cudaMalloc(&w.d_tables, sizeof(StepTables));
-        if (e == cudaSuccess) e = cudaMemcpy(w.d_tables, t, sizeof(StepTables), cudaMemcpyHostToDevice);
+        cudaError_t e = w.tables.reserve(1);
+        if (e == cudaSuccess) e = cudaMemcpy(w.tables.p, t, sizeof(StepTables), cudaMemcpyHostToDevice);
         delete t;
         K3_CUDA(e);
-        K3_CUDA(cudaHostAlloc(&w.h_counts, 64, cudaHostAllocDefault));
-        K3_CUDA(cudaMalloc(&w.counters, 32));
-        K3_CUDA(cudaMalloc(&w.long_points, 8));
+        K3_CUDA(w.h_counts.reserve(8));
+        K3_CUDA(w.counters.reserve(8));
+        K3_CUDA(w.long_points.reserve(1));
     }
     // list capacities: generous per frame; an overflow sends the whole call to the host stage (flag 8), never a wrong answer
     const size_t pixels = (size_t)p.w * p.h;
@@ -1480,53 +1455,31 @@ cudaError_t k3_begin(K3Workspace &ws, const K3Params &p, cudaStream_t stream) {
         const size_t alt = roomy < cap ? roomy : cap;
         if (alt > want_cands) want_cands = alt;
     }
-    if (want_cands > w.cands_cap) {
-        K3_CUDA(alloc_exact(w.cands, want_cands));
-        w.cands_cap = want_cands;
-    }
-    if (want_walkers > w.walkers_cap) {
-        K3_CUDA(alloc_exact(w.walkers, want_walkers));
-        K3_CUDA(alloc_exact(w.walker_slot, want_walkers));
-        w.walkers_cap = want_walkers;
-    }
+    K3_CUDA(w.cands.reserve(want_cands));
+    K3_CUDA(w.walkers.reserve(want_walkers));
+    K3_CUDA(w.walker_slot.reserve(want_walkers));
     const size_t want_ckpts = (size_t)p.n * (pixels / kSeg + 4096);  // one per kSeg walked points; an overflow flags the call (host stage)
-    if (want_ckpts > w.ckpt_cap) {
-        K3_CUDA(alloc_exact(w.ckpts, want_ckpts));
-        w.ckpt_cap = want_ckpts;
-    }
-    if (want_long > w.long_cap) {
-        K3_CUDA(alloc_exact(w.long_keys, want_long)); K3_CUDA(alloc_exact(w.long_keys_sorted, want_long));
-        K3_CUDA(alloc_exact(w.long_n, want_long)); K3_CUDA(alloc_exact(w.long_n_sorted, want_long)); K3_CUDA(alloc_exact(w.long_off, want_long));
-        K3_CUDA(alloc_exact(w.long_slot, want_long)); K3_CUDA(alloc_exact(w.long_slot_sorted, want_long)); K3_CUDA(alloc_exact(w.long_rank, want_long));
-        K3_CUDA(alloc_exact(w.long_off_slot, want_long));
-        w.long_cap = want_long;
+    K3_CUDA(w.ckpts.reserve(want_ckpts));
+    if (want_long > w.long_keys.cap) {
+        for (DevBuf<uint32_t> *b : {&w.long_n, &w.long_n_sorted, &w.long_off, &w.long_slot, &w.long_slot_sorted, &w.long_rank, &w.long_off_slot})
+            K3_CUDA(b->reserve(want_long));
+        K3_CUDA(w.long_keys_sorted.reserve(want_long));
         size_t need = 0;
-        K3_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, need, w.long_keys, w.long_keys_sorted, w.long_slot, w.long_slot_sorted, (int)want_long, 0, 64, stream));
-        if (need > w.cub_bytes) {
-            if (w.cub_tmp) cudaFree(w.cub_tmp);
-            w.cub_tmp = nullptr; w.cub_bytes = 0;
-            K3_CUDA(cudaMalloc(&w.cub_tmp, need));
-            w.cub_bytes = need;
-        }
+        K3_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, need, w.long_keys.p, w.long_keys_sorted.p, w.long_slot.p, w.long_slot_sorted.p, (int)want_long, 0, 64, stream));
+        K3_CUDA(w.cub_tmp.reserve(need));
+        K3_CUDA(w.long_keys.reserve(want_long));  // last: its capacity says that the other lists and the sort's storage have grown
     }
-    if (p.n > w.frames_cap) {
-        K3_CUDA(alloc_exact(w.frame_points, (size_t)p.n));
-        K3_CUDA(alloc_exact(w.frame_contours, (size_t)p.n));
-        K3_CUDA(alloc_exact(w.frame_long_count, (size_t)p.n));
-        w.frames_cap = p.n;
-    }
+    K3_CUDA(w.frame_points.reserve(p.n));
+    K3_CUDA(w.frame_contours.reserve(p.n));
+    K3_CUDA(w.frame_long_count.reserve(p.n));
     // per-frame lists of the long borders for k3_order: kOrderCap entries per frame, for calls of up to 4096 frames (48 MB of
     // lists; every CTA of k3_order also sums the counts of the frames before its own, which is quadratic in the frame count)
-    const bool frame_lists = p.n <= 4096 && !getenv("A3_K3_RADIX_SORT");
-    if (frame_lists && p.n > w.frame_lists_cap) {
-        K3_CUDA(alloc_exact(w.frame_keys, (size_t)p.n * kOrderCap));
-        K3_CUDA(alloc_exact(w.frame_slots, (size_t)p.n * kOrderCap));
-        w.frame_lists_cap = p.n;
+    const bool frame_lists = p.n <= 4096;
+    if (frame_lists) {
+        K3_CUDA(w.frame_keys.reserve((size_t)p.n * kOrderCap));
+        K3_CUDA(w.frame_slots.reserve((size_t)p.n * kOrderCap));
     }
-    if ((size_t)p.n * p.quad_cap > w.dead_cap) {
-        K3_CUDA(alloc_exact(w.dead, (size_t)p.n * p.quad_cap));
-        w.dead_cap = (size_t)p.n * p.quad_cap;
-    }
+    K3_CUDA(w.dead.reserve((size_t)p.n * p.quad_cap));
     // relays: the candidate cracks of every 16th row (32nd above 1200 rows).  A pure-noise frame has about w / 2 of them per
     // row; the lists are sized for that, capped at 48 M entries (an overflow sends the call to the host stage like any other list).
     // Relay walks are for calls of up to 16 frames (one front-end chunk of host input), where the time of the stage is the chain of the longest border (the reference
@@ -1544,40 +1497,33 @@ cudaError_t k3_begin(K3Workspace &ws, const K3Params &p, cudaStream_t stream) {
         const size_t c = strtoull(cap_env, nullptr, 10);
         if (want_relays > c) want_relays = c ? c : 1;
     }
-    if (want_relays > w.relay_cap) {
-        K3_CUDA(alloc_exact(w.relays, want_relays));
-        K3_CUDA(alloc_exact(w.segs, want_relays));
-        K3_CUDA(alloc_exact(w.seg_owner, want_relays));
-        K3_CUDA(alloc_exact(w.anchor_owner, want_relays));
-        K3_CUDA(alloc_exact(w.jumps, want_relays));
-        w.relay_cap = want_relays;
-    }
-    const size_t want_base = relays_off ? 0 : (size_t)p.n * nrr * ((p.w + 31) / 32);
-    if (want_base > w.relay_base_cap) {
-        K3_CUDA(alloc_exact(w.relay_base, want_base));
-        w.relay_base_cap = want_base;
-    }
-    K3_CUDA(cudaMemsetAsync(w.frame_points, 0, (size_t)p.n * 8, stream));
-    K3_CUDA(cudaMemsetAsync(w.frame_contours, 0, (size_t)p.n * 4, stream));
-    K3_CUDA(cudaMemsetAsync(w.frame_long_count, 0, (size_t)p.n * 4, stream));
+    K3_CUDA(w.relays.reserve(want_relays));
+    K3_CUDA(w.segs.reserve(want_relays));
+    K3_CUDA(w.seg_owner.reserve(want_relays));
+    K3_CUDA(w.anchor_owner.reserve(want_relays));
+    K3_CUDA(w.jumps.reserve(want_relays));
+    K3_CUDA(w.relay_base.reserve(relays_off ? 0 : (size_t)p.n * nrr * ((p.w + 31) / 32)));
+    K3_CUDA(cudaMemsetAsync(w.frame_points.p, 0, (size_t)p.n * 8, stream));
+    K3_CUDA(cudaMemsetAsync(w.frame_contours.p, 0, (size_t)p.n * 4, stream));
+    K3_CUDA(cudaMemsetAsync(w.frame_long_count.p, 0, (size_t)p.n * 4, stream));
     K3_CUDA(cudaMemsetAsync(p.frame_flags, 0, (size_t)p.n * 4, stream));
-    K3_CUDA(cudaMemsetAsync(w.counters, 0, 32, stream));
-    K3_CUDA(cudaMemsetAsync(w.long_points, 0, 8, stream));
+    K3_CUDA(cudaMemsetAsync(w.counters.p, 0, 32, stream));
+    K3_CUDA(cudaMemsetAsync(w.long_points.p, 0, 8, stream));
 
     timer.mark("begin");
     Lists l;
-    l.cands = w.cands; l.cands_cap = (uint32_t)(w.cands_cap > 0xffffffffull ? 0xffffffffull : w.cands_cap);
-    l.walkers = w.walkers; l.long_keys = w.long_keys; l.long_n = w.long_n; l.counters = w.counters; l.long_points = w.long_points;
-    l.walkers_cap = (uint32_t)(w.walkers_cap > 0xffffffffull ? 0xffffffffull : w.walkers_cap);
-    l.long_cap = (uint32_t)(w.long_cap > 0x7fffffffull ? 0x7fffffffull : w.long_cap);
-    l.frame_contours = w.frame_contours; l.frame_points = w.frame_points; l.frame_flags = p.frame_flags;
-    l.long_slot = w.long_slot; l.walker_slot = w.walker_slot; l.ckpts = w.ckpts;
-    l.long_off_slot = w.long_off_slot; l.frame_cap = frame_lists ? kOrderCap : 0u; l.frame_long_count = w.frame_long_count;
-    l.frame_keys = w.frame_keys; l.frame_slots = w.frame_slots;
-    l.ckpt_cap = (uint32_t)(w.ckpt_cap > 0x7fffffffull ? 0x7fffffffull : w.ckpt_cap);
-    l.relays = w.relays; l.segs = w.segs; l.seg_owner = w.seg_owner; l.relay_base = w.relay_base; l.relay_cap = (uint32_t)want_relays;
+    l.cands = w.cands.p; l.cands_cap = (uint32_t)(w.cands.cap > 0xffffffffull ? 0xffffffffull : w.cands.cap);
+    l.walkers = w.walkers.p; l.long_keys = w.long_keys.p; l.long_n = w.long_n.p; l.counters = w.counters.p; l.long_points = w.long_points.p;
+    l.walkers_cap = (uint32_t)(w.walkers.cap > 0xffffffffull ? 0xffffffffull : w.walkers.cap);
+    l.long_cap = (uint32_t)(w.long_keys.cap > 0x7fffffffull ? 0x7fffffffull : w.long_keys.cap);
+    l.frame_contours = w.frame_contours.p; l.frame_points = w.frame_points.p; l.frame_flags = p.frame_flags;
+    l.long_slot = w.long_slot.p; l.walker_slot = w.walker_slot.p; l.ckpts = w.ckpts.p;
+    l.long_off_slot = w.long_off_slot.p; l.frame_cap = frame_lists ? kOrderCap : 0u; l.frame_long_count = w.frame_long_count.p;
+    l.frame_keys = w.frame_keys.p; l.frame_slots = w.frame_slots.p;
+    l.ckpt_cap = (uint32_t)(w.ckpts.cap > 0x7fffffffull ? 0x7fffffffull : w.ckpts.cap);
+    l.relays = w.relays.p; l.segs = w.segs.p; l.seg_owner = w.seg_owner.p; l.relay_base = w.relay_base.p; l.relay_cap = (uint32_t)want_relays;
     l.relay_shift = relay_shift; l.nrr = nrr;
-    l.jumps = w.jumps; l.anchor_owner = w.anchor_owner;
+    l.jumps = w.jumps.p; l.anchor_owner = w.anchor_owner.p;
     {
         const char *jump_env = getenv("A3_K3_JUMP");  // test hook: short jumps exercise the multi-jump paths on small masks
         const unsigned long jh = jump_env ? strtoul(jump_env, nullptr, 10) : 32ul;
@@ -1586,6 +1532,7 @@ cudaError_t k3_begin(K3Workspace &ws, const K3Params &p, cudaStream_t stream) {
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const StepTables *tables = w.tables.p;
     {
         // about 8 blocks of 256 threads per SM (measured best: more, smaller shares than one resident wave), split over the frames
         // (blockIdx.x strides over the word columns of a frame, blockIdx.y over frames)
@@ -1608,13 +1555,13 @@ cudaError_t k3_begin(K3Workspace &ws, const K3Params &p, cudaStream_t stream) {
             if (gz > room) gz = room;
             if (gz < 1) gz = 1;
         }
-        if (l.relay_cap) k3_candidates<true><<<dim3(gx, gy, gz), bd, 0, stream>>>(g, w.d_tables, p.min_points, l);
-        else k3_candidates<false><<<dim3(gx, gy, gz), bd, 0, stream>>>(g, w.d_tables, p.min_points, l);
+        if (l.relay_cap) k3_candidates<true><<<dim3(gx, gy, gz), bd, 0, stream>>>(g, tables, p.min_points, l);
+        else k3_candidates<false><<<dim3(gx, gy, gz), bd, 0, stream>>>(g, tables, p.min_points, l);
     }
     K3_CUDA(cudaGetLastError());
     timer.mark("candidates");
     if (l.relay_cap) {
-        k3_segments<<<(uint32_t)sms * 8, 128, 0, stream>>>(g, w.d_tables, l);
+        k3_segments<<<(uint32_t)sms * 8, 128, 0, stream>>>(g, tables, l);
         K3_CUDA(cudaGetLastError());
         timer.mark("segments");
         k3_jumps<<<(uint32_t)sms * 4, 256, 0, stream>>>(l);
@@ -1623,175 +1570,161 @@ cudaError_t k3_begin(K3Workspace &ws, const K3Params &p, cudaStream_t stream) {
         K3_CUDA(cudaGetLastError());
         timer.mark("cycles");
     }
-    if (l.relay_cap) k3_walk_short<true><<<(uint32_t)sms * 8, 128, 0, stream>>>(g, w.d_tables, p.min_points, l);
-    else k3_walk_short<false><<<(uint32_t)sms * 8, 128, 0, stream>>>(g, w.d_tables, p.min_points, l);
+    if (l.relay_cap) k3_walk_short<true><<<(uint32_t)sms * 8, 128, 0, stream>>>(g, tables, p.min_points, l);
+    else k3_walk_short<false><<<(uint32_t)sms * 8, 128, 0, stream>>>(g, tables, p.min_points, l);
     K3_CUDA(cudaGetLastError());
     timer.mark("walk_short");
     // blocks of 2 / 4 / 6 / 8 steps measured: 0.207 / 0.188 / 0.186 / 0.184 ms (before the lighter step: 0.152 ms with 8)
-    if (l.relay_cap) k3_walkers<8, true><<<(uint32_t)sms * 8, 128, 0, stream>>>(g, w.d_tables, p.min_points, l);
-    else k3_walkers<8, false><<<(uint32_t)sms * 8, 128, 0, stream>>>(g, w.d_tables, p.min_points, l);
+    if (l.relay_cap) k3_walkers<8, true><<<(uint32_t)sms * 8, 128, 0, stream>>>(g, tables, p.min_points, l);
+    else k3_walkers<8, false><<<(uint32_t)sms * 8, 128, 0, stream>>>(g, tables, p.min_points, l);
     K3_CUDA(cudaGetLastError());
     timer.mark("walkers");
-    k3_flag_all<<<(p.n + 127) / 128, 128, 0, stream>>>(p.frame_flags, p.n, w.counters, 0);
+    k3_flag_all<<<(p.n + 127) / 128, 128, 0, stream>>>(p.frame_flags, p.n, w.counters.p, 0);
     K3_CUDA(cudaGetLastError());
-    K3_CUDA(cudaMemcpyAsync(&w.h_counts[0], w.counters, 32, cudaMemcpyDeviceToHost, stream));
-    K3_CUDA(cudaMemcpyAsync(&w.h_counts[4], w.long_points, 8, cudaMemcpyDeviceToHost, stream));
-    w.g = g; w.l = l; w.sms = sms;
+    K3_CUDA(cudaMemcpyAsync(&w.h_counts.p[0], w.counters.p, 32, cudaMemcpyDeviceToHost, stream));
+    K3_CUDA(cudaMemcpyAsync(&w.h_counts.p[4], w.long_points.p, 8, cudaMemcpyDeviceToHost, stream));
+    w.g = g; w.l = l;
     return cudaSuccess;
 }
 
-// Second half: waits for the counters (the only host synchronisation of the stage), then sort, emission, polygon
-// simplification and the per-frame filters.
-cudaError_t k3_finish(K3Workspace &ws, const K3Params &p, cudaStream_t stream) {
-    K3Workspace::Impl &w = *ws.impl;
-    if (p.n == 0) return cudaSuccess;
+// k3_begin's list sizes, from the pinned copy of the counters (once the stream has been synchronised)
+static ListSizes read_sizes(const K3Workspace::Impl &w) {
+    const uint32_t *c = reinterpret_cast<const uint32_t *>(w.h_counts.p);
+    ListSizes s;
+    s.n_long = c[kNumLong]; s.ckpts = c[kNumCkpts]; s.relays = c[kNumRelays]; s.frame_long = c[kMaxFrameLong];
+    s.points = w.h_counts.p[4];
+    s.overflow = c[kOverflow] != 0;
+    return s;
+}
+
+// the sizes of this call, for the speculative finish of the next call with the same geometry
+static void record_history(K3Workspace::Impl &w, const K3Params &p, const ListSizes &s) {
+    w.hist = {p.n, p.w, p.h, s, !s.overflow && s.points < 0xffffffffull};
+}
+
+// The second half: sort, emission, polygon simplification and the per-frame filters, launched for the sizes `s`.  k3_finish
+// passes the real sizes; k3_finish_speculative passes capacities and dyn = counters, where every kernel reads the real sizes
+// and where k3_spec_prepare stops the chain when they do not fit.
+static cudaError_t enqueue_finish(K3Workspace::Impl &w, const K3Params &p, const ListSizes &s, const uint32_t *dyn, cudaStream_t stream) {
+    const size_t fin_smem = (size_t)p.quad_cap * (32 + 4 + 1) + 16;
+    if (fin_smem > 200 * 1024) return cudaErrorInvalidValue;
+    const Geo &g = w.g;
+    const Lists &l = w.l;
+    const size_t words_per_frame = (size_t)g.h * g.wpr, nwords = words_per_frame * p.n;
     PhaseTimer timer(stream);
     timer.mark("begin");
-    const Geo g = w.g;
-    const Lists l = w.l;
-    const size_t words_per_frame = (size_t)g.h * g.wpr, nwords = words_per_frame * p.n;
-    K3_CUDA(cudaStreamSynchronize(stream));
-    timer.mark("sync");
-    const uint32_t *hc = reinterpret_cast<const uint32_t *>(&w.h_counts[0]);
-    uint32_t n_long = hc[1] < l.long_cap ? hc[1] : l.long_cap;
-    const unsigned long long n_points = w.h_counts[4];
-    const uint32_t n_ckpts = hc[4] < l.ckpt_cap ? hc[4] : l.ckpt_cap;
-    if (timer.on) fprintf(stderr, "k3 lists: %u candidates, %u walkers, %u long borders, %llu points, %u checkpoints, %u relay cracks\n", hc[3], hc[0], hc[1], n_points, hc[4], hc[6]);
-    w.hist_valid = !hc[2] && n_points < 0xffffffffull;
-    w.hist_n = p.n; w.hist_w = p.w; w.hist_h = p.h; w.hist_long = hc[1]; w.hist_ckpts = hc[4]; w.hist_points = n_points;
-    w.hist_frame_long = hc[7];
-    w.hist_relays = hc[6];
-    w.spec_long = 0;
-    const uint32_t n_relays = hc[6] < l.relay_cap ? hc[6] : l.relay_cap;
-    if (n_points >= 0xffffffffull && !hc[2]) {  // point offsets are 32-bit: hand the whole call to the host stage
-        k3_flag_all<<<(p.n + 127) / 128, 128, 0, stream>>>(p.frame_flags, p.n, w.counters, 1);
-        K3_CUDA(cudaGetLastError());
-    }
-    if (hc[2] || n_points >= 0xffffffffull) n_long = 0;  // overflow: every frame is flagged for the host stage
-    if (n_long) {
-        if ((size_t)n_long > w.contours_cap) {
-            K3_CUDA(alloc_exact(w.contours, (size_t)n_long + n_long / 4 + 1024));
-            K3_CUDA(alloc_exact(w.contour_quads, ((size_t)n_long + n_long / 4 + 1024) * 8));
-            w.contours_cap = (size_t)n_long + n_long / 4 + 1024;
+    if (s.n_long) {  // (speculative capacities are never 0)
+        if (s.n_long > w.contours.cap) {
+            const size_t c = (size_t)s.n_long + s.n_long / 4 + 1024;
+            K3_CUDA(w.contours.reserve(c));
+            K3_CUDA(w.contour_quads.reserve(c * 8));
         }
-        K3_CUDA(grow(w.points, w.points_cap, (size_t)n_points + 1));
-        if (l.frame_cap && hc[7] <= l.frame_cap) {
-            k3_order<<<p.n, 256, 0, stream>>>(l, p.n, w.long_keys_sorted, w.long_n_sorted, w.long_off, w.long_rank, nullptr);
+        const size_t need = (size_t)s.points + 1;
+        if (need > w.points.cap) K3_CUDA(w.points.reserve(need + need / 4 + 1024));
+        if (dyn) {
+            k3_spec_prepare<<<(s.n_long + 255) / 256, 256, 0, stream>>>(w.long_keys.p, w.long_slot.p, w.counters.p, w.long_points.p, s.n_long,
+                                                                        s.ckpts, s.points, s.frame_long, s.relays);
+            K3_CUDA(cudaGetLastError());
+        }
+        if (l.frame_cap && s.frame_long <= l.frame_cap) {
+            k3_order<<<p.n, 256, 0, stream>>>(l, p.n, w.long_keys_sorted.p, w.long_n_sorted.p, w.long_off.p, w.long_rank.p, dyn);
             K3_CUDA(cudaGetLastError());
         } else {
-            size_t tmp = w.cub_bytes;
+            size_t tmp = w.cub_tmp.cap;
             const int end_bit = 64 - __builtin_clzll(((unsigned long long)nwords << 6) | 1ull);
-            K3_CUDA(cub::DeviceRadixSort::SortPairs(w.cub_tmp, tmp, w.long_keys, w.long_keys_sorted, w.long_slot, w.long_slot_sorted, (int)n_long, 0, end_bit, stream));
-            k3_rank<<<(n_long + 255) / 256, 256, 0, stream>>>(w.long_slot_sorted, w.long_n, w.long_off_slot, n_long, w.long_n_sorted, w.long_off, w.long_rank);
+            K3_CUDA(cub::DeviceRadixSort::SortPairs(w.cub_tmp.p, tmp, w.long_keys.p, w.long_keys_sorted.p, w.long_slot.p, w.long_slot_sorted.p,
+                                                    (int)s.n_long, 0, end_bit, stream));
+            k3_rank<<<(s.n_long + 255) / 256, 256, 0, stream>>>(w.long_slot_sorted.p, w.long_n.p, w.long_off_slot.p, s.n_long, w.long_n_sorted.p,
+                                                               w.long_off.p, w.long_rank.p);
             K3_CUDA(cudaGetLastError());
         }
         timer.mark("order");
-        (emit_light(p.n) ? k3_emit<true> : k3_emit<false>)<<<(n_long + n_ckpts + n_relays + 127) / 128, 128, 0, stream>>>(g, w.d_tables, w.long_keys_sorted, w.long_n_sorted, w.long_off, n_long, w.long_rank,
-                                                                   w.walker_slot, w.ckpts, n_ckpts, w.contours, w.points, nullptr, w.relays, w.segs, w.seg_owner, n_relays);
+        // k3_emit's step: the register window when many segments are in flight (256 x 1080p: 0.094 ms against 0.115 ms), the
+        // walkers' lighter step for calls of a few frames, where the chain of one segment is what is waited for (noise frame:
+        // 0.025 against 0.040 ms)
+        (p.n <= 4 ? k3_emit<true> : k3_emit<false>)<<<(s.n_long + s.ckpts + s.relays + 127) / 128, 128, 0, stream>>>(
+            g, w.tables.p, w.long_keys_sorted.p, w.long_n_sorted.p, w.long_off.p, s.n_long, w.long_rank.p, w.walker_slot.p, w.ckpts.p, s.ckpts,
+            w.contours.p, w.points.p, dyn, w.relays.p, w.segs.p, w.seg_owner.p, s.relays);
         K3_CUDA(cudaGetLastError());
         timer.mark("emit");
-        k3_rdp<<<(n_long + 3) / 4, 128, 0, stream>>>(w.contours, w.points, n_long, p.eps_factor, p.min_edge_length, w.contour_quads, p.frame_flags, nullptr, p.w <= 16384 && p.h <= 16384);
+        k3_rdp<<<(s.n_long + 3) / 4, 128, 0, stream>>>(w.contours.p, w.points.p, s.n_long, p.eps_factor, p.min_edge_length, w.contour_quads.p,
+                                                        p.frame_flags, dyn, p.w <= 16384 && p.h <= 16384);
         K3_CUDA(cudaGetLastError());
     }
     timer.mark("rdp");
-    const size_t fin_smem = (size_t)p.quad_cap * (32 + 4 + 1) + 16;
-    if (fin_smem > 200 * 1024) return cudaErrorInvalidValue;
     K3_CUDA(cudaFuncSetAttribute(k3_finalize, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fin_smem));
-    k3_finalize<<<p.n, 32, fin_smem, stream>>>(w.contour_quads, w.long_keys_sorted, words_per_frame, n_long, p.n, p.min_corner_separation, p.quad_cap,
-                                        p.quads, p.quad_counts, p.before_discard, p.frame_flags, w.dead, nullptr);
+    k3_finalize<<<p.n, 32, fin_smem, stream>>>(w.contour_quads.p, w.long_keys_sorted.p, words_per_frame, s.n_long, p.n, p.min_corner_separation,
+                                               p.quad_cap, p.quads, p.quad_counts, p.before_discard, p.frame_flags, w.dead.p, dyn);
     K3_CUDA(cudaGetLastError());
     timer.mark("finalize");
-    if (p.frame_contours) K3_CUDA(cudaMemcpyAsync(p.frame_contours, w.frame_contours, (size_t)p.n * 4, cudaMemcpyDeviceToDevice, stream));
-    if (p.frame_points) K3_CUDA(cudaMemcpyAsync(p.frame_points, w.frame_points, (size_t)p.n * 8, cudaMemcpyDeviceToDevice, stream));
+    if (p.frame_contours) K3_CUDA(cudaMemcpyAsync(p.frame_contours, w.frame_contours.p, (size_t)p.n * 4, cudaMemcpyDeviceToDevice, stream));
+    if (p.frame_points) K3_CUDA(cudaMemcpyAsync(p.frame_points, w.frame_points.p, (size_t)p.n * 8, cudaMemcpyDeviceToDevice, stream));
     return cudaSuccess;
 }
 
-// Second half without the host synchronisation: the same kernels, launched with the list sizes of the previous call of
-// this geometry plus headroom; the real sizes stay on the device (`counters`).  *speculated = false (nothing enqueued)
-// when there is no such history.  The caller synchronises the stream later and asks k3_speculation_held(); when it did
-// not hold, k3_finish redoes the second half exactly (k3_begin's lists are untouched by a failed speculation).
+// Second half, exactly: waits for the counters (the only host synchronisation of the stage) and launches for the real sizes.
+cudaError_t k3_finish(K3Workspace &ws, const K3Params &p, cudaStream_t stream) {
+    K3Workspace::Impl &w = *ws.impl;
+    if (p.n == 0) return cudaSuccess;
+    K3_CUDA(cudaStreamSynchronize(stream));
+    const ListSizes s = read_sizes(w);
+    if (getenv("A3_K3_TIMING")) {
+        const uint32_t *hc = reinterpret_cast<const uint32_t *>(w.h_counts.p);
+        fprintf(stderr, "k3 lists: %u candidates, %u walkers, %u long borders, %llu points, %u checkpoints, %u relay cracks\n", hc[kNumCands],
+                hc[kNumWalkers], s.n_long, s.points, s.ckpts, s.relays);
+    }
+    record_history(w, p, s);
+    w.spec.reset();
+    const bool wide = s.points >= 0xffffffffull;
+    if (wide && !s.overflow) {  // point offsets are 32-bit: hand the whole call to the host stage
+        k3_flag_all<<<(p.n + 127) / 128, 128, 0, stream>>>(p.frame_flags, p.n, w.counters.p, 1);
+        K3_CUDA(cudaGetLastError());
+    }
+    const Lists &l = w.l;
+    ListSizes run = s;
+    run.n_long = s.overflow || wide ? 0 : std::min(s.n_long, l.long_cap);  // every frame is flagged for the host stage
+    run.ckpts = std::min(s.ckpts, l.ckpt_cap);
+    run.relays = std::min(s.relays, l.relay_cap);
+    return enqueue_finish(w, p, run, nullptr, stream);
+}
+
+// Second half without the host synchronisation: the same launches, sized from the previous call of this geometry plus
+// headroom; the real sizes stay on the device (`counters`).  *speculated = false (nothing enqueued) when there is no such
+// history.  The caller synchronises the stream later and asks k3_speculation_held(); when it did not hold, k3_finish redoes
+// the second half exactly (k3_begin's lists are untouched by a failed speculation).
 cudaError_t k3_finish_speculative(K3Workspace &ws, const K3Params &p, cudaStream_t stream, bool *speculated) {
     K3Workspace::Impl &w = *ws.impl;
     *speculated = false;
-    w.spec_long = 0;
-    if (p.n == 0 || !w.hist_valid || w.hist_n != p.n || w.hist_w != p.w || w.hist_h != p.h) return cudaSuccess;
-    const Geo g = w.g;
-    const Lists l = w.l;
-    const size_t words_per_frame = (size_t)g.h * g.wpr, nwords = words_per_frame * p.n;
-    const size_t fin_smem = (size_t)p.quad_cap * (32 + 4 + 1) + 16;
-    if (fin_smem > 200 * 1024) return cudaSuccess;
-    unsigned long long cap_long64 = (unsigned long long)w.hist_long + w.hist_long / 8 + 256;
-    if (cap_long64 > l.long_cap) cap_long64 = l.long_cap;
-    unsigned long long cap_ckpts64 = (unsigned long long)w.hist_ckpts + w.hist_ckpts / 8 + 1024;
-    if (cap_ckpts64 > l.ckpt_cap) cap_ckpts64 = l.ckpt_cap;
-    unsigned long long cap_points = w.hist_points + w.hist_points / 8 + 65536;
-    if (cap_points > 0xfffffffeull) cap_points = 0xfffffffeull;
-    const uint32_t cap_long = (uint32_t)cap_long64, cap_ckpts = (uint32_t)cap_ckpts64;
-    unsigned long long cap_relays64 = (unsigned long long)w.hist_relays + w.hist_relays / 8 + 1024;
-    if (cap_relays64 > l.relay_cap) cap_relays64 = l.relay_cap;
-    const uint32_t cap_relays = (uint32_t)cap_relays64;
-    if ((size_t)cap_long > w.contours_cap) {
-        K3_CUDA(alloc_exact(w.contours, (size_t)cap_long + cap_long / 4 + 1024));
-        K3_CUDA(alloc_exact(w.contour_quads, ((size_t)cap_long + cap_long / 4 + 1024) * 8));
-        w.contours_cap = (size_t)cap_long + cap_long / 4 + 1024;
-    }
-    K3_CUDA(grow(w.points, w.points_cap, (size_t)cap_points + 1));
-    PhaseTimer timer(stream);
-    timer.mark("begin");
+    w.spec.reset();
+    const K3Workspace::Impl::History &h = w.hist;
+    if (p.n == 0 || !h.valid || h.n != p.n || h.w != p.w || h.h != p.h) return cudaSuccess;
+    const Lists &l = w.l;
+    const ListSizes &last = h.sizes;
+    ListSizes cap;
+    cap.n_long = (uint32_t)std::min<unsigned long long>((unsigned long long)last.n_long + last.n_long / 8 + 256, l.long_cap);
+    cap.ckpts = (uint32_t)std::min<unsigned long long>((unsigned long long)last.ckpts + last.ckpts / 8 + 1024, l.ckpt_cap);
+    cap.relays = (uint32_t)std::min<unsigned long long>((unsigned long long)last.relays + last.relays / 8 + 1024, l.relay_cap);
+    cap.points = std::min(last.points + last.points / 8 + 65536, 0xfffffffeull);
     // which ordering: the per-frame ranking when the previous call's fullest frame fits its lists with room to spare
-    const bool per_frame = l.frame_cap && w.hist_frame_long + w.hist_frame_long / 4 + 16 <= l.frame_cap;
-    const uint32_t cap_frame_long = per_frame ? l.frame_cap : 0xffffffffu;
-    k3_spec_prepare<<<(cap_long + 255) / 256, 256, 0, stream>>>(w.long_keys, w.long_slot, w.counters, w.long_points, cap_long, cap_ckpts, cap_points,
-                                                                cap_frame_long, cap_relays);
-    K3_CUDA(cudaGetLastError());
-    if (per_frame) {
-        k3_order<<<p.n, 256, 0, stream>>>(l, p.n, w.long_keys_sorted, w.long_n_sorted, w.long_off, w.long_rank, w.counters);
-        K3_CUDA(cudaGetLastError());
-    } else {
-        size_t tmp = w.cub_bytes;
-        const int end_bit = 64 - __builtin_clzll(((unsigned long long)nwords << 6) | 1ull);
-        K3_CUDA(cub::DeviceRadixSort::SortPairs(w.cub_tmp, tmp, w.long_keys, w.long_keys_sorted, w.long_slot, w.long_slot_sorted, (int)cap_long, 0, end_bit, stream));
-        k3_rank<<<(cap_long + 255) / 256, 256, 0, stream>>>(w.long_slot_sorted, w.long_n, w.long_off_slot, cap_long, w.long_n_sorted, w.long_off, w.long_rank);
-        K3_CUDA(cudaGetLastError());
-    }
-    timer.mark("order");
-    (emit_light(p.n) ? k3_emit<true> : k3_emit<false>)<<<(cap_long + cap_ckpts + cap_relays + 127) / 128, 128, 0, stream>>>(g, w.d_tables, w.long_keys_sorted, w.long_n_sorted, w.long_off, cap_long, w.long_rank,
-                                                                   w.walker_slot, w.ckpts, cap_ckpts, w.contours, w.points, w.counters, w.relays, w.segs, w.seg_owner, cap_relays);
-    K3_CUDA(cudaGetLastError());
-    timer.mark("emit");
-    k3_rdp<<<(cap_long + 3) / 4, 128, 0, stream>>>(w.contours, w.points, cap_long, p.eps_factor, p.min_edge_length, w.contour_quads, p.frame_flags, w.counters, p.w <= 16384 && p.h <= 16384);
-    K3_CUDA(cudaGetLastError());
-    timer.mark("rdp");
-    K3_CUDA(cudaFuncSetAttribute(k3_finalize, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fin_smem));
-    k3_finalize<<<p.n, 32, fin_smem, stream>>>(w.contour_quads, w.long_keys_sorted, words_per_frame, cap_long, p.n, p.min_corner_separation, p.quad_cap,
-                                        p.quads, p.quad_counts, p.before_discard, p.frame_flags, w.dead, w.counters);
-    K3_CUDA(cudaGetLastError());
-    timer.mark("finalize");
-    if (p.frame_contours) K3_CUDA(cudaMemcpyAsync(p.frame_contours, w.frame_contours, (size_t)p.n * 4, cudaMemcpyDeviceToDevice, stream));
-    if (p.frame_points) K3_CUDA(cudaMemcpyAsync(p.frame_points, w.frame_points, (size_t)p.n * 8, cudaMemcpyDeviceToDevice, stream));
-    w.spec_long = cap_long ? cap_long : 1; w.spec_ckpts = cap_ckpts; w.spec_points = cap_points; w.spec_frame_long = cap_frame_long;
-    w.spec_relays = cap_relays;
+    cap.frame_long = l.frame_cap && last.frame_long + last.frame_long / 4 + 16 <= l.frame_cap ? l.frame_cap : 0xffffffffu;
+    K3_CUDA(enqueue_finish(w, p, cap, w.counters.p, stream));
+    w.spec = cap;
     *speculated = true;
     return cudaSuccess;
 }
 
 // Device word that is non-zero when the speculative finish in flight gave up (for kernels queued behind it).
-const uint32_t *k3_speculation_failed_flag(K3Workspace &ws) { return ws.impl->counters ? ws.impl->counters + kSpecFail : nullptr; }
+const uint32_t *k3_speculation_failed_flag(K3Workspace &ws) { return ws.impl->counters.p ? ws.impl->counters.p + kSpecFail : nullptr; }
 
-// After the stream of a speculative finish has been synchronised: did the real list sizes fit?  (The same test
-// k3_spec_prepare made on the device.)  Records the sizes for the next call either way.
+// After the stream of a speculative finish has been synchronised: did the real list sizes fit?  Records the sizes for the
+// next call either way.
 bool k3_speculation_held(K3Workspace &ws, const K3Params &p) {
     K3Workspace::Impl &w = *ws.impl;
-    if (!w.spec_long) return false;
-    const uint32_t *hc = reinterpret_cast<const uint32_t *>(&w.h_counts[0]);
-    const unsigned long long n_points = w.h_counts[4];
-    const bool held = !hc[2] && hc[1] <= w.spec_long && hc[4] <= w.spec_ckpts && n_points <= w.spec_points && hc[7] <= w.spec_frame_long &&
-                      hc[6] <= w.spec_relays;
-    w.hist_valid = !hc[2] && n_points < 0xffffffffull;
-    w.hist_n = p.n; w.hist_w = p.w; w.hist_h = p.h; w.hist_long = hc[1]; w.hist_ckpts = hc[4]; w.hist_points = n_points;
-    w.hist_frame_long = hc[7];
-    w.hist_relays = hc[6];
-    w.spec_long = 0;
+    if (!w.spec) return false;
+    const ListSizes s = read_sizes(w);
+    const bool held = s.fits(*w.spec);
+    record_history(w, p, s);
+    w.spec.reset();
     return held;
 }
 

@@ -7,7 +7,8 @@ counters and a digest of every output buffer.
 The matrix: host and device input; first and repeat call of a detector (the repeat takes the one-shot route where it can);
 markers only (lean) and full outputs; device and host contours; post-decode stages off, each alone, all together, and all with
 a lens distortion whose pose and board intrinsics are equal (one K7 set) or not (two); the ordinary route over several chunks
-and decode groups; and a call whose one-shot speculation fails and retries the ordinary way.
+and decode groups; a call whose one-shot speculation fails and retries the ordinary way; and a call of pure-noise frames after
+flat ones, whose K3 lists outgrow the speculation, so that K3's exact finish behind the failed speculative one is traced too.
 
 usage: python tools/route_trace.py --out FILE                    trace the library that A3_LIB_PATH (or the package) loads
        python tools/route_trace.py --compare OLD NEW [--out FILE]  compare two traces: kernel sequences, copies, counters, outputs"""
@@ -140,7 +141,7 @@ def run_case(name, board, imgs, mem, contours, full, stages, chunk=0, retry=Fals
     src = src_of(imgs)
     out = []
     with make_detector(board, stages, contours, chunk) as d:
-        if retry:  # blank frames set a small history (256 quads of headroom); the board frames then outgrow the speculated quad list
+        if retry:  # blank frames set a small history (256 quads of headroom); the traced frames then outgrow the speculated lists
             blank = src_of(np.full_like(imgs, 200))
             for _ in range(2):
                 detect(d, blank, kinds[mem], n, full)
@@ -157,6 +158,7 @@ def run_case(name, board, imgs, mem, contours, full, stages, chunk=0, retry=Fals
 
 
 def trace(path):
+    import numpy as np
     import torch
 
     from aruco3_b200 import _ffi
@@ -164,6 +166,7 @@ def trace(path):
     board, imgs = frames(5)
     imgs[2] = 200  # a frame without markers
     many = imgs[[i % 5 for i in range(40)]]  # 40 frames: two decode groups on the ordinary route
+    noise = np.random.default_rng(9).integers(0, 256, size=imgs.shape, dtype=np.uint8)  # far more long borders than flat frames
     traced(lambda: torch.zeros(1, device="cuda"))  # profiler start-up outside the cases
     cases = []
     for mem in ("host", "device"):
@@ -178,6 +181,8 @@ def trace(path):
             for full in (False, True):
                 cases += run_case(f"{mem} input, device contours, {'full' if full else 'lean'}, {stages}, 40 frames, one-shot retry", board,
                                   many, mem, "device", full, stages, retry=True)
+        cases += run_case(f"{mem} input, device contours, full, none, 5 noise frames after flat ones, K3 speculation fails", board, noise,
+                          mem, "device", True, "none", retry=True)
     res = {"library": _ffi.LIB_PATH.name, "card": card(), "calls": cases}
     Path(path).parent.mkdir(parents=True, exist_ok=True)
     Path(path).write_text(json.dumps(res, indent=1))
