@@ -1,17 +1,21 @@
 // C ABI of the detection path (include/aruco3_b200.h): detector handle, the batched pipeline and the stage probes.
 //
-// Pipeline of a3_detect_batch (frames are independent — src/aruco.rs:52-121 is a pure function of one image — so
-// frames, chunks and GPUs never exchange data):
+// a3_detect_batch (frames are independent — src/aruco.rs:52-121 is a pure function of one image — so frames, chunks and
+// GPUs never exchange data), ordinary route:
 //
-//   copy stream     H2D of front-end chunk j into a staging ring            (host input only)
-//   pixel stream    K1 (grey + 1-bit mask, k1_strips.cu) -> D2H of the mask bits -> event[j]
-//   host pool       persistent threads; frame f becomes runnable when event[chunk of f] has fired; one task = border
-//                   following + quad filters of one frame (host_quads.cpp)
-//   decode stream   per group of frames whose quads are ready: H2D quads -> K2 (k2_decode.cu) -> D2H decode records
-//   caller thread   feeds the pool, launches decode groups, finally assembles markers in frame / candidate order
+//   copy stream     H2D of front-end chunk j into a device staging ring (host input only)
+//   pixel stream    K1 (grey + 1-bit mask, k1_strips.cu), then K3 (k3_contours.cu) and D2H of its counters and quads, or
+//                   in host-contour mode D2H of the mask bits -> event[j]
+//   decode stream   per decode group of frames whose quads are ready: the quads (gathered from K3's output on the device,
+//                   or H2D from the host), K2 (k2_decode.cu) and the post-decode chain -> D2H of the group's outputs
 //
-// Device input runs K1 once over the whole (super-)batch; host input runs it per front-end chunk right behind the
-// copy, so the PCIe transfer, the host stage and the decode kernel all overlap.
+// Resident input runs K1 once per super-batch; host input runs it per chunk right behind that chunk's copy.
+// One-shot route (device contours, one K3 launch over the whole batch): the gather and the decode chain follow K3 on the
+// pixel stream, sized from the previous call, and everything comes back in one copy.
+//
+// Host threads: `pool` runs the host contour stage (host_quads.cpp), one task per frame, submitted when its chunk's event
+// has fired; `copy_pool` moves pageable caller memory through pinned rings.  The caller thread drives the chunks, redoes
+// the frames K3 flags, launches the decode groups and assembles markers in frame / candidate order.
 // There is no CPU fallback: without a CUDA device every compute entry point returns A3_ERR_CUDA.
 #include <immintrin.h>
 #include <math.h>
@@ -44,75 +48,15 @@ a3_status cuda_fail(cudaError_t e, const char *what) {
 
 namespace {
 
-// Persistent host threads.  A job is a function of a frame index; indices [0, ready) may be claimed.
-class WorkerPool {
+// Persistent host threads that run a FIFO of tasks.  Tasks do not finish in submission order; callers keep their own
+// completion counters (atomics) and sleep on them with wait(); a task calls notify() when a counter reaches its goal.
+class TaskPool {
 public:
-    ~WorkerPool() { stop(); }
-    void resize(uint32_t threads) {
+    ~TaskPool() { stop(); }
+    // `threads` workers, started on first use and restarted when the count changes; the pool must be idle
+    void ensure(uint32_t threads, int device) {
         if (threads == workers_.size()) return;
         stop();
-        quit_ = false;
-        for (uint32_t t = 0; t < threads; t++) workers_.emplace_back([this] { loop(); });
-    }
-    uint32_t size() const { return (uint32_t)workers_.size(); }
-    void begin(std::function<void(uint32_t)> fn, uint32_t total) {
-        std::lock_guard<std::mutex> lk(mu_);
-        fn_ = std::move(fn); total_ = total; next_ = 0; ready_ = 0; done_ = 0;
-    }
-    void publish(uint32_t upto) {
-        { std::lock_guard<std::mutex> lk(mu_); if (upto > ready_) ready_ = upto; }
-        cv_.notify_all();
-    }
-    // Tasks do not finish in index order; callers keep their own counters inside the job function and sleep on them
-    // with wait_caller(); the job calls notify_caller() when a counter reaches its goal.
-    void notify_caller() { { std::lock_guard<std::mutex> lk(mu_); } cv_done_.notify_all(); }
-    template <typename Pred>
-    void wait_caller(Pred pred) {
-        std::unique_lock<std::mutex> lk(mu_);
-        cv_done_.wait(lk, pred);
-    }
-    void finish() {  // block until all `total` tasks are done
-        std::unique_lock<std::mutex> lk(mu_);
-        cv_done_.wait(lk, [this] { return done_ >= total_; });
-        fn_ = nullptr;
-    }
-
-private:
-    void loop() {
-        std::unique_lock<std::mutex> lk(mu_);
-        for (;;) {
-            cv_.wait(lk, [this] { return quit_ || (fn_ && next_ < ready_); });
-            if (quit_) return;
-            const uint32_t i = next_++;
-            lk.unlock();
-            fn_(i);  // fn_ stays alive until finish(), which waits for this task
-            lk.lock();
-            if (++done_ >= total_) cv_done_.notify_all();
-        }
-    }
-    void stop() {
-        { std::lock_guard<std::mutex> lk(mu_); quit_ = true; }
-        cv_.notify_all();
-        for (auto &t : workers_) t.join();
-        workers_.clear();
-    }
-    std::vector<std::thread> workers_;
-    std::mutex mu_;
-    std::condition_variable cv_, cv_done_;
-    std::function<void(uint32_t)> fn_;
-    uint32_t total_ = 0, next_ = 0, ready_ = 0, done_ = 0;
-    bool quit_ = false;
-};
-
-// Host threads that move bytes between the caller's pageable memory and the pinned staging rings (a3_detect_batch with
-// A3_MEM_HOST frames that are not page-locked, and `Detection.grey` into a pageable buffer): a FIFO of small tasks.  Callers
-// keep their own completion counters (atomics) and sleep on them with wait(); a task calls notify() when a counter reaches
-// its goal.
-class CopyPool {
-public:
-    ~CopyPool() { stop(); }
-    void start(uint32_t threads, int device) {
-        if (!workers_.empty()) return;
         quit_ = false;
         for (uint32_t t = 0; t < threads; t++)
             workers_.emplace_back([this, device] {
@@ -134,14 +78,14 @@ public:
         std::unique_lock<std::mutex> lk(mu_);
         cv_done_.wait(lk, [this] { return q_.empty() && running_ == 0; });
     }
+
+private:
     void stop() {
         { std::lock_guard<std::mutex> lk(mu_); quit_ = true; }
         cv_.notify_all();
         for (auto &t : workers_) t.join();
         workers_.clear();
     }
-
-private:
     void loop() {
         std::unique_lock<std::mutex> lk(mu_);
         for (;;) {
@@ -181,7 +125,7 @@ __attribute__((target("avx2"))) void copy_stream_avx2(uint8_t *dst, const uint8_
     if (i < len) memcpy(dst + i, src + i, len - i);
 }
 void copy_stream(uint8_t *dst, const uint8_t *src, size_t len) {
-    static const bool avx2 = __builtin_cpu_supports("avx2") && !getenv("A3_PLAIN_MEMCPY");
+    static const bool avx2 = __builtin_cpu_supports("avx2");
     if (avx2 && len >= 4096) copy_stream_avx2(dst, src, len);
     else memcpy(dst, src, len);
 }
@@ -330,10 +274,7 @@ struct a3_detector {
     a3::DevBuf<int> d_meta;
     a3::EventPool events;
     std::vector<std::unique_ptr<a3::DecodeBlock>> blocks;
-    a3::WorkerPool pool;
-    // pageable host memory at the boundary: pinned rings + copy threads (created on first use)
-    a3::CopyPool copy_pool;
-    a3::PinBuf<uint8_t> h_stage_in, h_stage_out;
+    a3::PinBuf<uint8_t> h_stage_in, h_stage_out;  // pinned rings for pageable host memory at the boundary
     // GPU contour stage (K3)
     a3::K3Workspace k3;
     a3::DevBuf<uint32_t> d_planes, d_k3quads;
@@ -364,6 +305,9 @@ struct a3_detector {
     a3::DevBuf<a3_board_pose> d_probe_out;
     a3::DevBuf<float> d_und_in, d_und_out;  // a3_undistort_points, and K7's points for a3_solve_board
     a3::DevBuf<uint8_t> d_und_ok;
+    // host threads: the host contour stage (host_threads of them), and the copies between pageable caller memory and the
+    // pinned rings (up to 16).  Declared last, so that they stop before the buffers their tasks use go away.
+    a3::TaskPool pool, copy_pool;
 };
 
 namespace a3 {
@@ -823,8 +767,7 @@ void a3_detector_destroy(a3_detector *d) {
     cudaSetDevice(d->device);
     for (cudaStream_t s : {d->s_copy, d->s_pixel, d->s_decode})
         if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); }
-    d->copy_pool.stop();  // its tasks use the staging rings, which go with the handle
-    delete d;             // buffers and events free themselves, on the device set above
+    delete d;  // threads stop; buffers and events free themselves, on the device set above
 }
 
 a3_status a3_detector_set_host_threads(a3_detector *d, uint32_t threads) {
@@ -1042,7 +985,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
     memset(&st, 0, sizeof(st));
     st.n_frames = n;
     st.host_threads = d->host_threads;
-    if (d->pool.size() != d->host_threads) d->pool.resize(d->host_threads);
+    d->pool.ensure(d->host_threads, d->device);
     // Pageable host memory at the boundary (the Vec<u8> of a `DynamicImage`, a `Detection.grey` the caller got from malloc): a
     // cudaMemcpyAsync on it is neither asynchronous nor fast, so such buffers go through pinned rings that the copy threads
     // fill (input) or empty (grey) one front-end chunk ahead of / behind the DMA.
@@ -1051,10 +994,9 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
         if (cudaPointerGetAttributes(&at, ptr) != cudaSuccess) { cudaGetLastError(); return true; }
         return at.type == cudaMemoryTypeUnregistered;
     };
-    static const bool no_staging = getenv("A3_NO_HOST_STAGING") != nullptr;
-    const bool stage_in = mem == A3_MEM_HOST && !no_staging && (size_t)n * frame_stride >= ((size_t)1 << 20) && is_pageable(frames);
-    const bool stage_out = want_grey && !no_staging && (size_t)n * px >= ((size_t)1 << 20) && is_pageable(outs->grey);
-    if (stage_in || stage_out) d->copy_pool.start(d->host_threads < 16u ? d->host_threads : 16u, d->device);
+    const bool stage_in = mem == A3_MEM_HOST && (size_t)n * frame_stride >= ((size_t)1 << 20) && is_pageable(frames);
+    const bool stage_out = want_grey && (size_t)n * px >= ((size_t)1 << 20) && is_pageable(outs->grey);
+    if (stage_in || stage_out) d->copy_pool.ensure(d->host_threads < 16u ? d->host_threads : 16u, d->device);
     st.input_staged = stage_in ? 1u : 0u;
     st.output_staged = stage_out ? 1u : 0u;
 
@@ -1081,7 +1023,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
     // front-end chunk, e.g. a single frame — the second half of K3, the gather of its quads, K2 and K4 are all queued behind
     // K1 without a host synchronisation, sized from the previous call of the same geometry; the host synchronises once at the
     // end, checks that the sizes held and otherwise takes the ordinary route from where the speculation stopped.
-    const bool one_shot = gpu_contours && (mem == A3_MEM_DEVICE || n <= fe) && !getenv("A3_NO_ONE_SHOT");
+    const bool one_shot = gpu_contours && (mem == A3_MEM_DEVICE || n <= fe);
     if (one_shot) group = (uint32_t)sb;
     const uint32_t Hp = h + 2;                               // guarded column-major plane: words per 32-pixel column
     const size_t plane_words = (size_t)(wpr + 2) * Hp;       // words per frame
@@ -1291,7 +1233,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 A3_CUDA(cudaMemcpyAsync(outs->grey + (size_t)(s0 + f0) * px, d->d_grey.p + (size_t)f0 * px, (size_t)cn * px, cudaMemcpyDeviceToHost, d->s_pixel));
                 return A3_OK;
             }
-            CopyPool *cp = &d->copy_pool;
+            TaskPool *cp = &d->copy_pool;
             for (uint32_t sub = 0; sub < cn; sub += (uint32_t)out_slot_frames) {
                 const uint32_t m = cn - sub < out_slot_frames ? cn - sub : (uint32_t)out_slot_frames;
                 const size_t q = stg->out.size(), bytes = (size_t)m * px;
@@ -1359,7 +1301,7 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
         // c - kHostRing has completed.  Chunks are handed to the threads as early as that allows (without blocking), and the
         // caller only ever blocks for the chunk it is about to send (`must`).
         auto advance_stage_in = [&](uint32_t must) -> a3_status {
-            CopyPool *cp = &d->copy_pool;
+            TaskPool *cp = &d->copy_pool;
             while (stage_submitted < nfe) {
                 const uint32_t c = stage_submitted;
                 if (c >= kHostRing) {
@@ -1424,19 +1366,13 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             return bits_d2h(f0, cn, j);
         };
 
-        // ---- host stage: one task per frame (host-contour mode; in device-contour mode only flagged frames, inline) ----
-        const a3_config cfg = d->cfg;
-        uint32_t *h_bits = d->h_bits.p;
-        a3_detector *det = d;
-        if (!gpu_contours) {
-            d->pool.begin([&, h_bits, cfg, det](uint32_t i) {
-                const double t0 = now_ms();
-                quads_from_bits(h_bits + (size_t)i * bits_words, (uint32_t)wpr, w, h, cfg, frame_quads[i], &frame_stats[i]);
-                frame_ms[i] = now_ms() - t0;
-                const uint32_t g = i / group;
-                if (group_done[g].fetch_add(1) + 1 == group_size(g)) det->pool.notify_caller();
-            }, sn);
-        }
+        // ---- host stage of frame i on its row-major mask bits (host-contour mode: a pool task per frame; device-contour
+        // mode: the frames K3 flags, inline) ----
+        auto host_stage = [&](uint32_t i, const uint32_t *bits) {
+            const double t0 = now_ms();
+            quads_from_bits(bits, (uint32_t)wpr, w, h, d->cfg, frame_quads[i], &frame_stats[i]);
+            frame_ms[i] = now_ms() - t0;
+        };
         // device-contour mode: take frame i's quads from K3's output, or redo the frame on the host when K3 flagged it
         auto take_k3_frame = [&](uint32_t i) -> a3_status {
             if (hs.flags[i] == 0) {
@@ -1449,14 +1385,12 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 frame_quads[i].assign(d->h_k3quads.p + (size_t)i * quad_cap * 8, d->h_k3quads.p + (size_t)i * quad_cap * 8 + (size_t)m * 8);
                 hs.stats(i, frame_stats[i]);
             } else {
-                const double t0 = now_ms();
                 A3_CUDA(cudaMemcpyAsync(d->h_plane.p, d->d_planes.p + (size_t)i * plane_words, plane_words * 4, cudaMemcpyDeviceToHost, d->s_decode));
                 A3_CUDA(cudaStreamSynchronize(d->s_decode));
                 std::vector<uint32_t> rows(bits_words);  // back to the row-major mask the host stage reads
                 for (uint32_t k = 0; k < wpr; k++)
                     for (uint32_t y = 0; y < h; y++) rows[(size_t)y * wpr + k] = d->h_plane.p[(size_t)(k + 1) * Hp + (y + 1)];
-                quads_from_bits(rows.data(), (uint32_t)wpr, w, h, cfg, frame_quads[i], &frame_stats[i]);
-                frame_ms[i] = now_ms() - t0;
+                host_stage(i, rows.data());
                 st.host_fallback_frames++;
             }
             group_done[i / group].fetch_add(1);
@@ -1528,13 +1462,10 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
             A3_CUDA(cudaMemcpyAsync(b.h_out.p, b.d_out.p, lay.host_end, cudaMemcpyDeviceToHost, d->s_decode));
             return A3_OK;
         };
-        auto drain = [&](a3_status s) {  // an error: let the pool and the streams finish before the buffers go away
-            if (!gpu_contours) {
-                d->pool.publish(sn);
-                d->pool.finish();
-            }
+        auto drain = [&](a3_status s) {  // an error: the streams and the tasks already submitted finish before the buffers go away
             cudaStreamSynchronize(d->s_copy); cudaStreamSynchronize(d->s_pixel); cudaStreamSynchronize(d->s_decode);
-            if (stage_in || stage_out) d->copy_pool.drain();
+            d->pool.drain();
+            d->copy_pool.drain();
             return s;
         };
 
@@ -1556,24 +1487,29 @@ a3_status a3_detect_batch(a3_detector *d, const void *frames, a3_format format, 
                 if (k3_spec_inflight && (err = settle_one_shot())) break;
                 if ((mem == A3_MEM_HOST || j == 0) && !one_shot_done)  // resident input: K3 ran once over everything
                     for (uint32_t i = (mem == A3_MEM_HOST ? j * (uint32_t)fe : 0); i < (mem == A3_MEM_HOST ? upto : sn) && !err; i++) err = take_k3_frame(i);
-            } else {
-                d->pool.publish(upto);
+            } else {  // the mask bits of chunk j are on the host
+                for (uint32_t i = j * (uint32_t)fe; i < upto; i++)
+                    d->pool.submit([&, i] {
+                        host_stage(i, d->h_bits.p + (size_t)i * bits_words);
+                        const uint32_t g = i / group;
+                        if (group_done[g].fetch_add(1) + 1 == group_size(g)) d->pool.notify();
+                    });
             }
             while (next_group < ngroups && !err && group_done[next_group].load() == group_size(next_group)) err = launch_group(next_group++);
         }
         if (err) return drain(err);
         for (; next_group < ngroups; next_group++) {
             const uint32_t g = next_group;
-            if (!gpu_contours) d->pool.wait_caller([&] { return group_done[g].load() == group_size(g); });
+            if (!gpu_contours) d->pool.wait([&] { return group_done[g].load() == group_size(g); });
             if ((err = launch_group(g))) return drain(err);
         }
-        if (!gpu_contours) d->pool.finish();
+        d->pool.drain();
         st.ms_host_quads += now_ms() - t_host0;
 
         // ---- gather: stage timings, then markers in frame / candidate order (src/aruco.rs:75-113) ----
+        d->copy_pool.drain();  // the last grey sub-chunks reach the caller's buffer, before any return below
         A3_CUDA(cudaStreamSynchronize(d->s_decode));
         A3_CUDA(cudaStreamSynchronize(d->s_pixel));
-        if (stage_in || stage_out) d->copy_pool.drain();  // the last grey sub-chunks reach the caller's buffer
         if (trace) t_synced = now_ms();
         float ms = 0;
         for (uint32_t j = 0; j < nfe && stats; j++) {  // stage times only when the caller asked for statistics (about 2 us per query)

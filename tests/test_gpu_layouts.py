@@ -431,6 +431,7 @@ def _run_detect_case(a3, torch, name, layout, mem, variant):
     v = _VARIANTS[variant]
     want = _tight_records(name, variant)
     staged = int(mem == "pageable" and n * fs >= 1 << 20)
+    grey_staged = int(n * h * w >= 1 << 20)  # _detect's grey buffer is always pageable
     # the one-shot route needs the device contour stage and one front-end chunk per call (resident input always has one)
     one_shot_second = int(variant != "host_contours" and (variant != "chunk1" or mem == "device"))
     label = f"{name} {layout} {mem} {variant}"
@@ -445,6 +446,7 @@ def _run_detect_case(a3, torch, name, layout, mem, variant):
             del keep
             st = res["stats"]
             assert st["input_staged"] == staged, f"{label}: input_staged"
+            assert st["output_staged"] == grey_staged, f"{label}: output_staged"
             assert st["one_shot"] == (one_shot_second if call else 0), f"{label} call {call}: one_shot"
             if v.get("tuning") and mem != "device":
                 assert st["pixel_kernel_launches"] == n, f"{label}: one front-end chunk per frame"
@@ -478,6 +480,26 @@ def test_detect_layouts_variants(a3, torch, name, layout, variant):
     the tight call's byte for byte."""
     for mem in ("pageable", "pinned", "device"):
         _run_detect_case(a3, torch, name, layout, mem, variant)
+
+
+def test_host_threads_change_between_calls(a3):
+    """The host contour stage on one detector at 1 and then 3 host threads (a3_detector_set_host_threads between the
+    calls), with pageable input and grey large enough to go through both pinned rings: the host-stage and copy threads
+    restart at the new count, and every output is byte for byte the same."""
+    from aruco3_b200 import synth
+    frames = np.ascontiguousarray(synth.render_batch("C1", 4)[0])
+    n, h, w = frames.shape[:3]
+    res = []
+    with a3.Detector(contours="host") as d:
+        for threads in (1, 3):
+            _ffi.check(_ffi.lib().a3_detector_set_host_threads(d._h, threads))
+            r = _detect(d, frames.ctypes.data, "pageable", n, w, h, w * 3, w * 3 * h)
+            st = r["stats"]
+            assert (st["host_threads"], st["input_staged"], st["output_staged"]) == (threads, 1, 1)
+            res.append(r)
+    assert len(res[0]["markers"]) > 0
+    for k in ("markers", "grey", "mask", "cands", "cframe"):
+        assert res[0][k].tobytes() == res[1][k].tobytes(), k
 
 
 @pytest.mark.parametrize("fmt", ["rgb8", "luma8", "rgb16"])

@@ -7,8 +7,9 @@ counters and a digest of every output buffer.
 The matrix: host and device input; first and repeat call of a detector (the repeat takes the one-shot route where it can);
 markers only (lean) and full outputs; device and host contours; post-decode stages off, each alone, all together, and all with
 a lens distortion whose pose and board intrinsics are equal (one K7 set) or not (two); the ordinary route over several chunks
-and decode groups; a call whose one-shot speculation fails and retries the ordinary way; and a call of pure-noise frames after
-flat ones, whose K3 lists outgrow the speculation, so that K3's exact finish behind the failed speculative one is traced too.
+and decode groups, on host input also with host contours and both pinned rings; a call whose one-shot speculation fails and
+retries the ordinary way; and a call of pure-noise frames after flat ones, whose K3 lists outgrow the speculation, so that
+K3's exact finish behind the failed speculative one is traced too.
 
 usage: python tools/route_trace.py --out FILE                    trace the library that A3_LIB_PATH (or the package) loads
        python tools/route_trace.py --compare OLD NEW [--out FILE]  compare two traces: kernel sequences, copies, counters, outputs"""
@@ -183,6 +184,8 @@ def trace(path):
                                   many, mem, "device", full, stages, retry=True)
         cases += run_case(f"{mem} input, device contours, full, none, 5 noise frames after flat ones, K3 speculation fails", board, noise,
                           mem, "device", True, "none", retry=True)
+    # the host stage over several chunks and decode groups, from pageable frames into a pageable grey buffer
+    cases += run_case("host input, host contours, full, none, 40 frames in chunks of 8", board, many, "host", "host", True, "none", chunk=8)
     res = {"library": _ffi.LIB_PATH.name, "card": card(), "calls": cases}
     Path(path).parent.mkdir(parents=True, exist_ok=True)
     Path(path).write_text(json.dumps(res, indent=1))
