@@ -265,9 +265,8 @@ struct a3_detector {
     uint32_t max_taps = 0;
     a3::Options opt;
     cudaStream_t s_copy = nullptr, s_pixel = nullptr, s_decode = nullptr;
-    a3::DevBuf<uint8_t> d_src, d_grey, d_mask, d_patches, d_luma;  // d_luma: K0's Luma8 copy of LumaA8 / 16-bit frames
-    a3::DevBuf<uint32_t> d_bits, d_quads, d_qframe;
-    a3::DevBuf<a3_decode> d_dec;
+    a3::DevBuf<uint8_t> d_src, d_grey, d_mask, d_luma;  // d_luma: K0's Luma8 copy of LumaA8 / 16-bit frames
+    a3::DevBuf<uint32_t> d_bits;
     a3::PinBuf<uint32_t> h_bits;
     a3::DevBuf<uint64_t> d_codes;
     a3::DevBuf<float> d_taps;
@@ -292,19 +291,10 @@ struct a3_detector {
     a3::DevBuf<uint8_t> d_shot;
     a3::PinBuf<uint8_t> h_shot;
     uint32_t hist_nq = 0, hist_nq_n = 0, hist_nq_w = 0, hist_nq_h = 0;  // quads of the previous call with this geometry (0 = none)
-    a3::DevBuf<float> d_pose_in;      // standalone solve entry points: 8 x 4 bytes per marker (f32 points or u32 corners)
-    a3::DevBuf<a3_pose> d_pose_out;
-    a3::PinBuf<a3_pose> h_pose_out;
-    a3::DevBuf<float> d_refined;      // a3_refine_corners: refined corners and their flags
-    a3::DevBuf<uint8_t> d_refined_ok;
     // board pose (K6): the board as its id -> slot table and points on the device
     a3::DevBuf<uint16_t> d_board_slots;
     a3::DevBuf<float> d_board_pts;
-    a3::DevBuf<uint64_t> d_probe_ids;  // a3_solve_board
-    a3::DevBuf<uint32_t> d_probe_off;
-    a3::DevBuf<a3_board_pose> d_probe_out;
-    a3::DevBuf<float> d_und_in, d_und_out;  // a3_undistort_points, and K7's points for a3_solve_board
-    a3::DevBuf<uint8_t> d_und_ok;
+    a3::DevBuf<uint8_t> d_probe;  // the stage probes' inputs and outputs (probe_slices)
     // host threads: the host contour stage (host_threads of them), and the copies between pageable caller memory and the
     // pinned rings (up to 16).  Declared last, so that they stop before the buffers their tasks use go away.
     a3::TaskPool pool, copy_pool;
@@ -519,6 +509,36 @@ K2Params k2_params(const a3_detector *d, const uint8_t *grey, uint32_t w, uint32
     return p;
 }
 
+// What K6 reads from the detector (the board, its mode and intrinsics), the same for the chain and the board probe
+K6Params k6_params(const a3_detector *d, uint32_t image_w, uint32_t image_h) {
+    K6Params p;
+    p.slots = d->d_board_slots.p; p.n_codes = d->dict.n_codes; p.board = d->d_board_pts.p; p.n_board = d->opt.board_n;
+    p.mode = d->opt.board_mode; p.image_w = image_w; p.image_h = image_h; p.k = d->opt.board_k;
+    return p;
+}
+
+// K7's camera: the detector's distortion with the board's intrinsics (the corners K6 reads) or the pose's (K4's)
+K7Params k7_params(const a3_detector *d, bool board) {
+    K7Params p;
+    p.k = board ? d->opt.board_k : d->opt.pose_k; p.dist = d->opt.dist;
+    return p;
+}
+
+// A stage probe's inputs and outputs: slices (host source or null, bytes) 16-byte aligned in the detector's scratch d_probe,
+// as out_layout lays out a decode group.  The scratch grows once, slices with a source are copied up on `s`, and dev[i] is
+// slice i (null when empty).  Probes synchronise before they return, so they share it; the pipeline never touches it.
+struct ProbeSlice { const void *src; size_t bytes; };
+template <size_t N>
+cudaError_t probe_slices(a3_detector *d, const ProbeSlice (&sl)[N], cudaStream_t s, uint8_t *(&dev)[N]) {
+    size_t off[N], end = 0;
+    for (size_t i = 0; i < N; i++) { off[i] = end; end = align16(end + sl[i].bytes); }
+    cudaError_t e = d->d_probe.reserve(end);
+    for (size_t i = 0; i < N; i++) dev[i] = e == cudaSuccess && sl[i].bytes ? d->d_probe.p + off[i] : nullptr;
+    for (size_t i = 0; i < N && e == cudaSuccess; i++)
+        if (sl[i].src && sl[i].bytes) e = cudaMemcpyAsync(dev[i], sl[i].src, sl[i].bytes, cudaMemcpyHostToDevice, s);
+    return e;
+}
+
 StagePlan plan_stages(const a3_detector *d, bool poses, bool refine, bool board) {
     StagePlan sp;
     sp.poses = poses; sp.refine = refine; sp.board = board;
@@ -588,9 +608,8 @@ cudaError_t enqueue_chain(const a3_detector *d, const StagePlan &sp, const Chain
         e = timed(kUndistort, [&] {
             cudaError_t r = cudaSuccess;
             for (uint32_t j = 0; j < sp.und_sets && r == cudaSuccess; j++) {
-                K7Params p7;
+                K7Params p7 = k7_params(d, !(j == 0 && sp.und_pose));
                 p7.quads = in.quads; p7.corners_f32 = ref; p7.decodes = dec; p7.n = in.n; p7.n_dev = in.n_dev;
-                p7.k = (j == 0 && sp.und_pose) ? o.pose_k : o.board_k; p7.dist = o.dist;
                 p7.out = norm + (size_t)in.n * 8 * j; p7.ok = nok + (size_t)in.n * j;
                 r = k7_undistort(p7, s);
             }
@@ -605,10 +624,8 @@ cudaError_t enqueue_chain(const a3_detector *d, const StagePlan &sp, const Chain
         e = k4_pose(p4, s);
     }
     if (e == cudaSuccess && sp.board) {
-        K6Params p6;
+        K6Params p6 = k6_params(d, in.w, in.h);
         p6.decodes = dec; p6.quads = in.quads; p6.corners_f32 = ref; p6.offsets = in.offsets; p6.skip = in.skip; p6.n_frames = in.n_frames;
-        p6.slots = d->d_board_slots.p; p6.n_codes = d->dict.n_codes; p6.board = d->d_board_pts.p; p6.n_board = o.board_n;
-        p6.mode = o.board_mode; p6.image_w = in.w; p6.image_h = in.h; p6.k = o.board_k;
         p6.out = reinterpret_cast<a3_board_pose *>(out + l.board);
         if (sp.und_board) { p6.norm = norm + (size_t)in.n * 8 * sp.und_board_set; p6.norm_ok = nok + (size_t)in.n * sp.und_board_set; }
         e = timed(kBoard, [&] { return k6_board(p6, s); });
@@ -879,14 +896,12 @@ a3_status a3_quads_from_masks_device(a3_detector *d, const uint8_t *masks, uint3
             for (uint32_t x = 0; x < w; x++)
                 if (masks[((size_t)f * h + y) * w + x]) planes[(size_t)f * plane_words + (size_t)((x >> 5) + 1) * Hp + (y + 1)] |= 1u << (x & 31);
     cudaStream_t s = d->s_pixel;
-    d->planes_zeroed_words = 0;  // the pipeline's guard words are overwritten below
-    A3_CUDA(d->d_planes.reserve(planes.size()));
-    A3_CUDA(d->d_k3quads.reserve((size_t)n * quad_capacity * 8));
-    A3_CUDA(d->d_k3frames.reserve(K3Frames::bytes(n)));
-    A3_CUDA(cudaMemcpyAsync(d->d_planes.p, planes.data(), planes.size() * 4, cudaMemcpyHostToDevice, s));
-    const K3Frames k3f(d->d_k3frames.p, n);
-    A3_CUDA(k3_quads(d->k3, k3_params(d->cfg, d->d_planes.p, w, h, 0, n, d->d_k3quads.p, quad_capacity, k3f), s));
-    A3_CUDA(cudaMemcpyAsync(quads, d->d_k3quads.p, (size_t)n * quad_capacity * 32, cudaMemcpyDeviceToHost, s));
+    uint8_t *dev[3];
+    A3_CUDA(probe_slices(d, {{planes.data(), planes.size() * 4}, {nullptr, (size_t)n * quad_capacity * 32}, {nullptr, K3Frames::bytes(n)}}, s, dev));
+    const K3Frames k3f(dev[2], n);
+    A3_CUDA(k3_quads(d->k3, k3_params(d->cfg, reinterpret_cast<const uint32_t *>(dev[0]), w, h, 0, n, reinterpret_cast<uint32_t *>(dev[1]),
+                                      quad_capacity, k3f), s));
+    A3_CUDA(cudaMemcpyAsync(quads, dev[1], (size_t)n * quad_capacity * 32, cudaMemcpyDeviceToHost, s));
     A3_CUDA(cudaMemcpyAsync(counts, k3f.counts, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
     A3_CUDA(cudaMemcpyAsync(flags, k3f.flags, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
     if (contours) A3_CUDA(cudaMemcpyAsync(contours, k3f.contours, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
@@ -900,26 +915,22 @@ a3_status a3_decode_candidates(a3_detector *d, const uint8_t *grey, uint32_t n_f
                                uint8_t *patches) {
     if (!d || !grey || (!quads && n_quads) || (!decodes && n_quads)) return fail(A3_ERR_INVALID_ARGUMENT, "a3_decode_candidates: null argument");
     if (n_quads == 0) return A3_OK;
+    if (n_frames == 0 || w == 0 || h == 0) return fail(A3_ERR_INVALID_ARGUMENT, "a3_decode_candidates: empty grey frames");
     for (uint32_t i = 0; quad_frame && i < n_quads; i++)
         if (quad_frame[i] >= n_frames) return fail(A3_ERR_INVALID_ARGUMENT, "a3_decode_candidates: quad_frame out of range");
     A3_CUDA(cudaSetDevice(d->device));
     cudaStream_t s = d->s_decode;
     const size_t px = (size_t)w * h, np = (size_t)d->cfg.homography_sample_size * d->cfg.homography_sample_size;
-    A3_CUDA(d->d_grey.reserve(px * n_frames));
-    A3_CUDA(d->d_quads.reserve((size_t)n_quads * 8));
-    A3_CUDA(d->d_qframe.reserve(n_quads));
-    A3_CUDA(d->d_dec.reserve(n_quads));
-    if (patches) A3_CUDA(d->d_patches.reserve(n_quads * np));
-    A3_CUDA(cudaMemcpyAsync(d->d_grey.p, grey, px * n_frames, cudaMemcpyHostToDevice, s));
-    A3_CUDA(cudaMemcpyAsync(d->d_quads.p, quads, (size_t)n_quads * 32, cudaMemcpyHostToDevice, s));
-    if (quad_frame) A3_CUDA(cudaMemcpyAsync(d->d_qframe.p, quad_frame, (size_t)n_quads * 4, cudaMemcpyHostToDevice, s));
-    K2Params p = k2_params(d, d->d_grey.p, w, h);
-    p.quads = d->d_quads.p; p.quad_frame = quad_frame ? d->d_qframe.p : nullptr; p.n_quads = n_quads;
-    p.decodes = d->d_dec.p; p.patches = patches ? d->d_patches.p : nullptr;
+    uint8_t *dev[5];
+    A3_CUDA(probe_slices(d, {{grey, px * n_frames}, {quads, (size_t)n_quads * 32}, {quad_frame, quad_frame ? (size_t)n_quads * 4 : 0},
+                             {nullptr, (size_t)n_quads * sizeof(a3_decode)}, {nullptr, patches ? n_quads * np : 0}}, s, dev));
+    K2Params p = k2_params(d, dev[0], w, h);
+    p.quads = reinterpret_cast<const uint32_t *>(dev[1]); p.quad_frame = reinterpret_cast<const uint32_t *>(dev[2]); p.n_quads = n_quads;
+    p.decodes = reinterpret_cast<a3_decode *>(dev[3]); p.patches = dev[4];
     A3_CUDA(k2_queue(d, n_quads, nullptr, s, &p.queue));
     A3_CUDA(k2_decode(p, s));
-    A3_CUDA(cudaMemcpyAsync(decodes, d->d_dec.p, (size_t)n_quads * sizeof(a3_decode), cudaMemcpyDeviceToHost, s));
-    if (patches) A3_CUDA(cudaMemcpyAsync(patches, d->d_patches.p, n_quads * np, cudaMemcpyDeviceToHost, s));
+    A3_CUDA(cudaMemcpyAsync(decodes, dev[3], (size_t)n_quads * sizeof(a3_decode), cudaMemcpyDeviceToHost, s));
+    if (patches) A3_CUDA(cudaMemcpyAsync(patches, dev[4], n_quads * np, cudaMemcpyDeviceToHost, s));
     A3_CUDA(cudaStreamSynchronize(s));
     return A3_OK;
 }
@@ -934,20 +945,15 @@ a3_status a3_refine_corners(a3_detector *d, const uint8_t *grey, uint32_t n_fram
     A3_CUDA(cudaSetDevice(d->device));
     cudaStream_t s = d->s_decode;
     const size_t px = (size_t)w * h;
-    A3_CUDA(d->d_grey.reserve(px * n_frames));
-    A3_CUDA(d->d_quads.reserve((size_t)n * 8));
-    A3_CUDA(d->d_qframe.reserve(n));
-    A3_CUDA(d->d_refined.reserve((size_t)n * 8));
-    A3_CUDA(d->d_refined_ok.reserve(n));
-    A3_CUDA(cudaMemcpyAsync(d->d_grey.p, grey, px * n_frames, cudaMemcpyHostToDevice, s));
-    A3_CUDA(cudaMemcpyAsync(d->d_quads.p, corners, (size_t)n * 32, cudaMemcpyHostToDevice, s));
-    if (corner_frame) A3_CUDA(cudaMemcpyAsync(d->d_qframe.p, corner_frame, (size_t)n * 4, cudaMemcpyHostToDevice, s));
+    uint8_t *dev[5];
+    A3_CUDA(probe_slices(d, {{grey, px * n_frames}, {corners, (size_t)n * 32}, {corner_frame, corner_frame ? (size_t)n * 4 : 0},
+                             {nullptr, (size_t)n * 32}, {nullptr, n}}, s, dev));
     K5Params kp{};
-    kp.grey = d->d_grey.p; kp.w = w; kp.h = h; kp.quads = d->d_quads.p; kp.quad_frame = corner_frame ? d->d_qframe.p : nullptr;
-    kp.decodes = nullptr; kp.n = n; kp.corners = d->d_refined.p; kp.ok = d->d_refined_ok.p;
+    kp.grey = dev[0]; kp.w = w; kp.h = h; kp.quads = reinterpret_cast<const uint32_t *>(dev[1]); kp.quad_frame = reinterpret_cast<const uint32_t *>(dev[2]);
+    kp.decodes = nullptr; kp.n = n; kp.corners = reinterpret_cast<float *>(dev[3]); kp.ok = dev[4];
     A3_CUDA(k5_corners(kp, s));
-    A3_CUDA(cudaMemcpyAsync(refined, d->d_refined.p, (size_t)n * 32, cudaMemcpyDeviceToHost, s));
-    A3_CUDA(cudaMemcpyAsync(ok, d->d_refined_ok.p, n, cudaMemcpyDeviceToHost, s));
+    A3_CUDA(cudaMemcpyAsync(refined, dev[3], (size_t)n * 32, cudaMemcpyDeviceToHost, s));
+    A3_CUDA(cudaMemcpyAsync(ok, dev[4], n, cudaMemcpyDeviceToHost, s));
     A3_CUDA(cudaStreamSynchronize(s));
     return A3_OK;
 }
@@ -1702,28 +1708,21 @@ a3_status a3_solve_board(a3_detector *d, const uint64_t *ids, const float *corne
     for (uint32_t f = 0; f < n_frames; f++) off[f + 1] += off[f];
     A3_CUDA(cudaSetDevice(d->device));
     cudaStream_t s = d->s_decode;
-    A3_CUDA(d->d_probe_ids.reserve(n ? n : 1));
-    A3_CUDA(d->d_refined.reserve(n ? (size_t)n * 8 : 1));
-    A3_CUDA(d->d_probe_off.reserve(off.size()));
-    A3_CUDA(d->d_probe_out.reserve(n_frames));
-    if (n) {
-        A3_CUDA(cudaMemcpyAsync(d->d_probe_ids.p, ids, (size_t)n * 8, cudaMemcpyHostToDevice, s));
-        A3_CUDA(cudaMemcpyAsync(d->d_refined.p, corners, (size_t)n * 32, cudaMemcpyHostToDevice, s));
-    }
-    A3_CUDA(cudaMemcpyAsync(d->d_probe_off.p, off.data(), off.size() * 4, cudaMemcpyHostToDevice, s));
-    K6Params kp;
-    kp.ids = d->d_probe_ids.p; kp.corners_f32 = d->d_refined.p; kp.offsets = d->d_probe_off.p; kp.n_frames = n_frames;
-    kp.slots = d->d_board_slots.p; kp.n_codes = d->dict.n_codes; kp.board = d->d_board_pts.p; kp.n_board = d->opt.board_n;
-    kp.mode = d->opt.board_mode; kp.image_w = image_w; kp.image_h = image_h; kp.k = d->opt.board_k; kp.out = d->d_probe_out.p;
-    if (d->opt.dist_on && n) {  // K7 first, as a3_detect_batch runs it
-        A3_CUDA(d->d_und_out.reserve((size_t)n * 8)); A3_CUDA(d->d_und_ok.reserve(n));
-        K7Params up;
-        up.corners_f32 = d->d_refined.p; up.n = n; up.k = d->opt.board_k; up.dist = d->opt.dist; up.out = d->d_und_out.p; up.ok = d->d_und_ok.p;
+    const bool und = d->opt.dist_on && n;  // K7 first, as a3_detect_batch runs it
+    uint8_t *dev[6];
+    A3_CUDA(probe_slices(d, {{ids, (size_t)n * 8}, {corners, (size_t)n * 32}, {off.data(), off.size() * 4}, {nullptr, (size_t)n_frames * sizeof(a3_board_pose)},
+                             {nullptr, und ? (size_t)n * 32 : 0}, {nullptr, und ? n : 0}}, s, dev));
+    K6Params kp = k6_params(d, image_w, image_h);
+    kp.ids = reinterpret_cast<const uint64_t *>(dev[0]); kp.corners_f32 = reinterpret_cast<const float *>(dev[1]);
+    kp.offsets = reinterpret_cast<const uint32_t *>(dev[2]); kp.n_frames = n_frames; kp.out = reinterpret_cast<a3_board_pose *>(dev[3]);
+    if (und) {
+        K7Params up = k7_params(d, true);
+        up.corners_f32 = kp.corners_f32; up.n = n; up.out = reinterpret_cast<float *>(dev[4]); up.ok = dev[5];
         A3_CUDA(k7_undistort(up, s));
-        kp.norm = d->d_und_out.p; kp.norm_ok = d->d_und_ok.p;
+        kp.norm = up.out; kp.norm_ok = up.ok;
     }
     A3_CUDA(k6_board(kp, s));
-    A3_CUDA(cudaMemcpyAsync(out, d->d_probe_out.p, (size_t)n_frames * sizeof(a3_board_pose), cudaMemcpyDeviceToHost, s));
+    A3_CUDA(cudaMemcpyAsync(out, dev[3], (size_t)n_frames * sizeof(a3_board_pose), cudaMemcpyDeviceToHost, s));
     A3_CUDA(cudaStreamSynchronize(s));
     return A3_OK;
 }
@@ -1754,11 +1753,11 @@ a3_status a3_undistort_points(a3_detector *d, const float *points, uint32_t n, c
     if (n == 0) return A3_OK;
     A3_CUDA(cudaSetDevice(d->device));
     cudaStream_t s = d->s_decode;
-    A3_CUDA(d->d_und_in.reserve((size_t)n * 2)); A3_CUDA(d->d_und_out.reserve((size_t)n * 2)); A3_CUDA(d->d_und_ok.reserve(n));
-    A3_CUDA(cudaMemcpyAsync(d->d_und_in.p, points, (size_t)n * 8, cudaMemcpyHostToDevice, s));
-    A3_CUDA(k7_undistort_points(d->d_und_in.p, n, *k, *dist, d->d_und_out.p, d->d_und_ok.p, s));
-    A3_CUDA(cudaMemcpyAsync(out, d->d_und_out.p, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
-    A3_CUDA(cudaMemcpyAsync(ok, d->d_und_ok.p, n, cudaMemcpyDeviceToHost, s));
+    uint8_t *dev[3];
+    A3_CUDA(probe_slices(d, {{points, (size_t)n * 8}, {nullptr, (size_t)n * 8}, {nullptr, n}}, s, dev));
+    A3_CUDA(k7_undistort_points(reinterpret_cast<const float *>(dev[0]), n, *k, *dist, reinterpret_cast<float *>(dev[1]), dev[2], s));
+    A3_CUDA(cudaMemcpyAsync(out, dev[1], (size_t)n * 8, cudaMemcpyDeviceToHost, s));
+    A3_CUDA(cudaMemcpyAsync(ok, dev[2], n, cudaMemcpyDeviceToHost, s));
     A3_CUDA(cudaStreamSynchronize(s));
     return A3_OK;
 }
@@ -1770,17 +1769,17 @@ static a3_status solve_poses(a3_detector *d, uint32_t mode, const void *in, uint
     if (n == 0) return A3_OK;
     A3_CUDA(cudaSetDevice(d->device));
     cudaStream_t s = d->s_decode;
-    A3_CUDA(d->d_pose_in.reserve((size_t)n * 8)); A3_CUDA(d->d_pose_out.reserve((size_t)n * 2)); A3_CUDA(d->h_pose_out.reserve((size_t)n * 2));
-    A3_CUDA(cudaMemcpyAsync(d->d_pose_in.p, in, (size_t)n * 32, cudaMemcpyHostToDevice, s));
+    uint8_t *dev[2];  // 8 x 4 bytes per marker in (f32 points or u32 corners), K4's [2i] best and [2i + 1] alternative out
+    A3_CUDA(probe_slices(d, {{in, (size_t)n * 32}, {nullptr, (size_t)n * 2 * sizeof(a3_pose)}}, s, dev));
     K4Params kp{};
-    kp.mode = mode; kp.n = n; kp.marker_size = marker_size_mm; kp.image_w = iw; kp.image_h = ih; kp.poses = d->d_pose_out.p;
-    if (mode == A3_POSE_NORMALIZED) kp.points = d->d_pose_in.p;
-    else kp.corners = reinterpret_cast<const uint32_t *>(d->d_pose_in.p);
+    kp.mode = mode; kp.n = n; kp.marker_size = marker_size_mm; kp.image_w = iw; kp.image_h = ih; kp.poses = reinterpret_cast<a3_pose *>(dev[1]);
+    if (mode == A3_POSE_NORMALIZED) kp.points = reinterpret_cast<const float *>(dev[0]);
+    else kp.corners = reinterpret_cast<const uint32_t *>(dev[0]);
     if (k) kp.k = *k;
     A3_CUDA(k4_pose(kp, s));
-    A3_CUDA(cudaMemcpyAsync(d->h_pose_out.p, d->d_pose_out.p, (size_t)n * 2 * sizeof(a3_pose), cudaMemcpyDeviceToHost, s));
+    A3_CUDA(cudaMemcpy2DAsync(best, sizeof(a3_pose), dev[1], 2 * sizeof(a3_pose), sizeof(a3_pose), n, cudaMemcpyDeviceToHost, s));
+    A3_CUDA(cudaMemcpy2DAsync(alt, sizeof(a3_pose), dev[1] + sizeof(a3_pose), 2 * sizeof(a3_pose), sizeof(a3_pose), n, cudaMemcpyDeviceToHost, s));
     A3_CUDA(cudaStreamSynchronize(s));
-    for (uint32_t i = 0; i < n; i++) { best[i] = d->h_pose_out.p[2 * (size_t)i]; alt[i] = d->h_pose_out.p[2 * (size_t)i + 1]; }
     return A3_OK;
 }
 

@@ -280,12 +280,50 @@ def test_edges_and_errors(a3, det):
     assert e.value.status == _ffi.A3_ERR_INVALID_ARGUMENT
     with pytest.raises(a3.A3Error):
         a3.Detector(a3.DetectorConfig(contour_simplification_epsilon=0.0))
+    for shape in ((0, 480, 640), (1, 480, 0), (1, 0, 640)):  # a candidate but no grey to decode it on
+        with pytest.raises(a3.A3Error) as e:
+            det.decode_candidates(np.zeros(shape, np.uint8), np.zeros((1, 8), np.uint32))
+        assert e.value.status == _ffi.A3_ERR_INVALID_ARGUMENT
     imgs, _ = synth.render_batch("C1", 1)
     markers = (_ffi.A3Marker * 1)()
     n = C.c_uint32()
     st = _ffi.lib().a3_detect_batch(det._h, imgs.ctypes.data, _ffi.FMT_RGB8, _ffi.MEM_HOST, 1, 640, 480, 1920, 1920 * 480,
                                     C.cast(markers, C.c_void_p), 1, C.byref(n), None, None)
     assert st == _ffi.A3_ERR_CAPACITY and n.value > 1
+
+
+def test_probes_leave_the_pipeline_alone(a3):
+    """Every stage probe between two a3_detect_batch calls of one handle with every post-decode stage on: the probes keep
+    their inputs and outputs apart from the pipeline's buffers, so the second call returns every byte the first did."""
+    from aruco3_b200 import synth
+    from tests.test_gpu_board import _detect_all
+    frames, _ = synth.render_batch("C3", 3)
+    n, h, w = frames.shape[:3]
+    k = a3.CameraIntrinsics(w, h, 1400.0, 1400.0, w / 2, h / 2)
+    board = a3.Board.grid(6, 4, 40.0, 10.0)
+    rng = np.random.default_rng(8)
+    grey = rng.integers(0, 256, (2, 240, 320), np.uint8)
+    cx, cy, s = rng.integers(0, 270, 30), rng.integers(0, 190, 30), rng.integers(8, 48, 30)
+    quads = np.stack([cx, cy, cx + s, cy, cx + s, cy + s, cx, cy + s], 1).astype(np.uint32)
+    qf = np.sort(rng.integers(0, 2, 30)).astype(np.uint32)
+    with a3.Detector(corners="refined") as d:
+        d.set_pose(40.0, k)
+        d.set_board(board, k)
+        d.set_distortion(a3.CameraDistortion(-0.1, 0.02, 0.0, 0.0, 0.0))
+        first = _detect_all(a3, d, frames, full=True)
+        d.decode_candidates(grey, quads, qf)
+        d.refine_corners(grey, quads, qf)
+        d.quads_from_masks_device(rng.integers(0, 2, (2, 150, 200), np.uint8) * 255)
+        d.undistort_points(rng.uniform(0, 320, (50, 2)), k, a3.CameraDistortion(0.05, 0.0, 0.001, 0.0, 0.0))
+        d.solve_board(board.ids[rng.integers(0, len(board), 30)], quads.astype(np.float32), qf, 2, image_size=(320, 240))
+        a3.pose.solve_with_intrinsics(d, quads, 40.0, k)
+        a3.pose.solve_with_undistorted_points(d, quads, 40.0, (320, 240))
+        a3.pose.solve_with_normalized_points(d, quads.astype(np.float32) / 1000, 40.0)
+        second = _detect_all(a3, d, frames, full=True)
+    data, status, n_cands, n_markers, _ = first
+    assert status == 0 and n_markers > 0
+    # the counters are left out: they name the route, and the K3 probe replaces the size history the one-shot route reads
+    assert second[:4] == (data, status, n_cands, n_markers)
 
 
 def test_full_size_batch_properties(a3):
